@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the RISER read-classification hot path (contract: see DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path (median/MAD normalise + outlier smoothing ->
 12-layer ConvNet -> softmax -> accept/reject decision) over one fixed batch of
@@ -23,6 +23,10 @@ synthetic already-trimmed squiggle chunks: BASELINE.json configs[1], RNA004 mode
   latency  p50 / p99 per poll of the live loop (BASELINE config 5): 512 channels x 2 models, 3000 x 1.
 
     python bench.py --reads 1000000 [--gpus N]      BASELINE config 4: R reads of 12,048 samples sharded r mod G
+
+--dump-outputs DIR writes what the last timed step returned (rank 0), as float32: DIR/decisions.npy [B] (decision
+codes, include/riser_b200.h) and DIR/probs.npy [M, B, 2] (softmax per model).  The inputs and weights are seeded,
+so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -503,7 +507,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the host-side legs: cpu_baseline, torch_cuda_baseline, latency")
     ap.add_argument("--reads", type=int, default=0, help="BASELINE config 4: this many reads sharded r mod G (separate line)")
     ap.add_argument("--reads-length", type=int, default=12048)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's decisions and probabilities to DIR/*.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.reads):
+        ap.error("--dump-outputs applies to the flagship workload (--impl ours, no --reads)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -569,9 +579,12 @@ def main():
     for k in range(args.steps):
         flush.zero_()
         ev[k][0].record()
-        step(events=conv_events)
+        last = step(events=conv_events)
         ev[k][1].record()
     barrier()
+    # host copies now: the later legs reuse the classifier's device buffers
+    outputs = {"decisions": last[0].cpu().numpy().astype(np.float32),
+               "probs": last[1].cpu().numpy().astype(np.float32)} if args.dump_outputs else None
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = sum(step_ms)
     conv_ms = sum(a.elapsed_time(b) for a, b in conv_events) / args.steps
@@ -629,7 +642,7 @@ def main():
         live_clf = BatchedClassifier([mdl], proc, chunk=args.chunk)
         for _ in range(3):
             r_live = live_clf.classify_batch(sig_list, ids, {}, 0.9, "deplete")
-        n_live = max(3, min(args.steps, 10))
+        n_live = args.steps
         t0 = time.perf_counter()
         for _ in range(n_live):
             r_live = live_clf.classify_batch(sig_list, ids, {}, 0.9, "deplete")
@@ -725,6 +738,10 @@ def main():
                                    "promethion_3000ch_1model": sim.measure_latency(3000, 60, "RNA002", ("mRNA",))}
             except Exception as e:
                 line["latency"] = {"error": f"{type(e).__name__}: {e}"[:300]}
+        if outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in outputs.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
         _emit(line)
     if world > 1:
         dist.destroy_process_group()

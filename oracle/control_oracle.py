@@ -51,3 +51,48 @@ def run_batch(reads, states, version, cache, threshold, mode):
         if len(cache) >= 1000:
             cache = {}
     return decisions, p_on_out, p_off_out, sig_len, cache
+
+
+CSV_HEADER = 'batch_start,read_id,channel,sig_length,models,prob_targets,threshold,mode,decision\n'   # control.py:146
+
+
+def serial_target(client, models, proc, out_file, mode, threshold, unblock_duration=0.1):
+    """SequencerControl.target of riser/control.py:24-124 run until the client stops, its serial per-read body
+    driven through the ``proc`` (SignalProcessor) and ``models`` (Model) objects it is given, as the reference
+    calls them (control.py:36-82): poly(A) trim with the run's cache, fixed trim or skip, minimum-length skip,
+    cut to the kit's max length, ``mad_normalise``, ``classify`` per model, the decision rule.  One CSV row per
+    assessed read (control.py:145-153); rejects are unblocked by read number, rejects + accepts + exhausted
+    reads stop being received (control.py:100-106); the cache is wiped at 1000 entries (control.py:96-97)."""
+    import time
+    names = ";".join(m.target for m in models)
+    max_len = proc.get_max_length()
+    cache = {}
+    with open(f"{out_file}.csv", "a") as sink:
+        sink.write(CSV_HEADER)
+        while client.is_running():
+            batch_start = time.monotonic()
+            rejects, done = [], []
+            for channel, read in client.get_read_batch():
+                signal, trimmed = proc.trim_polyA(client.get_raw_signal(read), read.id, cache)
+                if not trimmed:
+                    if not proc.should_trim_fixed_length(signal):
+                        continue
+                    signal = proc.trim_polyA_fixed_length(signal)[:max_len]
+                else:
+                    if len(signal) < proc.get_min_length():
+                        continue
+                    signal = signal[:max_len]
+                signal = proc.mad_normalise(signal)
+                probs = [m.classify(signal) for m in models]
+                p_on = [p[1] for p in probs]
+                code = decide(p_on, [p[0] for p in probs], len(signal), max_len, threshold, mode)
+                sink.write(f"{batch_start:.0f},{read.id},{channel},{len(signal)},{names},"
+                           f"{';'.join(str(p.item()) for p in p_on)},{threshold},{mode},{NAMES[code]}\n")
+                if code == REJECT:
+                    rejects.append((channel, read.number))
+                if code in (REJECT, ACCEPT, NO_DECISION):
+                    done.append((channel, read.number))
+                if len(cache) >= 1000:
+                    cache = {}
+            client.reject_reads(rejects, unblock_duration)
+            client.finish_processing_reads(done)

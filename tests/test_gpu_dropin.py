@@ -12,6 +12,7 @@ import yaml
 from riser_b200 import Kit, SignalProcessor, Model, sim, synth
 from riser_b200.config import get_config, CNN_SHIPPED
 from oracle import refshim
+from oracle import control_oracle as ctl
 from oracle import preprocess_oracle as pp
 from oracle import convnet_oracle as net
 from tests.golden import make_golden_params as P
@@ -51,13 +52,11 @@ def test_model_from_pth_path_and_yaml_path(tmp_path):
         Model(str(tmp_path / "missing.pth"), get_config(yml), LOG, "mRNA")
 
 
-@pytest.mark.skipif(not refshim.available(), reason="reference importable neither from /root/reference nor oracle/_ref")
 @pytest.mark.parametrize("mode", ["deplete", "enrich"])
 def test_reference_control_loop_drives_riser_b200_objects(golden_dir, tmp_path, mode):
-    """INTEGRATION.md, import swap: the reference's UNMODIFIED SequencerControl.target (riser/control.py:11-124, its
-    serial per-read body) with riser_b200.Model / SignalProcessor behind it reproduces the rows, unblock and
-    stop-receiving calls the all-reference run produced (tests/golden/control_scenario.npz)."""
-    ref = refshim.load()
+    """INTEGRATION.md, import swap: the reference's serial SequencerControl.target (riser/control.py:11-124, restated
+    call for call in oracle/control_oracle.serial_target) with riser_b200.Model / SignalProcessor behind it reproduces
+    the rows, unblock and stop-receiving calls the all-reference run produced (tests/golden/control_scenario.npz)."""
     g = np.load(os.path.join(golden_dir, "control_scenario.npz"))
     reads = P.scenario_reads()
     client = sim.SimClient(reads, int(g["chunk"]), int(g["n_polls"]), first_len=int(g["first_len"]))
@@ -66,10 +65,8 @@ def test_reference_control_loop_drives_riser_b200_objects(golden_dir, tmp_path, 
     for t in [str(t) for t in g["targets"]]:
         pth, yml = _write_model_files(tmp_path, t)
         models.append(Model(pth, get_config(yml), LOG, t))
-    control = ref.control.SequencerControl(client, models, proc, LOG, str(tmp_path / f"ref_{mode}"))
-    control.start()
-    control.target(mode, 1, float(g["threshold"]))
-    control.finish()
+    client.start_streaming_reads()
+    ctl.serial_target(client, models, proc, str(tmp_path / f"ref_{mode}"), mode, float(g["threshold"]))
     with open(tmp_path / f"ref_{mode}.csv") as f:
         lines = [ln.rstrip("\n") for ln in f]
     assert lines[0] == str(g["header"])
