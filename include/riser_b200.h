@@ -127,6 +127,16 @@ int riser_polya_end(const int16_t* sig, const int64_t* off, const int32_t* n, in
                     int32_t* polya_end, int32_t* polya_start, int32_t* stats, int max_windows,
                     riser_stream_t stream);
 
+/* riser_polya_end for float32 (calibrated, pA) signal -- the secondary input mode: the same windows, scan,
+ * 512-window cap and -1 conventions, with every window statistic computed as numpy computes it for float32
+ * input (float32 median / MAD of the two middle values, np.mean's pairwise float32 sum, the rolling mean of
+ * the previous 1,000 samples as its own pairwise sum, the mean-change test in float32).  Read b is
+ * sig[off[b] .. off[b] + n[b]); 16-byte aligned reads take vector loads.
+ * stats (optional, may be NULL): float32 [B, max_windows, 4] = {median, MAD, mean, rolling mean}.          */
+int riser_polya_end_f32(const float* sig, const int64_t* off, const int32_t* n, int B,
+                        int32_t* polya_end, int32_t* polya_start, float* stats, int max_windows,
+                        riser_stream_t stream);
+
 /* Replaces the length gating of riser/control.py:36-60 (with preprocess.py:84-85,
  * 100, 104-106), batched: for read b of n[b] samples and poly(A) end `end` =
  * cached_end[b] if >= 0 else detected_end[b] (-1 = none found):

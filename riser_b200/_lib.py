@@ -25,6 +25,8 @@ SIGNATURES = {
     "riser_normalise_f32_live": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_i64, c_void_p, c_void_p]),
     "riser_polya_end": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int,
                                 c_void_p]),
+    "riser_polya_end_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int,
+                                    c_void_p]),
     "riser_select_window": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                     c_void_p]),
     "riser_model_create": (c_int, [P(c_void_p), c_int, P(c_int), P(c_void_p), P(c_void_p), c_void_p,

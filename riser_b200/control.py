@@ -14,6 +14,7 @@ import time
 import numpy as np
 
 from .pipeline import BatchedClassifier, DECISION_NAMES, SKIPPED, ACCEPT, REJECT, NO_DECISION
+from .preprocess import signal_dtype
 
 CSV_HEADER = 'batch_start,read_id,channel,sig_length,models,prob_targets,threshold,mode,decision\n'   # control.py:146
 TAKE_OVER_NOTICE = ('The sequencing run is being controlled by RISER, reads that are '
@@ -61,6 +62,7 @@ class SequencerControl():
         self.logger = logger
         self.out_filename = out_file
         self.classifier = BatchedClassifier(models, processor)
+        self.classifier_f32 = None     # built on the first poll of calibrated (float32) signal
         self.warm_up_batches = tuple(warm_up_batches)
         # Instrumentation (additive): seconds from "batch in hand" to "decisions on host" and the batch size of
         # the most recent non-empty polls.  Bounded -- ReadUntil's get_read_chunks does not block, so an idle
@@ -80,7 +82,9 @@ class SequencerControl():
     def target(self, mode, duration_h, threshold, unblock_duration=0.1):
         self.client.send_warning(TAKE_OVER_NOTICE)
         if self.warm_up_batches:
-            self.classifier.warm_up(self.warm_up_batches, threshold, mode)
+            calibrated = np.dtype(getattr(self.client, "signal_dtype", np.int16)) == np.float32
+            clf = self._classifier_f32() if calibrated else self.classifier
+            clf.warm_up(self.warm_up_batches, threshold, mode)
         model_names = ";".join(m.target for m in self.models)
         polyA_cache = {}       # one dict for the run; classify_batch stores found ends and wipes it at 1000 entries
         with open(f'{self.out_filename}.csv', 'a') as sink:
@@ -97,6 +101,16 @@ class SequencerControl():
                 self.logger.info(f'RISER has timed out after {duration_h} '
                                  'hours as requested.')
 
+    def _classifier_f32(self):
+        if self.classifier_f32 is None:
+            self.classifier_f32 = BatchedClassifier(self.models, self.proc, signal_dtype=np.float32)
+        return self.classifier_f32
+
+    def _classifier_for(self, signals):
+        """The classifier for a poll's arrays: the float32 one when they are float32 (a client run with calibrated
+        signal), the int16 one otherwise; a poll that mixes float32 with other dtypes raises TypeError."""
+        return self._classifier_f32() if signal_dtype(signals) == np.float32 else self.classifier
+
     # ------------------------------------------------------------------ one poll
     def _poll(self, sink, tally, polyA_cache, model_names, mode, threshold, unblock_duration):
         batch_start = time.monotonic()
@@ -110,7 +124,8 @@ class SequencerControl():
             return
         signals = [self.client.get_raw_signal(read) for _, read in batch]
         t0 = time.monotonic()
-        res = self.classifier.classify_batch(signals, [read.id for _, read in batch], polyA_cache, threshold, mode)
+        clf = self._classifier_for(signals)
+        res = clf.classify_batch(signals, [read.id for _, read in batch], polyA_cache, threshold, mode)
         self.batch_latencies.append(time.monotonic() - t0)
         self.batch_sizes.append(len(batch))
 

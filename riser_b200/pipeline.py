@@ -2,9 +2,10 @@
 rewritten ReadUntil loop calls once per ``get_read_batch()`` (SURVEY.md 8b), replacing
 the serial per-read body of riser/control.py:31-93.
 
-Everything between the H2D copy of the packed int16 signals and the D2H copy of the
-decision bytes / probabilities runs in the sm_100a kernels behind the C ABI, on the
-current CUDA stream, with one host synchronisation per batch.
+Everything between the H2D copy of the packed signals (int16 ADC counts, or float32
+calibrated signal with ``signal_dtype=np.float32``) and the D2H copy of the decision
+bytes / probabilities runs in the sm_100a kernels behind the C ABI, on the current CUDA
+stream, with one host synchronisation per batch.
 """
 import os
 
@@ -12,10 +13,11 @@ import numpy as np
 import torch
 
 from . import _lib
-from .preprocess import RaggedBatch, PinnedArena, _hostpack
+from .preprocess import RaggedBatch, PinnedArena, _hostpack, signal_dtype as _dtype_of
 from .model import decide, DEFAULT_CHUNK
 
 _EMPTY = np.zeros(0, dtype=np.int16)
+_EMPTY_F32 = np.zeros(0, dtype=np.float32)
 
 # decision codes (include/riser_b200.h)
 TRY_AGAIN, ACCEPT, REJECT, NO_DECISION, SKIPPED = 0, 1, 2, 3, 4
@@ -59,7 +61,15 @@ class BatchResult:
 
 
 class BatchedClassifier:
-    def __init__(self, models, processor, chunk=None):
+    def __init__(self, models, processor, chunk=None, signal_dtype=np.int16):
+        """``signal_dtype``: what the ReadUntil client hands over (riser/client.py:47).  np.int16 (raw ADC counts,
+        the default): integer prefixes are packed as int16, float ones refused.  np.float32 (calibrated signal):
+        float32 prefixes only; poly(A) detection and normalisation run in float32 as numpy does for such input
+        (riser_polya_end_f32, riser_normalise_f32_live)."""
+        self.signal_dtype = np.dtype(signal_dtype)
+        if self.signal_dtype not in (np.int16, np.float32):
+            raise TypeError(f"BatchedClassifier classifies int16 or float32 signal, not {self.signal_dtype}")
+        self.f32 = self.signal_dtype == np.float32
         self.models = list(models)
         self.proc = processor
         self.device = _lib.require_device()
@@ -69,7 +79,7 @@ class BatchedClassifier:
         self.fixed_trim = processor.get_fixed_trim_length()
         self.ld = (self.max_len + 3) & ~3
         self._bufs = {}
-        self._arena = PinnedArena(self.device)
+        self._arena = PinnedArena(self.device, dtype=torch.float32 if self.f32 else torch.int16)
         self._graphs = {}
         self.use_graphs = os.environ.get("RISER_LIVE_GRAPHS", "1") != "0"
 
@@ -95,9 +105,16 @@ class BatchedClassifier:
         B = batch.B
         buf = self._buffers(B)
         L = _lib.lib()
-        _lib.check(L.riser_normalise(_lib.ptr(batch.sig), _lib.ptr(batch.off), _lib.ptr(start), _lib.ptr(length),
-                                     B, self.max_len, _lib.ptr(buf["x"]), buf["x"].stride(0), None,
-                                     _lib.stream_ptr()), "riser_normalise")
+        if batch.sig.dtype == torch.float32:
+            # the float32 normaliser takes each window's own start: off + start
+            win_off = batch.off[:B] + start
+            _lib.check(L.riser_normalise_f32_live(_lib.ptr(batch.sig), _lib.ptr(win_off), _lib.ptr(length), B,
+                                                  self.max_len, _lib.ptr(buf["x"]), buf["x"].stride(0), None,
+                                                  _lib.stream_ptr()), "riser_normalise_f32_live")
+        else:
+            _lib.check(L.riser_normalise(_lib.ptr(batch.sig), _lib.ptr(batch.off), _lib.ptr(start),
+                                         _lib.ptr(length), B, self.max_len, _lib.ptr(buf["x"]), buf["x"].stride(0),
+                                         None, _lib.stream_ptr()), "riser_normalise")
         for m, model in enumerate(self.models):
             model.classify_batch(buf["x"], length, max_len=self.max_len, probs=buf["probs"][m],
                                  chunk=self.chunk, events=events)
@@ -115,9 +132,10 @@ class BatchedClassifier:
         # detection is only needed where nothing is cached; reads with a cache hit keep -1
         # (their prefix is skipped by giving them length 0 in the detection launch)
         n_detect = torch.where(cached >= 0, torch.zeros_like(batch.n), batch.n)
-        _lib.check(L.riser_polya_end(_lib.ptr(batch.sig), _lib.ptr(batch.off), _lib.ptr(n_detect), B,
-                                     _lib.ptr(buf["detected"]), None, None, 0, _lib.stream_ptr()),
-                   "riser_polya_end")
+        fn, name = ((L.riser_polya_end_f32, "riser_polya_end_f32") if batch.sig.dtype == torch.float32 else
+                    (L.riser_polya_end, "riser_polya_end"))
+        _lib.check(fn(_lib.ptr(batch.sig), _lib.ptr(batch.off), _lib.ptr(n_detect), B, _lib.ptr(buf["detected"]),
+                      None, None, 0, _lib.stream_ptr()), name)
         _lib.check(L.riser_select_window(_lib.ptr(batch.n), _lib.ptr(cached), _lib.ptr(buf["detected"]), B,
                                          self.min_len, self.max_len, self.fixed_trim, _lib.ptr(buf["start"]),
                                          _lib.ptr(buf["len"]), _lib.stream_ptr()), "riser_select_window")
@@ -141,11 +159,20 @@ class BatchedClassifier:
                                 "SignalProcessor.mad_normalise + Model.classify for float signal")
         return signals
 
+    @staticmethod
+    def _as_float32(signals):
+        """Calibrated mode: every prefix must be float32 (np.frombuffer(raw_data, float32) of a client run with
+        calibrated signal); anything else would be misread."""
+        if _dtype_of(signals) != np.float32:
+            raise TypeError("this BatchedClassifier was built for calibrated float32 signal: use one with "
+                            "signal_dtype=np.int16 for raw signal")
+        return signals
+
     # ------------------------------------------------------------------ public entry
     def classify_batch(self, signals, read_ids, polyA_cache, threshold, mode):
         """One pass of riser/control.py:31-97 over a batch.
 
-        signals: list of int16 arrays (the whole accumulated prefix of each read, as
+        signals: list of int16 (float32 in calibrated mode) arrays (the whole accumulated prefix of each read, as
         ``client.get_raw_signal`` returns it); read_ids: matching ids; polyA_cache: the
         loop's dict (updated here exactly as control.py does: found ends are stored, and
         the dict is cleared when it reaches 1000 entries after an assessed read).
@@ -160,12 +187,12 @@ class BatchedClassifier:
             res.h2d_bytes = res.d2h_bytes = 0
             return res
         n_real = B
-        signals = self._as_int16(signals)
+        signals = self._as_float32(signals) if self.f32 else self._as_int16(signals)
         B = bucket_size(n_real)                       # pad with empty reads up to the bucket
         cached = np.full(B, -1, dtype=np.int32)
         cached[:n_real] = np.fromiter((polyA_cache.get(r, -1) for r in read_ids), dtype=np.int32, count=n_real)
         if B > n_real:
-            signals = list(signals) + [_EMPTY] * (B - n_real)
+            signals = list(signals) + [_EMPTY_F32 if self.f32 else _EMPTY] * (B - n_real)
         # size the staging arena once for the longest prefixes the loop can hand over (a read is
         # classified, at the latest, once it exceeds fixed trim + max length: control.py:42-46)
         self._arena.reserve(B * (self.fixed_trim + self.max_len + 8192), B)
@@ -175,10 +202,10 @@ class BatchedClassifier:
         # whole (detection scans the whole prefix).
         n_all = np.zeros(B, dtype=np.int64)
         _hostpack().lengths(signals, n_all)
-        n_all >>= 1
+        n_all //= self.signal_dtype.itemsize
         skip, take = upload_ranges(n_all, cached, self.min_len, self.max_len)
         batch = RaggedBatch(signals, self.device, arena=self._arena, skip=skip, take=take, trusted=True,
-                            extra_i32=cached)
+                            extra_i32=cached, dtype=self.signal_dtype)
         # packed pinned result buffer: len | detected | probs | decisions (4-byte fields first)
         buf = self._buffers(B)
         host = buf["out_host"]
@@ -245,7 +272,8 @@ def _warm_up(self, batch_sizes, threshold, mode):
     for n in sorted(set(bucket_size(int(b)) for b in batch_sizes)):
         self._arena.reserve(n * (self.fixed_trim + self.max_len + 8192), n)
     for n in sorted(set(bucket_size(int(b)) for b in batch_sizes)):
-        self.classify_batch([_EMPTY] * n, [f"warm-up-{i}" for i in range(n)], {}, threshold, mode)
+        self.classify_batch([_EMPTY_F32 if self.f32 else _EMPTY] * n, [f"warm-up-{i}" for i in range(n)], {},
+                            threshold, mode)
 
 
 BatchedClassifier.warm_up = _warm_up

@@ -39,9 +39,11 @@ class Kit():
 
 class PinnedArena:
     """Grow-only pinned host buffer + device buffer pair reused across batches (pinning and
-    cudaMalloc per batch would dominate the latency of a live 512-read batch)."""
-    def __init__(self, device):
+    cudaMalloc per batch would dominate the latency of a live 512-read batch).  ``dtype``: the
+    sample type of the signal buffers (int16 ADC counts, or float32 for calibrated signal)."""
+    def __init__(self, device, dtype=torch.int16):
         self.device = device
+        self.dtype = dtype
         self.capacity = 0
         self.host = self.dev = self.meta_host = self.meta_dev = None
         self.meta_capacity = 0
@@ -50,8 +52,8 @@ class PinnedArena:
     def reserve(self, n_samples, n_reads):
         if n_samples > self.capacity:
             self.capacity = int(n_samples * 1.25) + 4096
-            self.host = torch.empty(self.capacity, dtype=torch.int16).pin_memory()
-            self.dev = torch.empty(self.capacity, dtype=torch.int16, device=self.device)
+            self.host = torch.empty(self.capacity, dtype=self.dtype).pin_memory()
+            self.dev = torch.empty(self.capacity, dtype=self.dtype, device=self.device)
             self.generation += 1
         if n_reads > self.meta_capacity:
             self.meta_capacity = int(n_reads * 1.25) + 64
@@ -79,7 +81,7 @@ def _hostpack():
 
 
 class RaggedBatch:
-    """int16 reads packed back to back on the device: ``sig`` [total], ``off`` int64
+    """Reads packed back to back on the device: ``sig`` [total], ``off`` int64
     [B+1], ``n`` int32 [B].  Built from host arrays through one pinned staging
     buffer and one H2D copy (two with metadata); pass a ``PinnedArena`` to reuse buffers.
 
@@ -90,15 +92,26 @@ class RaggedBatch:
     and the kernels need not know.  ``n`` is always the full prefix length.
     ``trusted=True`` skips the per-read dtype / contiguity check (the live loop's arrays come straight from
     ``np.frombuffer(raw_data, int16)``).  ``extra_i32`` (arena path only): an int32 [B] host array uploaded with the
-    metadata in the same copy, available as ``self.extra``."""
-    def __init__(self, signals, device, arena=None, skip=None, take=None, trusted=False, extra_i32=None):
+    metadata in the same copy, available as ``self.extra``.
+    ``dtype``: the sample type, int16 (ADC counts, the default) or float32 (calibrated signal); with an arena it
+    must be the arena's.  Every read starts on a 16-byte boundary: 8 int16 or 4 float32 samples."""
+    def __init__(self, signals, device, arena=None, skip=None, take=None, trusted=False, extra_i32=None,
+                 dtype=np.int16):
         B = len(signals)
+        dtype = np.dtype(dtype)
+        if dtype not in (np.int16, np.float32):
+            raise TypeError(f"RaggedBatch packs int16 or float32 samples, not {dtype}")
+        esz = dtype.itemsize
+        align = 16 // esz
+        tdtype = torch.int16 if dtype == np.int16 else torch.float32
+        if arena is not None and arena.dtype != tdtype:
+            raise TypeError(f"a {arena.dtype} arena cannot stage {dtype} samples")
         if not trusted:
-            signals = [np.ascontiguousarray(s, dtype=np.int16) for s in signals]
+            signals = [np.ascontiguousarray(s, dtype=dtype) for s in signals]
         nbytes = np.zeros(B, dtype=np.int64)
         hp = _hostpack()
         hp.lengths(signals, nbytes)
-        n = nbytes >> 1
+        n = nbytes // esz
         if take is None:
             skip = np.zeros(B, dtype=np.int64)
             take = n
@@ -106,25 +119,26 @@ class RaggedBatch:
             skip = np.ascontiguousarray(skip, dtype=np.int64)
             take = np.ascontiguousarray(take, dtype=np.int64)
         # keep every packed read 16-byte aligned so the kernels' vector loads need no peeling
-        padded = (take + 7) & ~7
+        padded = (take + (align - 1)) & ~(align - 1)
         pos = np.zeros(B + 1, dtype=np.int64)
         np.cumsum(padded, out=pos[1:])
-        total = int(pos[-1]) + 8
+        total = int(pos[-1]) + align
         off = pos.copy()
         off[:B] -= skip
         self.B = B
+        self.dtype = dtype
         self.n_host = n.astype(np.int32)
-        byte_pos = np.ascontiguousarray(pos[:B] << 1)
+        byte_pos = np.ascontiguousarray(pos[:B] * esz)
         if arena is None:
-            host = torch.empty(total, dtype=torch.int16).pin_memory()
-            hp.pack(signals, host.numpy(), byte_pos, skip << 1, take << 1, PACK_THREADS)
+            host = torch.empty(total, dtype=tdtype).pin_memory()
+            hp.pack(signals, host.numpy(), byte_pos, skip * esz, take * esz, PACK_THREADS)
             self.sig = host.to(device, non_blocking=True)
             self.off = torch.from_numpy(off).to(device, non_blocking=True)
             self.n = torch.from_numpy(self.n_host).to(device, non_blocking=True)
             self._host = host      # keep the pinned buffer alive until the copy has run
         else:
             arena.reserve(total, B)
-            hp.pack(signals, arena.host.numpy(), byte_pos, skip << 1, take << 1, PACK_THREADS)
+            hp.pack(signals, arena.host.numpy(), byte_pos, skip * esz, take * esz, PACK_THREADS)
             self.sig = arena.dev[:total]
             self.sig.copy_(arena.host[:total], non_blocking=True)
             mh = arena.meta_host.numpy()
@@ -139,7 +153,21 @@ class RaggedBatch:
             self.off = arena.meta_dev[:B + 1]
             self.n = arena.meta_dev[B + 1:B + 1 + half].view(torch.int32)[:B]
             self.extra = None if extra_i32 is None else arena.meta_dev[B + 1 + half:B + 1 + 2 * half].view(torch.int32)[:B]
-        self.h2d_bytes = total * 2 + off.nbytes + self.n_host.nbytes
+        self.h2d_bytes = total * esz + off.nbytes + self.n_host.nbytes
+
+
+_F32 = np.dtype(np.float32)
+
+
+def signal_dtype(signals):
+    """The sample type a list of signals is packed as: float32 when every one is float32 (calibrated signal, kept in
+    float32 as numpy keeps it), int16 when none is (other integer dtypes are converted); a mix raises TypeError."""
+    dtypes = {getattr(s, "dtype", None) for s in signals}
+    if _F32 not in dtypes:
+        return np.dtype(np.int16)
+    if len(dtypes) > 1:
+        raise TypeError(f"float32 (calibrated) signal mixed with other dtypes: {sorted(map(str, dtypes))}")
+    return _F32
 
 
 class SignalProcessor():
@@ -186,26 +214,39 @@ class SignalProcessor():
         return signal, trimmed
 
     def get_polyA_end_batch(self, signals, return_stats=False):
-        """Batched get_polyA_end: list of int16 arrays -> int32 [B] (-1 = None)."""
+        """Batched get_polyA_end: list of arrays -> int32 [B] (-1 = None).
+
+        float32 arrays (calibrated signal) go to ``riser_polya_end_f32``, which computes the window statistics in
+        float32 as numpy does for them; every other dtype is cast to int16 (``riser_polya_end``).  A list that
+        mixes float32 with other dtypes raises TypeError."""
         device = _lib.require_device()
         if not isinstance(signals, RaggedBatch) and len(signals) == 0:
             return np.zeros(0, dtype=np.int32)
-        batch = signals if isinstance(signals, RaggedBatch) else RaggedBatch(
-            [np.ascontiguousarray(s, dtype=np.int16) for s in signals], device)
+        if isinstance(signals, RaggedBatch):
+            batch = signals
+        else:
+            dtype = signal_dtype(signals)
+            batch = RaggedBatch([np.ascontiguousarray(s, dtype=dtype) for s in signals], device, dtype=dtype)
         ends = self.polya_end_device(batch, return_stats=return_stats)
         if return_stats:
             return ends[0].cpu().numpy(), ends[1].cpu().numpy()
         return ends.cpu().numpy()
 
     def polya_end_device(self, batch, return_stats=False, starts=None):
+        """Detection on a RaggedBatch already on the device.  stats (``return_stats``): int32 [B, W, 3] =
+        {sum, 2 * median, 4 * MAD} per window for int16 reads, float32 [B, W, 4] = {median, MAD, mean,
+        rolling mean} for float32 reads."""
         ends = torch.empty(batch.B, dtype=torch.int32, device=batch.sig.device)
+        f32 = batch.sig.dtype == torch.float32
         stats, max_w = None, 0
         if return_stats:
             max_w = max(1, int(batch.n_host.max()) // _TRIM_RESOLUTION)
-            stats = torch.zeros(batch.B, max_w, 3, dtype=torch.int32, device=batch.sig.device)
-        _lib.check(_lib.lib().riser_polya_end(_lib.ptr(batch.sig), _lib.ptr(batch.off), _lib.ptr(batch.n),
-                                              batch.B, _lib.ptr(ends), _lib.ptr(starts), _lib.ptr(stats), max_w,
-                                              _lib.stream_ptr()), "riser_polya_end")
+            stats = torch.zeros(batch.B, max_w, 4 if f32 else 3, dtype=torch.float32 if f32 else torch.int32,
+                                device=batch.sig.device)
+        fn, name = ((_lib.lib().riser_polya_end_f32, "riser_polya_end_f32") if f32 else
+                    (_lib.lib().riser_polya_end, "riser_polya_end"))
+        _lib.check(fn(_lib.ptr(batch.sig), _lib.ptr(batch.off), _lib.ptr(batch.n), batch.B, _lib.ptr(ends),
+                      _lib.ptr(starts), _lib.ptr(stats), max_w, _lib.stream_ptr()), name)
         return (ends, stats) if return_stats else ends
 
     # ------------------------------------------------------------ normalise

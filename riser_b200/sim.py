@@ -25,10 +25,14 @@ class SimClient:
     signal_dtype = np.int16
 
     def __init__(self, reads, chunk, n_polls, first_len=None, with_number=True):
-        """reads: list of (read_id, int16 full signal); channel c (1-based) carries
+        """reads: list of (read_id, full signal); channel c (1-based) carries
         reads[c-1].  Each poll exposes ``first_len + k*chunk`` samples (capped at the
-        read's length).  After ``n_polls`` polls ``is_running`` turns False."""
+        read's length).  After ``n_polls`` polls ``is_running`` turns False.
+        ``signal_dtype`` is that of the reads: int16 (raw ADC counts) or float32
+        (calibrated pA, what a client run with calibrated signal hands over)."""
         self.reads = reads
+        if reads:
+            self.signal_dtype = np.asarray(reads[0][1]).dtype
         self.chunk = int(chunk)
         self.first_len = int(first_len if first_len is not None else chunk)
         self.n_polls = int(n_polls)
@@ -116,12 +120,20 @@ class LiveSimClient(SimClient):
         return batch
 
 
+def calibrate(reads, scale, offset):
+    """Calibrated (pA) float32 copies of int16 reads, ``(adc + offset) * scale`` in float32 -- what a ReadUntil client
+    run with calibrated signal hands over."""
+    s, o = np.float32(scale), np.float32(offset)
+    return [(rid, ((sig.astype(np.float32) + o) * s).astype(np.float32)) for rid, sig in reads]
+
+
 def measure_latency(channels, polls, kit_version="RNA002", targets=("mRNA",), seed=7, skip=5, pool_reads=None,
-                    precision=None):
+                    precision=None, calibration=None):
     """BASELINE config 5: ``channels`` pores, every poll each live read's prefix grows by one second of samples
     (AccumulatingCache semantics, riser/client.py:29-31,44); the batched ``SequencerControl`` classifies every
     poll.  Returns p50 / p99 of the time from "batch in hand" to "decisions on host" over the polls after the
-    first ``skip`` (the ReadUntil decision budget is ~1 s), with the run's counters."""
+    first ``skip`` (the ReadUntil decision budget is ~1 s), with the run's counters.  ``calibration`` = (scale,
+    offset): the client hands over calibrated float32 signal, ``(adc + offset) * scale``, instead of int16."""
     import logging
     import os
     import tempfile
@@ -134,6 +146,8 @@ def measure_latency(channels, polls, kit_version="RNA002", targets=("mRNA",), se
     models = [Model(synth.state_dict(synth.TARGET_SEEDS[t]), shipped_config(), log, t, **kw) for t in targets]
     n_pool = int(pool_reads or min(2 * channels, 2048))
     reads = synth.raw_reads(seed, n_pool, min_body=14000, max_body=20000, frac_no_polya=0.05)
+    if calibration is not None:
+        reads = calibrate(reads, *calibration)
     client = LiveSimClient(reads, channels, chunk=kit.sampling_hz, n_polls=polls, first_len=kit.sampling_hz)
     with tempfile.TemporaryDirectory() as tmp:
         control = SequencerControl(client, models, SignalProcessor(kit), log, os.path.join(tmp, "live"),
@@ -145,7 +159,10 @@ def measure_latency(channels, polls, kit_version="RNA002", targets=("mRNA",), se
             rows = sum(1 for _ in f) - 1
     lat = np.array(control.batch_latencies) * 1e3
     steady = lat[skip:] if len(lat) > skip + 3 else lat
-    return {"channels": int(channels), "models": len(targets), "kit": kit_version, "polls": int(len(lat)),
+    out = {"channels": int(channels), "models": len(targets), "kit": kit_version, "polls": int(len(lat)),
             "p50_ms": round(float(np.median(steady)), 3), "p99_ms": round(float(np.percentile(steady, 99)), 3),
             "max_ms": round(float(steady.max()), 3), "batch_size_median": int(np.median(control.batch_sizes)),
             "assessed_rows": rows, "rejected": len(client.unblocked), "finished": len(client.finished)}
+    if calibration is not None:
+        out["calibration"] = [float(calibration[0]), float(calibration[1])]
+    return out
