@@ -60,11 +60,11 @@ enum { RISER_MODE_ENRICH = 0, RISER_MODE_DEPLETE = 1 };
  *   F16_X3 : three passes; weights AND activations split hi + lo
  *            (W_hi a_hi + W_lo a_hi + W_hi a_lo): fp32-class results.
  *   F16_F8 : the fp16 pass plus ONE e4m3 pass (kind::f8f6f4, twice the fp16 rate)
- *            that carries both correction terms, W_lo a + (W_hi 2^-9)(a_lo 2^9):
+ *            that carries both correction terms, (W_lo 2^3)(a 2^-3) + (W 2^-9)(a_lo 2^9):
  *            the corrections are ~2^-11 of the result, so 3 mantissa bits suffice
  *            (format error ~6e-5 on the probabilities).  Two pass-equivalents of
  *            tensor work instead of three; activation rows are
- *            [hi fp16 | e4m3(a) | e4m3(a_lo 2^9)] = the bytes of hi + lo.        */
+ *            [hi fp16 | e4m3(a 2^-3) | e4m3(a_lo 2^9)] = the bytes of hi + lo.   */
 enum { RISER_PREC_F16 = 0, RISER_PREC_F16_W2 = 1, RISER_PREC_F16_X3 = 2, RISER_PREC_F16_F8 = 3 };
 
 int riser_version(void);
@@ -224,7 +224,7 @@ int riser_plan_layer_eo(const riser_plan* p, int i);
  * mode (DESIGN.md section 2):
  *   1 = one fp16 plane [channels_padded];
  *   2 = fp16 hi | fp16 lo planes (a = hi + lo; the F16_X3 terms W_hi*a_hi + W_lo*a_hi + W_hi*a_lo);
- *   3 = fp16 hi | e4m3(a) | e4m3((a - hi) * 2^9): the operands of the fp16 pass and of the single
+ *   3 = fp16 hi | e4m3(a * 2^-3) | e4m3((a - hi) * 2^9): the operands of the fp16 pass and of the single
  *       e4m3 correction pass of RISER_PREC_F16_F8 (same bytes per row as format 2).
  * 0 for i outside that range, -1 when the buffer is never materialised (layer i is computed inside layer
  * i - 1's launch: conv_eo2_kernel).  Tests decode activations with it; bench.py derives the tensor passes

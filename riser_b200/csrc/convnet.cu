@@ -70,7 +70,7 @@ int pick_n_tile(int cout) {
 struct LayerPack {
   int cin = 0, cout = 0, cin_p = 0, cout_p = 0, n_tile = 0, n_tiles = 0;
   __half* w = nullptr;    // [passes][3][cout_p][cin_p] fp16 (layers >= 1)
-  uint8_t* w8 = nullptr;  // F16_F8 mode: [3][cout_p][2*cin_p] e4m3 = [W_lo | W_hi * 2^-9] (correction pass)
+  uint8_t* w8 = nullptr;  // F16_F8 mode: [3][cout_p][2*cin_p] e4m3 = [W_lo * 2^3 | W * 2^-9] (correction pass)
   __half* wkc = nullptr;  // layer 1, F16_X3 terms concatenated along K: [3][cout_p][64] = [W_hi | W_hi | W_lo | 0] (fused01 MODE 4)
   float* w0 = nullptr;    // layer 0 only: fp32 [cout][3]
   float* bias = nullptr;  // fp32 [cout_p], zero padded
@@ -204,8 +204,11 @@ struct riser_plan {
 namespace riser {
 namespace {
 
-// F16_F8 activation format: besides the fp16 value h = fp16(r), a row carries a8 = e4m3(r) (the operand of
-// the W_lo correction) and lo8 = e4m3((r - h) * 2^9) (the operand of the W_hi * 2^-9 correction).
+// F16_F8 activation format: besides the fp16 value h = fp16(r), a row carries a8 = e4m3(r * 2^-3) (the operand of
+// the W_lo * 2^3 correction) and lo8 = e4m3((r - h) * 2^9) (the operand of the W * 2^-9 correction).  The 2^-3
+// (model.py F8_A_SHIFT) keeps a8 below e4m3's 448 for |r| < 3584 (unshifted it saturated above 448); lo8 stays exact
+// in range to |r| = 2048.  A larger shift would push a8 of small activations into e4m3's subnormals (DESIGN.md 2).
+constexpr float kF8AScale = 1.f / 8.f;
 constexpr float kF8LoScale = 512.f;
 template <int N>
 __device__ __forceinline__ void store_f8_planes(const float (&r)[N], const __half2 (&h)[N / 2], uint8_t* a8,
@@ -218,7 +221,8 @@ __device__ __forceinline__ void store_f8_planes(const float (&r)[N], const __hal
     for (int e = 0; e < 2; ++e) {
       const int c = 4 * j + 2 * e;
       const float2 back = __half22float2(h[c / 2]);
-      wa[e] = __nv_cvt_float2_to_fp8x2(make_float2(r[c], r[c + 1]), __NV_SATFINITE, __NV_E4M3);
+      wa[e] = __nv_cvt_float2_to_fp8x2(make_float2(r[c] * kF8AScale, r[c + 1] * kF8AScale), __NV_SATFINITE,
+                                       __NV_E4M3);
       wl[e] = __nv_cvt_float2_to_fp8x2(make_float2((r[c] - back.x) * kF8LoScale, (r[c + 1] - back.y) * kF8LoScale),
                                        __NV_SATFINITE, __NV_E4M3);
     }
@@ -1242,7 +1246,7 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
           for (int ap = 0; ap < ((wp == 0 && !F8) ? PLANES : 1); ++ap)
             issue_group(a1s + ap * 2 * kF2A1Tile, w1_addr + wp * 3 * 2048, false, wp == 0 && ap == 0);
         }
-        if (F8)   // correction pass: [a8 | lo8] x [W_lo | W_hi * 2^-9], 64 e4m3 per row = 2 k-steps
+        if (F8)   // correction pass: [a8 | lo8] x [W_lo * 2^3 | W * 2^-9], 64 e4m3 per row = 2 k-steps
           issue_group(a1s + 2 * kF2A1Tile, w1_addr + 3 * 2048, true, false);
         umma_commit_p(leader, &s.a1_empty[st]);
         umma_commit_p(leader, &s.d1_full[st]);
@@ -1416,7 +1420,8 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
             for (int e = 0; e < 2; ++e) {
               const int c = 4 * j + 2 * e;
               const float2 back = __half22float2(hv[c / 2]);
-              wa[e] = __nv_cvt_float2_to_fp8x2(make_float2(v[c], v[c + 1]), __NV_SATFINITE, __NV_E4M3);
+              wa[e] = __nv_cvt_float2_to_fp8x2(make_float2(v[c] * kF8AScale, v[c + 1] * kF8AScale), __NV_SATFINITE,
+                                               __NV_E4M3);
               wl[e] = __nv_cvt_float2_to_fp8x2(
                   make_float2((v[c] - back.x) * kF8LoScale, (v[c + 1] - back.y) * kF8LoScale), __NV_SATFINITE, __NV_E4M3);
             }
@@ -2757,9 +2762,9 @@ extern "C" int riser_model_create(riser_model** out, int n_layers, const int* ch
             const size_t idx = (static_cast<size_t>(tap) * L.cout_p + co) * L.cin_p + ci;
             w[idx] = hi;
             if (L.passes == 2) w[per_pass + idx] = __float2half_rn(v - __half2float(hi));
-            if (L.f8) {   // correction operands: [W_lo | W_hi * 2^-9] e4m3 (pair with a8 and lo8 * 2^9)
+            if (L.f8) {   // correction operands: [W_lo * 2^3 | W * 2^-9] e4m3 (pair with a8 and lo8, store_f8_planes)
               const size_t i8 = (static_cast<size_t>(tap) * L.cout_p + co) * (2 * L.cin_p) + ci;
-              w8[i8] = __nv_cvt_float_to_fp8(v - __half2float(hi), __NV_SATFINITE, __NV_E4M3);
+              w8[i8] = __nv_cvt_float_to_fp8((v - __half2float(hi)) * (1.f / kF8AScale), __NV_SATFINITE, __NV_E4M3);
               w8[i8 + L.cin_p] = __nv_cvt_float_to_fp8(v * (1.f / kF8LoScale), __NV_SATFINITE, __NV_E4M3);
             }
           }

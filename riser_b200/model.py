@@ -20,6 +20,10 @@ PREC_F16_X3 = 2    # three passes, weights and activations split hi + lo: fp32-c
 PREC_F16_F8 = 3    # fp16 pass + one e4m3 pass carrying both hi/lo correction terms (2 pass-equivalents)
 DEFAULT_PRECISION = PREC_F16_F8
 MIN_LENGTH = 4096  # riser/preprocess.py:8 -- 12 stride-2 pools
+# F16_F8 rows carry a8 = e4m3(a * 2^-F8_A_SHIFT) and lo8 = e4m3((a - hi) * 2^(9 - F8_LO_SHIFT)); the weight operands
+# of the e4m3 pass carry the opposite powers of two (csrc/convnet.cu kF8AScale / kF8LoScale, which these must match)
+F8_A_SHIFT = 3
+F8_LO_SHIFT = 0
 DEFAULT_CHUNK = 0    # 0 = whole batch in one plan (the plan chunks the early layers itself)
 
 
@@ -55,12 +59,13 @@ class Plan:
         return {0: "conv_tc_kernel", 1: "conv_eo_kernel", 2: "conv_pair_kernel", 3: "fused01_kernel",
                 4: "conv_tc_kernel<FUSED>", 5: "conv_eo2_kernel"}.get(k, "?")
 
-    def activation(self, i, n_layers, planes=None):
-        """Layer i's input buffer as a [B, rows_per_read, channels] tensor (tests); `planes` = row format,
-        by default the one the plan reports (layer_format)."""
-        if planes is None:
-            planes = self.layer_format(i) or 1
-            if planes < 0:
+    def planes(self, i, n_layers, fmt=None):
+        """Layer i's input buffer as the planes it stores, each [B, rows_per_read, channels] in its stored dtype:
+        (hi, lo) fp16 for format 2, (hi fp16, a8 e4m3, lo8 e4m3) for format 3, (x,) otherwise (fp16; fp32 for the
+        head's input).  `fmt` = row format, by default the one the plan reports (layer_format)."""
+        if fmt is None:
+            fmt = self.layer_format(i) or 1
+            if fmt < 0:
                 raise ValueError(f"layer {i}'s input is never materialised in this plan (fused into the previous launch)")
         off, rows, cp, c, _ = self.layer_info(i)
         dt = torch.float32 if i == n_layers else torch.float16
@@ -71,15 +76,25 @@ class Plan:
             full = full.view(2, self.B, rows // 2, cp).permute(1, 2, 0, 3).reshape(self.B, rows, cp)
         else:
             full = full.view(self.B, rows, cp)
-        if planes == 2 and i != n_layers:      # hi + lo planes side by side
-            half = cp // 2
-            return full[:, :, :c].float() + full[:, :, half:half + c].float()
-        if planes == 3 and i != n_layers:      # F16_F8 rows: [hi fp16 | a8 e4m3 | lo8 e4m3 = (a - hi) * 2^9]
-            half = cp // 2
+        half = cp // 2
+        if fmt == 2 and i != n_layers:      # hi + lo planes side by side
+            return full[:, :, :c], full[:, :, half:half + c]
+        if fmt == 3 and i != n_layers:      # [hi fp16 | a8 e4m3 | lo8 e4m3] (bytes)
             raw = full.contiguous().view(torch.uint8).view(self.B, rows, cp * 2)
-            lo8 = raw[:, :, 3 * half:3 * half + c].contiguous().view(torch.float8_e4m3fn).float()
-            return full[:, :, :c].float() + lo8 / 512.0
-        return full[:, :, :c]
+            a8 = raw[:, :, 2 * half:2 * half + c].contiguous().view(torch.float8_e4m3fn)
+            lo8 = raw[:, :, 3 * half:3 * half + c].contiguous().view(torch.float8_e4m3fn)
+            return full[:, :, :c], a8, lo8
+        return (full[:, :, :c],)
+
+    def activation(self, i, n_layers, planes=None):
+        """Layer i's input buffer as a [B, rows_per_read, channels] tensor (tests); `planes` = row format,
+        by default the one the plan reports (layer_format)."""
+        p = self.planes(i, n_layers, planes)
+        if len(p) == 2:
+            return p[0].float() + p[1].float()
+        if len(p) == 3:                    # hi + (a - hi), the e4m3 a8 is only an MMA operand
+            return p[0].float() + p[2].float() * 2.0 ** -(9 - F8_LO_SHIFT)
+        return p[0]
 
     def __del__(self):
         try:
