@@ -266,8 +266,8 @@ int riser_stem_pool_cl(const float* x, int64_t ld_x, const int32_t* len_in, cons
  *               `residual` (= x for the identity shortcut), else nothing.  The intermediate stays on the SM.
  * Activations: fp32 channel-last [B][L_pad][C_p], channels padded to a multiple of 8 (padding channels zero),
  * 32-byte aligned; rows outside [0, len_in[b]) read as zero, rows >= len_out[b] are not written.
- * Weights: host-packed operand images (riser_b200/resnet.py pack_tc_weights): fp16 [plane hi, lo][tap][K block of
- * 32 channels][N rows][32] in the K-major SWIZZLE_64B layout, multiplied by a power of two whose inverse is
+ * Weights: host-packed operand images (riser_b200/resnet.py pack_tc_weights): fp16 [tap][K block of 32 channels]
+ * [plane hi, lo][N rows][32] in the K-major SWIZZLE_64B layout, multiplied by a power of two whose inverse is
  * inv_scale*.  n1 / n2: output channels padded to 16 (<= 256).  cmid_p: conv1's output channels (fused mode).
  * riser_res_tc_smem: shared memory a shape needs, 0 if unsupported (the caller falls back to riser_conv1d_cl). */
 size_t riser_res_tc_smem(int cin_p, int cmid_p, int n1, int n2, int taps, int stride, int fused, int shortcut_conv);
@@ -275,6 +275,26 @@ int riser_res_tc(const float* in, const int32_t* len_in, const int32_t* len_out,
                  const void* w1, const void* w2, const void* wsc, const float* bias1, const float* bias2,
                  float inv_scale1, float inv_scale2, int B, int Lin_pad, int Lout_pad, int cin_p, int cmid_p,
                  int cout_p, int n1, int n2, int taps, int stride, int relu, riser_stream_t stream);
+
+/* The same launches in a chosen arithmetic (RISER_PREC_*; with RISER_PREC_F16_X3 these ARE riser_res_tc_smem /
+ * riser_res_tc, bit for bit).  Per mode, the MMAs of a tap and 16-channel K step and the weight image (per tap and
+ * 32-channel K block, planes of N rows x 64 bytes, each SWIZZLE_64B, weights w = W * 2^e):
+ *   F16     a_hi W_hi                                    image [hi]: fp16(w)
+ *   F16_W2  a_hi [W_hi; W_lo] (one MMA when 2N <= 256)    image [hi, lo]: fp16(w), fp16(w - hi)
+ *   F16_X3  + a_lo W_hi                                  image [hi, lo] (as riser_res_tc)
+ *   F16_F8  a_hi W_hi, plus per K block two kind::f8f6f4 MMAs (K = 32) of the activation row
+ *           [e4m3(a 2^-3) x32 | e4m3((a - a_hi) 2^9) x32] against the weight row [e4m3((w - hi) 2^3) x32 |
+ *           e4m3(w 2^-9) x32]: image [hi, e4m3 row] (64 bytes per row, the size of an fp16 plane row).
+ * Activations stay fp32 in memory whatever the mode; the kernel converts them to the mode's operand tiles (the fused
+ * BasicBlock's intermediate too).  e4m3(a 2^-3) saturates at |a| = 3584.  riser_res_tc_smem_ex returns 0 for an
+ * unknown mode; F16 and F16_W2 need less shared memory than F16_X3 (no lo / e4m3 activation tiles; F16 no weight lo
+ * plane), so a block may fit in those modes and not in F16_X3.                                                  */
+size_t riser_res_tc_smem_ex(int cin_p, int cmid_p, int n1, int n2, int taps, int stride, int fused, int shortcut_conv,
+                            int precision);
+int riser_res_tc_ex(const float* in, const int32_t* len_in, const int32_t* len_out, float* out, const float* residual,
+                    const void* w1, const void* w2, const void* wsc, const float* bias1, const float* bias2,
+                    float inv_scale1, float inv_scale2, int B, int Lin_pad, int Lout_pad, int cin_p, int cmid_p,
+                    int cout_p, int n1, int n2, int taps, int stride, int relu, riser_stream_t stream, int precision);
 
 /* Conv1d(Cin->Cout, K, stride, padding) [+ residual] [+ ReLU] -- resnet.py:26-43,79-81.
  * w is packed [K][Cin][Cout]; rows outside [0, len_in[b]) are zero padding; rows

@@ -47,6 +47,8 @@ SIGNATURES = {
     "riser_stem_pool_cl": (c_int, [c_void_p, c_i64] + [c_void_p] * 6 + [c_int] * 6 + [c_void_p]),
     "riser_res_tc_smem": (c_size_t, [c_int] * 8),
     "riser_res_tc": (c_int, [c_void_p] * 10 + [c_float, c_float] + [c_int] * 11 + [c_void_p]),
+    "riser_res_tc_smem_ex": (c_size_t, [c_int] * 9),
+    "riser_res_tc_ex": (c_int, [c_void_p] * 10 + [c_float, c_float] + [c_int] * 11 + [c_void_p, c_int]),
     "riser_len_chain": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p]),
     "riser_maxpool1d_cl": (c_int, [c_void_p] * 4 + [c_int] * 4 + [c_void_p]),
     "riser_maxpool1d_pad_cl": (c_int, [c_void_p] * 4 + [c_int] * 5 + [c_void_p]),

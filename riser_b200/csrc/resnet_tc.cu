@@ -27,10 +27,19 @@
 // current item is worked on.  An identity shortcut is read back from that staging buffer.  Weights are copied into
 // shared memory once per CTA (persistent over items) from a host-packed image that already has the operand layout.
 //
-// Passes: with a = a_hi + a_lo and W = W_hi + W_lo the product is a_hi W_hi + a_lo W_hi + a_hi W_lo.  When 2 N <= 256
-// the two terms that share a_hi are ONE instruction -- B = [W_hi; W_lo] stacked, N doubled, the W_lo half landing in
-// its own accumulator columns, added by the epilogue -- so a tap and K step cost two MMAs instead of three (these
-// narrow MMAs are paced by their A-operand fetch, not by N).
+// Passes (precision mode P, include/riser_b200.h RISER_PREC_*): with a = a_hi + a_lo and W = W_hi + W_lo,
+//   F16_X3  a_hi W_hi + a_lo W_hi + a_hi W_lo (the default of riser_res_tc).  When 2 N <= 256 the two terms that
+//           share a_hi are ONE instruction -- B = [W_hi; W_lo] stacked, N doubled, the W_lo half landing in its own
+//           accumulator columns, added by the epilogue -- so a tap and K step cost two MMAs instead of three (these
+//           narrow MMAs are paced by their A-operand fetch, not by N).
+//   F16_W2  a_hi W_hi + a_hi W_lo: one stacked MMA per tap and K step when 2 N <= 256, else two.
+//   F16     a_hi W_hi.
+//   F16_F8  a_hi W_hi (kind::f16) + one e4m3 row per K block against the e4m3 weight row (kind::f8f6f4, K = 32 per
+//           instruction, two per K block): [e4m3(a 2^-3) x32 | e4m3((a - a_hi) 2^9) x32] . [e4m3(W_lo 2^3) x32 |
+//           e4m3(W 2^-9) x32], the two correction terms of X3 with 3 mantissa bits each (csrc/convnet.cu's F16_F8).
+// A tiles: hi fp16, plus (X3) the lo fp16 tile or (F8) the e4m3 tile in its place -- an e4m3 row of a 32-channel K
+// block is 64 bytes like an fp16 row, so it keeps the SWIZZLE_64B layout and the same descriptors; F16 and W2 have
+// no second A tile and need less shared memory.
 #include "common.cuh"
 
 #include <algorithm>
@@ -47,9 +56,9 @@ struct ResTcArgs {
   const int32_t* len_out;   // [B] valid output rows (after the stride; conv2 keeps the length)
   float* out;               // [B][Lout_pad][cout_p]
   const float* residual;    // identity shortcut / residual operand [B][Lout_pad][cout_p], or nullptr
-  const uint4* w1;          // packed image: [plane 2][tap][kb1][n1 rows][64 B]
-  const uint4* w2;          // fused: [plane 2][3][kb2][n2][64 B]; nullptr = single conv mode
-  const uint4* wsc;         // fused, shortcut conv: [plane 2][1][kb1][n2][64 B]; nullptr = none
+  const uint4* w1;          // packed image: [tap][kb1][plane (1 for F16, else 2)][n1 rows][64 B]
+  const uint4* w2;          // fused: [3][kb2][plane][n2][64 B]; nullptr = single conv mode
+  const uint4* wsc;         // fused, shortcut conv: [1][kb1][plane][n2][64 B]; nullptr = none
   const float* bias1;       // [n1]
   const float* bias2;       // [n2] (conv2 bias + shortcut-conv bias)
   float inv_scale1, inv_scale2;
@@ -64,7 +73,7 @@ struct ResTcArgs {
   uint32_t tiles_magic;          // floor(2^32 / tiles_per_read) + 1: item / tiles_per_read = umulhi(item, magic) (n_items < 2^20)
   int d2_col;                    // TMEM column of conv2's accumulator
   int tmem_cols;                 // columns allocated (power of two >= 32)
-  int cat1, cat2;                // conv1 / conv2: [W_hi; W_lo] stacked (accumulator = 2 n columns, two MMAs per step)
+  int cat1, cat2;                // conv1 / conv2: [W_hi; W_lo] stacked (accumulator = 2 n columns; W2 and X3 only)
   int raw_stages;                // raw fp32 input staging buffers (1 or 2)
   int raw_rows;                  // input rows an item stages
   uint32_t raw_bytes;            // bytes of one staging buffer
@@ -84,8 +93,22 @@ struct RtSmem {
 // paces these short MMAs).
 struct alignas(16) RtMma {
   uint64_t da, db;
-  uint32_t idesc, d_col, acc, pad_;
+  uint32_t idesc, d_col, acc, f8;      // f8: kind::f8f6f4 (the e4m3 pass of F16_F8), else kind::f16
 };
+
+constexpr int kPrecF16 = RISER_PREC_F16, kPrecW2 = RISER_PREC_F16_W2, kPrecX3 = RISER_PREC_F16_X3,
+              kPrecF8 = RISER_PREC_F16_F8;
+// A operand tiles per K block (hi, + lo or the e4m3 row) and weight planes per (tap, K block) of a mode
+__host__ __device__ constexpr int a_planes(int p) { return (p == kPrecX3 || p == kPrecF8) ? 2 : 1; }
+__host__ __device__ constexpr int w_planes(int p) { return p == kPrecF16 ? 1 : 2; }
+// the accumulator of a conv holds [a W_hi | a W_lo] side by side (the stacked B operand)
+__host__ __device__ constexpr bool cat_of(int p, int n) { return (p == kPrecX3 || p == kPrecW2) && 2 * n <= 256; }
+
+// F16_F8 row scales, the powers of two of riser_b200/model.py F8_A_SHIFT / F8_LO_SHIFT (as csrc/convnet.cu):
+// a8 = e4m3(a 2^-3) pairs with the W_lo 2^3 weight row, lo8 = e4m3((a - a_hi) 2^9) with the W 2^-9 row.
+// e4m3(a 2^-3) saturates at |a| = 3584.
+constexpr float kRtF8AScale = 1.f / 8.f;
+constexpr float kRtF8LoScale = 512.f;
 
 // fp32 x 8 -> fp16 hi (8 halfs = one 16-byte chunk) and lo = fp16(v - hi)
 __device__ __forceinline__ void split8(const float (&v)[8], uint4& hi, uint4& lo) {
@@ -101,39 +124,119 @@ __device__ __forceinline__ void split8(const float (&v)[8], uint4& hi, uint4& lo
   lo = *reinterpret_cast<const uint4*>(l);
 }
 
+// fp32 x 8 -> fp16 hi only (F16, W2)
+__device__ __forceinline__ uint4 half8(const float (&v)[8]) {
+  __half2 h[4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j)
+    h[j] = __hmin2(__hmax2(__floats2half2_rn(v[2 * j], v[2 * j + 1]), __floats2half2_rn(-65504.f, -65504.f)),
+                   __floats2half2_rn(65504.f, 65504.f));
+  return *reinterpret_cast<const uint4*>(h);
+}
+
+// fp32 x 8 -> fp16 hi, a8 = e4m3(v 2^-3) and lo8 = e4m3((v - hi) 2^9) (8 bytes each; F16_F8)
+__device__ __forceinline__ void split8_f8(const float (&v)[8], uint4& hi, uint2& a8, uint2& lo8) {
+  hi = half8(v);
+  const __half2* h = reinterpret_cast<const __half2*>(&hi);
+  uint32_t pa[2], pl[2];
+#pragma unroll
+  for (int j = 0; j < 2; ++j) {
+    uint32_t wa[2], wl[2];
+#pragma unroll
+    for (int e = 0; e < 2; ++e) {
+      const int c = 4 * j + 2 * e;
+      const float2 back = __half22float2(h[c / 2]);
+      wa[e] = __nv_cvt_float2_to_fp8x2(make_float2(v[c] * kRtF8AScale, v[c + 1] * kRtF8AScale), __NV_SATFINITE,
+                                       __NV_E4M3);
+      wl[e] = __nv_cvt_float2_to_fp8x2(make_float2((v[c] - back.x) * kRtF8LoScale, (v[c + 1] - back.y) * kRtF8LoScale),
+                                       __NV_SATFINITE, __NV_E4M3);
+    }
+    pa[j] = wa[0] | (wa[1] << 16);
+    pl[j] = wl[0] | (wl[1] << 16);
+  }
+  a8 = make_uint2(pa[0], pa[1]);
+  lo8 = make_uint2(pl[0], pl[1]);
+}
+
+// Byte offset of (row r, byte) in a SWIZZLE_64B tile: 16-byte chunk c of a row lands at c ^ ((r >> 1) & 3)
+__device__ __forceinline__ uint32_t sw64(int r, int byte) {
+  return static_cast<uint32_t>(r * 64 + ((((byte >> 4) ^ (r >> 1)) & 3) << 4) + (byte & 15));
+}
+
+// The operand tiles of 8 channels (group g, K block g >> 2) of row r in the mode's format: hi at `hi_tile`, and the
+// lo fp16 (X3) or the a8 / lo8 bytes (F8) at the same place in the tile `lo_off` bytes further
+template <int P>
+__device__ __forceinline__ void store_act8(unsigned char* hi_tile, uint32_t lo_off, int g, int r, const float (&v)[8]) {
+  unsigned char* t = hi_tile + (g >> 2) * kRtTile;
+  if (P == kPrecX3) {
+    uint4 hi, lo;
+    split8(v, hi, lo);
+    *reinterpret_cast<uint4*>(t + sw64(r, 16 * (g & 3))) = hi;
+    *reinterpret_cast<uint4*>(t + lo_off + sw64(r, 16 * (g & 3))) = lo;
+  } else if (P == kPrecF8) {
+    uint4 hi;
+    uint2 a8, lo8;
+    split8_f8(v, hi, a8, lo8);
+    *reinterpret_cast<uint4*>(t + sw64(r, 16 * (g & 3))) = hi;
+    *reinterpret_cast<uint2*>(t + lo_off + sw64(r, 8 * (g & 3))) = a8;          // e4m3 row bytes [0, 32): a8
+    *reinterpret_cast<uint2*>(t + lo_off + sw64(r, 32 + 8 * (g & 3))) = lo8;    // bytes [32, 64): lo8
+  } else {
+    *reinterpret_cast<uint4*>(t + sw64(r, 16 * (g & 3))) = half8(v);
+  }
+}
+
 __device__ __forceinline__ uint64_t rt_desc(uint32_t addr) {      // K-major SWIZZLE_64B, 8-row atoms of 512 B
   constexpr uint64_t kHi = (static_cast<uint64_t>(1) << 16) | (static_cast<uint64_t>(512 >> 4) << 32) |
                            (static_cast<uint64_t>(1) << 46) | (static_cast<uint64_t>(4) << 61);
   return kHi | static_cast<uint64_t>(addr >> 4);
 }
 
-// weight image: [tap][K block][plane hi, lo][n rows][64 B] -- for a (tap, K block) the hi rows are followed by the lo
-// rows, so the stacked operand [W_hi; W_lo] is one contiguous 2n-row tile
+// weight image: [tap][K block][plane][n rows][64 B] -- for a (tap, K block) the hi rows are followed by the lo rows
+// (W2, X3: the stacked operand [W_hi; W_lo] is one contiguous 2n-row tile) or the e4m3 rows (F8); F16 has hi only
+template <int P>
 __device__ __forceinline__ uint32_t w_tile(uint32_t base, int tap, int kb, int n_kb, int n) {
-  return base + static_cast<uint32_t>((tap * n_kb + kb) * 2 * n * 64);
+  return base + static_cast<uint32_t>((tap * n_kb + kb) * w_planes(P) * n * 64);
 }
 
-// The MMAs of one term  D += A(view) * W(tap)  over the K blocks:  a_hi x [W_hi; W_lo] + a_lo x W_hi  (cat), or the three
-// products one by one, appended to a replay list.  a_hi / a_lo: shared-memory addresses of the hi / lo A tiles of K
-// block 0 (consecutive K blocks kRtTile apart), already shifted to the view's first row.
+// The MMAs of one term  D += A(view) * W(tap)  over the K blocks, appended to a replay list.  X3: a_hi x [W_hi; W_lo] +
+// a_lo x W_hi (cat), or the three products one by one; W2: a_hi x [W_hi; W_lo] (cat) or its two products; F16:
+// a_hi x W_hi; F8: a_hi x W_hi per K step, then the two e4m3 steps of the K block.  a_hi / a_lo: shared-memory
+// addresses of the hi / second A tiles of K block 0 (consecutive K blocks kRtTile apart), already shifted to the
+// view's first row.
+template <int P>
 __device__ __forceinline__ int list_term(RtMma* list, int n_list, uint32_t d_col, uint32_t a_hi, uint32_t a_lo,
                                          uint32_t w_base, int tap, int n_kb, int k_ch, int n, bool cat,
                                          uint32_t idesc_n, uint32_t idesc_2n) {
   for (int kb = 0; kb < n_kb; ++kb) {
     const int nk = min(2, (k_ch - 32 * kb + 15) >> 4);
-    const uint32_t wt = w_tile(w_base, tap, kb, n_kb, n);
+    const uint32_t wt = w_tile<P>(w_base, tap, kb, n_kb, n);
     for (int k = 0; k < nk; ++k) {
       const uint64_t ah = rt_desc(a_hi + kb * kRtTile) + 2 * k, al = rt_desc(a_lo + kb * kRtTile) + 2 * k;
       const uint64_t wh = rt_desc(wt) + 2 * k, wl = rt_desc(wt + n * 64) + 2 * k;
       const uint32_t acc = n_list ? 1u : 0u;
-      if (cat) {
-        list[n_list++] = RtMma{ah, wh, idesc_2n, d_col, acc, 0u};   // columns [0, n): a_hi W_hi, [n, 2n): a_hi W_lo
-        list[n_list++] = RtMma{al, wh, idesc_n, d_col, 1u, 0u};     // columns [0, n) += a_lo W_hi
+      if (P == kPrecX3) {
+        if (cat) {
+          list[n_list++] = RtMma{ah, wh, idesc_2n, d_col, acc, 0u};   // columns [0, n): a_hi W_hi, [n, 2n): a_hi W_lo
+          list[n_list++] = RtMma{al, wh, idesc_n, d_col, 1u, 0u};     // columns [0, n) += a_lo W_hi
+        } else {
+          list[n_list++] = RtMma{ah, wh, idesc_n, d_col, acc, 0u};
+          list[n_list++] = RtMma{al, wh, idesc_n, d_col, 1u, 0u};
+          list[n_list++] = RtMma{ah, wl, idesc_n, d_col, 1u, 0u};
+        }
+      } else if (P == kPrecW2) {
+        if (cat) {
+          list[n_list++] = RtMma{ah, wh, idesc_2n, d_col, acc, 0u};
+        } else {
+          list[n_list++] = RtMma{ah, wh, idesc_n, d_col, acc, 0u};
+          list[n_list++] = RtMma{ah, wl, idesc_n, d_col, 1u, 0u};
+        }
       } else {
         list[n_list++] = RtMma{ah, wh, idesc_n, d_col, acc, 0u};
-        list[n_list++] = RtMma{al, wh, idesc_n, d_col, 1u, 0u};
-        list[n_list++] = RtMma{ah, wl, idesc_n, d_col, 1u, 0u};
       }
+    }
+    if (P == kPrecF8) {       // [a8 | lo8] x [W_lo 2^3 | W 2^-9]: 64 e4m3 per row = two K = 32 steps of 32 bytes
+      const uint64_t a8 = rt_desc(a_lo + kb * kRtTile), w8 = rt_desc(wt + n * 64);
+      for (int k = 0; k < 2; ++k) list[n_list++] = RtMma{a8 + 2 * k, w8 + 2 * k, idesc_n, d_col, 1u, 1u};
     }
   }
   return n_list;
@@ -144,37 +247,54 @@ __device__ __forceinline__ int list_term(RtMma* list, int n_list, uint32_t d_col
 #ifndef RISER_RT_REPLAY
 #define RISER_RT_REPLAY 1      // measured: the replayed list 1.009 ms, the uniform loop nest 1.045 ms (512 x 12,048, basic)
 #endif
+template <int P>
 __device__ __forceinline__ void issue_term_uniform(bool leader, uint32_t d, uint32_t a_hi, uint32_t a_lo, uint32_t w_base,
                                                    int tap, int n_kb, int k_ch, int n, bool cat, uint32_t idesc_n,
                                                    uint32_t idesc_2n, uint32_t& acc) {
   for (int kb = 0; kb < n_kb; ++kb) {
     const int nk = min(2, (k_ch - 32 * kb + 15) >> 4);
-    const uint32_t wt = w_tile(w_base, tap, kb, n_kb, n);
+    const uint32_t wt = w_tile<P>(w_base, tap, kb, n_kb, n);
     const uint64_t ah0 = rt_desc(a_hi + kb * kRtTile), al0 = rt_desc(a_lo + kb * kRtTile);
     const uint64_t wh0 = rt_desc(wt), wl0 = rt_desc(wt + n * 64);
     if (leader) {
 #pragma unroll
       for (int k = 0; k < 2; ++k)
         if (k < nk) {
-          if (cat) {
-            umma_f16(d, ah0 + 2 * k, wh0 + 2 * k, idesc_2n, (k == 0) ? acc : 1u);
-            umma_f16(d, al0 + 2 * k, wh0 + 2 * k, idesc_n, 1u);
+          const uint32_t a0 = (k == 0) ? acc : 1u;
+          if (P == kPrecX3) {
+            if (cat) {
+              umma_f16(d, ah0 + 2 * k, wh0 + 2 * k, idesc_2n, a0);
+              umma_f16(d, al0 + 2 * k, wh0 + 2 * k, idesc_n, 1u);
+            } else {
+              umma_f16(d, ah0 + 2 * k, wh0 + 2 * k, idesc_n, a0);
+              umma_f16(d, al0 + 2 * k, wh0 + 2 * k, idesc_n, 1u);
+              umma_f16(d, ah0 + 2 * k, wl0 + 2 * k, idesc_n, 1u);
+            }
+          } else if (P == kPrecW2) {
+            umma_f16(d, ah0 + 2 * k, wh0 + 2 * k, cat ? idesc_2n : idesc_n, a0);
+            if (!cat) umma_f16(d, ah0 + 2 * k, wl0 + 2 * k, idesc_n, 1u);
           } else {
-            umma_f16(d, ah0 + 2 * k, wh0 + 2 * k, idesc_n, (k == 0) ? acc : 1u);
-            umma_f16(d, al0 + 2 * k, wh0 + 2 * k, idesc_n, 1u);
-            umma_f16(d, ah0 + 2 * k, wl0 + 2 * k, idesc_n, 1u);
+            umma_f16(d, ah0 + 2 * k, wh0 + 2 * k, idesc_n, a0);
           }
         }
+      if (P == kPrecF8) {
+#pragma unroll
+        for (int k = 0; k < 2; ++k) umma_f8(d, al0 + 2 * k, wl0 + 2 * k, idesc_n, 1u);
+      }
     }
     acc = 1u;
   }
 }
 
+template <int P>
 __device__ __forceinline__ void replay(const RtMma* list, int n, uint32_t tmem_base) {
 #pragma unroll 4
   for (int i = 0; i < n; ++i) {
     const RtMma e = list[i];
-    umma_f16(tmem_base + e.d_col, e.da, e.db, e.idesc, e.acc);
+    if (P == kPrecF8 && e.f8)
+      umma_f8(tmem_base + e.d_col, e.da, e.db, e.idesc, e.acc);
+    else
+      umma_f16(tmem_base + e.d_col, e.da, e.db, e.idesc, e.acc);
   }
 }
 
@@ -195,17 +315,19 @@ __device__ __forceinline__ void cta_wait(uint64_t* bar, uint32_t parity) {
   }
 }
 
+template <int P>
 __global__ void __launch_bounds__(kRtThreads)
 res_tc_kernel(const ResTcArgs a) {
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* base = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
   const bool fused = a.w2 != nullptr;
   const int parts = a.stride == 2 ? 2 : 1;                       // staged input tiles per plane: X, or E and O
-  const uint32_t w1_bytes = 2u * a.taps * a.kb1 * a.n1 * 64u;
-  const uint32_t w2_bytes = fused ? 2u * 3 * a.kb2 * a.n2 * 64u : 0u;
-  const uint32_t wsc_bytes = a.wsc ? 2u * a.kb1 * a.n2 * 64u : 0u;
-  const uint32_t a1_bytes = 2u * parts * a.kb1 * kRtTile;
-  const uint32_t a2_bytes = fused ? 2u * a.kb2 * kRtTile : 0u;
+  constexpr uint32_t kWp = w_planes(P), kAp = a_planes(P);
+  const uint32_t w1_bytes = kWp * a.taps * a.kb1 * a.n1 * 64u;
+  const uint32_t w2_bytes = fused ? kWp * 3 * a.kb2 * a.n2 * 64u : 0u;
+  const uint32_t wsc_bytes = a.wsc ? kWp * a.kb1 * a.n2 * 64u : 0u;
+  const uint32_t a1_bytes = kAp * parts * a.kb1 * kRtTile;
+  const uint32_t a2_bytes = fused ? kAp * a.kb2 * kRtTile : 0u;
   unsigned char* w1s = base;
   unsigned char* w2s = w1s + w1_bytes;
   unsigned char* wscs = w2s + w2_bytes;
@@ -251,7 +373,7 @@ res_tc_kernel(const ResTcArgs a) {
   const uint32_t idesc2 = umma_idesc_f16(128, a.n2), idesc2c = umma_idesc_f16(128, 2 * a.n2);
   const uint32_t w1_addr = smem_u32(w1s), w2_addr = smem_u32(w2s), wsc_addr = smem_u32(wscs);
   const uint32_t a1_addr = smem_u32(a1s), a2_addr = smem_u32(a2s);
-  const uint32_t a1_lo = parts * a.kb1 * kRtTile, a2_lo = a.kb2 * kRtTile;     // hi -> lo plane offsets
+  const uint32_t a1_lo = parts * a.kb1 * kRtTile, a2_lo = a.kb2 * kRtTile;     // hi -> lo / e4m3 tile offsets (X3, F8)
   const int groups = a.cin_p >> 3;                               // 8-channel groups per input row
   const int pad = (a.taps - 1) >> 1;
   const int row_bytes = a.cin_p * 4;
@@ -267,19 +389,19 @@ res_tc_kernel(const ResTcArgs a) {
         else { part = 1; shift = (tap == 2) ? 1 : 0; }                  // w0 O[m-1], w2 O[m]
       }
       const uint32_t av = a1_addr + part * a.kb1 * kRtTile + shift * 64;
-      n = list_term(list1, n, 0u, av, av + a1_lo, w1_addr, tap, a.kb1, a.cin_p, a.n1, a.cat1 != 0, idesc1, idesc1c);
+      n = list_term<P>(list1, n, 0u, av, av + a1_lo, w1_addr, tap, a.kb1, a.cin_p, a.n1, a.cat1 != 0, idesc1, idesc1c);
     }
     if (fused) {
       // conv2 (+ 1x1 shortcut conv): D2[i] = sum_t W2_t A2[i + t]  (+ Wsc x[s (p0 + i)])
       n = 0;
       for (int tap = 0; tap < 3; ++tap) {
         const uint32_t av = a2_addr + tap * 64;
-        n = list_term(list2, n, a.d2_col, av, av + a2_lo, w2_addr, tap, a.kb2, a.cmid_p, a.n2, a.cat2 != 0, idesc2, idesc2c);
+        n = list_term<P>(list2, n, a.d2_col, av, av + a2_lo, w2_addr, tap, a.kb2, a.cmid_p, a.n2, a.cat2 != 0, idesc2, idesc2c);
       }
       if (a.wsc) {
         // x[s (p0 + i)]: stride 1 -> X row i + 1 + pad; stride 2 -> E row i + 1
         const uint32_t av = a1_addr + ((a.stride == 2) ? 1 : 1 + pad) * 64;
-        n = list_term(list2, n, a.d2_col, av, av + a1_lo, wsc_addr, 0, a.kb1, a.cin_p, a.n2, a.cat2 != 0, idesc2, idesc2c);
+        n = list_term<P>(list2, n, a.d2_col, av, av + a1_lo, wsc_addr, 0, a.kb1, a.cin_p, a.n2, a.cat2 != 0, idesc2, idesc2c);
       }
     }
     mbar_wait(&s.w_full, 0);                                     // the weight images have landed
@@ -330,7 +452,7 @@ res_tc_kernel(const ResTcArgs a) {
     // two staging buffers: the next item's rows start to arrive now, while this item is worked on
     if (a.raw_stages == 2 && tid == 0 && nxt < a.n_items) prefetch(nxt, slot ^ 1);
 
-    // ---------------- convert: raw fp32 rows -> fp16 hi / lo tiles (swizzled K-major)
+    // ---------------- convert: raw fp32 rows -> the mode's A tiles (swizzled K-major)
     // stride 1: X row r = x[q0 - pad + r];  stride 2: E row r = x[2 (q0 + r)], O row r = x[2 (q0 - 1 + r) + 1]
     cta_wait(&s.raw_full[slot], (a.raw_stages == 2) ? ((k >> 1) & 1) : (k & 1));
     const float* raw = reinterpret_cast<const float*>(raws + slot * a.raw_bytes);
@@ -358,12 +480,7 @@ res_tc_kernel(const ResTcArgs a) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) v[j] = 0.f;
       }
-      uint4 hi, lo;
-      split8(v, hi, lo);
-      const uint32_t off = static_cast<uint32_t>((part * a.kb1 + (g >> 2)) * kRtTile + r * 64 +
-                                                 (((g & 3) ^ ((r >> 1) & 3)) << 4));
-      *reinterpret_cast<uint4*>(a1s + off) = hi;
-      *reinterpret_cast<uint4*>(a1s + a1_lo + off) = lo;
+      store_act8<P>(a1s + part * a.kb1 * kRtTile, a1_lo, g, r, v);
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     tc_fence_before();
@@ -376,7 +493,7 @@ res_tc_kernel(const ResTcArgs a) {
     if (RISER_RT_REPLAY) {
       if (tid == 0) {
         tc_fence_after();
-        replay(list1, a.n_mma1, tmem_base);
+        replay<P>(list1, a.n_mma1, tmem_base);
         umma_commit(&s.bar);
       }
     } else if (warp == 0) {
@@ -390,7 +507,7 @@ res_tc_kernel(const ResTcArgs a) {
           else { part = 1; shift = (tap == 2) ? 1 : 0; }                  // w0 O[m-1], w2 O[m]
         }
         const uint32_t av = a1_addr + part * a.kb1 * kRtTile + shift * 64;
-        issue_term_uniform(leader, tmem_base, av, av + a1_lo, w1_addr, tap, a.kb1, a.cin_p, a.n1, a.cat1 != 0, idesc1,
+        issue_term_uniform<P>(leader, tmem_base, av, av + a1_lo, w1_addr, tap, a.kb1, a.cin_p, a.n1, a.cat1 != 0, idesc1,
                            idesc1c, acc);
       }
       umma_commit_p(leader ? 1u : 0u, &s.bar);
@@ -403,7 +520,8 @@ res_tc_kernel(const ResTcArgs a) {
     const int row = 32 * quad + lane;                              // this thread's accumulator row (TMEM lane)
     const uint32_t t_lane = tmem_base + (static_cast<uint32_t>(32 * quad) << 16);
     if (fused) {
-      // ---------------- mid-epilogue: bias + ReLU + length mask -> conv2's A operand (row j = mid row q0 + j)
+      // ---------------- mid-epilogue: bias + ReLU + length mask -> conv2's A operand in the mode's format (row j =
+      // mid row q0 + j)
       const int m = q0 + row;
       const bool live = (m >= 0 && m < n_out);
       for (int c16 = 16 * half; c16 < a.n1; c16 += 32) {
@@ -422,12 +540,7 @@ res_tc_kernel(const ResTcArgs a) {
             if (a.cat1) acc += __uint_as_float(w[8 * h8 + j]);
             r[j] = live ? fmaxf(fmaf(acc, a.inv_scale1, bias1s[c + j]), 0.f) : 0.f;
           }
-          uint4 hi, lo;
-          split8(r, hi, lo);
-          const int g = c >> 3;
-          const uint32_t off = static_cast<uint32_t>((g >> 2) * kRtTile + row * 64 + (((g & 3) ^ ((row >> 1) & 3)) << 4));
-          *reinterpret_cast<uint4*>(a2s + off) = hi;
-          *reinterpret_cast<uint4*>(a2s + a2_lo + off) = lo;
+          store_act8<P>(a2s, a2_lo, c >> 3, row, r);
         }
       }
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -438,7 +551,7 @@ res_tc_kernel(const ResTcArgs a) {
       if (RISER_RT_REPLAY) {
         if (tid == 0) {
           tc_fence_after();
-          replay(list2, a.n_mma2, tmem_base);
+          replay<P>(list2, a.n_mma2, tmem_base);
           umma_commit(&s.bar);
         }
       } else if (warp == 0) {
@@ -448,12 +561,12 @@ res_tc_kernel(const ResTcArgs a) {
         const uint32_t d2 = tmem_base + a.d2_col;
         for (int tap = 0; tap < 3; ++tap) {
           const uint32_t av = a2_addr + tap * 64;
-          issue_term_uniform(leader, d2, av, av + a2_lo, w2_addr, tap, a.kb2, a.cmid_p, a.n2, a.cat2 != 0, idesc2, idesc2c, acc);
+          issue_term_uniform<P>(leader, d2, av, av + a2_lo, w2_addr, tap, a.kb2, a.cmid_p, a.n2, a.cat2 != 0, idesc2, idesc2c, acc);
         }
         if (a.wsc) {
           // x[s (p0 + i)]: stride 1 -> X row i + 1 + pad; stride 2 -> E row i + 1
           const uint32_t av = a1_addr + ((a.stride == 2) ? 1 : 1 + pad) * 64;
-          issue_term_uniform(leader, d2, av, av + a1_lo, wsc_addr, 0, a.kb1, a.cin_p, a.n2, a.cat2 != 0, idesc2, idesc2c, acc);
+          issue_term_uniform<P>(leader, d2, av, av + a1_lo, wsc_addr, 0, a.kb1, a.cin_p, a.n2, a.cat2 != 0, idesc2, idesc2c, acc);
         }
         umma_commit_p(leader ? 1u : 0u, &s.bar);
       }
@@ -542,45 +655,62 @@ using namespace riser;
 namespace riser {
 namespace {
 int raw_rows_of(int taps, int stride) { return stride == 2 ? 258 : 128 + (taps - 1); }
-int mma_count(int taps, int k_ch, int n) {       // MMAs of `taps` terms over k_ch channels (two per step stacked, else three)
+// MMAs of `taps` terms over k_ch channels in mode p (list_term): per fp16 K step X3 two stacked / three, W2 one stacked /
+// two, F16 one, F8 one; F8 adds two e4m3 steps per K block
+int mma_count(int taps, int k_ch, int n, int p) {
   int steps = 0;
-  for (int kb = 0; kb < (k_ch + 31) / 32; ++kb) steps += std::min(2, (k_ch - 32 * kb + 15) >> 4);
-  return taps * steps * (2 * n <= 256 ? 2 : 3);
+  const int kb = (k_ch + 31) / 32;
+  for (int b = 0; b < kb; ++b) steps += std::min(2, (k_ch - 32 * b + 15) >> 4);
+  const bool cat = cat_of(p, n);
+  const int per = p == kPrecX3 ? (cat ? 2 : 3) : p == kPrecW2 ? (cat ? 1 : 2) : 1;
+  return taps * (steps * per + (p == kPrecF8 ? 2 * kb : 0));
 }
+int acc_cols(int n, int p) { return ((cat_of(p, n) ? 2 * n : n) + 31) / 32 * 32; }
+bool prec_ok(int p) { return p == kPrecF16 || p == kPrecW2 || p == kPrecX3 || p == kPrecF8; }
 size_t raw_bytes_of(int cin_p, int taps, int stride) {
   return (static_cast<size_t>(raw_rows_of(taps, stride)) * cin_p * 4 + 127) & ~size_t(127);
 }
 }  // namespace
 }  // namespace riser
 
-// Shared memory the kernel needs for a shape with ONE raw staging buffer (0 = the shape is not supported).
-extern "C" size_t riser_res_tc_smem(int cin_p, int cmid_p, int n1, int n2, int taps, int stride, int fused,
-                                    int shortcut_conv) {
+// Shared memory the kernel needs for a shape with ONE raw staging buffer (0 = the shape or the mode is not supported).
+// Modes without a second A tile (F16, W2) or without a weight lo plane (F16) need less.
+extern "C" size_t riser_res_tc_smem_ex(int cin_p, int cmid_p, int n1, int n2, int taps, int stride, int fused,
+                                       int shortcut_conv, int precision) {
+  if (!prec_ok(precision)) return 0;
   if (cin_p <= 0 || (cin_p & 7) || n1 <= 0 || (n1 & 15) || n1 > 256 || (taps != 1 && taps != 3) ||
       (stride != 1 && stride != 2))
     return 0;
   if (fused && (cmid_p <= 0 || (cmid_p & 7) || n2 <= 0 || (n2 & 15) || n2 > 256 || taps != 3)) return 0;
   const int kb1 = (cin_p + 31) / 32, kb2 = fused ? (cmid_p + 31) / 32 : 0;
   const int parts = stride == 2 ? 2 : 1;
-  size_t bytes = 1024 + 2u * taps * kb1 * n1 * 64u + 2u * parts * kb1 * kRtTile + raw_bytes_of(cin_p, taps, stride) +
+  const size_t wp = w_planes(precision), ap = a_planes(precision);
+  size_t bytes = 1024 + wp * taps * kb1 * n1 * 64u + ap * parts * kb1 * kRtTile + raw_bytes_of(cin_p, taps, stride) +
                  sizeof(float) * n1 + sizeof(RtSmem) + 64 +
-                 sizeof(RtMma) * (mma_count(taps, cin_p, n1) + (fused ? mma_count(3, cmid_p, n2) + (shortcut_conv ? mma_count(1, cin_p, n2) : 0) : 0));
+                 sizeof(RtMma) * (mma_count(taps, cin_p, n1, precision) +
+                                  (fused ? mma_count(3, cmid_p, n2, precision) +
+                                               (shortcut_conv ? mma_count(1, cin_p, n2, precision) : 0) : 0));
   if (fused) {
-    bytes += 2u * 3 * kb2 * n2 * 64u + 2u * kb2 * kRtTile + sizeof(float) * n2;
-    if (shortcut_conv) bytes += ((2u * kb1 * n2 * 64u) + 511u) & ~size_t(511);
-    const int cols = ((2 * n1 <= 256 ? 2 * n1 : n1) + 31) / 32 * 32 + ((2 * n2 <= 256 ? 2 * n2 : n2) + 31) / 32 * 32;
-    if (cols > 512) return 0;
+    bytes += wp * 3 * kb2 * n2 * 64u + ap * kb2 * kRtTile + sizeof(float) * n2;
+    if (shortcut_conv) bytes += ((wp * kb1 * n2 * 64u) + 511u) & ~size_t(511);
+    if (acc_cols(n1, precision) + acc_cols(n2, precision) > 512) return 0;
   }
   return bytes;
 }
 
+extern "C" size_t riser_res_tc_smem(int cin_p, int cmid_p, int n1, int n2, int taps, int stride, int fused,
+                                    int shortcut_conv) {
+  return riser_res_tc_smem_ex(cin_p, cmid_p, n1, n2, taps, stride, fused, shortcut_conv, RISER_PREC_F16_X3);
+}
+
 // Replaces one conv_block (+ optional residual) or one whole BasicBlock of riser/nets/resnet.py on the tensor
-// pipe; see the header for the argument conventions.
-extern "C" int riser_res_tc(const float* in, const int32_t* len_in, const int32_t* len_out, float* out,
-                            const float* residual, const void* w1, const void* w2, const void* wsc,
-                            const float* bias1, const float* bias2, float inv_scale1, float inv_scale2, int B,
-                            int Lin_pad, int Lout_pad, int cin_p, int cmid_p, int cout_p, int n1, int n2, int taps,
-                            int stride, int relu, riser_stream_t stream) {
+// pipe in the given precision mode; see the header for the argument conventions.
+extern "C" int riser_res_tc_ex(const float* in, const int32_t* len_in, const int32_t* len_out, float* out,
+                               const float* residual, const void* w1, const void* w2, const void* wsc,
+                               const float* bias1, const float* bias2, float inv_scale1, float inv_scale2, int B,
+                               int Lin_pad, int Lout_pad, int cin_p, int cmid_p, int cout_p, int n1, int n2, int taps,
+                               int stride, int relu, riser_stream_t stream, int precision) {
+  RISER_REQUIRE(prec_ok(precision), "riser_res_tc: unknown precision mode %d", precision);
   RISER_REQUIRE(in && len_in && len_out && out && w1 && bias1, "riser_res_tc: null pointer");
   RISER_REQUIRE(B > 0 && Lin_pad > 0 && Lout_pad > 0, "riser_res_tc: bad shape");
   const int fused = w2 != nullptr;
@@ -590,7 +720,7 @@ extern "C" int riser_res_tc(const float* in, const int32_t* len_in, const int32_
   RISER_REQUIRE(((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out) |
                   reinterpret_cast<uintptr_t>(residual)) & 31) == 0,
                 "riser_res_tc: activation buffers must be 32-byte aligned");
-  const size_t smem = riser_res_tc_smem(cin_p, cmid_p, n1, n2, taps, stride, fused, wsc != nullptr);
+  const size_t smem = riser_res_tc_smem_ex(cin_p, cmid_p, n1, n2, taps, stride, fused, wsc != nullptr, precision);
   RISER_REQUIRE(smem > 0, "riser_res_tc: unsupported shape (cin_p %d, n1 %d, n2 %d, taps %d, stride %d)", cin_p, n1,
                 n2, taps, stride);
   int dev = 0, sms = 148, max_smem = 0;
@@ -612,12 +742,12 @@ extern "C" int riser_res_tc(const float* in, const int32_t* len_in, const int32_
   a.n_items = B * a.tiles_per_read;
   RISER_REQUIRE(a.n_items < (1 << 20), "riser_res_tc: %d work items (B x tiles per read) exceed 2^20", a.n_items);
   a.tiles_magic = static_cast<uint32_t>((1ull << 32) / static_cast<unsigned>(a.tiles_per_read)) + 1u;
-  a.cat1 = (2 * n1 <= 256) ? 1 : 0;
-  a.cat2 = (fused && 2 * n2 <= 256) ? 1 : 0;
-  a.d2_col = ((a.cat1 ? 2 * n1 : n1) + 31) & ~31;
-  a.tmem_cols = pow2_at_least(a.d2_col + (fused ? (((a.cat2 ? 2 * n2 : n2) + 31) & ~31) : 0));
-  a.n_mma1 = mma_count(taps, cin_p, n1);
-  a.n_mma2 = fused ? mma_count(3, cmid_p, n2) + (wsc ? mma_count(1, cin_p, n2) : 0) : 0;
+  a.cat1 = cat_of(precision, n1) ? 1 : 0;
+  a.cat2 = (fused && cat_of(precision, n2)) ? 1 : 0;
+  a.d2_col = acc_cols(n1, precision);
+  a.tmem_cols = pow2_at_least(a.d2_col + (fused ? acc_cols(n2, precision) : 0));
+  a.n_mma1 = mma_count(taps, cin_p, n1, precision);
+  a.n_mma2 = fused ? mma_count(3, cmid_p, n2, precision) + (wsc ? mma_count(1, cin_p, n2, precision) : 0) : 0;
   a.raw_rows = raw_rows_of(taps, stride);
   a.raw_bytes = static_cast<uint32_t>(raw_bytes_of(cin_p, taps, stride));
   // CTAs per SM: as many as shared memory allows, but their TMEM allocations must fit the 512 columns of an SM
@@ -632,9 +762,23 @@ extern "C" int riser_res_tc(const float* in, const int32_t* len_in, const int32_
   size_t request = smem + (a.raw_stages == 2 ? a.raw_bytes : 0);
   const size_t floor_for_cap = static_cast<size_t>(227 * 1024) / (ctas + 1) + 1;      // > 1/(ctas+1) of the SM's shared memory
   if (request < floor_for_cap) request = std::min<size_t>(floor_for_cap, max_smem);
-  RISER_CUDA_TRY(cudaFuncSetAttribute(res_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
+  void (*kernel)(const ResTcArgs) = precision == kPrecF16 ? res_tc_kernel<kPrecF16>
+                                    : precision == kPrecW2  ? res_tc_kernel<kPrecW2>
+                                    : precision == kPrecF8  ? res_tc_kernel<kPrecF8>
+                                                            : res_tc_kernel<kPrecX3>;
+  RISER_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
   const int grid = std::min(a.n_items, sms * ctas);
-  res_tc_kernel<<<grid, kRtThreads, request, as_stream(stream)>>>(a);
+  kernel<<<grid, kRtThreads, request, as_stream(stream)>>>(a);
   RISER_CUDA_TRY(cudaGetLastError());
   return RISER_OK;
+}
+
+extern "C" int riser_res_tc(const float* in, const int32_t* len_in, const int32_t* len_out, float* out,
+                            const float* residual, const void* w1, const void* w2, const void* wsc,
+                            const float* bias1, const float* bias2, float inv_scale1, float inv_scale2, int B,
+                            int Lin_pad, int Lout_pad, int cin_p, int cmid_p, int cout_p, int n1, int n2, int taps,
+                            int stride, int relu, riser_stream_t stream) {
+  return riser_res_tc_ex(in, len_in, len_out, out, residual, w1, w2, wsc, bias1, bias2, inv_scale1, inv_scale2, B,
+                         Lin_pad, Lout_pad, cin_p, cmid_p, cout_p, n1, n2, taps, stride, relu, stream,
+                         RISER_PREC_F16_X3);
 }

@@ -4,8 +4,9 @@ in csrc/convnet.cu.
 ``Model(state, config, logger, target)`` and ``Model.classify(signal)`` keep the
 reference's signature and behaviour (riser/model.py:7-28) so ``riser.py:41`` and
 ``control.py:69`` work unchanged; ``classify_batch`` is the additive batched entry
-the rewritten loop uses.  There is no CPU fallback: constructing a Model without an
-sm_100 device raises.
+the rewritten loop uses.  A config with ``model: resnet`` (train.py:177-178) builds the
+ResNet variant instead (``resnet.ResNetModel``, same call surface).  There is no CPU
+fallback: constructing a Model without an sm_100 device raises.
 """
 import ctypes
 
@@ -105,6 +106,14 @@ class Plan:
 
 
 class Model():
+    def __new__(cls, state=None, config=None, logger=None, target=None, precision=None):
+        # a checkpoint trained with `model: resnet` (the reference's train.py) comes with a `resnet:` section and no
+        # `cnn:` one: Model then is the ResNet variant (riser_b200/resnet.py), with the same call surface
+        if cls is Model and getattr(config, "model", "cnn") == "resnet":
+            from .resnet import ResNetModel
+            return ResNetModel(state, config, logger, target, precision=precision)
+        return super().__new__(cls)
+
     def __init__(self, state, config, logger, target, precision=None):
         self.target = target
 

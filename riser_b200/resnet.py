@@ -5,13 +5,18 @@ The reference can only select it in train.py:177-178 (``config.model == 'resnet'
 whatever the caller's config says: ``channels, kernel, padding, stride, block, n_layers,
 blocks, n_classes`` (resnet.py:73-102).  BatchNorm (eval mode) is folded into the convolution
 weights here on the host.  The residual blocks run on the tensor pipe (csrc/resnet_tc.cu: tcgen05 implicit GEMM,
-fp16 hi + lo operand planes, fp32 accumulation in TMEM) -- a BasicBlock as ONE launch whose intermediate
+fp16 operand planes, fp32 accumulation in TMEM) -- a BasicBlock as ONE launch whose intermediate
 activation never leaves the SM, the convolutions of a BottleneckBlock (and blocks whose weights do not fit
 shared memory fused) one launch each with the residual added in the epilogue; the stem (Cin = 1, K = 19: 3 % of the
 FLOPs), its max-pool and the head stay on the fp32 CUDA-core kernels of csrc/resnet.cu, which also remain the
 fallback for shapes the tensor-core kernel does not take (``RISER_RESNET_TC=0`` forces them everywhere).
 Activations are fp32 channel-last [B][L][C_p] with the channels padded to a multiple of 8 (zero weights / biases in
 the padding, so the padding channels stay zero through every layer).
+
+Precision (``ResNetModel(..., precision=)``, the PREC_* modes of model.py) applies to the tensor-core launches only:
+F16_X3 (the default, ``precision=None``: a_hi W_hi + a_lo W_hi + a_hi W_lo), F16_W2 (a_hi (W_hi + W_lo)), F16 (a_hi
+W_hi) and F16_F8 (a_hi W_hi + one e4m3 pass carrying both correction terms, as the ConvNet's default).  The stem, its
+max-pool, the head and every convolution that falls back to the CUDA cores stay fp32 whatever the mode.
 """
 import os
 
@@ -19,6 +24,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .model import F8_A_SHIFT, F8_LO_SHIFT, PREC_F16, PREC_F16_F8, PREC_F16_W2, PREC_F16_X3
 
 EPS = 1e-5
 
@@ -40,28 +46,51 @@ def _scale_exponent(*ws):
     return int(max(-24, min(24, 12 - np.frexp(wmax)[1])))
 
 
-def pack_tc_weights(w, n_pad, cin_p, e):
-    """Folded conv weight [Cout, Cin, K] fp32 -> the operand image riser_res_tc reads: fp16
-    [tap][K block of 32 channels][plane hi, lo][n_pad rows][32 channels] (for a tap and K block the hi rows are
-    followed by the lo rows: the stacked operand [W_hi; W_lo] is one tile), every 64-byte row with its 16-byte
-    chunks at ``chunk ^ ((row >> 1) & 3)`` (K-major SWIZZLE_64B), weights multiplied by 2^e."""
+E4M3_MAX = 448.0
+
+
+def e4m3_bytes(x):
+    """float32 -> e4m3 bytes, rounded to nearest and saturated to +-448 (__nv_cvt_float_to_fp8 with __NV_SATFINITE;
+    torch's cast alone gives NaN above the range)."""
+    return x.clamp(-E4M3_MAX, E4M3_MAX).to(torch.float8_e4m3fn).view(torch.uint8)
+
+
+def pack_tc_weights(w, n_pad, cin_p, e, precision=PREC_F16_X3):
+    """Folded conv weight [Cout, Cin, K] fp32 -> the operand image riser_res_tc_ex reads in mode `precision`:
+    [tap][K block of 32 channels][plane][n_pad rows][64 bytes], every 64-byte row with its 16-byte chunks at
+    ``chunk ^ ((row >> 1) & 3)`` (K-major SWIZZLE_64B), weights w = W 2^e.  Planes: F16 [hi]; F16_W2 and F16_X3 [hi, lo]
+    (hi = fp16(w), lo = fp16(w - hi): for a tap and K block the hi rows are followed by the lo rows, so the stacked
+    operand [W_hi; W_lo] is one tile); F16_F8 [hi, e4m3 row] with the row [e4m3((w - hi) 2^F8_A_SHIFT) x32 |
+    e4m3(w 2^-(9 - F8_LO_SHIFT)) x32] of the K block's 32 channels."""
     cout, cin, K = w.shape
     kb = (cin_p + 31) // 32
     ws = (w.double() * (2.0 ** e)).float()
     hi = ws.half()
-    lo = (ws - hi.float()).half()
-    img = torch.zeros(K, kb, 2, n_pad, 32, dtype=torch.float16)
-    for plane, src in enumerate((hi, lo)):
-        full = torch.zeros(K, n_pad, kb * 32, dtype=torch.float16)
+    d = ws - hi.float()                                          # exact in float32
+
+    def plane(src):                       # [cout, cin, K] -> bytes [K][kb][n_pad][32 x element]
+        full = torch.zeros(K, n_pad, kb * 32, dtype=src.dtype)
         full[:, :cout, :cin] = src.permute(2, 0, 1)
-        img[:, :, plane] = full.view(K, n_pad, kb, 32).permute(0, 2, 1, 3)
-    chunks = img.view(K, kb, 2, n_pad, 4, 8)
+        return full.view(K, n_pad, kb, 32).permute(0, 2, 1, 3).contiguous().view(torch.uint8)
+
+    if precision == PREC_F16:
+        planes = [plane(hi)]
+    elif precision in (PREC_F16_W2, PREC_F16_X3):
+        planes = [plane(hi), plane(d.half())]
+    elif precision == PREC_F16_F8:
+        w8 = torch.cat([plane(e4m3_bytes(d * 2.0 ** F8_A_SHIFT)), plane(e4m3_bytes(ws * 2.0 ** -(9 - F8_LO_SHIFT)))],
+                       dim=3)
+        planes = [plane(hi), w8]
+    else:
+        raise ValueError(f"unknown precision mode {precision}")
+    P = len(planes)
+    chunks = torch.stack(planes, dim=2).view(K, kb, P, n_pad, 4, 16)
     rows = torch.arange(n_pad)
     out = torch.empty_like(chunks)
     for c in range(4):
         dst = c ^ ((rows >> 1) & 3)
         out[:, :, :, rows, dst] = chunks[:, :, :, rows, c]
-    return out.contiguous().view(torch.uint8).view(-1)
+    return out.contiguous().view(-1)
 
 
 def _fold(w, b, bn):
@@ -98,31 +127,33 @@ class _Conv:
         return self.k in (1, 3) and self.stride in (1, 2) and self.pad == (self.k - 1) // 2 and self.cin_p % 8 == 0 \
             and _pad16(self.cout) <= 256
 
-    def build_tc(self, device, max_smem):
-        """Operand image for the single-conv mode of riser_res_tc (None if the shape is not supported)."""
+    def build_tc(self, device, max_smem, precision=PREC_F16_X3):
+        """Operand image for the single-conv mode of riser_res_tc_ex (None if the shape is not supported)."""
         if not self.tc_ok():
             return None
         n1 = _pad16(self.cout)
-        need = _lib.lib().riser_res_tc_smem(self.cin_p, 0, n1, 0, self.k, self.stride, 0, 0)
+        need = _lib.lib().riser_res_tc_smem_ex(self.cin_p, 0, n1, 0, self.k, self.stride, 0, 0, precision)
         if need == 0 or need > max_smem:
             return None
         e = _scale_exponent(self.w_host)
         bias = torch.zeros(n1)
         bias[:self.cout] = self.b_host
-        self.tc = dict(w=pack_tc_weights(self.w_host, n1, self.cin_p, e).to(device), bias=bias.to(device),
-                       inv=float(2.0 ** -e), n1=n1)
+        self.tc = dict(w=pack_tc_weights(self.w_host, n1, self.cin_p, e, precision).to(device), bias=bias.to(device),
+                       inv=float(2.0 ** -e), e=e, n1=n1)
         return self.tc
 
 
 class _FusedBasic:
     """Operand images of a whole BasicBlock for the fused mode of riser_res_tc."""
-    def __init__(self, conv1, conv2, shortcut, device):
+    def __init__(self, conv1, conv2, shortcut, device, precision=PREC_F16_X3):
         n1, n2 = _pad16(conv1.cout), _pad16(conv2.cout)
         e1 = _scale_exponent(conv1.w_host)
         e2 = _scale_exponent(conv2.w_host, *([shortcut.w_host] if shortcut is not None else []))
-        self.w1 = pack_tc_weights(conv1.w_host, n1, conv1.cin_p, e1).to(device)
-        self.w2 = pack_tc_weights(conv2.w_host, n2, conv2.cin_p, e2).to(device)
-        self.wsc = None if shortcut is None else pack_tc_weights(shortcut.w_host, n2, shortcut.cin_p, e2).to(device)
+        self.w1 = pack_tc_weights(conv1.w_host, n1, conv1.cin_p, e1, precision).to(device)
+        self.w2 = pack_tc_weights(conv2.w_host, n2, conv2.cin_p, e2, precision).to(device)
+        self.wsc = None if shortcut is None else \
+            pack_tc_weights(shortcut.w_host, n2, shortcut.cin_p, e2, precision).to(device)
+        self.e1, self.e2 = e1, e2
         b1 = torch.zeros(n1)
         b1[:conv1.cout] = conv1.b_host
         b2 = torch.zeros(n2)
@@ -135,8 +166,12 @@ class _FusedBasic:
 
 
 class ResNetModel():
-    def __init__(self, state, config, logger, target):
+    def __init__(self, state, config, logger, target, precision=None):
+        """precision: PREC_F16, PREC_F16_W2, PREC_F16_X3 or PREC_F16_F8 for the tensor-core launches; None = F16_X3."""
         self.target = target
+        self.precision = PREC_F16_X3 if precision is None else int(precision)
+        if self.precision not in (PREC_F16, PREC_F16_W2, PREC_F16_X3, PREC_F16_F8):
+            raise ValueError(f"unknown precision mode {precision}")
         self.logger = logger
         self.device = _lib.require_device()
         self.logger.info('Using %s device', self.device)
@@ -179,13 +214,14 @@ class ResNetModel():
                 fused = None
                 if self.use_tc:
                     if c.block != "bottleneck" and all(cv.tc_ok() for cv in convs):
-                        need = L_.riser_res_tc_smem(convs[0].cin_p, convs[1].cin_p, _pad16(convs[0].cout),
-                                                    _pad16(convs[1].cout), 3, stride, 1, 1 if shortcut is not None else 0)
+                        need = L_.riser_res_tc_smem_ex(convs[0].cin_p, convs[1].cin_p, _pad16(convs[0].cout),
+                                                       _pad16(convs[1].cout), 3, stride, 1,
+                                                       1 if shortcut is not None else 0, self.precision)
                         if 0 < need <= max_smem:
-                            fused = _FusedBasic(convs[0], convs[1], shortcut, dev)
+                            fused = _FusedBasic(convs[0], convs[1], shortcut, dev, self.precision)
                     if fused is None:
                         for cv in convs + ([shortcut] if shortcut is not None else []):
-                            cv.build_tc(dev, max_smem)
+                            cv.build_tc(dev, max_smem, self.precision)
                 if fused is not None:
                     self.n_tc_fused += 1
                 else:
@@ -221,16 +257,27 @@ class ResNetModel():
             t = self._acts[(key,) + shape] = torch.empty(*shape, dtype=torch.float32, device=self.device)
         return t
 
+    def _conv_args(self, cv, x, n_in, L_in, n_out, out, residual, relu):
+        """Arguments of riser_res_tc(_ex) for a single-conv launch, up to the stream."""
+        t = cv.tc
+        return (_lib.ptr(x), _lib.ptr(n_in), _lib.ptr(n_out), _lib.ptr(out), _lib.ptr(residual), _lib.ptr(t["w"]), None,
+                None, _lib.ptr(t["bias"]), None, t["inv"], 1.0, x.shape[0], L_in, out.shape[1], cv.cin_p, 0, cv.cout_p,
+                t["n1"], 0, cv.k, cv.stride, 1 if relu else 0)
+
+    def _fused_args(self, fb, convs, x, n_in, L_in, n_out, out, residual):
+        """Arguments of riser_res_tc(_ex) for a fused BasicBlock launch, up to the stream."""
+        c1, c2 = convs
+        return (_lib.ptr(x), _lib.ptr(n_in), _lib.ptr(n_out), _lib.ptr(out), _lib.ptr(residual), _lib.ptr(fb.w1),
+                _lib.ptr(fb.w2), _lib.ptr(fb.wsc), _lib.ptr(fb.b1), _lib.ptr(fb.b2), fb.inv1, fb.inv2, x.shape[0], L_in,
+                out.shape[1], c1.cin_p, c2.cin_p, c2.cout_p, fb.n1, fb.n2, 3, c1.stride, 1)
+
     def _conv(self, cv, x, n_in, L_in, n_out, residual=None, relu=True):
         B = x.shape[0]
         L_out = max(1, (L_in + 2 * cv.pad - cv.k) // cv.stride + 1)
         out = self._buf(id(cv), B, L_out, cv.cout_p)
         if cv.tc is not None:
-            t = cv.tc
-            _lib.check(_lib.lib().riser_res_tc(_lib.ptr(x), _lib.ptr(n_in), _lib.ptr(n_out), _lib.ptr(out),
-                                               _lib.ptr(residual), _lib.ptr(t["w"]), None, None, _lib.ptr(t["bias"]), None,
-                                               t["inv"], 1.0, B, L_in, L_out, cv.cin_p, 0, cv.cout_p, t["n1"], 0,
-                                               cv.k, cv.stride, 1 if relu else 0, _lib.stream_ptr()), "riser_res_tc")
+            _lib.check(_lib.lib().riser_res_tc_ex(*self._conv_args(cv, x, n_in, L_in, n_out, out, residual, relu),
+                                                  _lib.stream_ptr(), self.precision), "riser_res_tc")
             return out, L_out
         _lib.check(_lib.lib().riser_conv1d_cl(_lib.ptr(x), _lib.ptr(n_in), _lib.ptr(cv.w), _lib.ptr(cv.b),
                                               _lib.ptr(residual), _lib.ptr(out), _lib.ptr(n_out), B, L_in, L_out,
@@ -245,11 +292,8 @@ class ResNetModel():
         L_out = max(1, (L_in + 2 - 3) // c1.stride + 1)
         out = self._buf(id(fb), B, L_out, c2.cout_p)
         residual = x if shortcut is None else None              # identity shortcut: same layout as the output
-        _lib.check(_lib.lib().riser_res_tc(_lib.ptr(x), _lib.ptr(n_in), _lib.ptr(n_out), _lib.ptr(out),
-                                           _lib.ptr(residual), _lib.ptr(fb.w1), _lib.ptr(fb.w2), _lib.ptr(fb.wsc),
-                                           _lib.ptr(fb.b1), _lib.ptr(fb.b2), fb.inv1, fb.inv2, B, L_in, L_out,
-                                           c1.cin_p, c2.cin_p, c2.cout_p, fb.n1, fb.n2, 3, c1.stride, 1,
-                                           _lib.stream_ptr()), "riser_res_tc")
+        _lib.check(_lib.lib().riser_res_tc_ex(*self._fused_args(fb, convs, x, n_in, L_in, n_out, out, residual),
+                                              _lib.stream_ptr(), self.precision), "riser_res_tc")
         return out, L_out
 
     def classify_batch(self, x, lens, max_len=None, probs=None, **_unused):
