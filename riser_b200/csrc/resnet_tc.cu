@@ -70,7 +70,9 @@ struct ResTcArgs {
   int relu;                      // single conv mode: ReLU in the epilogue
   int tile_rows;                 // output rows per item: 128 (single) or 126 (fused)
   int tiles_per_read, n_items;
-  uint32_t tiles_magic;          // floor(2^32 / tiles_per_read) + 1: item / tiles_per_read = umulhi(item, magic) (n_items < 2^20)
+  // floor(2^40 / tiles_per_read) + 1: item / tiles_per_read = (item * magic) >> 40, exact while
+  // item * tiles_per_read < 2^40 (n_items < 2^20 and tiles_per_read <= n_items); tiles_per_read = 1 included
+  uint64_t tiles_magic;
   int d2_col;                    // TMEM column of conv2's accumulator
   int tmem_cols;                 // columns allocated (power of two >= 32)
   int cat1, cat2;                // conv1 / conv2: [W_hi; W_lo] stacked (accumulator = 2 n columns; W2 and X3 only)
@@ -410,7 +412,7 @@ res_tc_kernel(const ResTcArgs a) {
 
   // item -> (read, first output row); an item whose rows all lie beyond its read's valid length is skipped
   auto decode = [&](int item, int& b, int& p0) {
-    b = static_cast<int>(__umulhi(static_cast<uint32_t>(item), a.tiles_magic));     // item / tiles_per_read
+    b = static_cast<int>((static_cast<uint64_t>(item) * a.tiles_magic) >> 40);     // item / tiles_per_read
     p0 = (item - b * a.tiles_per_read) * a.tile_rows;
   };
   auto next_active = [&](int item) {
@@ -741,7 +743,7 @@ extern "C" int riser_res_tc_ex(const float* in, const int32_t* len_in, const int
   a.tiles_per_read = (Lout_pad + a.tile_rows - 1) / a.tile_rows;
   a.n_items = B * a.tiles_per_read;
   RISER_REQUIRE(a.n_items < (1 << 20), "riser_res_tc: %d work items (B x tiles per read) exceed 2^20", a.n_items);
-  a.tiles_magic = static_cast<uint32_t>((1ull << 32) / static_cast<unsigned>(a.tiles_per_read)) + 1u;
+  a.tiles_magic = (1ull << 40) / static_cast<uint64_t>(a.tiles_per_read) + 1ull;
   a.cat1 = cat_of(precision, n1) ? 1 : 0;
   a.cat2 = (fused && cat_of(precision, n2)) ? 1 : 0;
   a.d2_col = acc_cols(n1, precision);

@@ -299,6 +299,10 @@ class ResNetModel():
     def classify_batch(self, x, lens, max_len=None, probs=None, **_unused):
         """x: fp32 [B, ld] normalised signals on the device, lens int32 [B].  -> probs [B, n_classes]."""
         B = x.shape[0]
+        if probs is None:
+            probs = torch.empty(B, self.n_classes, dtype=torch.float32, device=self.device)
+        if B == 0:
+            return probs
         L0 = int(max_len if max_len is not None else x.shape[1])
         lens = lens.to(torch.int32)
         # valid lengths after every op of the main chain, one launch (stem conv, stem pool, every block conv)
@@ -344,8 +348,6 @@ class ResNetModel():
                 ny = n_all[j]
                 j += 1
             h, n, L = y, ny, Ly
-        if probs is None:
-            probs = torch.empty(B, self.n_classes, dtype=torch.float32, device=self.device)
         _lib.check(_lib.lib().riser_gap_linear_softmax(_lib.ptr(h), _lib.ptr(n), _lib.ptr(self.fc_w),
                                                        _lib.ptr(self.fc_b), _lib.ptr(probs), B, L, self.c_last_p,
                                                        self.n_classes, _lib.stream_ptr()),
