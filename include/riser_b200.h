@@ -233,9 +233,8 @@ int riser_plan_layer_format(const riser_plan* p, int i);
 
 /* Which kernel runs conv layer i (1..n_layers-1) in this plan: 0 = conv_tc_kernel (one CTA per SM),
  * 1 = conv_eo_kernel (even / odd planes, resident weights), 2 = conv_pair_kernel (cta_group::2 CTA
- * pairs), 3 = fused01_kernel (layers 0 + 1 in one launch), 4 = conv_tc_kernel with the CUDA-core
- * layer-0 converter warps, 5 = conv_eo2_kernel (this layer and its neighbour in one launch, the
- * activation between them kept in shared memory).  -1 outside the range.  For bench.py's launch description. */
+ * pairs), 3 = fused01_kernel (layers 0 + 1 in one launch), 5 = conv_eo2_kernel (this layer and its
+ * neighbour in one launch, the activation between them kept in shared memory).  -1 outside the range.  For bench.py's launch description. */
 int riser_plan_layer_kernel(const riser_plan* p, int i);
 
 /* Replaces the decision rule of riser/control.py:75-82 for M models:

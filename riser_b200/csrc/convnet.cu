@@ -128,7 +128,7 @@ struct ConvArgs {
   int out_f8;             // output rows in that format
   int out_eo;             // output rows in the even / odd plane layout of conv_eo_kernel (else flat [B * Lp_out])
   int n_pairs_out, half_lp_out;
-  // fused layer 0 (layer 1 only): A tiles are computed in-kernel from the normalised signal
+  // fused01_kernel (layers 0 + 1): layer 0 is computed in-kernel from the normalised signal
   const float* x;
   long long ld_x;
   const float* w0;        // layer-0 weights [cout0][3], bias [cout0]
@@ -158,6 +158,17 @@ struct Eo2Args {
   float inv_scale1, inv_scale2;
 };
 
+typedef void (*ConvKernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap,
+                             const ConvArgs);
+typedef void (*EoKernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const ConvArgs);
+typedef void (*PairKernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap,
+                             const CUtensorMap, const ConvArgs);
+typedef void (*FusedKernelFn)(const CUtensorMap, const CUtensorMap, const ConvArgs);
+typedef void (*Eo2KernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const Eo2Args);
+
+// Which kernel runs a conv layer: the codes of riser_plan_layer_kernel (include/riser_b200.h)
+enum LayerKind { kTcKernel = 0, kEoKernel = 1, kPairKernel = 2, kFused01Kernel = 3, kEo2Kernel = 5 };
+
 struct ActivityLayer {
   int Lp_in, rows_in, rows_per_super, shift, n_supers, flag_off;
 };
@@ -170,17 +181,20 @@ struct LayerPlan {
   CUtensorMap tm_a, tm_b, tm_a8, tm_b8;   // (EO layers: tm_a = E plane, tm_a8 = O plane)
   CUtensorMap tm_bl, tm_b8l;              // conv_pair_kernel: weight maps whose box is half of the LAST N tile
   int eo = 0;                             // input in the even / odd plane layout -> conv_eo_kernel
-  int pair = 0;                           // CTA pairs (cta_group::2) -> conv_pair_kernel
-  int kc = 0;                             // fused01_kernel<4>: layer 1's hi / lo terms concatenated along K
-  int fuse_next = 0;                      // this layer and the next one run as ONE conv_eo2_kernel launch
   int fused_prev = 0;                     // computed inside the previous layer's launch: its input buffer is never written
-  Eo2Args eo2;                            // fuse_next: arguments of the two-layer launch
-  size_t eo2_smem = 0;
-  ConvArgs args;
-  int n_supers_total = 0;
-  int rows_per_super = 0;   // flat input rows one work item covers (ms * 128; 510 for the fused layers 0+1)
-  int flag_off = 0;
+  int kind = kTcKernel;                   // kEo2Kernel: this layer and the next one run as ONE conv_eo2_kernel launch
+  union {                                 // the kernel of `kind` (unset when fused_prev)
+    ConvKernelFn tc;
+    EoKernelFn eo;
+    PairKernelFn pair;
+    FusedKernelFn fused01;
+    Eo2KernelFn eo2;
+  } fn = {nullptr};
+  int grid = 0, block = 0;                // launch configuration of fn
   size_t smem = 0;
+  ConvArgs args;                          // everything but len0, x, ld_x, which each forward fills in
+  Eo2Args eo2;                            // kEo2Kernel: arguments of the two-layer launch (but len0)
+  int rows_per_super = 0;   // flat input rows one work item covers (ms * 128; 510 for the fused layers 0+1)
 };
 
 }  // namespace
@@ -189,12 +203,9 @@ struct LayerPlan {
 struct riser_plan {
   const riser_model* model = nullptr;
   int B = 0, max_len = 0;
-  int fuse_l0 = 0;                      // layer 0 computed inside layer 1's launch: 1 = CUDA-core converter warps
-                                        // (conv_tc_kernel<FUSED>), 2 = both layers on the tensor pipe (fused01_kernel)
+  int fuse_l0 = 0;                      // 1 = layers 0 + 1 run as one fused01_kernel launch
   uint8_t* flags = nullptr;             // tile activity flags (plan-owned), see tile_activity_kernel
   riser::ActivityArgs activity;
-  int chunk_reads = 0, n_chunked = 0;   // early layers 0..n_chunked-1 run chunk by chunk (L2 residency)
-  int Lmax[riser::kMaxLayers + 1];
   int Lp[riser::kMaxLayers + 1];
   size_t act_off[riser::kMaxLayers + 1];
   char* ws = nullptr;
@@ -318,9 +329,7 @@ layer0_kernel(const float* __restrict__ x, int64_t ld_x, const int32_t* __restri
 // Roles: warp 0 = TMA producer, warp 1 = MMA issuer + TMEM owner, warps 2..9 = two epilogue
 // sets (each covers the four TMEM lane quadrants; the sets split the 16-column chunks).
 constexpr int kMaxAStages = 8, kMaxBStages = 8, kMaxAccStages = 4;
-constexpr int kConvThreads = 320;
-constexpr int kCvtThreads = 288;         // fused layer 0: converter warps 10..18 (514 rows = 2 passes)
-constexpr int kMaxEpiSets = 4;             // plain kernels: up to four sets (warps 2..17)
+constexpr int kMaxEpiSets = 4;             // up to four sets (warps 2..17)
 
 struct ConvSmem {
   uint64_t a_full[kMaxAStages], a_empty[kMaxAStages];
@@ -331,7 +340,7 @@ struct ConvSmem {
   uint64_t tmem_empty[kMaxAccStages][4];     // per accumulator stage AND sub-tile: released as soon as drained
   uint32_t tmem_base;
   alignas(16) float bias[2][kMaxNTile];
-  float4 w0q[32];        // fused layer 0: {w[c][0], w[c][1], w[c][2], bias[c]} per output channel
+  float4 w0q[32];        // unused; its bytes still count in the plans' shared-memory budgets
 };
 
 // fp32 pair -> fp16 pair, saturated to the fp16 range (inf -> 65504) in the half2 domain
@@ -479,8 +488,8 @@ struct ItemFlags {
   }
 };
 
-template <int MS, int PLANES, int WPLANES, bool RESIDENT, bool FUSED = false, bool K32 = false, bool F8 = false>
-__global__ void __launch_bounds__(FUSED ? kConvThreads + kCvtThreads : 96 + 128 * kMaxEpiSets, 1)
+template <int MS, int PLANES, int WPLANES, bool RESIDENT, bool K32 = false, bool F8 = false>
+__global__ void __launch_bounds__(96 + 128 * kMaxEpiSets, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
                const __grid_constant__ CUtensorMap tm_a8, const __grid_constant__ CUtensorMap tm_b8,
                const ConvArgs a) {
@@ -489,12 +498,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
   // shared address space, so the compiler emits LDS/STS instead of generic LD/ST
   unsigned char* base = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
   constexpr int kATiles = MS * PLANES;                       // A tiles per K block
-  // fused layer 0: one contiguous (MS*128 + 2)-row tile per plane instead of MS haloed tiles
   constexpr int kRowBytes = K32 ? 64 : 128;                  // bytes per operand row (one K block)
   constexpr int kKElems = kRowBytes / 2;                     // fp16 elements per K block
   constexpr uint32_t kATile = 136 * kRowBytes;               // smem stride of one haloed A tile
-  constexpr uint32_t kFusedTileBytes = (MS * kBlockM + 8) * kRowBytes;
-  constexpr uint32_t kAGroupBytes = FUSED ? PLANES * kFusedTileBytes : kATiles * kATile;
+  constexpr uint32_t kAGroupBytes = kATiles * kATile;
   const uint32_t b_bytes = a.n_tile * kRowBytes;
   unsigned char* a_ring = base;
   unsigned char* b_region = base + static_cast<size_t>(a.a_stages) * kAGroupBytes;
@@ -515,7 +522,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
     }
     const uint32_t n_issuers = a.dual ? 2 : 1;     // every issuer commits to the operand "empty" barriers
     for (int i = 0; i < a.a_stages; ++i) {
-      mbar_init(&s.a_full[i], FUSED ? kCvtThreads : 1);
+      mbar_init(&s.a_full[i], 1);
       mbar_init(&s.a_empty[i], n_issuers);
     }
     for (int i = 0; i < a.b_stages; ++i) {
@@ -561,7 +568,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
       const uint32_t a_tx = kATiles * a.a_tx_bytes;
       ItemCursor cur(blockIdx.x, gridDim.x, a.n_tiles, a.super0);
       ItemFlags fl(a.flags, cur.super, blockIdx.x < n_items);
-      for (int item = blockIdx.x; !FUSED && item < n_items; item += gridDim.x, cur.next()) {
+      for (int item = blockIdx.x; item < n_items; item += gridDim.x, cur.next()) {
         if (!fl.take(cur, item + gridDim.x < n_items)) continue;
         const int m0 = cur.super * (MS * kBlockM) - 1;
         const int n0 = cur.n * a.n_tile;
@@ -606,7 +613,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
         }
       }
     }
-  } else if (warp == 1 || (!FUSED && a.dual && warp == 2 + 4 * a.epi_sets)) {
+  } else if (warp == 1 || (a.dual && warp == 2 + 4 * a.epi_sets)) {
     // ===================== MMA issuer(s) =====================
     // One thread issues every MMA of an item -- or, `dual` (MS == 2), one thread per sub-tile: the two walk the same
     // operand stages on their own (both commit to the "empty" barriers), so the thread whose accumulator is still
@@ -614,8 +621,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
     // accumulator stage (N > 128) both sub-tiles of an item used to finish together and the pipe idled for the
     // whole drain (profiles/README.md, round 2: 22 % of the issuing thread's time in layer 6) -- and the
     // instruction stream between two MMAs (~16 SASS instructions on one thread) is shared by two threads.
-    const int ms_lo = (!FUSED && a.dual) ? (warp == 1 ? 0 : 1) : 0;
-    const int ms_hi = (!FUSED && a.dual) ? ms_lo + 1 : MS;
+    const int ms_lo = a.dual ? (warp == 1 ? 0 : 1) : 0;
+    const int ms_hi = a.dual ? ms_lo + 1 : MS;
     // the whole warp runs the loop (uniform registers); only the elected lane executes the MMAs / commits
     const uint32_t leader = (RISER_UNIFORM_ISSUE ? elect_one() : (lane == 0)) ? 1u : 0u;
     if (RISER_UNIFORM_ISSUE || lane == 0) {
@@ -663,9 +670,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
                 }
 #pragma unroll
                 for (int ap = 0; ap < (wp == 0 ? PLANES : 1); ++ap) {   // W_lo only meets the hi plane
-                  const uint64_t da =
-                      FUSED ? sw_desc<K32>(a_addr + ap * kFusedTileBytes + (ms * kBlockM + tap) * kRowBytes)
-                            : sw_desc<K32>(a_addr + (ms * PLANES + ap) * kATile + tap * kRowBytes);
+                  const uint64_t da = sw_desc<K32>(a_addr + (ms * PLANES + ap) * kATile + tap * kRowBytes);
                   if (leader) {      // one elected lane issues; the K steps of a view in one go
 #pragma unroll
                     for (int k = 0; k < kKElems / 16; ++k)
@@ -701,88 +706,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
           stage = 0;
           acc_phase ^= 1;
         }
-      }
-    }
-  } else if (FUSED && warp >= 10) {
-    // ===================== fused layer 0: converter warps 10..17 =====================
-    // Compute layer 1's A operand (layer 0 = Conv1d(1->C0,k3,same)+ReLU+MaxPool(2,2), fp32 on
-    // CUDA cores, nets/cnn.py:55-64) straight into shared memory in the SWIZZLE_128B K-major
-    // layout the MMA reads: row j of the tile at byte j*128, 16-byte chunk c at (c ^ (j & 7))
-    // (K32: 64-byte rows, chunk c at (c ^ ((j >> 1) & 3)) -- SWIZZLE_64B).
-    const int ct = threadIdx.x - kConvThreads;
-    for (int c = ct; c < 32; c += kCvtThreads)
-      s.w0q[c] = (c < a.cout0) ? make_float4(a.w0[c * 3], a.w0[c * 3 + 1], a.w0[c * 3 + 2], a.b0[c])
-                               : make_float4(0.f, 0.f, 0.f, 0.f);
-    asm volatile("bar.sync 2, %0;" ::"n"(kCvtThreads) : "memory");
-    constexpr int kRows = MS * kBlockM + 2;
-    int sa = 0;
-    uint32_t pa = 0;
-    ItemCursor cur(blockIdx.x, gridDim.x, a.n_tiles, a.super0);
-    ItemFlags fl(a.flags, cur.super, blockIdx.x < n_items);
-    for (int item = blockIdx.x; item < n_items; item += gridDim.x, cur.next()) {
-      if (!fl.take(cur, item + gridDim.x < n_items)) continue;
-      const int r0 = cur.super * (MS * kBlockM) - 1;
-      mbar_wait_relaxed(&s.a_empty[sa], pa ^ 1);
-      unsigned char* dst = a_ring + static_cast<size_t>(sa) * kAGroupBytes;
-      for (int j = ct; j < kRows; j += kCvtThreads) {
-        const int r = r0 + j;
-        // all global loads of the row are issued together (none depends on another's result);
-        // validity is applied afterwards
-        const bool inb = (r >= 0 && r < a.rows_in);
-        const uint32_t pidx = static_cast<uint32_t>(inb ? r : 0) >> 1;
-        const int b = static_cast<int>((static_cast<unsigned long long>(pidx) * a.pair_magic) >> 40);
-        const int tp = (inb ? r : 0) - b * a.Lp_in;
-        const float* xr = a.x + static_cast<long long>(b) * a.ld_x + 2 * tp;
-        const bool in_row = inb && (2 * tp + 1 < a.ld_x);
-        const int L = inb ? __ldg(a.len0 + b) : 0;
-        const float2 x01 = in_row ? __ldg(reinterpret_cast<const float2*>(xr)) : make_float2(0.f, 0.f);
-        float xm1 = (in_row && tp > 0) ? __ldg(xr - 1) : 0.f;
-        float x2 = (in_row && 2 * tp + 2 < a.ld_x) ? __ldg(xr + 2) : 0.f;
-        const float x0 = x01.x, x1 = x01.y;
-        const bool live = in_row && tp < (L >> 1);
-        if (2 * tp + 2 >= L) x2 = 0.f;
-        unsigned char* row = dst + j * kRowBytes;
-        const int sw = K32 ? ((j >> 1) & 3) : (j & 7);      // 16-byte-chunk XOR of the row (SWIZZLE_64B / _128B)
-        if (!live) {
-#pragma unroll
-          for (int c8 = 0; c8 < 4; ++c8) {
-            *reinterpret_cast<uint4*>(row + ((c8 ^ sw) << 4)) = make_uint4(0, 0, 0, 0);
-            if (PLANES == 2) *reinterpret_cast<uint4*>(row + kFusedTileBytes + ((c8 ^ sw) << 4)) = make_uint4(0, 0, 0, 0);
-          }
-          continue;
-        }
-        // (FFMA2 was tried here: same FMA-pipe time, twice the weight loads -> slower.)
-#pragma unroll
-        for (int c8 = 0; c8 < 4; ++c8) {
-          __half2 hv[4], lv[4];
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            float v[2] = {0.f, 0.f};
-            if (c8 * 8 + 2 * e < a.cout0) {          // uniform: skips the zero-padded channels
-#pragma unroll
-              for (int h = 0; h < 2; ++h) {
-                const float4 w = s.w0q[c8 * 8 + 2 * e + h];
-                const float y0 = fmaf(w.z, x1, fmaf(w.y, x0, fmaf(w.x, xm1, w.w)));
-                const float y1 = fmaf(w.z, x2, fmaf(w.y, x1, fmaf(w.x, x0, w.w)));
-                v[h] = fmaxf(fmaxf(y0, y1), 0.f);
-              }
-            }
-            hv[e] = sat_half2(v[0], v[1]);
-            if (PLANES == 2) {
-              const float2 back = __half22float2(hv[e]);
-              lv[e] = __floats2half2_rn(v[0] - back.x, v[1] - back.y);
-            }
-          }
-          const int off = (c8 ^ sw) << 4;
-          *reinterpret_cast<uint4*>(row + off) = *reinterpret_cast<const uint4*>(hv);
-          if (PLANES == 2) *reinterpret_cast<uint4*>(row + kFusedTileBytes + off) = *reinterpret_cast<const uint4*>(lv);
-        }
-      }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic writes -> visible to the MMA
-      mbar_arrive(&s.a_full[sa]);
-      if (++sa == a.a_stages) {
-        sa = 0;
-        pa ^= 1;
       }
     }
   } else if (warp < 2 + 4 * a.epi_sets) {
@@ -881,52 +804,42 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
   }
 }
 
-typedef void (*ConvKernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap,
-                             const ConvArgs);
-
-template <int MS, bool RESIDENT, bool FUSED, bool K32>
+template <int MS, bool RESIDENT, bool K32>
 ConvKernelFn pick_conv_planes(int planes, int wplanes) {
-  if (planes == 1 && wplanes == 1) return conv_tc_kernel<MS, 1, 1, RESIDENT, FUSED, K32>;
-  if (planes == 1 && wplanes == 2) return conv_tc_kernel<MS, 1, 2, RESIDENT, FUSED, K32>;
-  return conv_tc_kernel<MS, 2, 2, RESIDENT, FUSED, K32>;
+  if (planes == 1 && wplanes == 1) return conv_tc_kernel<MS, 1, 1, RESIDENT, K32>;
+  if (planes == 1 && wplanes == 2) return conv_tc_kernel<MS, 1, 2, RESIDENT, K32>;
+  return conv_tc_kernel<MS, 2, 2, RESIDENT, K32>;
 }
 template <bool K32>
-ConvKernelFn pick_conv_k(int ms, int planes, int wplanes, int resident, int fused) {
-  if (fused) {
-    if (ms == 4) return pick_conv_planes<4, true, true, K32>(planes, wplanes);
-    if (ms == 2) return pick_conv_planes<2, true, true, K32>(planes, wplanes);
-    return pick_conv_planes<1, true, true, K32>(planes, wplanes);
-  }
+ConvKernelFn pick_conv_k(int ms, int planes, int wplanes, int resident) {
   if (resident) {
-    if (ms == 4) return pick_conv_planes<4, true, false, K32>(planes, wplanes);
-    if (ms == 2) return pick_conv_planes<2, true, false, K32>(planes, wplanes);
-    return pick_conv_planes<1, true, false, K32>(planes, wplanes);
+    if (ms == 4) return pick_conv_planes<4, true, K32>(planes, wplanes);
+    if (ms == 2) return pick_conv_planes<2, true, K32>(planes, wplanes);
+    return pick_conv_planes<1, true, K32>(planes, wplanes);
   }
-  if (ms == 4) return pick_conv_planes<4, false, false, K32>(planes, wplanes);
-  if (ms == 2) return pick_conv_planes<2, false, false, K32>(planes, wplanes);
-  return pick_conv_planes<1, false, false, K32>(planes, wplanes);
+  if (ms == 4) return pick_conv_planes<4, false, K32>(planes, wplanes);
+  if (ms == 2) return pick_conv_planes<2, false, K32>(planes, wplanes);
+  return pick_conv_planes<1, false, K32>(planes, wplanes);
 }
 // F16_F8 mode: one activation / weight plane per K block, the e4m3 correction blocks after the fp16 ones
 template <bool K32>
 ConvKernelFn pick_conv_f8(int ms, int resident) {
   if (resident) {
-    if (ms == 4) return conv_tc_kernel<4, 1, 1, true, false, K32, true>;
-    if (ms == 2) return conv_tc_kernel<2, 1, 1, true, false, K32, true>;
-    return conv_tc_kernel<1, 1, 1, true, false, K32, true>;
+    if (ms == 4) return conv_tc_kernel<4, 1, 1, true, K32, true>;
+    if (ms == 2) return conv_tc_kernel<2, 1, 1, true, K32, true>;
+    return conv_tc_kernel<1, 1, 1, true, K32, true>;
   }
-  if (ms == 4) return conv_tc_kernel<4, 1, 1, false, false, K32, true>;
-  if (ms == 2) return conv_tc_kernel<2, 1, 1, false, false, K32, true>;
-  return conv_tc_kernel<1, 1, 1, false, false, K32, true>;
+  if (ms == 4) return conv_tc_kernel<4, 1, 1, false, K32, true>;
+  if (ms == 2) return conv_tc_kernel<2, 1, 1, false, K32, true>;
+  return conv_tc_kernel<1, 1, 1, false, K32, true>;
 }
-ConvKernelFn pick_conv_kernel(int ms, int planes, int wplanes, int resident, int fused = 0, int k32 = 0,
-                              int f8 = 0) {
+ConvKernelFn pick_conv_kernel(int ms, int planes, int wplanes, int resident, int k32, int f8) {
   if (f8) return k32 ? pick_conv_f8<true>(ms, resident) : pick_conv_f8<false>(ms, resident);
-  return k32 ? pick_conv_k<true>(ms, planes, wplanes, resident, fused)
-             : pick_conv_k<false>(ms, planes, wplanes, resident, fused);
+  return k32 ? pick_conv_k<true>(ms, planes, wplanes, resident) : pick_conv_k<false>(ms, planes, wplanes, resident);
 }
 
 // ------------------------------------------------------------------------------------
-// Layers 0 + 1 in one launch, BOTH on the tensor pipe (RISER_FUSE_L0=2, the default).
+// Layers 0 + 1 in one launch, BOTH on the tensor pipe (the default; RISER_FUSE_L0=0 runs layer0_kernel instead).
 //
 // Layer 0 (Conv1d(1->C0,k3,same)+ReLU+MaxPool, nets/cnn.py:55-64) is a GEMM with K = 16:
 // row p of its A operand is the signal window x[2p-1 .. 2p+2] split into fp16 hi and lo
@@ -1545,7 +1458,6 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
   }
 }
 
-typedef void (*FusedKernelFn)(const CUtensorMap, const CUtensorMap, const ConvArgs);
 FusedKernelFn pick_fused01(int mode) {
   if (mode == 0) return fused01_kernel<0>;
   if (mode == 1) return fused01_kernel<1>;
@@ -1795,7 +1707,6 @@ conv_eo_kernel(const __grid_constant__ CUtensorMap tm_e, const __grid_constant__
   }
 }
 
-typedef void (*EoKernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const ConvArgs);
 EoKernelFn pick_conv_eo(int ms, int planes, int wplanes) {
   if (ms == 2) {
     if (planes == 1 && wplanes == 1) return conv_eo_kernel<2, 1, 1>;
@@ -2495,8 +2406,6 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
   }
 }
 
-typedef void (*PairKernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap,
-                             const CUtensorMap, const ConvArgs);
 PairKernelFn pick_conv_pair(int ms) { return ms == 2 ? conv_pair_kernel<2> : conv_pair_kernel<1>; }
 
 // ------------------------------------------------------------------------------------
@@ -2830,15 +2739,26 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
   RISER_REQUIRE(out && m && workspace, "riser_plan_create: null pointer");
   RISER_REQUIRE(B > 0 && max_len >= kMinLen, "riser_plan_create: need B > 0 and max_len >= %d", kMinLen);
   RISER_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "riser_plan_create: workspace not 256-byte aligned");
+  // These switches exist so that the test suite can reach, on the shipped network, the kernels that other shapes
+  // select on their own.  RISER_PAIR_DBG_SKIP is a timing experiment (wrong results).
+  const bool fuse_l0 = env_int("RISER_FUSE_L0", 1) != 0;
+  const bool eo_on = env_int("RISER_EO", 1) != 0;
+  const bool pair_on = env_int("RISER_PAIR", 1) != 0;
+  const int pair_ms = env_int("RISER_PAIR_MS", 1);
+  const int pair_from = env_int("RISER_PAIR_FROM", 6);
+  const int pair_ntile = env_int("RISER_PAIR_NTILE", kMaxNTile);
+  const bool dual_issue = env_int("RISER_DUAL_ISSUE", 1) != 0;
+  const bool kc_on = env_int("RISER_KC", 1) != 0;
+  const bool fuse23 = env_int("RISER_FUSE23", 1) != 0;
+  const int pair_dbg_skip = env_int("RISER_PAIR_DBG_SKIP", 0);
   std::unique_ptr<riser_plan, int (*)(riser_plan*)> owner(new riser_plan(), riser_plan_destroy);   // freed on every error return
   riser_plan* p = owner.get();
   p->model = m;
   p->B = B;
   p->max_len = max_len;
   p->ws = static_cast<char*>(workspace);
-  const bool allow_resident = env_int("RISER_CONV_RESIDENT", 1) != 0;
-  const int max_ms = std::max(1, std::min(2, env_int("RISER_CONV_MS", 2)));
-  plan_lengths(m, max_len, p->Lmax, p->Lp);
+  int Lmax[kMaxLayers + 1];
+  plan_lengths(m, max_len, Lmax, p->Lp);
   const size_t need = plan_offsets(m, B, p->Lp, p->act_off);
   if (workspace_bytes < need) {
     return fail(RISER_ENOMEM, "riser_plan_create: workspace %zu < %zu bytes", workspace_bytes, need);
@@ -2848,44 +2768,14 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
   int max_smem = 0;
   RISER_CUDA_TRY(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, m->device));
 
-  // Early layers run read-chunk by read-chunk so that their activations stay in the L2:
-  // layer i is "chunked" while streaming its input + output through HBM would take longer
-  // than its tensor work (both per read).  From the first compute-bound layer on, layers run
-  // over the whole batch (more tiles per launch, weights amortised).
-  {
-    const double hbm_bw = 6.4e12, tensor_peak = 1.4e15;
-    const int n_terms = (m->act_planes == 2) ? 3 : m->passes;
-    int n_chunked = 1;   // layer 0 goes with layer 1
-    size_t pair_bytes = 0;
-    for (int i = 1; i < m->n_layers; ++i) {
-      const bool last = (i == m->n_layers - 1);
-      const double in_b = static_cast<double>(p->Lp[i]) * m->layer[i - 1].cout_p * m->act_planes * 2;
-      const double out_b = static_cast<double>(p->Lp[i + 1]) * m->layer[i].cout_p * (last ? 4 : m->act_planes * 2);
-      const double flops = 2.0 * 3 * m->layer[i].cin_p * m->layer[i].cout_p * p->Lp[i] * n_terms;
-      if ((in_b + out_b) / hbm_bw > 0.7 * flops / tensor_peak && n_chunked == i) {
-        n_chunked = i + 1;
-        pair_bytes = std::max(pair_bytes, static_cast<size_t>(in_b + out_b));
-      }
-    }
-    if (n_chunked == 1) n_chunked = 0;
-    const size_t l2_budget = static_cast<size_t>(env_int("RISER_L2_BUDGET_MB", 72)) << 20;
-    int chunk = pair_bytes ? static_cast<int>(std::max<size_t>(8, l2_budget / pair_bytes)) : B;
-    // Measured on B200 (profiles/README.md): with the current kernels the extra launches and
-    // wave tails of chunking cost more than the L2 hits give back, so it is opt-in.
-    if (!env_int("RISER_CHUNKING", 0)) chunk = B;
-    p->chunk_reads = std::max(1, std::min(B, env_int("RISER_CHUNK_READS", chunk)));
-    if (p->chunk_reads >= B) n_chunked = 0;
-    p->n_chunked = std::max(0, std::min(m->n_layers, env_int("RISER_CHUNKED_LAYERS", n_chunked)));
-  }
-
-  // Even / odd plane layout (conv_eo_kernel) for the narrow resident-weight layers after layer 1
-  if (env_int("RISER_EO", 1))
-    for (int i = 2; i < m->n_layers - 1; ++i) {
+  // Even / odd plane layout (conv_eo_kernel) for the narrow resident-weight layers 2..4
+  if (eo_on)
+    for (int i = 2; i < m->n_layers - 1 && i <= 4; ++i) {
       const LayerPack& L = m->layer[i];
       const size_t w_all = static_cast<size_t>(L.passes) * ((L.cin_p + 31) / 32) * 3 * L.n_tile * 64;
       const size_t group1 = static_cast<size_t>(m->act_planes) * 2 * kEoTile;
       if (!L.f8 && L.cin_p <= 80 && L.n_tiles == 1 && 2 * L.n_tile <= kMaxNTile &&
-          w_all + 2 * group1 + 1024 + sizeof(ConvSmem) + 64 <= static_cast<size_t>(max_smem) && i <= env_int("RISER_EO_LAST", 4))
+          w_all + 2 * group1 + 1024 + sizeof(ConvSmem) + 64 <= static_cast<size_t>(max_smem))
         p->layer[i].eo = 1;
     }
 
@@ -2894,13 +2784,12 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
     LayerPlan& lp = p->layer[i];
     const int rows_in = B * p->Lp[i];
     const bool last = (i == m->n_layers - 1);
-    const int a_box_rows = env_int("RISER_A_BOX_ROWS", 136);   // 130 needed; a multiple of 8 is what TMA likes
+    const int a_box_rows = 136;   // 130 needed; a multiple of 8 is what TMA likes
+    const bool fuse01 = (i == 1 && fuse_l0 && L.cin_p == 32 && L.n_tile == 32 && L.n_tiles == 1 &&
+                         m->layer[0].cout <= 24);
     // 32-channel K blocks (64-byte rows, SWIZZLE_64B) for narrow layers: no zero-filled half rows,
     // twice the pipeline depth / sub-tiles per item in the same shared memory
-    const int want_fuse = env_int("RISER_FUSE_L0", 2);
-    const bool fuse2 = (i == 1 && want_fuse == 2 && L.cin_p == 32 && L.n_tile == 32 && L.n_tiles == 1 &&
-                        m->layer[0].cout <= 24);
-    const bool k32 = fuse2 || L.cin_p <= env_int("RISER_K32_MAX_CIN", 80);
+    const bool k32 = fuse01 || L.cin_p <= 80;
     const int row_bytes = k32 ? 64 : 128;
     const int k_elems = row_bytes / 2;
     int st = make_tmap(&lp.tm_a, p->ws + p->act_off[i], static_cast<uint64_t>(L.cin_p) * m->act_planes, rows_in,
@@ -2950,13 +2839,12 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
     const size_t avail = static_cast<size_t>(max_smem) - fixed;
     const size_t w_all = static_cast<size_t>(L.passes) * 3 * a.k_blocks * b_bytes;
     const size_t a_group1 = static_cast<size_t>(kplanes) * 136 * row_bytes;
-    if (allow_resident && L.n_tiles == 1 && w_all + 2 * a_group1 <= avail) {
+    if (L.n_tiles == 1 && w_all + 2 * a_group1 <= avail) {
       // resident weights; as many 128-row sub-tiles per work item as leave >= 2 accumulator
       // stages and >= 2 A groups in flight (amortises the per-item bookkeeping of small-N layers)
       a.resident = 1;
       a.ms = 1;
-      const int want_ms = std::max(1, std::min(4, env_int("RISER_CONV_MS_RES", 4)));
-      for (int ms = want_ms; ms > 1; ms >>= 1)
+      for (int ms = 4; ms > 1; ms >>= 1)
         if (2 * ms * a.acc_cols <= kTmemCols && w_all + 2 * ms * a_group1 <= avail &&
             static_cast<int64_t>(rows_in) / (ms * kBlockM) >= 2 * m->sm_count) {
           a.ms = ms;
@@ -2965,28 +2853,10 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
       a.b_stages = 1;
       a.a_stages = std::min<int>(kMaxAStages, static_cast<int>((avail - w_all) / (a.ms * a_group1)));
       lp.smem = fixed + w_all + static_cast<size_t>(a.a_stages) * a.ms * a_group1;
-      if (i == 1 && L.cin_p == 32 && want_fuse == 1 && !m->f8) {
-        // fused layer 0: A tiles are written by converter warps; one contiguous
-        // (ms*128 + 8)-row tile per plane and stage
-        for (int ms = want_ms; ms >= 1; ms >>= 1) {
-          const size_t group = static_cast<size_t>(m->act_planes) * (ms * kBlockM + 8) * row_bytes;
-          if (2 * ms * a.acc_cols <= kTmemCols && w_all + 2 * group <= avail) {
-            p->fuse_l0 = 1;
-            a.ms = ms;
-            a.a_stages = std::min<int>(kMaxAStages, static_cast<int>((avail - w_all) / group));
-            lp.smem = fixed + w_all + static_cast<size_t>(a.a_stages) * group;
-            a.w0 = m->layer[0].w0;
-            a.b0 = m->layer[0].bias;
-            a.cout0 = m->layer[0].cout;
-            break;
-          }
-        }
-      }
     } else {
       a.resident = 0;
-      a.ms = (2 * a.acc_cols <= kTmemCols) ? max_ms : 1;
-      if (max_ms == 2 && 4 * a.acc_cols <= kTmemCols && 2 * 4 * a_group1 + 3 * b_bytes <= avail &&
-          env_int("RISER_CONV_MS4_STREAM", 1))
+      a.ms = (2 * a.acc_cols <= kTmemCols) ? 2 : 1;
+      if (4 * a.acc_cols <= kTmemCols && 2 * 4 * a_group1 + 3 * b_bytes <= avail)
         a.ms = 4;       // more rows per streamed weight tile (narrow layers / 32-channel K blocks)
       // smem split: at least 2 A groups and 2 B stages; prefer 3+ B stages
       while (a.ms > 1 && 2 * a.ms * a_group1 + 2 * b_bytes > avail) a.ms >>= 1;
@@ -3002,28 +2872,29 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
       lp.smem = fixed + static_cast<size_t>(a.a_stages) * a_group + static_cast<size_t>(a.b_stages) * b_bytes;
     }
     a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / (a.ms * a.acc_cols)));
-    a.dual = (a.ms == 2 && !a.resident && env_int("RISER_DUAL_ISSUE", 1)) ? 1 : 0;
-    // four epilogue sets when there are enough 16-column chunks to split (the fused kernel keeps
-    // two: its thread budget goes to the layer-0 converter warps)
-    a.epi_sets = (i == 1 && p->fuse_l0) ? 2 : std::max(2, std::min(env_int("RISER_EPI_SETS", kMaxEpiSets), 4));
+    a.dual = (a.ms == 2 && !a.resident && dual_issue) ? 1 : 0;
+    a.epi_sets = kMaxEpiSets;
     lp.rows_per_super = a.ms * kBlockM;
-    if (fuse2) {
+    bool kc = false;
+    if (fuse01) {
       // layers 0 + 1 on the tensor pipe (fused01_kernel): work item = 255 pooled outputs = 510 input rows
-      p->fuse_l0 = 2;
+      p->fuse_l0 = 1;
+      lp.kind = kFused01Kernel;
       a.w0 = m->layer[0].w0;
       a.b0 = m->layer[0].bias;
       a.cout0 = m->layer[0].cout;
       lp.rows_per_super = 2 * kF2Pairs;
       lp.smem = fused01_smem(m->act_planes, L.f8 ? 2 : L.passes);
       a.planes = m->act_planes;     // fused01_kernel's own modes (see pick_fused01)
-      if (L.wkc && m->layer[0].cout <= 20 && env_int("RISER_KC", 1)) {
-        lp.kc = 1;      // the three hi / lo terms concatenated along K (fused01_kernel<4>); same shared-memory footprint
+      if (L.wkc && m->layer[0].cout <= 20 && kc_on) {
+        kc = true;      // the three hi / lo terms concatenated along K (fused01_kernel<4>); same shared-memory footprint
         const int st3 = make_tmap(&lp.tm_b, L.wkc, 64, 3ull * L.cout_p, 32, false);
         if (st3) return st3;
       }
     }
     if (lp.eo) {
       // conv_eo_kernel: E plane = rows [0, n_pairs), O plane = rows [n_pairs, 2 n_pairs) of the same buffer
+      lp.kind = kEoKernel;
       const uint64_t n_pairs = static_cast<uint64_t>(rows_in) / 2;
       const uint64_t pitch = static_cast<uint64_t>(L.cin_p) * m->act_planes;     // fp16 elements per row
       int st2 = make_tmap(&lp.tm_a, p->ws + p->act_off[i], pitch, n_pairs, 136, true);
@@ -3032,7 +2903,7 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
       a.acc_cols = round_up(2 * L.n_tile, 32);
       const size_t w_eo = static_cast<size_t>(L.passes) * a.k_blocks * 3 * b_bytes;
       const size_t group1 = static_cast<size_t>(m->act_planes) * 2 * kEoTile;
-      a.ms = (2 * 2 * a.acc_cols <= kTmemCols && w_eo + 2 * 2 * group1 <= avail && env_int("RISER_EO_MS", 2) >= 2) ? 2 : 1;
+      a.ms = (2 * 2 * a.acc_cols <= kTmemCols && w_eo + 2 * 2 * group1 <= avail) ? 2 : 1;
       a.resident = 1;
       a.a_stages = std::min<int>(kMaxAStages, static_cast<int>((avail - w_eo) / (a.ms * group1)));
       a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / (a.ms * a.acc_cols)));
@@ -3040,17 +2911,14 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
       lp.smem = fixed + w_eo + static_cast<size_t>(a.a_stages) * a.ms * group1;
       lp.rows_per_super = a.ms * 2 * kBlockM;
     }
-    if (L.f8 && !a.resident && !k32 && !lp.eo && (L.n_tile % 16) == 0 && env_int("RISER_PAIR", 1) &&
-        (i >= env_int("RISER_PAIR_FROM", 6) ||
-         (L.n_tiles == 1 && static_cast<size_t>(3) * a.k_blocks * (L.cout_p / 2) * 128 + 3 * 136 * 128 <= avail &&
-          env_int("RISER_PAIR_RESIDENT", 1)))) {
+    if (L.f8 && !a.resident && !k32 && !lp.eo && (L.n_tile % 16) == 0 && pair_on &&
+        (i >= pair_from ||
+         (L.n_tiles == 1 && static_cast<size_t>(3) * a.k_blocks * (L.cout_p / 2) * 128 + 3 * 136 * 128 <= avail))) {
       // conv_pair_kernel: M = 256 over two CTAs, each holds 128 rows of A and half of every weight tile
       // N tiles of the pair kernel: 256 wide (the widest M = 256 MMA: fewest shared-memory operand bytes per MAC)
       // with ONE narrower last tile instead of equal tiles -- cout_p itself (the next layer's K) is unchanged
-      lp.pair = 1;
-      char ntile_key[32];
-      snprintf(ntile_key, sizeof ntile_key, "RISER_PAIR_NTILE_L%d", i);      // per-layer override (tuning)
-      const int wide = std::max(64, std::min(kMaxNTile, env_int(ntile_key, env_int("RISER_PAIR_NTILE", kMaxNTile))) & ~15);
+      lp.kind = kPairKernel;
+      const int wide = std::max(64, std::min(kMaxNTile, pair_ntile) & ~15);
       a.n_tile = std::min(wide, L.cout_p);
       a.n_tiles = (L.cout_p + a.n_tile - 1) / a.n_tile;
       a.n_last = L.cout_p - (a.n_tiles - 1) * a.n_tile;
@@ -3066,33 +2934,60 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
       // 0.47 / 0.37 / 0.38 / 0.46 / 0.49 ms against 0.41 / 0.47 / 0.40 / 0.43 / 0.48 / 0.55 with two sub-tiles, which
       // halve the weight bytes streamed per MAC but leave the TMEM one item deep; `dual` then gives each sub-tile its
       // own issuing warp so that one computes while the other is drained -- RISER_PAIR_MS=2 keeps that variant testable).
-      a.ms = (2 * a.acc_cols <= kTmemCols && env_int("RISER_PAIR_MS", 1) >= 2) ? 2 : 1;
+      a.ms = (2 * a.acc_cols <= kTmemCols && pair_ms >= 2) ? 2 : 1;
       const size_t a_group = static_cast<size_t>(a.ms) * 136 * 128, half_b = static_cast<size_t>(a.n_tile / 2) * 128;
-      a.a_stages = std::max(2, std::min(kMaxAStages, env_int("RISER_PAIR_ASTAGES", a.ms == 2 ? 3 : 5)));
+      a.a_stages = a.ms == 2 ? 3 : 5;
       while (a.a_stages > 2 && a.a_stages * a_group + 4 * half_b > avail) --a.a_stages;
       a.b_stages = std::max(2, std::min<int>(kMaxBStages, static_cast<int>((avail - a.a_stages * a_group) / half_b)));
       a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / (a.ms * a.acc_cols)));
-      a.dual = (a.ms == 2 && env_int("RISER_DUAL_ISSUE", 1)) ? 1 : 0;
-      a.dbg_skip = env_int("RISER_PAIR_DBG_SKIP", 0);       // timing experiments only
-      a.nt_magic = 0;      // (set below, once n_tiles is final)
+      a.dual = (a.ms == 2 && dual_issue) ? 1 : 0;
+      a.dbg_skip = pair_dbg_skip;
       a.resident = 0;
       size_t b_total = a.b_stages * half_b;
       const size_t w_half = static_cast<size_t>(3) * a.k_blocks * half_b;      // this CTA's half of every tap and K block
-      if (a.n_tiles == 1 && w_half + 3 * a_group <= avail && env_int("RISER_PAIR_RESIDENT", 1)) {
+      if (a.n_tiles == 1 && w_half + 3 * a_group <= avail) {
         a.resident = 1;
         a.a_stages = std::min<int>(kMaxAStages, static_cast<int>((avail - w_half) / a_group));
         b_total = w_half;
       }
       a.epi_sets = 4;
-      a.nt_magic = (env_int("RISER_PAIR_MAGIC", 1) && a.n_tiles > 1) ? static_cast<uint32_t>((1ull << 32) / static_cast<unsigned>(a.n_tiles)) + 1u : 0u;
+      // item / n_tiles by multiply-high; with one N tile the magic would overflow, and the kernel divides instead
+      a.nt_magic = a.n_tiles > 1 ? static_cast<uint32_t>((1ull << 32) / static_cast<unsigned>(a.n_tiles)) + 1u : 0u;
       lp.smem = fixed + a.a_stages * a_group + b_total;
       lp.rows_per_super = a.ms * 256;
     }
-    lp.n_supers_total = (rows_in + lp.rows_per_super - 1) / lp.rows_per_super;
+    // every launch covers the whole batch
+    a.n_supers = (rows_in + lp.rows_per_super - 1) / lp.rows_per_super;
+    const int n_items = a.n_supers * a.n_tiles;
+    lp.grid = std::min(n_items, m->sm_count);
+    const void* fn = nullptr;
+    switch (lp.kind) {
+      case kFused01Kernel:
+        lp.fn.fused01 = pick_fused01(kc ? 4 : a.f8 ? 3 : (a.planes == 2 ? 2 : (a.wplanes == 2 ? 1 : 0)));
+        lp.block = kF2Threads;
+        fn = reinterpret_cast<const void*>(lp.fn.fused01);
+        break;
+      case kEoKernel:
+        lp.fn.eo = pick_conv_eo(a.ms, a.planes, a.wplanes);
+        lp.block = 64 + 128 * a.epi_sets;
+        fn = reinterpret_cast<const void*>(lp.fn.eo);
+        break;
+      case kPairKernel:
+        lp.fn.pair = pick_conv_pair(a.ms);
+        lp.grid = std::min(2 * n_items, m->sm_count & ~1);
+        lp.block = 64 + 128 * a.epi_sets + (a.dual ? 32 : 0);
+        fn = reinterpret_cast<const void*>(lp.fn.pair);
+        break;
+      default:
+        lp.fn.tc = pick_conv_kernel(a.ms, a.planes, a.wplanes, a.resident, a.k32, a.f8);
+        lp.block = 64 + 128 * a.epi_sets + (a.dual ? 32 : 0);
+        fn = reinterpret_cast<const void*>(lp.fn.tc);
+    }
+    RISER_CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
   }
   // Two consecutive even / odd layers as ONE launch (conv_eo2_kernel): the first such pair (layers 2 + 3 of the shipped
   // network), when both are hi + lo plane layers, the accumulators fit the TMEM and everything fits shared memory.
-  if (env_int("RISER_FUSE23", 1) && m->act_planes == 2 && p->n_chunked == 0)
+  if (fuse23 && m->act_planes == 2)
     for (int i = 2; i + 1 < m->n_layers - 1; ++i) {
       LayerPlan& l1 = p->layer[i];
       LayerPlan& l2 = p->layer[i + 1];
@@ -3131,8 +3026,11 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
       e.idesc2_2n = umma_idesc_f16(kBlockM, 2 * e.n2);
       e.inv_scale1 = L1.w_inv_scale;
       e.inv_scale2 = L2.w_inv_scale;
-      l1.fuse_next = 1;
-      l1.eo2_smem = smem;
+      l1.kind = l2.kind = kEo2Kernel;
+      l1.fn.eo2 = conv_eo2_kernel;
+      l1.grid = std::min(e.B * e.n_seg, m->sm_count);
+      l1.block = kE2Threads;
+      l1.smem = smem;
       l2.fused_prev = 1;
       RISER_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(conv_eo2_kernel),
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
@@ -3141,44 +3039,24 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
   // tile activity flags (ragged batches / skipped reads): one byte per M super-tile and layer
   p->activity.n_layers = 0;
   p->activity.total = 0;
-  if (env_int("RISER_TILE_SKIP", 1)) {
-    for (int i = 1; i < m->n_layers; ++i) {
-      const ConvArgs& a = p->layer[i].args;
-      ActivityLayer& al = p->activity.layer[p->activity.n_layers++];
-      al.Lp_in = a.Lp_in;
-      al.rows_in = a.rows_in;
-      al.rows_per_super = p->layer[i].rows_per_super;
-      al.shift = a.shift;
-      al.n_supers = p->layer[i].n_supers_total;
-      al.flag_off = p->activity.total;
-      p->layer[i].flag_off = al.flag_off;
-      p->activity.total += al.n_supers;
-    }
-    RISER_CUDA_TRY(cudaMalloc(&p->flags, p->activity.total));
+  for (int i = 1; i < m->n_layers; ++i) {
+    const ConvArgs& a = p->layer[i].args;
+    ActivityLayer& al = p->activity.layer[p->activity.n_layers++];
+    al.Lp_in = a.Lp_in;
+    al.rows_in = a.rows_in;
+    al.rows_per_super = p->layer[i].rows_per_super;
+    al.shift = a.shift;
+    al.n_supers = a.n_supers;
+    al.flag_off = p->activity.total;
+    p->activity.total += al.n_supers;
   }
-  for (int k32v = 0; k32v < 2; ++k32v)
-    for (int ms = 1; ms <= 4; ms <<= 1)
-      for (int pl = 0; pl < 3; ++pl)
-        for (int mode = 0; mode < 3; ++mode)     // 0 streamed, 1 resident, 2 resident + fused layer 0
-          RISER_CUDA_TRY(cudaFuncSetAttribute(
-              reinterpret_cast<const void*>(pick_conv_kernel(ms, pl == 2 ? 2 : 1, pl == 0 ? 1 : 2, mode >= 1,
-                                                             mode == 2, k32v)),
-              cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-  for (int ms = 1; ms <= 2; ++ms)
-    for (int pl = 0; pl < 3; ++pl)
-      RISER_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(pick_conv_eo(ms, pl == 2 ? 2 : 1, pl == 0 ? 1 : 2)),
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-  for (int ms = 1; ms <= 2; ++ms)
-    RISER_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(pick_conv_pair(ms)),
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-  for (int pl = 0; pl < 5; ++pl)
-    RISER_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(pick_fused01(pl)),
-                                        cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-  for (int k32v = 0; k32v < 2; ++k32v)
-    for (int ms = 1; ms <= 4; ms <<= 1)
-      for (int res = 0; res < 2; ++res)
-        RISER_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(pick_conv_kernel(ms, 1, 1, res, 0, k32v, 1)),
-                                            cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
+  RISER_CUDA_TRY(cudaMalloc(&p->flags, p->activity.total));
+  for (int i = 1; i < m->n_layers; ++i) {
+    LayerPlan& lp = p->layer[i];
+    // fused01_kernel stages its CTA's flags in shared memory; past kF2MaxLocalItems items per CTA it runs every item
+    if (lp.kind != kFused01Kernel || (lp.args.n_supers + lp.grid - 1) / lp.grid <= kF2MaxLocalItems)
+      lp.args.flags = p->flags + p->activity.layer[i - 1].flag_off;
+  }
   *out = owner.release();
   return RISER_OK;
 }
@@ -3191,12 +3069,10 @@ extern "C" int riser_plan_destroy(riser_plan* p) {
 
 extern "C" int riser_forward_launches(const riser_plan* p) {
   if (!p) return 0;
-  const int n = p->model->n_layers;
-  const int chunks = p->n_chunked > 0 ? (p->B + p->chunk_reads - 1) / p->chunk_reads : 0;
-  const int l0 = p->fuse_l0 ? (p->n_chunked > 0 ? chunks : 1) : 0;   // layer-0 launches that fusion removes
-  int fused = 0;
-  for (int i = 1; i < n; ++i) fused += p->layer[i].fused_prev;
-  return chunks * p->n_chunked + (n - p->n_chunked) + 1 - l0 - fused + (p->flags ? 1 : 0);
+  // tile_activity_kernel, layer 0, the conv layers and the head, less the layers computed inside another launch
+  int inside = p->fuse_l0;
+  for (int i = 1; i < p->model->n_layers; ++i) inside += p->layer[i].fused_prev;
+  return p->model->n_layers + 2 - inside;
 }
 
 extern "C" int riser_plan_fused_layer0(const riser_plan* p) { return p ? p->fuse_l0 : 0; }
@@ -3214,11 +3090,7 @@ extern "C" int riser_plan_layer_format(const riser_plan* p, int i) {
 
 extern "C" int riser_plan_layer_kernel(const riser_plan* p, int i) {
   if (!p || i < 1 || i >= p->model->n_layers) return -1;
-  if (i == 1 && p->fuse_l0 == 2) return 3;
-  if (i == 1 && p->fuse_l0 == 1) return 4;
-  if (p->layer[i].pair) return 2;
-  if (p->layer[i].fuse_next || p->layer[i].fused_prev) return 5;
-  return p->layer[i].eo ? 1 : 0;
+  return p->layer[i].kind;
 }
 
 extern "C" int riser_plan_layer_info(const riser_plan* p, int i, int64_t* offset, int* rows_per_read,
@@ -3237,83 +3109,62 @@ extern "C" int riser_plan_layer_info(const riser_plan* p, int i, int64_t* offset
 namespace riser {
 namespace {
 
-int launch_layer0(const riser_plan* p, const float* x, int64_t ld_x, const int32_t* len, int b0, int nb,
-                  cudaStream_t st) {
+int launch_layer0(const riser_plan* p, const float* x, int64_t ld_x, const int32_t* len, cudaStream_t st) {
   const riser_model* m = p->model;
   if (p->fuse_l0) return RISER_OK;       // computed inside layer 1's kernel
   const LayerPack& L = m->layer[0];
-  const int64_t total = static_cast<int64_t>(nb) * p->Lp[1] * (L.cout_p / 8);
+  const int64_t total = static_cast<int64_t>(p->B) * p->Lp[1] * (L.cout_p / 8);
   const int grid = static_cast<int>(std::min<int64_t>((total + 255) / 256, static_cast<int64_t>(m->sm_count) * 32));
-  __half* out = reinterpret_cast<__half*>(p->ws + p->act_off[1]) +
-                static_cast<int64_t>(b0) * p->Lp[1] * L.cout_p * m->act_planes;
-  layer0_kernel<<<grid, 256, 0, st>>>(x + static_cast<int64_t>(b0) * ld_x, ld_x, len + b0, L.w0, L.bias, out, nb,
-                                      p->Lp[1], L.cout, L.cout_p, m->act_planes, m->layer[1].f8);
+  __half* out = reinterpret_cast<__half*>(p->ws + p->act_off[1]);
+  layer0_kernel<<<grid, 256, 0, st>>>(x, ld_x, len, L.w0, L.bias, out, p->B, p->Lp[1], L.cout, L.cout_p,
+                                      m->act_planes, m->layer[1].f8);
   RISER_CUDA_TRY(cudaGetLastError());
   return RISER_OK;
 }
 
-// conv layer i over reads [b0, b0 + nb): the super-tiles that touch those reads' rows
-int launch_conv(const riser_plan* p, int i, const float* x, int64_t ld_x, const int32_t* len, int b0, int nb,
-                cudaStream_t st) {
+// conv layer i, through the kernel the plan chose for it
+int launch_conv(const riser_plan* p, int i, const float* x, int64_t ld_x, const int32_t* len, cudaStream_t st) {
   const LayerPlan& lp = p->layer[i];
   if (lp.fused_prev) return RISER_OK;      // computed inside layer i - 1's launch
-  if (lp.fuse_next) {
-    RISER_REQUIRE(b0 == 0 && nb == p->B, "conv_eo2_kernel runs over the whole batch");
-    Eo2Args e = lp.eo2;
-    e.len0 = len;
-    const int n_items = e.B * e.n_seg;
-    conv_eo2_kernel<<<std::min(n_items, p->model->sm_count), kE2Threads, lp.eo2_smem, st>>>(
-        lp.tm_a, lp.tm_a8, lp.tm_b, p->layer[i + 1].tm_b, e);
-    RISER_CUDA_TRY(cudaGetLastError());
-    return RISER_OK;
-  }
   ConvArgs a = lp.args;
   a.len0 = len;
-  const int fused = (i == 1 && p->fuse_l0 == 1) ? 1 : 0;
-  const bool fused2 = (i == 1 && p->fuse_l0 == 2);
-  a.flags = p->flags ? p->flags + lp.flag_off : nullptr;
-  if (fused || fused2) {
-    RISER_REQUIRE(x, "riser_forward: null x");
-    a.x = x;
-    a.ld_x = ld_x;
+  switch (lp.kind) {
+    case kEo2Kernel: {
+      Eo2Args e = lp.eo2;
+      e.len0 = len;
+      lp.fn.eo2<<<lp.grid, lp.block, lp.smem, st>>>(lp.tm_a, lp.tm_a8, lp.tm_b, p->layer[i + 1].tm_b, e);
+      break;
+    }
+    case kFused01Kernel:
+      RISER_REQUIRE(x, "riser_forward: null x");
+      RISER_REQUIRE((ld_x & 3) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0,
+                    "riser_forward: x must be 16-byte aligned with ld_x a multiple of 4 (bulk copies of the signal)");
+      a.x = x;
+      a.ld_x = ld_x;
+      lp.fn.fused01<<<lp.grid, lp.block, lp.smem, st>>>(lp.tm_b, lp.tm_b8, a);
+      break;
+    case kPairKernel: {
+      cudaLaunchConfig_t cfg = {};
+      cfg.gridDim = dim3(static_cast<unsigned>(lp.grid));
+      cfg.blockDim = dim3(static_cast<unsigned>(lp.block));
+      cfg.dynamicSmemBytes = lp.smem;
+      cfg.stream = st;
+      cudaLaunchAttribute attr[1];
+      attr[0].id = cudaLaunchAttributeClusterDimension;
+      attr[0].val.clusterDim.x = 2;
+      attr[0].val.clusterDim.y = 1;
+      attr[0].val.clusterDim.z = 1;
+      cfg.attrs = attr;
+      cfg.numAttrs = 1;
+      RISER_CUDA_TRY(cudaLaunchKernelEx(&cfg, lp.fn.pair, lp.tm_a, lp.tm_b, lp.tm_a8, lp.tm_b8, lp.tm_bl, lp.tm_b8l, a));
+      return RISER_OK;
+    }
+    case kEoKernel:
+      lp.fn.eo<<<lp.grid, lp.block, lp.smem, st>>>(lp.tm_a, lp.tm_a8, lp.tm_b, a);
+      break;
+    default:
+      lp.fn.tc<<<lp.grid, lp.block, lp.smem, st>>>(lp.tm_a, lp.tm_b, lp.tm_a8, lp.tm_b8, a);
   }
-  const int64_t rows_per_super = lp.rows_per_super;
-  const int64_t row0 = static_cast<int64_t>(b0) * a.Lp_in, row1 = static_cast<int64_t>(b0 + nb) * a.Lp_in;
-  a.super0 = static_cast<int>(row0 / rows_per_super);
-  a.n_supers = static_cast<int>((row1 + rows_per_super - 1) / rows_per_super) - a.super0;
-  const int grid = std::min(a.n_supers * a.n_tiles, p->model->sm_count);
-  if (fused2) {
-    if ((a.n_supers + grid - 1) / grid > kF2MaxLocalItems) a.flags = nullptr;   // (every item treated as active)
-    RISER_REQUIRE((ld_x & 3) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0,
-                  "riser_forward: x must be 16-byte aligned with ld_x a multiple of 4 (bulk copies of the signal)");
-    pick_fused01(lp.kc ? 4 : a.f8 ? 3 : (a.planes == 2 ? 2 : (a.wplanes == 2 ? 1 : 0)))<<<grid, kF2Threads, lp.smem, st>>>(
-        lp.tm_b, lp.tm_b8, a);
-    RISER_CUDA_TRY(cudaGetLastError());
-    return RISER_OK;
-  }
-  if (lp.pair) {
-    cudaLaunchConfig_t cfg = {};
-    const int n_items = a.n_supers * a.n_tiles;
-    cfg.gridDim = dim3(static_cast<unsigned>(std::min(2 * n_items, p->model->sm_count & ~1)));
-    cfg.blockDim = dim3(64 + 128 * a.epi_sets + (a.dual ? 32 : 0));
-    cfg.dynamicSmemBytes = lp.smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    RISER_CUDA_TRY(cudaLaunchKernelEx(&cfg, pick_conv_pair(a.ms), lp.tm_a, lp.tm_b, lp.tm_a8, lp.tm_b8, lp.tm_bl, lp.tm_b8l, a));
-    return RISER_OK;
-  }
-  if (lp.eo) {
-    pick_conv_eo(a.ms, a.planes, a.wplanes)<<<grid, 64 + 128 * a.epi_sets, lp.smem, st>>>(lp.tm_a, lp.tm_a8, lp.tm_b, a);
-    RISER_CUDA_TRY(cudaGetLastError());
-    return RISER_OK;
-  }
-  pick_conv_kernel(a.ms, a.planes, a.wplanes, a.resident, fused, a.k32, a.f8)<<<grid, fused ? kConvThreads + kCvtThreads : 64 + 128 * a.epi_sets + (a.dual ? 32 : 0), lp.smem, st>>>(lp.tm_a, lp.tm_b, lp.tm_a8, lp.tm_b8, a);
   RISER_CUDA_TRY(cudaGetLastError());
   return RISER_OK;
 }
@@ -3321,8 +3172,8 @@ int launch_conv(const riser_plan* p, int i, const float* x, int64_t ld_x, const 
 }  // namespace
 }  // namespace riser
 
-// stage 0: the chunked early layers (layer 0 + conv layers < n_chunked), chunk by chunk;
-// stage 1: the remaining conv layers over the whole batch; stage 2: head.
+// stage 0: tile activity flags and layer 0 (unless fused into layer 1's launch); stage 1: the conv layers;
+// stage 2: head; stage 3: layer 0 alone; stage 16 + i: conv layer i alone.
 extern "C" int riser_forward_stage(const riser_plan* p, int stage, const float* x, int64_t ld_x,
                                    const int32_t* len, float* probs, float* feat, riser_stream_t stream) {
   RISER_REQUIRE(p && len, "riser_forward_stage: null pointer");
@@ -3333,20 +3184,12 @@ extern "C" int riser_forward_stage(const riser_plan* p, int stage, const float* 
     RISER_REQUIRE(x, "riser_forward_stage: null x");
     RISER_REQUIRE(ld_x >= p->max_len && (ld_x & 1) == 0 && (reinterpret_cast<uintptr_t>(x) & 7) == 0,
                   "riser_forward: x must be 8-byte aligned with even ld_x >= max_len");
-    if (p->flags) {
-      tile_activity_kernel<<<(p->activity.total + 255) / 256, 256, 0, st>>>(len, p->activity, p->flags);
-      RISER_CUDA_TRY(cudaGetLastError());
-    }
-    if (p->n_chunked == 0) return launch_layer0(p, x, ld_x, len, 0, p->B, st);
-    for (int b0 = 0; b0 < p->B; b0 += p->chunk_reads) {
-      const int nb = std::min(p->chunk_reads, p->B - b0);
-      if ((rc = launch_layer0(p, x, ld_x, len, b0, nb, st))) return rc;
-      for (int i = 1; i < p->n_chunked; ++i)
-        if ((rc = launch_conv(p, i, x, ld_x, len, b0, nb, st))) return rc;
-    }
+    tile_activity_kernel<<<(p->activity.total + 255) / 256, 256, 0, st>>>(len, p->activity, p->flags);
+    RISER_CUDA_TRY(cudaGetLastError());
+    return launch_layer0(p, x, ld_x, len, st);
   } else if (stage == 1) {
-    for (int i = std::max(1, p->n_chunked); i < m->n_layers; ++i)
-      if ((rc = launch_conv(p, i, x, ld_x, len, 0, p->B, st))) return rc;
+    for (int i = 1; i < m->n_layers; ++i)
+      if ((rc = launch_conv(p, i, x, ld_x, len, st))) return rc;
   } else if (stage == 2) {
     RISER_REQUIRE(probs, "riser_forward_stage: null probs");
     const int n = m->n_layers;
@@ -3354,14 +3197,12 @@ extern "C" int riser_forward_stage(const riser_plan* p, int stage, const float* 
                                                m->fc_b, probs, feat, p->B, p->Lp[n], m->layer[n - 1].cout_p,
                                                m->c_last, n);
     RISER_CUDA_TRY(cudaGetLastError());
-  } else if (stage == 3) {   // layer-0 launches only (timing aid: see bench.py)
+  } else if (stage == 3) {   // layer-0 launch only (timing aid: see bench.py)
     RISER_REQUIRE(x, "riser_forward_stage: null x");
-    if (p->n_chunked == 0) return launch_layer0(p, x, ld_x, len, 0, p->B, st);
-    for (int b0 = 0; b0 < p->B; b0 += p->chunk_reads)
-      if ((rc = launch_layer0(p, x, ld_x, len, b0, std::min(p->chunk_reads, p->B - b0), st))) return rc;
+    return launch_layer0(p, x, ld_x, len, st);
   } else if (stage >= 16 && stage < 16 + m->n_layers) {   // conv layer (stage - 16) alone (timing aid: tools/layer_events.py)
-    RISER_REQUIRE(stage - 16 >= 1 && p->n_chunked == 0, "riser_forward_stage: single-layer stages need layer >= 1, no chunking");
-    return launch_conv(p, stage - 16, x, ld_x, len, 0, p->B, st);
+    RISER_REQUIRE(stage - 16 >= 1, "riser_forward_stage: single-layer stages need layer >= 1");
+    return launch_conv(p, stage - 16, x, ld_x, len, st);
   } else {
     return fail(RISER_EINVAL, "riser_forward_stage: stage %d outside 0..3 / 16..", stage);
   }

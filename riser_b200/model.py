@@ -25,7 +25,7 @@ MIN_LENGTH = 4096  # riser/preprocess.py:8 -- 12 stride-2 pools
 # of the e4m3 pass carry the opposite powers of two (csrc/convnet.cu kF8AScale / kF8LoScale, which these must match)
 F8_A_SHIFT = 3
 F8_LO_SHIFT = 0
-DEFAULT_CHUNK = 0    # 0 = whole batch in one plan (the plan chunks the early layers itself)
+DEFAULT_CHUNK = 0    # 0 = whole batch in one plan (every launch covers the whole batch)
 
 
 class Plan:
@@ -58,7 +58,7 @@ class Plan:
         """Name of the kernel that runs conv layer i in this plan (riser_plan_layer_kernel)."""
         k = int(_lib.lib().riser_plan_layer_kernel(self._handle, i))
         return {0: "conv_tc_kernel", 1: "conv_eo_kernel", 2: "conv_pair_kernel", 3: "fused01_kernel",
-                4: "conv_tc_kernel<FUSED>", 5: "conv_eo2_kernel"}.get(k, "?")
+                5: "conv_eo2_kernel"}.get(k, "?")
 
     def planes(self, i, n_layers, fmt=None):
         """Layer i's input buffer as the planes it stores, each [B, rows_per_read, channels] in its stored dtype:
@@ -226,9 +226,8 @@ class Model():
         ld), lens: int32 [B] valid lengths (>= 4096; shorter -> NaN row).
         Returns probs fp32 [B, 2] on the device.  No synchronisation.
 
-        chunk: optionally run the network over sub-batches of this many reads (the
-        library already runs the memory-bound early layers chunk by chunk inside one
-        plan so their activations stay in the 126 MB L2; this only bounds workspace).
+        chunk: optionally run the network over sub-batches of this many reads, one plan
+        and one forward each (bounds the workspace; each launch covers its whole sub-batch).
         events: optional list; (start, end) torch.cuda.Event pairs bracketing layer 0 +
         the tcgen05 conv layers of every sub-batch are appended (bench.py's roofline;
         ``time_layer0`` gives the layer-0 share to subtract)."""
@@ -252,7 +251,7 @@ class Model():
                 _lib.check(L.riser_forward(p._handle, _lib.ptr(xs), x.stride(0), _lib.ptr(ls), _lib.ptr(ps),
                                            _lib.ptr(fs), stream), "riser_forward")
                 continue
-            # stages 0 (layer 0 + chunked early conv layers) and 1 (remaining conv layers) bracketed
+            # stages 0 (tile activity flags + layer 0 unless fused) and 1 (the conv layers) bracketed
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
             for stage in range(3):

@@ -48,15 +48,17 @@ def oracle_layers(state, x):
     return outs
 
 
-@pytest.mark.parametrize("fuse,precision", [(0, PREC_F16), (0, PREC_F16_W2), (0, PREC_F16_X3), (1, PREC_F16),
-                                            (1, PREC_F16_W2), (1, PREC_F16_X3), (2, PREC_F16), (2, PREC_F16_W2),
-                                            (2, PREC_F16_X3), (0, PREC_F16_F8), (2, PREC_F16_F8),
+# pytest numbers the tuple-valued cases by position ("precision11"); their ids are pinned so that a case keeps its
+# id when the list in front of it changes
+@pytest.mark.parametrize("fuse,precision", [(0, PREC_F16), (0, PREC_F16_W2), (0, PREC_F16_X3),
+                                            (2, PREC_F16), (2, PREC_F16_W2), (2, PREC_F16_X3), (0, PREC_F16_F8), (2, PREC_F16_F8)] +
+                         [pytest.param(f, p, id=f"{f}-precision{k}") for k, (f, p) in enumerate([
                                             (0, (PREC_F16_F8, 1)), (2, (PREC_F16_F8, 1)), (2, (PREC_F16_F8, 3)),
                                             (2, (PREC_F16_X3, "flat")), (0, (PREC_F16, "flat")),
                                             (2, (PREC_F16_F8, "nopair")), (2, (PREC_F16_F8, "pair2")), (2, (PREC_F16_F8, "pair5")),
                                             (2, (PREC_F16_F8, "pair192")), (2, (PREC_F16_F8, 6)),
                                             (2, (PREC_F16_F8, "nofuse23")), (2, (PREC_F16_X3, "nofuse23")),
-                                            (2, (PREC_F16_X3, "nokc")), (2, (PREC_F16_F8, "nokc"))])
+                                            (2, (PREC_F16_X3, "nokc")), (2, (PREC_F16_F8, "nokc"))], 11)])
 def test_every_layer_against_oracle(fuse, precision, monkeypatch):
     monkeypatch.setenv("RISER_FUSE_L0", str(fuse))
     if isinstance(precision, tuple) and precision[1] == "flat":     # without the even / odd plane layout

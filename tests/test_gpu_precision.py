@@ -37,7 +37,6 @@ POISON = 7.5
 # name -> (RISER_FUSE_L0, precision, extra environment); the variants of test_every_layer_against_oracle
 VARIANTS = {
     "f0-f16": (0, PREC_F16, {}), "f0-w2": (0, PREC_F16_W2, {}), "f0-x3": (0, PREC_F16_X3, {}),
-    "f1-f16": (1, PREC_F16, {}), "f1-w2": (1, PREC_F16_W2, {}), "f1-x3": (1, PREC_F16_X3, {}),
     "f2-f16": (2, PREC_F16, {}), "f2-w2": (2, PREC_F16_W2, {}), "f2-x3": (2, PREC_F16_X3, {}),
     "f0-f8": (0, PREC_F16_F8, {}), "f2-f8": (2, PREC_F16_F8, {}),
     "f0-f8-from1": (0, PREC_F16_F8, {"RISER_F8_FROM": "1"}), "f2-f8-from1": (2, PREC_F16_F8, {"RISER_F8_FROM": "1"}),
@@ -152,8 +151,7 @@ def run_variant(fuse, precision, env, monkeypatch, scale=None):
             rows_in, rows_out = L0 >> i, L0 >> (j + 1)
             if src is None:                                   # layer 0 inside layer 1's launch
                 xs = x[b, :L0]
-                a0 = pe.layer0_tc(xs, state["layers.0.0.weight"].cuda(), state["layers.0.0.bias"].cuda()) \
-                    if fuse == 2 else pe.exact_layer(xs.double()[:, None], W[0], Bs[0])
+                a0 = pe.layer0_tc(xs, state["layers.0.0.weight"].cuda(), state["layers.0.0.bias"].cuda())
                 s_in = pe.layer0_bound(xs, W[0], Bs[0])
                 planes = pe.split_act(a0, fmt_in)
             else:
