@@ -114,6 +114,31 @@ int riser_normalise_f32(const float* sig, const int64_t* off, const int32_t* len
 int riser_normalise_f32_live(const float* sig, const int64_t* off, const int32_t* len, int B, int max_len,
                              float* out, int64_t ld_out, float* med_mad, riser_stream_t stream);
 
+/* Windows of any length (max_len up to INT32_MAX): the three entry points above hold a whole window in one
+ * CTA's shared memory and refuse longer ones; these keep it in global memory and work on it with many CTAs
+ * (exact multi-pass radix select for median and MAD, then the elementwise normalise and the sequential
+ * outlier smoothing).  The results are those of riser_normalise / riser_normalise_f32(_live) bit for bit, at
+ * any length, short windows included.  The arguments mean what they mean there, except:
+ *   - out needs no alignment and ld_out only ld_out >= max_len; elements i >= len[b] of a row are not
+ *     written, len[b] == 0 writes nothing, and a window longer than max_len is processed as its first
+ *     max_len samples (riser_normalise_f32_long too);
+ *   - riser_normalise_f32_long: outlier_lim and zero_if_mad0 choose between riser_normalise_f32 (the
+ *     caller's limit, 0 = no MAD == 0 guard: IEEE inf / nan) and riser_normalise_f32_live (3.5, 1 = zeros
+ *     when MAD == 0); med_mad (optional) as riser_normalise_f32_live's;
+ *   - workspace: device memory of at least riser_normalise_long_workspace_bytes(B, max_len) bytes, 16-byte
+ *     aligned, any content (RISER_ENOMEM when smaller).  Its contents are scratch between calls; two calls in
+ *     flight at once need two workspaces.
+ * Each call launches a fixed sequence of kernels for a given (B, max_len), so it can be captured in a CUDA
+ * graph.  On short windows the shared-memory entry points are faster; callers pick by length
+ * (SignalProcessor.mad_normalise_batch sends only windows above riser_normalise_max_len() here).          */
+size_t riser_normalise_long_workspace_bytes(int B, int max_len);
+int riser_normalise_long(const int16_t* sig, const int64_t* off, const int32_t* start, const int32_t* len, int B,
+                         int max_len, float* out, int64_t ld_out, int32_t* med2_mad4,
+                         void* workspace, size_t workspace_bytes, riser_stream_t stream);
+int riser_normalise_f32_long(const float* sig, const int64_t* off, const int32_t* len, int B, int max_len,
+                             float outlier_lim, int zero_if_mad0, float* out, int64_t ld_out, float* med_mad,
+                             void* workspace, size_t workspace_bytes, riser_stream_t stream);
+
 /* Replaces SignalProcessor.get_polyA_end (riser/preprocess.py:42-79), batched.
  * Read b is sig[off[b] .. off[b] + n[b]).  polya_end[b] = the returned window
  * start index, or -1 for None.  Window statistics are exact integers; the

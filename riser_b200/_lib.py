@@ -23,6 +23,11 @@ SIGNATURES = {
     "riser_normalise_f32_max_len": (c_int, []),
     "riser_normalise_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_float, c_void_p, c_i64, c_void_p]),
     "riser_normalise_f32_live": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_i64, c_void_p, c_void_p]),
+    "riser_normalise_long_workspace_bytes": (c_size_t, [c_int, c_int]),
+    "riser_normalise_long": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_i64,
+                                     c_void_p, c_void_p, c_size_t, c_void_p]),
+    "riser_normalise_f32_long": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_float, c_int, c_void_p, c_i64,
+                                         c_void_p, c_void_p, c_size_t, c_void_p]),
     "riser_polya_end": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int,
                                 c_void_p]),
     "riser_polya_end_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int,

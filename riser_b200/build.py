@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libriser_b200.so")
-SOURCES = ["preprocess.cu", "normalise_f32.cu", "polya_f32.cu", "convnet.cu", "resnet.cu", "resnet_tc.cu"]
+SOURCES = ["preprocess.cu", "normalise_f32.cu", "normalise_long.cu", "polya_f32.cu", "convnet.cu", "resnet.cu", "resnet_tc.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "-cudart", "static"]
 

@@ -287,19 +287,35 @@ class SignalProcessor():
             return np.zeros(n, dtype=np.int64)
         return out[0, :n].double().cpu().numpy()
 
+    def _long_workspace(self, B, max_len):
+        """Workspace of riser_normalise_long / riser_normalise_f32_long for (B, max_len), kept for the next call of
+        the same shape."""
+        key = (B, max_len)
+        ws = getattr(self, "_long_ws", None)
+        if ws is None or ws[0] != key:
+            nbytes = _lib.lib().riser_normalise_long_workspace_bytes(B, max_len)
+            ws = (key, torch.empty(max(nbytes, 16), dtype=torch.uint8, device=_lib.require_device()))
+            self._long_ws = ws
+        return ws[1]
+
     def _mad_normalise_f32(self, signal):
         device = _lib.require_device()
         n = signal.shape[0]
-        if n > _lib.lib().riser_normalise_f32_max_len():
-            raise ValueError(f"signal of {n} samples exceeds riser_normalise_f32_max_len()")
         sig = torch.from_numpy(np.ascontiguousarray(signal)).to(device)
         off = torch.tensor([0, n], dtype=torch.int64, device=device)
         ln = torch.tensor([n], dtype=torch.int32, device=device)
         out = torch.empty(1, n, dtype=torch.float32, device=device)
         med_mad = torch.empty(1, 2, dtype=torch.float32, device=device)
-        _lib.check(_lib.lib().riser_normalise_f32_live(_lib.ptr(sig), _lib.ptr(off), _lib.ptr(ln), 1, n,
-                                                       _lib.ptr(out), out.stride(0), _lib.ptr(med_mad),
-                                                       _lib.stream_ptr()), "riser_normalise_f32_live")
+        if n > _lib.lib().riser_normalise_f32_max_len():
+            ws = self._long_workspace(1, n)
+            _lib.check(_lib.lib().riser_normalise_f32_long(_lib.ptr(sig), _lib.ptr(off), _lib.ptr(ln), 1, n, 3.5, 1,
+                                                           _lib.ptr(out), out.stride(0), _lib.ptr(med_mad),
+                                                           _lib.ptr(ws), ws.numel(), _lib.stream_ptr()),
+                       "riser_normalise_f32_long")
+        else:
+            _lib.check(_lib.lib().riser_normalise_f32_live(_lib.ptr(sig), _lib.ptr(off), _lib.ptr(ln), 1, n,
+                                                           _lib.ptr(out), out.stride(0), _lib.ptr(med_mad),
+                                                           _lib.stream_ptr()), "riser_normalise_f32_live")
         if float(med_mad[0, 1]) == 0.0:
             return np.zeros(n, dtype=np.int64)
         return out[0].cpu().numpy()
@@ -310,7 +326,11 @@ class SignalProcessor():
         signals: list of int16 arrays, or a RaggedBatch already on the device.
         start / length (optional int32 arrays): window of each read
         (``sig[start:start+length]``); default the whole read.
-        Returns (out fp32 [B, ld] on the device, lengths int32 device tensor)."""
+        Returns (out fp32 [B, ld] on the device, lengths int32 device tensor).
+
+        Windows longer than ``riser_normalise_max_len()`` go to ``riser_normalise_long`` (same results, global-memory
+        passes instead of one CTA's shared memory); the rest to ``riser_normalise``, each launch seeing the other's
+        windows as length 0."""
         device = _lib.require_device()
         batch = signals if isinstance(signals, RaggedBatch) else RaggedBatch(
             [np.ascontiguousarray(s, dtype=np.int16) for s in signals], device)
@@ -319,17 +339,27 @@ class SignalProcessor():
         else:
             len_host = np.asarray(length, dtype=np.int32)
         max_len = int(len_host.max()) if batch.B else 0
-        if max_len > _lib.lib().riser_normalise_max_len():
-            raise ValueError(f"window of {max_len} samples exceeds riser_normalise_max_len()")
+        limit = _lib.lib().riser_normalise_max_len()
         ld = (max_len + 3) & ~3
         if out is None:
             out = torch.zeros(batch.B, max(ld, 4), dtype=torch.float32, device=device)
         start_t = None if start is None else torch.as_tensor(np.asarray(start, dtype=np.int32)).to(device)
         len_t = batch.n if (length is None and start is None) else torch.from_numpy(len_host).to(device)
         stats = torch.zeros(batch.B, 2, dtype=torch.int32, device=device) if return_stats else None
+        short_t = len_t
+        if max_len > limit:
+            is_long = len_host > limit
+            short_t = torch.from_numpy(np.where(is_long, 0, len_host).astype(np.int32)).to(device)
+            long_t = torch.from_numpy(np.where(is_long, len_host, 0).astype(np.int32)).to(device)
+            ws = self._long_workspace(batch.B, max_len)
+            _lib.check(_lib.lib().riser_normalise_long(_lib.ptr(batch.sig), _lib.ptr(batch.off), _lib.ptr(start_t),
+                                                       _lib.ptr(long_t), batch.B, max_len, _lib.ptr(out),
+                                                       out.stride(0), _lib.ptr(stats), _lib.ptr(ws), ws.numel(),
+                                                       _lib.stream_ptr()), "riser_normalise_long")
+            max_len = limit
         if batch.B and max_len > 0:
             _lib.check(_lib.lib().riser_normalise(_lib.ptr(batch.sig), _lib.ptr(batch.off), _lib.ptr(start_t),
-                                                  _lib.ptr(len_t), batch.B, max_len, _lib.ptr(out),
+                                                  _lib.ptr(short_t), batch.B, max_len, _lib.ptr(out),
                                                   out.stride(0), _lib.ptr(stats), _lib.stream_ptr()),
                        "riser_normalise")
         if return_stats:
