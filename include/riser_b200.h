@@ -351,6 +351,45 @@ int riser_gap_linear_softmax(const float* in, const int32_t* len, const float* f
                              float* probs, int B, int L_pad, int C, int n_classes,
                              riser_stream_t stream);
 
+/* ------------------------------------------------------------------ training (backward pass of the ConvNet)
+ * riser/nets/cnn.py:8-65 trained with nn.CrossEntropyLoss (the reference's train.py); riser_b200/training.py drives
+ * them.  Activations are fp32 channel-last [B][L_pad][C] with per-read valid lengths, as for riser_conv1d_cl.  The
+ * forward pass and the input gradients use riser_conv1d_cl (dgrad: the weight [K][Cout][Cin] with the taps flipped,
+ * relu 0, zero bias), riser_maxpool1d_pad_cl (pad 0) and riser_len_chain.                                    */
+
+/* Weight and bias gradients of Conv1d(Cin -> Cout, K odd, stride 1, padding (K - 1) / 2):
+ *   dw[co][ci][j] = sum_b sum_{t < len[b]} dz[b][t][co] * x[b][t + j - (K - 1) / 2][ci]   (x = 0 outside [0, len[b]))
+ *   db[co]        = sum_b sum_{t < len[b]} dz[b][t][co]
+ * dz [B][L_pad][Cout], x [B][L_pad][Cin]; rows t >= len[b] of either are never read (NaN there changes nothing).
+ * tcgen05 with the rows as the reduction dimension: operands converted to bf16 hi + lo planes, the products
+ * hi*hi + hi*lo + lo*hi accumulated in fp32, the row splits of the reduction added in a fixed order (bitwise the same
+ * on every run).  K <= 31.  workspace: at least riser_conv1d_wgrad_workspace_bytes(...) bytes (0 = unsupported
+ * shape), any content; RISER_ENOMEM when smaller.                                                            */
+size_t riser_conv1d_wgrad_workspace_bytes(int B, int L_pad, int Cin, int Cout, int K);
+int riser_conv1d_wgrad_cl(const float* dz, const float* x, const int32_t* len, int B, int L_pad, int Cin, int Cout,
+                          int K, float* dw, float* db, void* workspace, size_t workspace_bytes, riser_stream_t stream);
+
+/* Gradient through ReLU + MaxPool1d(2, 2) (pool = 1) or ReLU alone (pool = 0).  y [B][L_pad][C]: the saved
+ * post-ReLU convolution output, valid for t < len[b]; dp: the gradient of the pooled output [B][Lp_pad][C] (valid
+ * for t < len[b] / 2) or, pool = 0, of y itself [B][L_pad][C] (Lp_pad == L_pad).  Writes every row of dz
+ * [B][L_pad][C]: the pooled gradient goes to the larger of each pair (the first on a tie, torch's rule), times
+ * (y > 0); the odd trailing row the floor pool drops and rows t >= len[b] get 0.                              */
+int riser_relu_pool_bwd_cl(const float* y, const float* dp, const int32_t* len, float* dz, int B, int L_pad,
+                           int Lp_pad, int C, int pool, riser_stream_t stream);
+
+/* AdaptiveAvgPool1d(1) + Flatten + Linear(C, n_classes) + nn.CrossEntropyLoss() (mean) forward and backward
+ * (the 'gap_fc' head, cnn.py:28-33; 'gap', cnn.py:35-39, is the same linear map).  h [B][L_pad][C], valid for
+ * t < len[b]; fc_w [n_classes][C]; labels int64 [B].  Computed in float64, stored as fp32:
+ *   loss [B] = logsumexp(z) - z[y], loss_mean [1], logits [B][n_classes] = z, dlogits = (softmax(z) - onehot) / B,
+ *   feat [B][C] the pooled features, dfc_w [n_classes][C] and dfc_b [n_classes] summed over reads in order,
+ *   dh [B][L_pad][C] = (fc_w^T dlogits) / len[b] on rows t < len[b], 0 on the others.
+ * A read with len 0 or a label outside [0, n_classes) gets a NaN loss (so loss_mean is NaN) and no gradient.
+ * n_classes <= 32.                                                                                             */
+int riser_gap_linear_ce_bwd(const float* h, const int32_t* len, const float* fc_w, const float* fc_b,
+                            const int64_t* labels, int B, int L_pad, int C, int n_classes, float* loss,
+                            float* loss_mean, float* logits, float* dlogits, float* feat, float* dfc_w, float* dfc_b,
+                            float* dh, riser_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -20,6 +20,15 @@ from . import _lib
 from .resnet import _Conv, _pad8
 
 
+def check_supported(c):
+    """Raise NotImplementedError for the ConvNet configurations riser_b200 does not implement (module docstring)."""
+    if c.classifier not in ('gap_fc', 'gap'):
+        raise NotImplementedError(f"classifier {c.classifier!r}: riser_b200 implements 'gap_fc' and 'gap' "
+                                  "(the reference's 'fc' head is hard-coded to one input width, riser/nets/cnn.py:24-29)")
+    if any(int(k) % 2 == 0 or int(k) < 1 for k in c.kernels[:int(c.n_layers)]):
+        raise NotImplementedError("riser_b200 implements odd kernel sizes (padding='same' is asymmetric for even ones)")
+
+
 class GenericConvNet:
     def __init__(self, sd, c, device, logger=None):
         self.device = device
@@ -28,11 +37,7 @@ class GenericConvNet:
         self.n_classes = int(c.n_classes)
         channels = [int(x) for x in c.channels[:n]]
         kernels = [int(k) for k in c.kernels[:n]]
-        if c.classifier not in ('gap_fc', 'gap'):
-            raise NotImplementedError(f"classifier {c.classifier!r}: riser_b200 implements 'gap_fc' and 'gap' "
-                                      "(the reference's 'fc' head is hard-coded to one input width, riser/nets/cnn.py:24-29)")
-        if any(k % 2 == 0 or k < 1 for k in kernels):
-            raise NotImplementedError("riser_b200 implements odd kernel sizes (padding='same' is asymmetric for even ones)")
+        check_supported(c)
         # expected keys and shapes: what ConvNet(config.cnn).load_state_dict enforces (cnn.py:13-41, 52-65)
         expected = {}
         cin = 1
