@@ -60,11 +60,6 @@ __device__ __forceinline__ bool elect_one() {
 // two 16-byte stores to the same sector are two half-filled sector writes and two tag look-ups at the L2,
 // which is what bounded the narrow layers (profiles/README.md, round 2).
 __device__ __forceinline__ void st_global_256(void* p, const uint4& a, const uint4& b) {
-#ifdef RISER_ST128   // A/B timing builds: the two 16-byte stores this replaces
-  reinterpret_cast<uint4*>(p)[0] = a;
-  reinterpret_cast<uint4*>(p)[1] = b;
-  return;
-#endif
   asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
                ::"l"(p), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w)
                : "memory");
@@ -98,16 +93,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
 }
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   while (!mbar_try_wait(bar, parity)) {
-  }
-}
-// Wait of the many-thread roles (converter / epilogue warps): back off between polls so that
-// their spinning does not take issue slots from the warps that are doing work.
-#ifndef RISER_SPIN_NS
-#define RISER_SPIN_NS 0
-#endif
-__device__ __forceinline__ void mbar_wait_relaxed(uint64_t* bar, uint32_t parity) {
-  while (!mbar_try_wait(bar, parity)) {
-    if (RISER_SPIN_NS > 0) __nanosleep(RISER_SPIN_NS);
   }
 }
 

@@ -31,18 +31,6 @@
 namespace riser {
 namespace {
 
-// Timing experiments only (results are wrong when set): fused01_kernel 1 = one MMA per layer-1 accumulator,
-// 2 = no global stores, 4 / 8 = mid-epilogue / epilogue skip their TMEM loads, 16 = mid-epilogue idle,
-// 32 = cvt1 idle; conv_tc_kernel 64 = one MMA per accumulator, 128 = epilogue idle after its TMEM loads,
-// 256 = epilogue skips its TMEM loads.
-#ifndef RISER_DBG
-#define RISER_DBG 0
-#endif
-// 1: the MMA-issuing loops are run by the whole warp with the instruction predicated on the elected lane (A/B timing
-// builds: 0 = the loop under `if (lane == 0)`)
-#ifndef RISER_UNIFORM_ISSUE
-#define RISER_UNIFORM_ISSUE 1
-#endif
 constexpr int kMaxLayers = 16;
 constexpr int kBlockM = 128;          // rows per tile (UMMA M)
 constexpr int kBlockK = 64;           // fp16 elements per K block = 128 bytes = one swizzle row
@@ -109,7 +97,7 @@ struct ConvArgs {
   const uint8_t* flags;   // per M super-tile: 0 = every row pair lies beyond its read's valid length + 1 -> skip
   int rows_in, Lp_in, Lp_out, shift;
   int cin_p, cout_p, n_tile, n_tiles, k_blocks;
-  int super0, n_supers;   // range of M super-tiles this launch covers (x n_tiles work items)
+  int n_supers;           // M super-tiles of the batch (x n_tiles work items)
   int ms;                 // 128-row M sub-tiles per work item (they share every weight tile)
   int planes;             // activation planes read (1, or 2 = hi + lo)
   int wplanes;            // weight planes (1, or 2 = hi + lo)
@@ -117,7 +105,6 @@ struct ConvArgs {
   int a_stages, b_stages, acc_stages, resident;
   int epi_sets;           // epilogue warp sets (each = 4 warps covering the TMEM lane quadrants)
   int dual;               // conv_tc_kernel, MS == 2: one MMA-issuing thread PER SUB-TILE (warp 1 and the last warp)
-  int dbg_skip;           // conv_pair_kernel timing experiments (WRONG results): 1 = no weight loads, 2 = no activation loads
   uint32_t nt_magic;      // conv_pair_kernel: floor(2^32 / n_tiles) + 1 -- item / n_tiles = umulhi(item, nt_magic) (items < 2^24); 0 = divide
   int acc_cols;           // TMEM columns per accumulator slot (n_tile rounded up to 32)
   int half_lp;            // Lp_in / 2
@@ -429,12 +416,7 @@ __device__ __forceinline__ void epilogue_row16(const uint32_t (&ve)[16], const u
       const float2 back = __half22float2(hv[c]);
       lv[c] = __floats2half2_rn(r[2 * c] - back.x, r[2 * c + 1] - back.y);
     }
-#ifdef RISER_DBG_TRAFFIC   // timing experiment (wrong results): the lo plane is written over the hi plane
-    uint4* ol = reinterpret_cast<uint4*>(ohi);
-#else
-    uint4* ol = reinterpret_cast<uint4*>(ohi + lo_off);
-#endif
-    st_global_256(ol, *reinterpret_cast<const uint4*>(lv), *reinterpret_cast<const uint4*>(lv + 4));
+    st_global_256(ohi + lo_off, *reinterpret_cast<const uint4*>(lv), *reinterpret_cast<const uint4*>(lv + 4));
   }
   if (f8) store_f8_planes<16>(r, hv, f8, f8_stride);
 }
@@ -454,8 +436,8 @@ __device__ __forceinline__ uint64_t sw_desc(uint32_t addr) {
 // Decoding is kept incremental (no division in the single-thread roles' loops).
 struct ItemCursor {
   int super, n, step_super, step_n, n_tiles;
-  __device__ __forceinline__ ItemCursor(int first, int grid, int n_tiles_, int super0) : n_tiles(n_tiles_) {
-    super = super0 + first / n_tiles_;
+  __device__ __forceinline__ ItemCursor(int first, int grid, int n_tiles_) : n_tiles(n_tiles_) {
+    super = first / n_tiles_;
     n = first % n_tiles_;
     step_super = grid / n_tiles_;
     step_n = grid % n_tiles_;
@@ -566,7 +548,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
       int sa = 0, sb = 0;
       uint32_t pa = 0, pb = 0;
       const uint32_t a_tx = kATiles * a.a_tx_bytes;
-      ItemCursor cur(blockIdx.x, gridDim.x, a.n_tiles, a.super0);
+      ItemCursor cur(blockIdx.x, gridDim.x, a.n_tiles);
       ItemFlags fl(a.flags, cur.super, blockIdx.x < n_items);
       for (int item = blockIdx.x; item < n_items; item += gridDim.x, cur.next()) {
         if (!fl.take(cur, item + gridDim.x < n_items)) continue;
@@ -624,88 +606,86 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
     const int ms_lo = a.dual ? (warp == 1 ? 0 : 1) : 0;
     const int ms_hi = a.dual ? ms_lo + 1 : MS;
     // the whole warp runs the loop (uniform registers); only the elected lane executes the MMAs / commits
-    const uint32_t leader = (RISER_UNIFORM_ISSUE ? elect_one() : (lane == 0)) ? 1u : 0u;
-    if (RISER_UNIFORM_ISSUE || lane == 0) {
-      if (RESIDENT) {
-        mbar_wait(&s.w_full, 0);
+    const uint32_t leader = elect_one() ? 1u : 0u;
+    if (RESIDENT) {
+      mbar_wait(&s.w_full, 0);
+      tc_fence_after();
+    }
+    int sa = 0, sb = 0, stage = 0;
+    uint32_t pa = 0, pb = 0, acc_phase = 0;
+    const uint32_t a_ring_addr = smem_u32(a_ring), b_region_addr = smem_u32(b_region);
+    const int nk_last = (a.cin_p - (a.kb16 - 1) * kKElems) / 16;
+    const int nk_last8 = F8 ? (2 * a.cin_p - (a.k_blocks - a.kb16 - 1) * kRowBytes) / 32 : 0;
+    const uint32_t acc_stride = MS * a.acc_cols;
+    ItemCursor cur(blockIdx.x, gridDim.x, a.n_tiles);
+    ItemFlags fl(a.flags, cur.super, blockIdx.x < n_items);
+    for (int item = blockIdx.x; item < n_items; item += gridDim.x, cur.next()) {
+      if (!fl.take(cur, item + gridDim.x < n_items)) continue;
+      const uint32_t d_base = tmem_base + stage * acc_stride;
+      for (int kb = 0; kb < a.k_blocks; ++kb) {
+        const bool is8 = F8 && kb >= a.kb16;     // e4m3 correction blocks follow the fp16 blocks
+        const int nk = is8 ? ((kb == a.k_blocks - 1) ? nk_last8 : (kKElems / 16))
+                           : ((kb == a.kb16 - 1) ? nk_last : (kKElems / 16));
+        mbar_wait(&s.a_full[sa], pa);
         tc_fence_after();
-      }
-      int sa = 0, sb = 0, stage = 0;
-      uint32_t pa = 0, pb = 0, acc_phase = 0;
-      const uint32_t a_ring_addr = smem_u32(a_ring), b_region_addr = smem_u32(b_region);
-      const int nk_last = (a.cin_p - (a.kb16 - 1) * kKElems) / 16;
-      const int nk_last8 = F8 ? (2 * a.cin_p - (a.k_blocks - a.kb16 - 1) * kRowBytes) / 32 : 0;
-      const uint32_t acc_stride = MS * a.acc_cols;
-      ItemCursor cur(blockIdx.x, gridDim.x, a.n_tiles, a.super0);
-      ItemFlags fl(a.flags, cur.super, blockIdx.x < n_items);
-      for (int item = blockIdx.x; item < n_items; item += gridDim.x, cur.next()) {
-        if (!fl.take(cur, item + gridDim.x < n_items)) continue;
-        const uint32_t d_base = tmem_base + stage * acc_stride;
-        for (int kb = 0; kb < a.k_blocks; ++kb) {
-          const bool is8 = F8 && kb >= a.kb16;     // e4m3 correction blocks follow the fp16 blocks
-          const int nk = is8 ? ((kb == a.k_blocks - 1) ? nk_last8 : (kKElems / 16))
-                             : ((kb == a.kb16 - 1) ? nk_last : (kKElems / 16));
-          mbar_wait(&s.a_full[sa], pa);
-          tc_fence_after();
-          const uint32_t a_addr = a_ring_addr + sa * kAGroupBytes;
+        const uint32_t a_addr = a_ring_addr + sa * kAGroupBytes;
 #pragma unroll
-          for (int tap = 0; tap < 3; ++tap) {
+        for (int tap = 0; tap < 3; ++tap) {
 #pragma unroll
-            for (int wp = 0; wp < WPLANES; ++wp) {
-              uint32_t b_addr;
-              if (RESIDENT) {
-                b_addr = b_region_addr + ((wp * 3 + tap) * a.k_blocks + kb) * b_bytes;
-              } else {
-                mbar_wait(&s.b_full[sb], pb);
+          for (int wp = 0; wp < WPLANES; ++wp) {
+            uint32_t b_addr;
+            if (RESIDENT) {
+              b_addr = b_region_addr + ((wp * 3 + tap) * a.k_blocks + kb) * b_bytes;
+            } else {
+              mbar_wait(&s.b_full[sb], pb);
+              tc_fence_after();
+              b_addr = b_region_addr + sb * b_bytes;
+            }
+            const uint64_t db = sw_desc<K32>(b_addr);
+#pragma unroll
+            for (int ms = 0; ms < MS; ++ms) {
+              if (ms < ms_lo || ms >= ms_hi) continue;      // (the other issuer's sub-tile)
+              if (kb == 0 && tap == 0 && wp == 0) {   // first touch of this accumulator: wait until drained
+                mbar_wait(&s.tmem_empty[stage][ms], acc_phase ^ 1);
                 tc_fence_after();
-                b_addr = b_region_addr + sb * b_bytes;
               }
-              const uint64_t db = sw_desc<K32>(b_addr);
 #pragma unroll
-              for (int ms = 0; ms < MS; ++ms) {
-                if (ms < ms_lo || ms >= ms_hi) continue;      // (the other issuer's sub-tile)
-                if (kb == 0 && tap == 0 && wp == 0) {   // first touch of this accumulator: wait until drained
-                  mbar_wait(&s.tmem_empty[stage][ms], acc_phase ^ 1);
-                  tc_fence_after();
-                }
+              for (int ap = 0; ap < (wp == 0 ? PLANES : 1); ++ap) {   // W_lo only meets the hi plane
+                const uint64_t da = sw_desc<K32>(a_addr + (ms * PLANES + ap) * kATile + tap * kRowBytes);
+                if (leader) {      // one elected lane issues; the K steps of a view in one go
 #pragma unroll
-                for (int ap = 0; ap < (wp == 0 ? PLANES : 1); ++ap) {   // W_lo only meets the hi plane
-                  const uint64_t da = sw_desc<K32>(a_addr + (ms * PLANES + ap) * kATile + tap * kRowBytes);
-                  if (leader) {      // one elected lane issues; the K steps of a view in one go
-#pragma unroll
-                    for (int k = 0; k < kKElems / 16; ++k)
-                      if (k < nk && !((RISER_DBG & 64) && (kb | tap | wp | ap | k) != 0)) {
-                        if (is8)
-                          umma_f8(d_base + ms * a.acc_cols, da + 2 * k, db + 2 * k, a.idesc, 1);
-                        else
-                          umma_f16(d_base + ms * a.acc_cols, da + 2 * k, db + 2 * k, a.idesc,
-                                   (kb | tap | wp | ap | k) != 0);
-                      }
-                  }
-                }
-              }
-              if (!RESIDENT) {
-                umma_commit_p(leader, &s.b_empty[sb]);
-                if (++sb == a.b_stages) {
-                  sb = 0;
-                  pb ^= 1;
+                  for (int k = 0; k < kKElems / 16; ++k)
+                    if (k < nk) {
+                      if (is8)
+                        umma_f8(d_base + ms * a.acc_cols, da + 2 * k, db + 2 * k, a.idesc, 1);
+                      else
+                        umma_f16(d_base + ms * a.acc_cols, da + 2 * k, db + 2 * k, a.idesc,
+                                 (kb | tap | wp | ap | k) != 0);
+                    }
                 }
               }
             }
-          }
-          umma_commit_p(leader, &s.a_empty[sa]);
-          if (++sa == a.a_stages) {
-            sa = 0;
-            pa ^= 1;
+            if (!RESIDENT) {
+              umma_commit_p(leader, &s.b_empty[sb]);
+              if (++sb == a.b_stages) {
+                sb = 0;
+                pb ^= 1;
+              }
+            }
           }
         }
+        umma_commit_p(leader, &s.a_empty[sa]);
+        if (++sa == a.a_stages) {
+          sa = 0;
+          pa ^= 1;
+        }
+      }
 #pragma unroll
-        for (int ms = 0; ms < MS; ++ms)
-          if (ms >= ms_lo && ms < ms_hi) umma_commit_p(leader, &s.tmem_full_ms[stage][ms]);
-        if (++stage == a.acc_stages) {
-          stage = 0;
-          acc_phase ^= 1;
-        }
+      for (int ms = 0; ms < MS; ++ms)
+        if (ms >= ms_lo && ms < ms_hi) umma_commit_p(leader, &s.tmem_full_ms[stage][ms]);
+      if (++stage == a.acc_stages) {
+        stage = 0;
+        acc_phase ^= 1;
       }
     }
   } else if (warp < 2 + 4 * a.epi_sets) {
@@ -725,7 +705,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
     }
     int stage = 0, it = -1;
     uint32_t acc_phase = 0;
-    ItemCursor cur(blockIdx.x, gridDim.x, a.n_tiles, a.super0);
+    ItemCursor cur(blockIdx.x, gridDim.x, a.n_tiles);
     ItemFlags fl(a.flags, cur.super, blockIdx.x < n_items);
     for (int item = blockIdx.x; item < n_items; item += gridDim.x, cur.next()) {
       if (!fl.take(cur, item + gridDim.x < n_items)) continue;
@@ -760,7 +740,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
       int u = eset;
 #pragma unroll
       for (int ms = 0; ms < MS; ++ms) {
-        mbar_wait_relaxed(&s.tmem_full_ms[stage][ms], acc_phase);      // this sub-tile's accumulator is complete
+        mbar_wait(&s.tmem_full_ms[stage][ms], acc_phase);      // this sub-tile's accumulator is complete
         tc_fence_after();
         void* orow = a.out_fp32
                          ? static_cast<void*>(static_cast<float*>(a.out) + out_row[ms] * row_elems + n0)
@@ -770,14 +750,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
         for (; u < (ms + 1) * n_chunks; u += a.epi_sets) {
           const int c = u - ms * n_chunks;
           uint32_t v[16];
-          if (RISER_DBG & 256) {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) v[j] = 0u;
-          } else {
-            tmem_ld_32x16(t_addr + c * 16, v);
-          }
+          tmem_ld_32x16(t_addr + c * 16, v);
           tmem_ld_wait();
-          if ((RISER_DBG & 128) && a.Lp_out > 0) continue;
           uint8_t* f8_row = nullptr;
           if (a.out_f8)
             f8_row = static_cast<uint8_t*>(a.out) + out_row[ms] * row_elems * 2 + 2 * a.cout_p + n0;
@@ -862,15 +836,15 @@ ConvKernelFn pick_conv_kernel(int ms, int planes, int wplanes, int resident, int
 //   warps 8..15   mid-epilogue: layer-0 accumulators -> max, ReLU, fp16 hi (+ lo) -> layer-1 A tiles
 //   warps 16..23  epilogue: layer-1 accumulators -> max, bias, ReLU, mask -> act_2 in HBM
 constexpr int kF2Pairs = 255;
-#ifndef RISER_F2_CVT_WARPS
-#define RISER_F2_CVT_WARPS 6
-#endif
-constexpr int kF2Threads = 576 + 32 * RISER_F2_CVT_WARPS;     // producer + issuer + cvt1 + 8 mid-epilogue + 8 epilogue warps
+// cvt1 warps: 257 rows in two passes (two warps were ~100 % busy; with four the issuer still waited on a0_full:
+// 4 -> 6 -> 9 warps 1.04 / 1.01 / 1.00 ms on one box)
+constexpr int kF2CvtWarps = 6;
+constexpr int kF2Threads = 576 + 32 * kF2CvtWarps;     // producer + issuer + cvt1 + 8 mid-epilogue + 8 epilogue warps
 constexpr uint32_t kF2A1Tile = 264 * 64;   // 256 rows + the slack row the shifted taps of row 255 touch
 constexpr uint32_t kF2A0Tile = 256 * 64;   // per row: [E window (K=16) | O window (K=16)]
 constexpr int kF2N0 = 48;
 constexpr int kF2D0Col = 256;              // TMEM: layer-1 accumulators [0,256), layer-0 at 256 + 48*k
-constexpr int kF2CvtThreads = 32 * RISER_F2_CVT_WARPS;     // six cvt1 warps: 257 rows in two passes (two warps were ~100 % busy; with four the issuer still waited on a0_full: 4 -> 6 -> 9 warps 1.04 / 1.01 / 1.00 ms on one box)
+constexpr int kF2CvtThreads = 32 * kF2CvtWarps;
 constexpr int kF2XStages = 4;
 constexpr int kF2MaxLocalItems = 2048;   // work items per CTA whose activity flags fit the shared-memory copy
 constexpr uint32_t kF2XStage = 260 * 16;     // pairs i = -2 .. 256 (4 samples each) + pad
@@ -938,8 +912,7 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
   const int lane = threadIdx.x & 31;
   const int n_items = a.n_supers;
   const int n_pairs = a.rows_in >> 1;
-  const uint8_t* flags0 = a.flags ? a.flags + a.super0 : nullptr;
-  const uint8_t* flags_l = flags0 ? s.my_flags : nullptr;
+  const uint8_t* flags_l = a.flags ? s.my_flags : nullptr;
 
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&tm_b);
@@ -969,9 +942,9 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
   for (uint32_t i = threadIdx.x; i < (2 * kF2A0Tile + 2 * kA1Stage + kF2XStages * kF2XStage) / 16; i += kF2Threads)
     reinterpret_cast<uint4*>(a0_ring)[i] = make_uint4(0, 0, 0, 0);
   if (threadIdx.x < 32) s.bias[threadIdx.x] = a.bias[threadIdx.x];
-  if (flags0)
+  if (a.flags)
     for (int i = threadIdx.x, it = blockIdx.x + threadIdx.x * gridDim.x; it < n_items; i += kF2Threads, it += kF2Threads * gridDim.x)
-      s.my_flags[i] = flags0[it];
+      s.my_flags[i] = a.flags[it];
   if (threadIdx.x < kF2N0) {
     // layer-0 B operand, row n: channel n % 24 at conv position 2p + n / 24 (SWIZZLE_64B rows)
     const int n = threadIdx.x, c = n % 24, odd = n / 24;
@@ -1030,7 +1003,7 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
         const int st = k % kF2XStages;
         mbar_wait(&s.x_empty[st], ((k / kF2XStages) & 1) ^ 1);
         unsigned char* dst = x_ring + st * kF2XStage;
-        long long u_lo = static_cast<long long>(a.super0 + item) * kF2Pairs - 2;
+        long long u_lo = static_cast<long long>(item) * kF2Pairs - 2;
         long long u_hi = u_lo + 258;                            // inclusive
         const int i_lo = (u_lo < 0) ? static_cast<int>(-u_lo) - 2 : -2;
         if (u_lo < 0) u_lo = 0;
@@ -1060,112 +1033,109 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     // (the whole warp runs the loop so that the descriptor arithmetic stays in uniform registers; the elected lane issues)
-    const bool leader = RISER_UNIFORM_ISSUE ? elect_one() : (lane == 0);
-    if (RISER_UNIFORM_ISSUE || lane == 0) {
-      mbar_wait(&s.w_full, 0);
+    const bool leader = elect_one();
+    mbar_wait(&s.w_full, 0);
+    tc_fence_after();
+    const uint32_t w1_addr = smem_u32(w1), b0_addr = smem_u32(b0);
+    const uint32_t a0_addr = smem_u32(a0_ring), a1_addr = smem_u32(a1_ring);
+    const uint32_t idesc0 = umma_idesc_f16(kBlockM, kF2N0);
+    const uint32_t idesc64 = umma_idesc_f16(kBlockM, 64);
+    const uint64_t db0 = sw_desc<true>(b0_addr);
+    F2Iter iter(flags_l, n_items);
+    int k0 = 0;                       // items whose layer 0 has been issued
+    auto issue_layer0 = [&]() {
+      const int st = k0 & 1;
+      mbar_wait(&s.a0_full[st], (k0 >> 1) & 1);
       tc_fence_after();
-      const uint32_t w1_addr = smem_u32(w1), b0_addr = smem_u32(b0);
-      const uint32_t a0_addr = smem_u32(a0_ring), a1_addr = smem_u32(a1_ring);
-      const uint32_t idesc0 = umma_idesc_f16(kBlockM, kF2N0);
-      const uint32_t idesc64 = umma_idesc_f16(kBlockM, 64);
-      const uint64_t db0 = sw_desc<true>(b0_addr);
-      F2Iter iter(flags_l, n_items);
-      int k0 = 0;                       // items whose layer 0 has been issued
-      auto issue_layer0 = [&]() {
-        const int st = k0 & 1;
-        mbar_wait(&s.a0_full[st], (k0 >> 1) & 1);
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        mbar_wait(&s.d0_empty[h], (k0 & 1) ^ 1);
         tc_fence_after();
+        if (leader) {
 #pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          mbar_wait(&s.d0_empty[h], (k0 & 1) ^ 1);
-          tc_fence_after();
-          if (leader) {
-#pragma unroll
-            for (int sub = 0; sub < 2; ++sub)
-              umma_f16(tmem_base + kF2D0Col + (h * 2 + sub) * kF2N0,
-                       sw_desc<true>(a0_addr + st * kF2A0Tile + sub * 128 * 64) + 2 * h, db0, idesc0, 0);
-          }
-          umma_commit_p(leader, &s.d0_full[h]);
+          for (int sub = 0; sub < 2; ++sub)
+            umma_f16(tmem_base + kF2D0Col + (h * 2 + sub) * kF2N0,
+                     sw_desc<true>(a0_addr + st * kF2A0Tile + sub * 128 * 64) + 2 * h, db0, idesc0, 0);
         }
-        umma_commit_p(leader, &s.a0_empty[st]);
-        ++k0;
-      };
-      int cur = iter.take();
-      if (cur >= 0) issue_layer0();
-      int k1 = 0;                       // items whose layer 1 has been issued
-      while (cur >= 0) {
-        const int nxt = iter.take();
-        if (nxt >= 0) issue_layer0();
-        const int st = k1 & 1;
-        mbar_wait(&s.a1_full[st], (k1 >> 1) & 1);
-        tc_fence_after();
-        const uint32_t a1s = a1_addr + st * kA1Stage;
-#pragma unroll
-        for (int sub = 0; sub < 2; ++sub) {
-          mbar_wait(&s.d1_empty[st][sub], ((k1 >> 1) & 1) ^ 1);
-          tc_fence_after();
-        }
-        // even position 2j: w0*O[j-1] + w1*E[j] + w2*O[j];  odd position 2j+1: w0*E[j] + w1*O[j] + w2*E[j+1]
-        // (tile rows: E[j] = E row j, O[j] = O row j + 1; weight slot of tap t = 2 - t).
-        // Consecutive MMAs go to DIFFERENT accumulators (sub-tile x parity, round-robin): back-to-back
-        // MMAs into the same TMEM tile serialise on the accumulator (~80 cycles each at N = 32).
-        auto issue_group = [&](uint32_t a_tiles, uint32_t w_set, bool f8, bool first) {
-          if (!leader) return;
-#pragma unroll
-          for (int tap = 0; tap < 3; ++tap) {
-#pragma unroll
-            for (int k = 0; k < 2; ++k) {
-              const uint64_t db = sw_desc<true>(w_set + (2 - tap) * 2048) + 2 * k;
-#pragma unroll
-              for (int sub = 0; sub < 2; ++sub) {
-#pragma unroll
-                for (int pe = 0; pe < 2; ++pe) {
-                  const int par = (pe == 0) ? ((tap == 1) ? 0 : 1) : ((tap == 1) ? 1 : 0);
-                  const int shift = (pe == 0) ? ((tap == 2) ? 1 : 0) : ((tap == 0) ? 0 : 1);
-                  const uint64_t da = sw_desc<true>(a_tiles + par * kF2A1Tile + (sub * 128 + shift) * 64) + 2 * k;
-                  const uint32_t d = tmem_base + st * 128 + (2 * sub + pe) * 32;
-                  if ((RISER_DBG & 1) && !(first && tap == 0 && k == 0)) continue;
-                  if (f8) umma_f8(d, da, db, a.idesc, 1);
-                  else umma_f16(d, da, db, a.idesc, !(first && tap == 0 && k == 0));
-                }
-              }
-            }
-          }
-        };
-        if (KC) {
-          // one 64-channel K block per tap set: 4 K steps x 4 MMAs per sub-tile (E tile at a1s, O tile behind it;
-          // rows of 128 bytes; weight slots [w2; w1; w0] of 4 KB)
-          if (leader) {
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const uint64_t w21 = sw_desc<false>(w1_addr) + 2 * k;
-              const uint64_t w10 = sw_desc<false>(w1_addr + 4096) + 2 * k;
-              const uint64_t w0 = sw_desc<false>(w1_addr + 8192) + 2 * k;
-#pragma unroll
-              for (int sub = 0; sub < 2; ++sub) {
-                const uint32_t e_rows = a1s + sub * 128 * 128, o_rows = e_rows + 2 * kF2A1Tile;
-                const uint32_t d_even = tmem_base + st * 128 + 2 * sub * 32, d_odd = d_even + 32;
-                umma_f16(d_even, sw_desc<false>(e_rows) + 2 * k, w10, idesc64, k != 0);      // E[j]   -> (even | odd)
-                umma_f16(d_even, sw_desc<false>(o_rows + 128) + 2 * k, w21, idesc64, 1);     // O[j]   -> (even | odd)
-                umma_f16(d_even, sw_desc<false>(o_rows) + 2 * k, w0, a.idesc, 1);            // O[j-1] -> even
-                umma_f16(d_odd, sw_desc<false>(e_rows + 128) + 2 * k, w21, a.idesc, 1);      // E[j+1] x w2 -> odd
-              }
-            }
-          }
-        } else {
-#pragma unroll
-        for (int wp = 0; wp < WPLANES; ++wp)
-#pragma unroll
-          for (int ap = 0; ap < ((wp == 0 && !F8) ? PLANES : 1); ++ap)
-            issue_group(a1s + ap * 2 * kF2A1Tile, w1_addr + wp * 3 * 2048, false, wp == 0 && ap == 0);
-        }
-        if (F8)   // correction pass: [a8 | lo8] x [W_lo * 2^3 | W * 2^-9], 64 e4m3 per row = 2 k-steps
-          issue_group(a1s + 2 * kF2A1Tile, w1_addr + 3 * 2048, true, false);
-        umma_commit_p(leader, &s.a1_empty[st]);
-        umma_commit_p(leader, &s.d1_full[st]);
-        ++k1;
-        cur = nxt;
+        umma_commit_p(leader, &s.d0_full[h]);
       }
+      umma_commit_p(leader, &s.a0_empty[st]);
+      ++k0;
+    };
+    int cur = iter.take();
+    if (cur >= 0) issue_layer0();
+    int k1 = 0;                       // items whose layer 1 has been issued
+    while (cur >= 0) {
+      const int nxt = iter.take();
+      if (nxt >= 0) issue_layer0();
+      const int st = k1 & 1;
+      mbar_wait(&s.a1_full[st], (k1 >> 1) & 1);
+      tc_fence_after();
+      const uint32_t a1s = a1_addr + st * kA1Stage;
+#pragma unroll
+      for (int sub = 0; sub < 2; ++sub) {
+        mbar_wait(&s.d1_empty[st][sub], ((k1 >> 1) & 1) ^ 1);
+        tc_fence_after();
+      }
+      // even position 2j: w0*O[j-1] + w1*E[j] + w2*O[j];  odd position 2j+1: w0*E[j] + w1*O[j] + w2*E[j+1]
+      // (tile rows: E[j] = E row j, O[j] = O row j + 1; weight slot of tap t = 2 - t).
+      // Consecutive MMAs go to DIFFERENT accumulators (sub-tile x parity, round-robin): back-to-back
+      // MMAs into the same TMEM tile serialise on the accumulator (~80 cycles each at N = 32).
+      auto issue_group = [&](uint32_t a_tiles, uint32_t w_set, bool f8, bool first) {
+        if (!leader) return;
+#pragma unroll
+        for (int tap = 0; tap < 3; ++tap) {
+#pragma unroll
+          for (int k = 0; k < 2; ++k) {
+            const uint64_t db = sw_desc<true>(w_set + (2 - tap) * 2048) + 2 * k;
+#pragma unroll
+            for (int sub = 0; sub < 2; ++sub) {
+#pragma unroll
+              for (int pe = 0; pe < 2; ++pe) {
+                const int par = (pe == 0) ? ((tap == 1) ? 0 : 1) : ((tap == 1) ? 1 : 0);
+                const int shift = (pe == 0) ? ((tap == 2) ? 1 : 0) : ((tap == 0) ? 0 : 1);
+                const uint64_t da = sw_desc<true>(a_tiles + par * kF2A1Tile + (sub * 128 + shift) * 64) + 2 * k;
+                const uint32_t d = tmem_base + st * 128 + (2 * sub + pe) * 32;
+                if (f8) umma_f8(d, da, db, a.idesc, 1);
+                else umma_f16(d, da, db, a.idesc, !(first && tap == 0 && k == 0));
+              }
+            }
+          }
+        }
+      };
+      if (KC) {
+        // one 64-channel K block per tap set: 4 K steps x 4 MMAs per sub-tile (E tile at a1s, O tile behind it;
+        // rows of 128 bytes; weight slots [w2; w1; w0] of 4 KB)
+        if (leader) {
+#pragma unroll
+          for (int k = 0; k < 4; ++k) {
+            const uint64_t w21 = sw_desc<false>(w1_addr) + 2 * k;
+            const uint64_t w10 = sw_desc<false>(w1_addr + 4096) + 2 * k;
+            const uint64_t w0 = sw_desc<false>(w1_addr + 8192) + 2 * k;
+#pragma unroll
+            for (int sub = 0; sub < 2; ++sub) {
+              const uint32_t e_rows = a1s + sub * 128 * 128, o_rows = e_rows + 2 * kF2A1Tile;
+              const uint32_t d_even = tmem_base + st * 128 + 2 * sub * 32, d_odd = d_even + 32;
+              umma_f16(d_even, sw_desc<false>(e_rows) + 2 * k, w10, idesc64, k != 0);      // E[j]   -> (even | odd)
+              umma_f16(d_even, sw_desc<false>(o_rows + 128) + 2 * k, w21, idesc64, 1);     // O[j]   -> (even | odd)
+              umma_f16(d_even, sw_desc<false>(o_rows) + 2 * k, w0, a.idesc, 1);            // O[j-1] -> even
+              umma_f16(d_odd, sw_desc<false>(e_rows + 128) + 2 * k, w21, a.idesc, 1);      // E[j+1] x w2 -> odd
+            }
+          }
+        }
+      } else {
+#pragma unroll
+      for (int wp = 0; wp < WPLANES; ++wp)
+#pragma unroll
+        for (int ap = 0; ap < ((wp == 0 && !F8) ? PLANES : 1); ++ap)
+          issue_group(a1s + ap * 2 * kF2A1Tile, w1_addr + wp * 3 * 2048, false, wp == 0 && ap == 0);
+      }
+      if (F8)   // correction pass: [a8 | lo8] x [W_lo * 2^3 | W * 2^-9], 64 e4m3 per row = 2 k-steps
+        issue_group(a1s + 2 * kF2A1Tile, w1_addr + 3 * 2048, true, false);
+      umma_commit_p(leader, &s.a1_empty[st]);
+      umma_commit_p(leader, &s.d1_full[st]);
+      ++k1;
+      cur = nxt;
     }
   } else if (warp < 2 + kF2CvtThreads / 32) {
     // ===================== cvt1: signal -> layer-0 A rows =====================
@@ -1176,12 +1146,12 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
     for (int item = iter.take(); item >= 0; item = iter.take(), ++k) {
       const int st = k & 1;
       const int xst = k % kF2XStages;
-      mbar_wait_relaxed(&s.x_full[xst], (k / kF2XStages) & 1);
-      mbar_wait_relaxed(&s.a0_empty[st], ((k >> 1) & 1) ^ 1);
+      mbar_wait(&s.x_full[xst], (k / kF2XStages) & 1);
+      mbar_wait(&s.a0_empty[st], ((k >> 1) & 1) ^ 1);
       unsigned char* tile = a0_ring + st * kF2A0Tile;
       const float* xs = reinterpret_cast<const float*>(x_ring + xst * kF2XStage) + 8;   // xs[4*i + e]
-      const long long u0 = static_cast<long long>(a.super0 + item) * kF2Pairs;
-      for (int i = ct - 1; i <= 255 && !(RISER_DBG & 32); i += kF2CvtThreads) {
+      const long long u0 = static_cast<long long>(item) * kF2Pairs;
+      for (int i = ct - 1; i <= 255; i += kF2CvtThreads) {
         const long long u = u0 + i;
         const bool inb = (u >= 0 && u < n_pairs);
         const uint32_t uu = inb ? static_cast<uint32_t>(u) : 0u;
@@ -1246,25 +1216,17 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
     int k = 0;
     for (int item = iter.take(); item >= 0; item = iter.take(), ++k) {
       const int st = k & 1;
-      mbar_wait_relaxed(&s.a1_empty[st], ((k >> 1) & 1) ^ 1);
-      mbar_wait_relaxed(&s.d0_full[h], k & 1);
+      mbar_wait(&s.a1_empty[st], ((k >> 1) & 1) ^ 1);
+      mbar_wait(&s.d0_full[h], k & 1);
       tc_fence_after();
       unsigned char* tile_hi = a1_ring + st * kA1Stage + h * kF2A1Tile;
 #pragma unroll
       for (int sub = 0; sub < 2; ++sub) {
         const uint32_t taddr = tmem_base + (static_cast<uint32_t>(32 * q) << 16) + kF2D0Col + (h * 2 + sub) * kF2N0;
         uint32_t e0[16], e1[8], o0[16], o1[8];
-        if (RISER_DBG & 4) {
-#pragma unroll
-          for (int j = 0; j < 16; ++j) e0[j] = o0[j] = 0u;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) e1[j] = o1[j] = 0u;
-        } else {
         tmem_ld_32x16(taddr, e0);
         tmem_ld_32x16(taddr + 24, o0);
-        }
-        if (RISER_DBG & 4) {
-        } else if (a.cout0 > 20) {        // TMEM reads are 64 B/clk per SM: do not fetch the zero columns
+        if (a.cout0 > 20) {        // TMEM reads are 64 B/clk per SM: do not fetch the zero columns
           tmem_ld_32x8(taddr + 16, e1);
           tmem_ld_32x8(taddr + 40, o1);
         } else {
@@ -1279,7 +1241,6 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
           __syncwarp();
           if (lane == 0) mbar_arrive(&s.d0_empty[h]);
         }
-        if (RISER_DBG & 16) continue;
         const int row = sub * 128 + 32 * q + lane;
         unsigned char* rp = tile_hi + row * 64;
         const int sw = (row >> 1) & 3;
@@ -1364,7 +1325,7 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
     for (int item = iter.take(); item >= 0; item = iter.take(), ++k) {
       const int st = k & 1;
       const int j = sub * 128 + 32 * q + lane;
-      const long long u = static_cast<long long>(a.super0 + item) * kF2Pairs + j;
+      const long long u = static_cast<long long>(item) * kF2Pairs + j;
       const bool ok = (j < kF2Pairs) && (u < n_pairs);
       const uint32_t uu = ok ? static_cast<uint32_t>(u) : 0u;
       const int b = static_cast<int>((static_cast<unsigned long long>(uu) * a.pair_magic) >> 40);
@@ -1374,12 +1335,12 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
       const int64_t out_row = a.out_eo ? static_cast<int64_t>(tp & 1) * a.n_pairs_out + static_cast<int64_t>(b) * a.half_lp_out + (tp >> 1)
                                        : static_cast<int64_t>(b) * a.Lp_out + tp;
       __half* orow = static_cast<__half*>(a.out) + out_row * row_elems;
-      mbar_wait_relaxed(&s.d1_full[st], (k >> 1) & 1);
+      mbar_wait(&s.d1_full[st], (k >> 1) & 1);
       tc_fence_after();
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(32 * q) << 16) + st * 128 + 2 * sub * 32;
       // m[c] = max of the two conv positions of a pool pair (accumulator units); bias, ReLU, mask, fp16 hi + lo, stores
       auto finish = [&](int c16, const float (&m)[16]) {
-        if (!(writable && !((RISER_DBG & 2) && a.Lp_out > 0))) return;
+        if (!writable) return;
         float r[16];
         if (valid) {
 #pragma unroll
@@ -1419,25 +1380,15 @@ fused01_kernel(const __grid_constant__ CUtensorMap tm_b, const __grid_constant__
       float m0[16];
       {
         uint32_t ve[16], vo[16];
-        if (RISER_DBG & 8) {
-#pragma unroll
-          for (int j = 0; j < 16; ++j) ve[j] = vo[j] = 0u;
-        } else {
-          tmem_ld_32x16(taddr, ve);
-          tmem_ld_32x16(taddr + 32, vo);
-        }
+        tmem_ld_32x16(taddr, ve);
+        tmem_ld_32x16(taddr + 32, vo);
         tmem_ld_wait();
 #pragma unroll
         for (int j = 0; j < 16; ++j) m0[j] = fmaxf(__uint_as_float(ve[j]), __uint_as_float(vo[j]));
       }
       uint32_t ve1[16], vo1[16];
-      if (RISER_DBG & 8) {
-#pragma unroll
-        for (int j = 0; j < 16; ++j) ve1[j] = vo1[j] = 0u;
-      } else {
-        tmem_ld_32x16(taddr + 16, ve1);
-        tmem_ld_32x16(taddr + 32 + 16, vo1);
-      }
+      tmem_ld_32x16(taddr + 16, ve1);
+      tmem_ld_32x16(taddr + 32 + 16, vo1);
       finish(0, m0);
       tmem_ld_wait();
       tc_fence_before();
@@ -1541,7 +1492,7 @@ conv_eo_kernel(const __grid_constant__ CUtensorMap tm_e, const __grid_constant__
                         &s.w_full, kb * 32, (wp * 3 + tap) * a.cout_p);
       int sa = 0;
       uint32_t pa = 0;
-      ItemCursor cur(blockIdx.x, gridDim.x, 1, a.super0);
+      ItemCursor cur(blockIdx.x, gridDim.x, 1);
       ItemFlags fl(a.flags, cur.super, blockIdx.x < n_items);
       for (int item = blockIdx.x; item < n_items; item += gridDim.x, cur.next()) {
         if (!fl.take(cur, item + gridDim.x < n_items)) continue;
@@ -1555,11 +1506,7 @@ conv_eo_kernel(const __grid_constant__ CUtensorMap tm_e, const __grid_constant__
 #pragma unroll
             for (int ap = 0; ap < PLANES; ++ap) {
               unsigned char* t = dst + (ms * PLANES + ap) * 2 * kEoTile;
-#ifdef RISER_DBG_TRAFFIC   // timing experiment (wrong results): the lo plane is read from the hi plane's bytes
-              const int apc = 0;
-#else
               const int apc = ap * a.cin_p;
-#endif
               tma_load_2d(t, &tm_e, &s.a_full[sa], apc + kb * 32, u0 + ms * kBlockM);              // E[j ..]
               tma_load_2d(t + kEoTile, &tm_o, &s.a_full[sa], apc + kb * 32, u0 + ms * kBlockM - 1);  // O[j-1 ..]
             }
@@ -1573,66 +1520,64 @@ conv_eo_kernel(const __grid_constant__ CUtensorMap tm_e, const __grid_constant__
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     // (the whole warp runs the loop so that the descriptor arithmetic stays in uniform registers; the elected lane issues)
-    const bool leader = RISER_UNIFORM_ISSUE ? elect_one() : (lane == 0);
-    if (RISER_UNIFORM_ISSUE || lane == 0) {
-      mbar_wait(&s.w_full, 0);
-      tc_fence_after();
-      int sa = 0, stage = 0;
-      uint32_t pa = 0, acc_phase = 0;
-      const uint32_t a_ring_addr = smem_u32(a_ring), b_region_addr = smem_u32(b_region);
-      const int nk_last = (a.cin_p - (a.k_blocks - 1) * 32) / 16;
-      const uint32_t idesc1 = a.idesc;                                  // N = n_tile
-      const uint32_t idesc2 = umma_idesc_f16(kBlockM, 2 * a.n_tile);    // N = 2 n_tile: (even | odd)
-      ItemCursor cur(blockIdx.x, gridDim.x, 1, a.super0);
-      ItemFlags fl(a.flags, cur.super, blockIdx.x < n_items);
-      for (int item = blockIdx.x; item < n_items; item += gridDim.x, cur.next()) {
-        if (!fl.take(cur, item + gridDim.x < n_items)) continue;
-        const uint32_t d_base = tmem_base + stage * (MS * acc2);
-        for (int kb = 0; kb < a.k_blocks; ++kb) {
-          const int nk = (kb == a.k_blocks - 1) ? nk_last : 2;
-          mbar_wait(&s.a_full[sa], pa);
-          tc_fence_after();
-          const uint32_t a_addr = a_ring_addr + sa * kGroup;
+    const bool leader = elect_one();
+    mbar_wait(&s.w_full, 0);
+    tc_fence_after();
+    int sa = 0, stage = 0;
+    uint32_t pa = 0, acc_phase = 0;
+    const uint32_t a_ring_addr = smem_u32(a_ring), b_region_addr = smem_u32(b_region);
+    const int nk_last = (a.cin_p - (a.k_blocks - 1) * 32) / 16;
+    const uint32_t idesc1 = a.idesc;                                  // N = n_tile
+    const uint32_t idesc2 = umma_idesc_f16(kBlockM, 2 * a.n_tile);    // N = 2 n_tile: (even | odd)
+    ItemCursor cur(blockIdx.x, gridDim.x, 1);
+    ItemFlags fl(a.flags, cur.super, blockIdx.x < n_items);
+    for (int item = blockIdx.x; item < n_items; item += gridDim.x, cur.next()) {
+      if (!fl.take(cur, item + gridDim.x < n_items)) continue;
+      const uint32_t d_base = tmem_base + stage * (MS * acc2);
+      for (int kb = 0; kb < a.k_blocks; ++kb) {
+        const int nk = (kb == a.k_blocks - 1) ? nk_last : 2;
+        mbar_wait(&s.a_full[sa], pa);
+        tc_fence_after();
+        const uint32_t a_addr = a_ring_addr + sa * kGroup;
 #pragma unroll
-          for (int wp = 0; wp < WPLANES; ++wp) {
-            const uint32_t w_set = b_region_addr + ((wp * a.k_blocks + kb) * 3) * b_bytes;   // slots: w2, w1, w0
+        for (int wp = 0; wp < WPLANES; ++wp) {
+          const uint32_t w_set = b_region_addr + ((wp * a.k_blocks + kb) * 3) * b_bytes;   // slots: w2, w1, w0
 #pragma unroll
-            for (int ms = 0; ms < MS; ++ms) {
-              if (kb == 0 && wp == 0) {      // first touch of this accumulator: wait until drained
-                mbar_wait(&s.tmem_empty[stage][ms], acc_phase ^ 1);
-                tc_fence_after();
-              }
-              const uint32_t d_even = d_base + ms * acc2, d_odd = d_even + a.n_tile;
+          for (int ms = 0; ms < MS; ++ms) {
+            if (kb == 0 && wp == 0) {      // first touch of this accumulator: wait until drained
+              mbar_wait(&s.tmem_empty[stage][ms], acc_phase ^ 1);
+              tc_fence_after();
+            }
+            const uint32_t d_even = d_base + ms * acc2, d_odd = d_even + a.n_tile;
 #pragma unroll
-              for (int ap = 0; ap < (wp == 0 ? PLANES : 1); ++ap) {      // W_lo only meets the hi plane
-                const uint32_t e_rows = a_addr + (ms * PLANES + ap) * 2 * kEoTile, o_rows = e_rows + kEoTile;
-                if (leader) {
+            for (int ap = 0; ap < (wp == 0 ? PLANES : 1); ++ap) {      // W_lo only meets the hi plane
+              const uint32_t e_rows = a_addr + (ms * PLANES + ap) * 2 * kEoTile, o_rows = e_rows + kEoTile;
+              if (leader) {
 #pragma unroll
-                  for (int k = 0; k < 2; ++k)
-                    if (k < nk) {
-                      const uint64_t w21 = sw_desc<true>(w_set) + 2 * k;
-                      const uint64_t w10 = sw_desc<true>(w_set + b_bytes) + 2 * k;
-                      const uint64_t w0 = sw_desc<true>(w_set + 2 * b_bytes) + 2 * k;
-                      umma_f16(d_even, sw_desc<true>(e_rows) + 2 * k, w10, idesc2, (kb | wp | ap | k) != 0);   // E[j]
-                      umma_f16(d_even, sw_desc<true>(o_rows + 64) + 2 * k, w21, idesc2, 1);                    // O[j]
-                      umma_f16(d_even, sw_desc<true>(o_rows) + 2 * k, w0, idesc1, 1);                          // O[j-1]
-                      umma_f16(d_odd, sw_desc<true>(e_rows + 64) + 2 * k, w21, idesc1, 1);                     // E[j+1] x w2
-                    }
-                }
+                for (int k = 0; k < 2; ++k)
+                  if (k < nk) {
+                    const uint64_t w21 = sw_desc<true>(w_set) + 2 * k;
+                    const uint64_t w10 = sw_desc<true>(w_set + b_bytes) + 2 * k;
+                    const uint64_t w0 = sw_desc<true>(w_set + 2 * b_bytes) + 2 * k;
+                    umma_f16(d_even, sw_desc<true>(e_rows) + 2 * k, w10, idesc2, (kb | wp | ap | k) != 0);   // E[j]
+                    umma_f16(d_even, sw_desc<true>(o_rows + 64) + 2 * k, w21, idesc2, 1);                    // O[j]
+                    umma_f16(d_even, sw_desc<true>(o_rows) + 2 * k, w0, idesc1, 1);                          // O[j-1]
+                    umma_f16(d_odd, sw_desc<true>(e_rows + 64) + 2 * k, w21, idesc1, 1);                     // E[j+1] x w2
+                  }
               }
             }
           }
-          umma_commit_p(leader, &s.a_empty[sa]);
-          if (++sa == a.a_stages) {
-            sa = 0;
-            pa ^= 1;
-          }
         }
-        umma_commit_p(leader, &s.tmem_full[stage]);
-        if (++stage == a.acc_stages) {
-          stage = 0;
-          acc_phase ^= 1;
+        umma_commit_p(leader, &s.a_empty[sa]);
+        if (++sa == a.a_stages) {
+          sa = 0;
+          pa ^= 1;
         }
+      }
+      umma_commit_p(leader, &s.tmem_full[stage]);
+      if (++stage == a.acc_stages) {
+        stage = 0;
+        acc_phase ^= 1;
       }
     }
   } else if (warp < 2 + 4 * a.epi_sets) {
@@ -1649,7 +1594,7 @@ conv_eo_kernel(const __grid_constant__ CUtensorMap tm_e, const __grid_constant__
     asm volatile("bar.sync 1, %0;" ::"r"(epi_threads) : "memory");
     int stage = 0;
     uint32_t acc_phase = 0;
-    ItemCursor cur(blockIdx.x, gridDim.x, 1, a.super0);
+    ItemCursor cur(blockIdx.x, gridDim.x, 1);
     ItemFlags fl(a.flags, cur.super, blockIdx.x < n_items);
     for (int item = blockIdx.x; item < n_items; item += gridDim.x, cur.next()) {
       if (!fl.take(cur, item + gridDim.x < n_items)) continue;
@@ -1670,7 +1615,7 @@ conv_eo_kernel(const __grid_constant__ CUtensorMap tm_e, const __grid_constant__
                                  : static_cast<int64_t>(b) * a.Lp_out + tp;
         }
       }
-      mbar_wait_relaxed(&s.tmem_full[stage], acc_phase);
+      mbar_wait(&s.tmem_full[stage], acc_phase);
       tc_fence_after();
       int uw = eset;       // work units = (sub-tile, 16-column chunk), dealt round-robin to the epilogue sets
 #pragma unroll
@@ -1966,9 +1911,9 @@ conv_eo2_kernel(const __grid_constant__ CUtensorMap tm_e, const __grid_constant_
       const int sw = (idx >> 1) & 3;
       unsigned char* row0 = a3 + static_cast<size_t>(eo) * kEoTile + idx * 64;
       const uint32_t qq = 2 * k + t, slot = qq % 3;
-      mbar_wait_relaxed(&s.acc1_full[slot], (qq / 3) & 1);
+      mbar_wait(&s.acc1_full[slot], (qq / 3) & 1);
       tc_fence_after();
-      mbar_wait_relaxed(&s.a3_empty, (k & 1) ^ 1);          // the second layer of the previous item has read the tiles
+      mbar_wait(&s.a3_empty, (k & 1) ^ 1);          // the second layer of the previous item has read the tiles
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(32 * q4) << 16) + slot * a.acc1;
       for (int c = 0; c < n_chunks; ++c) {
         uint32_t ve[16], vo[16];
@@ -2039,7 +1984,7 @@ conv_eo2_kernel(const __grid_constant__ CUtensorMap tm_e, const __grid_constant_
       const int64_t out_row = a.out_eo ? static_cast<int64_t>(j & 1) * a.n_pairs_out + static_cast<int64_t>(b) * a.half_lp_out + (j >> 1)
                                        : static_cast<int64_t>(b) * a.Lp_out + j;
       __half* orow = static_cast<__half*>(a.out) + out_row * row_elems;
-      mbar_wait_relaxed(&s.acc2_full, k & 1);
+      mbar_wait(&s.acc2_full, k & 1);
       tc_fence_after();
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(32 * q4) << 16) + 3 * a.acc1;
       for (int c = eset; c < n_chunks; c += 2) {
@@ -2084,9 +2029,8 @@ size_t conv_eo2_smem(int n1, int n2, int kb1, int kb2) {
 // (cp.async.bulk.tensor ... cta_group::2 with the peer bit cleared), tcgen05.commit multicasts the
 // "empty" / "accumulator full" arrivals to both CTAs, and the peer's epilogue warps release the
 // accumulators on the leader's barrier (mapa + remote arrive).
-// Work item of a pair = (MS sub-tiles of 256 flat rows, N tile); both CTAs walk the same item list.
-template <int MS>
-__global__ void __launch_bounds__(96 + 128 * kMaxEpiSets, 1)
+// Work item of a pair = (256 flat rows, N tile); both CTAs walk the same item list.
+__global__ void __launch_bounds__(64 + 128 * kMaxEpiSets, 1)
 conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
                  const __grid_constant__ CUtensorMap tm_a8, const __grid_constant__ CUtensorMap tm_b8,
                  const __grid_constant__ CUtensorMap tm_bl, const __grid_constant__ CUtensorMap tm_b8l,
@@ -2094,10 +2038,9 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* base = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
   constexpr uint32_t kATile = 136 * 128;
-  constexpr uint32_t kAGroup = MS * kATile;
   const uint32_t b_bytes = (a.n_tile / 2) * 128;           // this CTA's half of a (full-width) weight tile
   unsigned char* a_ring = base;
-  unsigned char* b_region = base + static_cast<size_t>(a.a_stages) * kAGroup;
+  unsigned char* b_region = base + static_cast<size_t>(a.a_stages) * kATile;
   // (`resident`: one N tile whose halves fit -- every CTA keeps ITS half of all taps and K blocks for the whole kernel,
   //  [tap][K block][n_tile / 2 rows x 128 B], and nothing but activations is streamed: layer 5)
   const size_t b_region_bytes = a.resident ? static_cast<size_t>(3) * a.k_blocks * b_bytes : static_cast<size_t>(a.b_stages) * b_bytes;
@@ -2117,21 +2060,18 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
     tma_prefetch_desc(&tm_b8);
     tma_prefetch_desc(&tm_bl);
     tma_prefetch_desc(&tm_b8l);
-    const uint32_t n_issuers = a.dual ? 2 : 1;     // every issuer's commit arrives on the operand "empty" barriers
     for (int i = 0; i < a.a_stages; ++i) {
       mbar_init(&s.a_full[i], 1);
-      mbar_init(&s.a_empty[i], n_issuers);
+      mbar_init(&s.a_empty[i], 1);
     }
     for (int i = 0; i < a.b_stages; ++i) {
       mbar_init(&s.b_full[i], 1);
-      mbar_init(&s.b_empty[i], n_issuers);
+      mbar_init(&s.b_empty[i], 1);
     }
     mbar_init(&s.w_full, 1);
     for (int i = 0; i < a.acc_stages; ++i) {
-      for (int ms = 0; ms < MS; ++ms) {
-        mbar_init(&s.tmem_full_ms[i][ms], 1);
-        mbar_init(&s.tmem_empty[i][ms], 2 * 4 * a.epi_sets);   // both CTAs' warps
-      }
+      mbar_init(&s.tmem_full[i], 1);
+      mbar_init(&s.tmem_empty[i][0], 2 * 4 * a.epi_sets);   // both CTAs' warps
     }
     fence_mbar_init();
   }
@@ -2154,7 +2094,6 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
     if (a.n_tiles == 1) return x;
     return a.nt_magic ? static_cast<int>(__umulhi(static_cast<uint32_t>(x), a.nt_magic)) : x / a.n_tiles;
   };
-  auto item_super = [&](int item) { return a.super0 + div_nt(item); };
   auto item_n = [&](int item) {
     const int q = div_nt(item), t = item - q * a.n_tiles + q;          // item % n_tiles + item / n_tiles
     return t - div_nt(t) * a.n_tiles;
@@ -2163,15 +2102,15 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
   // (a global load per item otherwise sits on the critical path of the single-thread roles).
   struct PairFlags {
     const uint8_t* flags;
-    int n_tiles, super0, stride, n_items;
+    int n_tiles, stride, n_items;
     uint32_t next;
     uint32_t magic;
     __device__ __forceinline__ uint32_t load(int item) const {
       const int q = (n_tiles == 1) ? item : magic ? static_cast<int>(__umulhi(static_cast<uint32_t>(item), magic)) : item / n_tiles;
-      return (flags && item < n_items) ? __ldg(flags + super0 + q) : 1u;
+      return (flags && item < n_items) ? __ldg(flags + q) : 1u;
     }
-    __device__ __forceinline__ PairFlags(const uint8_t* f, int nt, int s0, int first, int stride_, int n, uint32_t mg = 0)
-        : flags(f), n_tiles(nt), super0(s0), stride(stride_), n_items(n), magic(mg) { next = load(first); }
+    __device__ __forceinline__ PairFlags(const uint8_t* f, int nt, int first, int stride_, int n, uint32_t mg = 0)
+        : flags(f), n_tiles(nt), stride(stride_), n_items(n), magic(mg) { next = load(first); }
     __device__ __forceinline__ bool take(int item) {      // call once per item, in order
       const uint32_t now = next;
       next = load(item + stride);
@@ -2194,10 +2133,10 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
       }
       int sa = 0, sb = 0;
       uint32_t pa = 0, pb = 0;
-      PairFlags fl(a.flags, a.n_tiles, a.super0, pair, n_pairs_grid, n_items, a.nt_magic);
+      PairFlags fl(a.flags, a.n_tiles, pair, n_pairs_grid, n_items, a.nt_magic);
       for (int item = pair; item < n_items; item += n_pairs_grid) {
         if (!fl.take(item)) continue;
-        const int m0 = item_super(item) * (MS * 256) + static_cast<int>(rank) * kBlockM - 1;
+        const int m0 = div_nt(item) * 256 + static_cast<int>(rank) * kBlockM - 1;
         const int n_idx = item_n(item);
         const bool last_n = (n_idx == a.n_tiles - 1);
         const int n_half = (last_n ? a.n_last : a.n_tile) / 2;       // weight rows this CTA stages per tile
@@ -2208,20 +2147,12 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
         for (int kb = 0; kb < a.k_blocks; ++kb) {
           const bool is8 = kb >= a.kb16;
           mbar_wait(&s.a_empty[sa], pa ^ 1);
-          if (a.dbg_skip & 2) {
-            if (leader) mbar_arrive(&s.a_full[sa]);
-          } else if (leader) {
-            mbar_arrive_expect_tx(&s.a_full[sa], 2 * MS * kATile);
-          }
-          unsigned char* dst = a_ring + static_cast<size_t>(sa) * kAGroup;
-#pragma unroll
-          for (int ms = 0; ms < MS; ++ms) {
-            if (a.dbg_skip & 2) break;
-            if (is8)
-              tma_load_2d_pair(dst + ms * kATile, &tm_a8, &s.a_full[sa], 2 * a.cin_p + (kb - a.kb16) * 128, m0 + ms * 256);
-            else
-              tma_load_2d_pair(dst + ms * kATile, &tm_a, &s.a_full[sa], kb * 64, m0 + ms * 256);
-          }
+          if (leader) mbar_arrive_expect_tx(&s.a_full[sa], 2 * kATile);
+          unsigned char* dst = a_ring + static_cast<size_t>(sa) * kATile;
+          if (is8)
+            tma_load_2d_pair(dst, &tm_a8, &s.a_full[sa], 2 * a.cin_p + (kb - a.kb16) * 128, m0);
+          else
+            tma_load_2d_pair(dst, &tm_a, &s.a_full[sa], kb * 64, m0);
           if (++sa == a.a_stages) {
             sa = 0;
             pa ^= 1;
@@ -2230,17 +2161,13 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
           for (int tap = 0; tap < 3; ++tap) {
             if (a.resident) break;
             mbar_wait(&s.b_empty[sb], pb ^ 1);
-            if (a.dbg_skip & 1) {
-              if (leader) mbar_arrive(&s.b_full[sb]);
-            } else {
-              if (leader) mbar_arrive_expect_tx(&s.b_full[sb], 2 * b_tx);
-              if (is8)
-                tma_load_2d_pair(b_region + static_cast<size_t>(sb) * b_bytes, tb8, &s.b_full[sb], (kb - a.kb16) * 128,
-                                 tap * a.cout_p + n0);
-              else
-                tma_load_2d_pair(b_region + static_cast<size_t>(sb) * b_bytes, tb, &s.b_full[sb], kb * 64,
-                                 tap * a.cout_p + n0);
-            }
+            if (leader) mbar_arrive_expect_tx(&s.b_full[sb], 2 * b_tx);
+            if (is8)
+              tma_load_2d_pair(b_region + static_cast<size_t>(sb) * b_bytes, tb8, &s.b_full[sb], (kb - a.kb16) * 128,
+                               tap * a.cout_p + n0);
+            else
+              tma_load_2d_pair(b_region + static_cast<size_t>(sb) * b_bytes, tb, &s.b_full[sb], kb * 64,
+                               tap * a.cout_p + n0);
             if (++sb == a.b_stages) {
               sb = 0;
               pb ^= 1;
@@ -2249,38 +2176,31 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
         }
       }
     }
-  } else if (warp == 1 || (a.dual && warp == 2 + 4 * a.epi_sets)) {
-    // ===================== MMA issuer(s) (leader CTA only) =====================
-    // One warp issues every MMA of an item -- or, `dual` (MS == 2), one warp PER SUB-TILE: with 2 x 256 accumulator
-    // columns the TMEM holds one item, so a single issuer would idle for the whole drain of both sub-tiles; the two
-    // issuers walk the same operand stages on their own (both commit to the "empty" barriers), and the one whose
-    // accumulator is still being drained falls a few weight tiles behind while the other keeps the tensor pipe busy.
+  } else if (warp == 1) {
+    // ===================== MMA issuer (leader CTA only) =====================
     // (The whole warp runs the loop -- uniform registers, see umma_f16_p -- and the elected lane issues.)
     if (leader) {
-      const int ms_lo = a.dual ? (warp == 1 ? 0 : 1) : 0;
-      const int ms_hi = a.dual ? ms_lo + 1 : MS;
       const uint32_t lead = elect_one() ? 1u : 0u;
       int sa = 0, sb = 0, stage = 0;
       uint32_t pa = 0, pb = 0, acc_phase = 0;
       const uint32_t a_ring_addr = smem_u32(a_ring), b_region_addr = smem_u32(b_region);
       const int nk_last = (a.cin_p - (a.kb16 - 1) * 64) / 16;
       const int nk_last8 = (2 * a.cin_p - (a.k_blocks - a.kb16 - 1) * 128) / 32;
-      const uint32_t acc_stride = MS * a.acc_cols;
       if (a.resident) {
         mbar_wait(&s.w_full, 0);
         tc_fence_after();
       }
-      PairFlags fl(a.flags, a.n_tiles, a.super0, pair, n_pairs_grid, n_items, a.nt_magic);
+      PairFlags fl(a.flags, a.n_tiles, pair, n_pairs_grid, n_items, a.nt_magic);
       for (int item = pair; item < n_items; item += n_pairs_grid) {
         if (!fl.take(item)) continue;
-        const uint32_t d_base = tmem_base + stage * acc_stride;
+        const uint32_t d = tmem_base + stage * a.acc_cols;
         const uint32_t idesc = (item_n(item) == a.n_tiles - 1) ? a.idesc_last : a.idesc;
         for (int kb = 0; kb < a.k_blocks; ++kb) {
           const bool is8 = kb >= a.kb16;
           const int nk = is8 ? ((kb == a.k_blocks - 1) ? nk_last8 : 4) : ((kb == a.kb16 - 1) ? nk_last : 4);
           mbar_wait(&s.a_full[sa], pa);
           tc_fence_after();
-          const uint32_t a_addr = a_ring_addr + sa * kAGroup;
+          const uint32_t a_addr = a_ring_addr + sa * kATile;
 #pragma unroll
           for (int tap = 0; tap < 3; ++tap) {
             if (!a.resident) {
@@ -2289,21 +2209,17 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
             }
             const uint64_t db = sw_desc<false>(a.resident ? b_region_addr + (tap * a.k_blocks + kb) * b_bytes
                                                           : b_region_addr + sb * b_bytes);
-#pragma unroll
-            for (int ms = 0; ms < MS; ++ms) {
-              if (ms < ms_lo || ms >= ms_hi) continue;      // (the other issuer's sub-tile)
-              if (kb == 0 && tap == 0) {       // first touch of this accumulator: both CTAs have drained it
-                mbar_wait(&s.tmem_empty[stage][ms], acc_phase ^ 1);
-                tc_fence_after();
-              }
-              const uint64_t da = sw_desc<false>(a_addr + ms * kATile + tap * 128);
-#pragma unroll
-              for (int k = 0; k < 4; ++k)
-                if (k < nk) {
-                  if (is8) umma_f8_pair_p(lead, d_base + ms * a.acc_cols, da + 2 * k, db + 2 * k, idesc, 1);
-                  else umma_f16_pair_p(lead, d_base + ms * a.acc_cols, da + 2 * k, db + 2 * k, idesc, (kb | tap | k) != 0);
-                }
+            if (kb == 0 && tap == 0) {       // first touch of this accumulator: both CTAs have drained it
+              mbar_wait(&s.tmem_empty[stage][0], acc_phase ^ 1);
+              tc_fence_after();
             }
+            const uint64_t da = sw_desc<false>(a_addr + tap * 128);
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+              if (k < nk) {
+                if (is8) umma_f8_pair_p(lead, d, da + 2 * k, db + 2 * k, idesc, 1);
+                else umma_f16_pair_p(lead, d, da + 2 * k, db + 2 * k, idesc, (kb | tap | k) != 0);
+              }
             if (!a.resident) {
               umma_commit_pair_p(lead, &s.b_empty[sb]);
               if (++sb == a.b_stages) {
@@ -2318,9 +2234,7 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
             pa ^= 1;
           }
         }
-#pragma unroll
-        for (int ms = 0; ms < MS; ++ms)
-          if (ms >= ms_lo && ms < ms_hi) umma_commit_pair_p(lead, &s.tmem_full_ms[stage][ms]);
+        umma_commit_pair_p(lead, &s.tmem_full[stage]);
         if (++stage == a.acc_stages) {
           stage = 0;
           acc_phase ^= 1;
@@ -2338,11 +2252,11 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
     const int lo_off = (a.out_planes == 2 && !a.out_f8) ? a.cout_p : 0;
     int stage = 0, it = -1;
     uint32_t acc_phase = 0;
-    PairFlags fl(a.flags, a.n_tiles, a.super0, pair, n_pairs_grid, n_items, a.nt_magic);
+    PairFlags fl(a.flags, a.n_tiles, pair, n_pairs_grid, n_items, a.nt_magic);
     for (int item = pair; item < n_items; item += n_pairs_grid) {
       if (!fl.take(item)) continue;
       ++it;
-      const int m0 = item_super(item) * (MS * 256) + static_cast<int>(rank) * kBlockM;
+      const int m0 = div_nt(item) * 256 + static_cast<int>(rank) * kBlockM;
       const int n_idx = item_n(item);
       const int n_cur = (n_idx == a.n_tiles - 1) ? a.n_last : a.n_tile;
       const int n_chunks = n_cur >> 4;
@@ -2350,46 +2264,34 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
       float* bias_s = s.bias[it & 1];
       for (int i = et; i < n_cur; i += epi_threads) bias_s[i] = a.bias[n0 + i];
       asm volatile("bar.sync 1, %0;" ::"r"(epi_threads) : "memory");
-      bool valid[MS], writable[MS];
-      int64_t out_row[MS];
-#pragma unroll
-      for (int ms = 0; ms < MS; ++ms) {
-        valid[ms] = writable[ms] = false;
-        out_row[ms] = 0;
-        const int r_even = (m0 + ms * 256 + 32 * q + lane) & ~1;
-        if (r_even < a.rows_in) {
-          const uint32_t pidx = static_cast<uint32_t>(r_even) >> 1;
-          const int b = static_cast<int>((static_cast<unsigned long long>(pidx) * a.pair_magic) >> 40);
-          const int tp = static_cast<int>(pidx) - b * a.half_lp;
-          valid[ms] = tp < (__ldg(a.len0 + b) >> a.shift);
-          writable[ms] = tp < a.Lp_out;
-          out_row[ms] = static_cast<int64_t>(b) * a.Lp_out + tp;
-        }
+      bool valid = false, writable = false;
+      int64_t out_row = 0;
+      const int r_even = (m0 + 32 * q + lane) & ~1;
+      if (r_even < a.rows_in) {
+        const uint32_t pidx = static_cast<uint32_t>(r_even) >> 1;
+        const int b = static_cast<int>((static_cast<unsigned long long>(pidx) * a.pair_magic) >> 40);
+        const int tp = static_cast<int>(pidx) - b * a.half_lp;
+        valid = tp < (__ldg(a.len0 + b) >> a.shift);
+        writable = tp < a.Lp_out;
+        out_row = static_cast<int64_t>(b) * a.Lp_out + tp;
       }
-      int u = eset;
-#pragma unroll
-      for (int ms = 0; ms < MS; ++ms) {
-        mbar_wait_relaxed(&s.tmem_full_ms[stage][ms], acc_phase);      // this sub-tile's accumulator is complete
-        tc_fence_after();
-        void* orow = a.out_fp32
-                         ? static_cast<void*>(static_cast<float*>(a.out) + out_row[ms] * row_elems + n0)
-                         : static_cast<void*>(static_cast<__half*>(a.out) + out_row[ms] * row_elems + n0);
-        const uint32_t t_addr = tmem_base + (static_cast<uint32_t>(32 * q) << 16) + (stage * MS + ms) * a.acc_cols;
-        for (; u < (ms + 1) * n_chunks; u += a.epi_sets) {
-          const int c = u - ms * n_chunks;
-          uint32_t v[16];
-          tmem_ld_32x16(t_addr + c * 16, v);
-          tmem_ld_wait();
-          uint8_t* f8_row = nullptr;
-          if (a.out_f8)
-            f8_row = static_cast<uint8_t*>(a.out) + out_row[ms] * row_elems * 2 + 2 * a.cout_p + n0;
-          epilogue_chunk16(v, bias_s, c * 16, odd, valid[ms], writable[ms], orow, a.out_fp32, lo_off,
-                           a.w_inv_scale, f8_row, a.cout_p);
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_remote_relaxed(&s.tmem_empty[stage][ms], 0);   // on the leader's barrier
+      mbar_wait(&s.tmem_full[stage], acc_phase);      // the accumulator is complete
+      tc_fence_after();
+      void* orow = a.out_fp32 ? static_cast<void*>(static_cast<float*>(a.out) + out_row * row_elems + n0)
+                              : static_cast<void*>(static_cast<__half*>(a.out) + out_row * row_elems + n0);
+      const uint32_t t_addr = tmem_base + (static_cast<uint32_t>(32 * q) << 16) + stage * a.acc_cols;
+      for (int c = eset; c < n_chunks; c += a.epi_sets) {
+        uint32_t v[16];
+        tmem_ld_32x16(t_addr + c * 16, v);
+        tmem_ld_wait();
+        uint8_t* f8_row = nullptr;
+        if (a.out_f8) f8_row = static_cast<uint8_t*>(a.out) + out_row * row_elems * 2 + 2 * a.cout_p + n0;
+        epilogue_chunk16(v, bias_s, c * 16, odd, valid, writable, orow, a.out_fp32, lo_off, a.w_inv_scale, f8_row,
+                         a.cout_p);
       }
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive_remote_relaxed(&s.tmem_empty[stage][0], 0);   // on the leader's barrier
       if (++stage == a.acc_stages) {
         stage = 0;
         acc_phase ^= 1;
@@ -2405,8 +2307,6 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
     tmem_dealloc_pair(tmem_base, kTmemCols);
   }
 }
-
-PairKernelFn pick_conv_pair(int ms) { return ms == 2 ? conv_pair_kernel<2> : conv_pair_kernel<1>; }
 
 // ------------------------------------------------------------------------------------
 // Per-layer activity flags of the M super-tiles: a super-tile is active when at least one of
@@ -2740,17 +2640,12 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
   RISER_REQUIRE(B > 0 && max_len >= kMinLen, "riser_plan_create: need B > 0 and max_len >= %d", kMinLen);
   RISER_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "riser_plan_create: workspace not 256-byte aligned");
   // These switches exist so that the test suite can reach, on the shipped network, the kernels that other shapes
-  // select on their own.  RISER_PAIR_DBG_SKIP is a timing experiment (wrong results).
+  // select on their own.
   const bool fuse_l0 = env_int("RISER_FUSE_L0", 1) != 0;
   const bool eo_on = env_int("RISER_EO", 1) != 0;
   const bool pair_on = env_int("RISER_PAIR", 1) != 0;
-  const int pair_ms = env_int("RISER_PAIR_MS", 1);
-  const int pair_from = env_int("RISER_PAIR_FROM", 6);
-  const int pair_ntile = env_int("RISER_PAIR_NTILE", kMaxNTile);
-  const bool dual_issue = env_int("RISER_DUAL_ISSUE", 1) != 0;
   const bool kc_on = env_int("RISER_KC", 1) != 0;
   const bool fuse23 = env_int("RISER_FUSE23", 1) != 0;
-  const int pair_dbg_skip = env_int("RISER_PAIR_DBG_SKIP", 0);
   std::unique_ptr<riser_plan, int (*)(riser_plan*)> owner(new riser_plan(), riser_plan_destroy);   // freed on every error return
   riser_plan* p = owner.get();
   p->model = m;
@@ -2872,7 +2767,7 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
       lp.smem = fixed + static_cast<size_t>(a.a_stages) * a_group + static_cast<size_t>(a.b_stages) * b_bytes;
     }
     a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / (a.ms * a.acc_cols)));
-    a.dual = (a.ms == 2 && !a.resident && dual_issue) ? 1 : 0;
+    a.dual = (a.ms == 2 && !a.resident) ? 1 : 0;
     a.epi_sets = kMaxEpiSets;
     lp.rows_per_super = a.ms * kBlockM;
     bool kc = false;
@@ -2911,15 +2806,17 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
       lp.smem = fixed + w_eo + static_cast<size_t>(a.a_stages) * a.ms * group1;
       lp.rows_per_super = a.ms * 2 * kBlockM;
     }
+    // CTA pairs take the streamed-weight F16_F8 layers from layer kPairFrom on, and earlier ones (layer 5 of the shipped
+    // network) only when each CTA's half of the weights stays resident
+    constexpr int kPairFrom = 6;
     if (L.f8 && !a.resident && !k32 && !lp.eo && (L.n_tile % 16) == 0 && pair_on &&
-        (i >= pair_from ||
+        (i >= kPairFrom ||
          (L.n_tiles == 1 && static_cast<size_t>(3) * a.k_blocks * (L.cout_p / 2) * 128 + 3 * 136 * 128 <= avail))) {
       // conv_pair_kernel: M = 256 over two CTAs, each holds 128 rows of A and half of every weight tile
       // N tiles of the pair kernel: 256 wide (the widest M = 256 MMA: fewest shared-memory operand bytes per MAC)
       // with ONE narrower last tile instead of equal tiles -- cout_p itself (the next layer's K) is unchanged
       lp.kind = kPairKernel;
-      const int wide = std::max(64, std::min(kMaxNTile, pair_ntile) & ~15);
-      a.n_tile = std::min(wide, L.cout_p);
+      a.n_tile = std::min(kMaxNTile, L.cout_p);
       a.n_tiles = (L.cout_p + a.n_tile - 1) / a.n_tile;
       a.n_last = L.cout_p - (a.n_tiles - 1) * a.n_tile;
       a.acc_cols = round_up(a.n_tile, 32);
@@ -2932,16 +2829,15 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
       a.idesc_last = umma_idesc_f16(256, a.n_last);
       // One 256-row sub-tile per item and two accumulator stages is the measured optimum (layers 6-11 in situ: 0.38 /
       // 0.47 / 0.37 / 0.38 / 0.46 / 0.49 ms against 0.41 / 0.47 / 0.40 / 0.43 / 0.48 / 0.55 with two sub-tiles, which
-      // halve the weight bytes streamed per MAC but leave the TMEM one item deep; `dual` then gives each sub-tile its
-      // own issuing warp so that one computes while the other is drained -- RISER_PAIR_MS=2 keeps that variant testable).
-      a.ms = (2 * a.acc_cols <= kTmemCols && pair_ms >= 2) ? 2 : 1;
-      const size_t a_group = static_cast<size_t>(a.ms) * 136 * 128, half_b = static_cast<size_t>(a.n_tile / 2) * 128;
-      a.a_stages = a.ms == 2 ? 3 : 5;
+      // halve the weight bytes streamed per MAC but leave the TMEM one item deep, even with one issuing warp per
+      // sub-tile).
+      a.ms = 1;
+      const size_t a_group = static_cast<size_t>(136) * 128, half_b = static_cast<size_t>(a.n_tile / 2) * 128;
+      a.a_stages = 5;
       while (a.a_stages > 2 && a.a_stages * a_group + 4 * half_b > avail) --a.a_stages;
       a.b_stages = std::max(2, std::min<int>(kMaxBStages, static_cast<int>((avail - a.a_stages * a_group) / half_b)));
-      a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / (a.ms * a.acc_cols)));
-      a.dual = (a.ms == 2 && dual_issue) ? 1 : 0;
-      a.dbg_skip = pair_dbg_skip;
+      a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / a.acc_cols));
+      a.dual = 0;
       a.resident = 0;
       size_t b_total = a.b_stages * half_b;
       const size_t w_half = static_cast<size_t>(3) * a.k_blocks * half_b;      // this CTA's half of every tap and K block
@@ -2954,7 +2850,7 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
       // item / n_tiles by multiply-high; with one N tile the magic would overflow, and the kernel divides instead
       a.nt_magic = a.n_tiles > 1 ? static_cast<uint32_t>((1ull << 32) / static_cast<unsigned>(a.n_tiles)) + 1u : 0u;
       lp.smem = fixed + a.a_stages * a_group + b_total;
-      lp.rows_per_super = a.ms * 256;
+      lp.rows_per_super = 256;
     }
     // every launch covers the whole batch
     a.n_supers = (rows_in + lp.rows_per_super - 1) / lp.rows_per_super;
@@ -2973,9 +2869,9 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
         fn = reinterpret_cast<const void*>(lp.fn.eo);
         break;
       case kPairKernel:
-        lp.fn.pair = pick_conv_pair(a.ms);
+        lp.fn.pair = conv_pair_kernel;
         lp.grid = std::min(2 * n_items, m->sm_count & ~1);
-        lp.block = 64 + 128 * a.epi_sets + (a.dual ? 32 : 0);
+        lp.block = 64 + 128 * a.epi_sets;
         fn = reinterpret_cast<const void*>(lp.fn.pair);
         break;
       default:

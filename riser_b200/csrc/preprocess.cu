@@ -25,14 +25,14 @@ constexpr int kSubBins = 128;           // refinement pass (shift <= 7)
 constexpr int kMaxLen = 98304;          // samples staged in smem (192 KB)
 constexpr int kMaxRuns = 512;           // outlier-run start indices collected per read (more: rescan path)
 
-constexpr int kDefaultF64 = 1;            // samples per group of four on the float64 pipe (RISER_NORM_F64; 0 / 1 / 4: 0.1106 / 0.1085 / 0.1085 ms)
+constexpr int kDefaultF64 = 1;          // samples per group of four on the float64 pipe (0 / 1 / 4: 0.1106 / 0.1085 / 0.1085 ms)
 
 constexpr double kOutlierLimit = 3.5;   // riser/preprocess.py:6
 constexpr double kScalingFactor = 1.4826;  // riser/preprocess.py:7
 
 struct SelectScratch {
-  uint64_t bar[2];      // one mbarrier per staging buffer (bulk-copy completion)
-  uint32_t hist[kBins];
+  uint64_t bar;         // bulk-copy completion of the staging buffer
+  alignas(16) uint32_t hist[kBins];
   uint32_t sub[kSubBins];
   uint32_t warp_sums[kWarps];
   uint32_t res[4];      // bin1, before1, bin2, before2
@@ -213,8 +213,8 @@ __device__ __forceinline__ double clip_outlier(double v) {
 
 // Kernel structure (one CTA per read, persistent over reads b = blockIdx.x, + gridDim.x, ...):
 //   stage    one 1-D bulk copy (cp.async.bulk, mbarrier complete_tx) of the 16-byte blocks that hold the
-//            window; with two staging buffers the copy of the CTA's NEXT read is issued before the
-//            current one is processed, so the global-load latency is off the critical path
+//            window; the CTA's NEXT read is prefetched into L2 while the current one is processed, so its
+//            copy is an L2 hit
 //   min/max  packed 16-bit min / max over the staged chunks
 //   median   histogram radix select (select_two); MAD from the same histogram by a warp-wide
 //            32-ary search on the distance (or a second select when the range needed a shift)
@@ -225,29 +225,28 @@ __global__ void __launch_bounds__(kThreads, 5)
 normalise_kernel(const int16_t* __restrict__ sig, const int64_t* __restrict__ off,
                  const int32_t* __restrict__ start, const int32_t* __restrict__ len, int B,
                  float* __restrict__ out, int64_t ld_out, int32_t* __restrict__ med2_mad4,
-                 int nbuf, int buf_samples, int max_len, int dbg) {
+                 int max_len) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   SelectScratch& s = *reinterpret_cast<SelectScratch*>(smem_raw);
-  int16_t* stage_base = reinterpret_cast<int16_t*>(smem_raw + ((sizeof(SelectScratch) + 127) & ~size_t(127)));
+  int16_t* stage = reinterpret_cast<int16_t*>(smem_raw + ((sizeof(SelectScratch) + 127) & ~size_t(127)));
   const int tid = threadIdx.x;
   const int lane = tid & 31, warp = tid >> 5;
 
   if (tid == 0) {
-    mbar_init(&s.bar[0], 1);
-    mbar_init(&s.bar[1], 1);
+    mbar_init(&s.bar, 1);
     fence_mbar_init();
   }
   __syncthreads();
-  // thread 0: bulk copy of a window of nr samples at gr (whole 16-byte blocks) into staging buffer `buf`
-  auto issue = [&](int nr, const int16_t* gr, int buf) {
+  // thread 0: bulk copy of a window of nr samples at gr (whole 16-byte blocks) into the staging buffer
+  auto issue = [&](int nr, const int16_t* gr) {
     if (nr <= 0) return;
     const int ar = static_cast<int>((reinterpret_cast<uintptr_t>(gr) >> 1) & 7);
     const uint32_t bytes = static_cast<uint32_t>(((ar + nr + 7) >> 3) << 4);
-    mbar_arrive_expect_tx(&s.bar[buf], bytes);
-    bulk_load_1d(stage_base + static_cast<size_t>(buf) * buf_samples, gr - ar, bytes, &s.bar[buf]);
+    mbar_arrive_expect_tx(&s.bar, bytes);
+    bulk_load_1d(stage, gr - ar, bytes, &s.bar);
   };
-  // one staging buffer: the NEXT read's blocks are pulled into L2 while this one is processed, so that its
-  // copy at the top of the next iteration is an L2 hit and the HBM reads spread over the compute phases
+  // the NEXT read's blocks are pulled into L2 while this one is processed, so that its copy at the top of the
+  // next iteration is an L2 hit and the HBM reads spread over the compute phases
   auto prefetch = [&](int nr, const int16_t* gr) {
     if (nr <= 0) return;
     const int ar = static_cast<int>((reinterpret_cast<uintptr_t>(gr) >> 1) & 7);
@@ -266,28 +265,22 @@ normalise_kernel(const int16_t* __restrict__ sig, const int64_t* __restrict__ of
   int n_cur, n_nxt;
   const int16_t *g_cur, *g_nxt;
   meta(blockIdx.x, n_cur, g_cur);
-  if (nbuf == 2 && tid == 0) issue(n_cur, g_cur, 0);
-  uint32_t phase_bits = 0;             // bit `buf` = parity the next wait on bar[buf] uses
+  uint32_t phase = 0;                  // parity the next wait on bar uses
 
-  int it = 0;
-  for (int b = blockIdx.x; b < B; b += gridDim.x, ++it, n_cur = n_nxt, g_cur = g_nxt) {
-    const int buf = (nbuf == 2) ? (it & 1) : 0;
-    if (tid == 0 && nbuf == 1) issue(n_cur, g_cur, 0);
+  for (int b = blockIdx.x; b < B; b += gridDim.x, n_cur = n_nxt, g_cur = g_nxt) {
+    if (tid == 0) issue(n_cur, g_cur);
     meta(b + gridDim.x, n_nxt, g_nxt);
-    if (tid == 0) {
-      if (nbuf == 2) issue(n_nxt, g_nxt, buf ^ 1); else prefetch(n_nxt, g_nxt);
-    }
+    if (tid == 0) prefetch(n_nxt, g_nxt);
     const int n = n_cur;
     if (n <= 0) continue;                 // block-uniform; nothing was issued for this read
     const int16_t* g = g_cur;
     float* o = out + static_cast<int64_t>(b) * ld_out;
     const int a = static_cast<int>((reinterpret_cast<uintptr_t>(g) >> 1) & 7);
-    const int16_t* stage = stage_base + static_cast<size_t>(buf) * buf_samples;
     const StagedWindow x{stage, a, n};     // x[i] == g[i]
     // (the value histogram of the fused pass below is cleared while the read's copy is in flight)
     for (int i = tid; i < kBins / 4; i += kThreads) reinterpret_cast<uint4*>(s.hist)[i] = make_uint4(0u, 0u, 0u, 0u);
-    mbar_wait(&s.bar[buf], (phase_bits >> buf) & 1u);
-    phase_bits ^= 1u << buf;
+    mbar_wait(&s.bar, phase);
+    phase ^= 1u;
     __syncthreads();
 
     // ---- min / max of the window AND its value histogram in one pass over the staged chunks: a sample is counted in
@@ -429,8 +422,7 @@ normalise_kernel(const int16_t* __restrict__ sig, const int64_t* __restrict__ of
       // and the float64 pipe is what bounds this kernel: when the value range fits the histogram, the fp32 result
       // of every VALUE is tabulated once (in the histogram's storage, free after the MAD search) and the per-sample
       // work becomes one shared-memory look-up.
-      const int n_f64 = dbg & 7;            // samples of every group of four whose quotient is computed, not looked up
-      const bool use_lut = (shift_used == 0) && n_f64 < 4;
+      const bool use_lut = (shift_used == 0);
       float* lut = reinterpret_cast<float*>(s.hist);
       if (use_lut)
         for (int u = tid; u <= range; u += kThreads)      // (circular by VALUE: the entry of sample value v sits at v & (kBins - 1))
@@ -585,10 +577,9 @@ normalise_kernel(const int16_t* __restrict__ sig, const int64_t* __restrict__ of
           asm volatile("ld.shared.f32 %0, [%1];" : "=f"(f) : "r"(lut_addr + (static_cast<uint32_t>(x4) & (4u * (kBins - 1)))));
           return f;
         };
-        if (n_f64 == 2) dispatch(std::integral_constant<int, 2>{}, lut_value, lut_x4);
-        else if (n_f64 == 1) dispatch(std::integral_constant<int, 1>{}, lut_value, lut_x4);
-        else if (n_f64 == 3) dispatch(std::integral_constant<int, 3>{}, lut_value, lut_x4);
-        else dispatch(std::integral_constant<int, 0>{}, lut_value, lut_x4);
+        // kDefaultF64 of every group of four samples take their quotient from the float64 pipe rather than the table
+        // (same results: the table's bank conflicts load the LSU pipe, which then bounds the kernel)
+        dispatch(std::integral_constant<int, kDefaultF64>{}, lut_value, lut_x4);
       } else {
         dispatch(std::integral_constant<int, 4>{}, f64_value, f64_x4);
       }
@@ -1044,19 +1035,12 @@ extern "C" int riser_normalise(const int16_t* sig, const int64_t* off, const int
                 max_len, kMaxLen);
   RISER_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0 && (ld_out & 3) == 0 && ld_out >= max_len,
                 "riser_normalise: out must be 16-byte aligned, ld_out a multiple of 4 and >= max_len");
-  // staging buffers of whole 16-byte blocks: window + up to 7 samples of phase + tail block, 128-byte pitch
+  // staging buffer of whole 16-byte blocks: window + up to 7 samples of phase + tail block, 128-byte pitch
   const int buf_samples = (max_len + 16 + 63) & ~63;
   const size_t scratch = (sizeof(SelectScratch) + 127) & ~size_t(127);
-  static int nbuf_env = -1;
-  if (nbuf_env < 0) {
-    const char* e = getenv("RISER_NORM_NBUF");
-    nbuf_env = e ? atoi(e) : 0;
-  }
-  // One staging buffer + L2 prefetch of the next read by default: a second buffer (RISER_NORM_NBUF=2, the next
-  // read's copy in flight during this read's work) costs a resident CTA per SM and measured slower.
-  int nbuf = (nbuf_env == 2) ? 2 : 1;
-  if (scratch + 2 * static_cast<size_t>(nbuf) * buf_samples > 227 * 1024) nbuf = 1;
-  const size_t smem = scratch + 2 * static_cast<size_t>(nbuf) * buf_samples;
+  // One staging buffer + L2 prefetch of the next read: a second buffer (the next read's copy in flight during this
+  // read's work) costs a resident CTA per SM and measured slower.
+  const size_t smem = scratch + 2 * static_cast<size_t>(buf_samples);
   static size_t configured[64] = {0};   // per device
   int dev = 0;
   RISER_CUDA_TRY(cudaGetDevice(&dev));
@@ -1068,20 +1052,9 @@ extern "C" int riser_normalise(const int16_t* sig, const int64_t* off, const int
   int per_sm = 0;
   RISER_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, normalise_kernel, kThreads, smem));
   if (per_sm < 1) per_sm = 1;
-  // RISER_NORM_CTAS caps the resident CTAs per SM (timing experiments); RISER_NORM_F64 = 0..4 sets how many samples
-  // of every group of four take their quotient from the float64 pipe instead of the per-value look-up table in
-  // shared memory (same results; the table's bank conflicts load the LSU pipe that bounds the kernel, 4 = no table)
-  static int ctas_env = -1, dbg = 0;
-  if (ctas_env < 0) {
-    const char* e = getenv("RISER_NORM_CTAS");
-    ctas_env = e ? atoi(e) : 0;
-    e = getenv("RISER_NORM_F64");
-    dbg = e ? std::max(0, std::min(4, atoi(e))) : kDefaultF64;
-  }
-  if (ctas_env > 0) per_sm = std::min(per_sm, ctas_env);
   const int grid = std::min(B, sm_count() * per_sm);
   normalise_kernel<<<grid, kThreads, smem, as_stream(stream)>>>(sig, off, start, len, B, out, ld_out,
-                                                               med2_mad4, nbuf, buf_samples, max_len, dbg);
+                                                               med2_mad4, max_len);
   RISER_CUDA_TRY(cudaGetLastError());
   return RISER_OK;
 }

@@ -244,50 +244,8 @@ __device__ __forceinline__ int list_term(RtMma* list, int n_list, uint32_t d_col
   return n_list;
 }
 
-// The same MMAs issued from a warp-uniform loop nest (the whole warp runs it, the descriptor arithmetic stays in uniform
-// registers, the elected lane executes the instructions): no shared-memory list, no R2UR per operand.
-#ifndef RISER_RT_REPLAY
-#define RISER_RT_REPLAY 1      // measured: the replayed list 1.009 ms, the uniform loop nest 1.045 ms (512 x 12,048, basic)
-#endif
-template <int P>
-__device__ __forceinline__ void issue_term_uniform(bool leader, uint32_t d, uint32_t a_hi, uint32_t a_lo, uint32_t w_base,
-                                                   int tap, int n_kb, int k_ch, int n, bool cat, uint32_t idesc_n,
-                                                   uint32_t idesc_2n, uint32_t& acc) {
-  for (int kb = 0; kb < n_kb; ++kb) {
-    const int nk = min(2, (k_ch - 32 * kb + 15) >> 4);
-    const uint32_t wt = w_tile<P>(w_base, tap, kb, n_kb, n);
-    const uint64_t ah0 = rt_desc(a_hi + kb * kRtTile), al0 = rt_desc(a_lo + kb * kRtTile);
-    const uint64_t wh0 = rt_desc(wt), wl0 = rt_desc(wt + n * 64);
-    if (leader) {
-#pragma unroll
-      for (int k = 0; k < 2; ++k)
-        if (k < nk) {
-          const uint32_t a0 = (k == 0) ? acc : 1u;
-          if (P == kPrecX3) {
-            if (cat) {
-              umma_f16(d, ah0 + 2 * k, wh0 + 2 * k, idesc_2n, a0);
-              umma_f16(d, al0 + 2 * k, wh0 + 2 * k, idesc_n, 1u);
-            } else {
-              umma_f16(d, ah0 + 2 * k, wh0 + 2 * k, idesc_n, a0);
-              umma_f16(d, al0 + 2 * k, wh0 + 2 * k, idesc_n, 1u);
-              umma_f16(d, ah0 + 2 * k, wl0 + 2 * k, idesc_n, 1u);
-            }
-          } else if (P == kPrecW2) {
-            umma_f16(d, ah0 + 2 * k, wh0 + 2 * k, cat ? idesc_2n : idesc_n, a0);
-            if (!cat) umma_f16(d, ah0 + 2 * k, wl0 + 2 * k, idesc_n, 1u);
-          } else {
-            umma_f16(d, ah0 + 2 * k, wh0 + 2 * k, idesc_n, a0);
-          }
-        }
-      if (P == kPrecF8) {
-#pragma unroll
-        for (int k = 0; k < 2; ++k) umma_f8(d, al0 + 2 * k, wl0 + 2 * k, idesc_n, 1u);
-      }
-    }
-    acc = 1u;
-  }
-}
-
+// One thread replays the list: measured 1.009 ms against 1.045 ms for the same MMAs issued from a warp-uniform loop
+// nest (512 x 12,048, basic).
 template <int P>
 __device__ __forceinline__ void replay(const RtMma* list, int n, uint32_t tmem_base) {
 #pragma unroll 4
@@ -297,23 +255,6 @@ __device__ __forceinline__ void replay(const RtMma* list, int n, uint32_t tmem_b
       umma_f8(tmem_base + e.d_col, e.da, e.db, e.idesc, e.acc);
     else
       umma_f16(tmem_base + e.d_col, e.da, e.db, e.idesc, e.acc);
-  }
-}
-
-// The CTA waits for an mbarrier phase: ONE thread polls it, the others park at the hardware barrier (256 threads
-// spinning on try_wait took an eighth of the kernel's issue slots from the co-resident CTAs that had work to do).
-#ifndef RISER_RT_CTAWAIT
-#define RISER_RT_CTAWAIT 0
-#endif
-#ifndef RISER_RT_RES_GLOBAL
-#define RISER_RT_RES_GLOBAL 0
-#endif
-__device__ __forceinline__ void cta_wait(uint64_t* bar, uint32_t parity) {
-  if (RISER_RT_CTAWAIT) {
-    if (threadIdx.x == 0) mbar_wait(bar, parity);
-    __syncthreads();
-  } else {
-    mbar_wait(bar, parity);
   }
 }
 
@@ -456,7 +397,7 @@ res_tc_kernel(const ResTcArgs a) {
 
     // ---------------- convert: raw fp32 rows -> the mode's A tiles (swizzled K-major)
     // stride 1: X row r = x[q0 - pad + r];  stride 2: E row r = x[2 (q0 + r)], O row r = x[2 (q0 - 1 + r) + 1]
-    cta_wait(&s.raw_full[slot], (a.raw_stages == 2) ? ((k >> 1) & 1) : (k & 1));
+    mbar_wait(&s.raw_full[slot], (a.raw_stages == 2) ? ((k >> 1) & 1) : (k & 1));
     const float* raw = reinterpret_cast<const float*>(raws + slot * a.raw_bytes);
     // unit u = (raw row rr, 8-channel group g), u = rr * groups + g; a thread's units are kRtThreads apart
     int g = tid % groups, rr = tid / groups;                      // raw row = input position pos0 + rr
@@ -488,33 +429,16 @@ res_tc_kernel(const ResTcArgs a) {
     tc_fence_before();
     __syncthreads();
     // one staging buffer: it is free again unless the epilogue reads the identity shortcut from it
-    const bool res_from_raw = fused && a.residual && !a.wsc && a.stride == 1 && (a.raw_stages == 2 || !RISER_RT_RES_GLOBAL);
+    const bool res_from_raw = fused && a.residual && a.stride == 1 && !a.wsc;
     if (a.raw_stages == 1 && !res_from_raw && tid == 0 && nxt < a.n_items) prefetch(nxt, 0);
 
     // ---------------- conv1: D1[128 x n1] = sum over taps / K of A1(view) * W1
-    if (RISER_RT_REPLAY) {
-      if (tid == 0) {
-        tc_fence_after();
-        replay<P>(list1, a.n_mma1, tmem_base);
-        umma_commit(&s.bar);
-      }
-    } else if (warp == 0) {
-      const bool leader = elect_one();
+    if (tid == 0) {
       tc_fence_after();
-      uint32_t acc = 0u;
-      for (int tap = 0; tap < a.taps; ++tap) {
-        int part = 0, shift = tap;
-        if (a.stride == 2) {
-          if (a.taps == 1 || tap == 1) { part = 0; shift = 0; }           // E[m]  (w1 E[m])
-          else { part = 1; shift = (tap == 2) ? 1 : 0; }                  // w0 O[m-1], w2 O[m]
-        }
-        const uint32_t av = a1_addr + part * a.kb1 * kRtTile + shift * 64;
-        issue_term_uniform<P>(leader, tmem_base, av, av + a1_lo, w1_addr, tap, a.kb1, a.cin_p, a.n1, a.cat1 != 0, idesc1,
-                           idesc1c, acc);
-      }
-      umma_commit_p(leader ? 1u : 0u, &s.bar);
+      replay<P>(list1, a.n_mma1, tmem_base);
+      umma_commit(&s.bar);
     }
-    cta_wait(&s.bar, phase);
+    mbar_wait(&s.bar, phase);
     phase ^= 1;
     tc_fence_after();
 
@@ -550,29 +474,12 @@ res_tc_kernel(const ResTcArgs a) {
       __syncthreads();
 
       // ---------------- conv2 (+ 1x1 shortcut conv): D2[i] = sum_t W2_t A2[i + t]  (+ Wsc x[s (p0 + i)])
-      if (RISER_RT_REPLAY) {
-        if (tid == 0) {
-          tc_fence_after();
-          replay<P>(list2, a.n_mma2, tmem_base);
-          umma_commit(&s.bar);
-        }
-      } else if (warp == 0) {
-        const bool leader = elect_one();
+      if (tid == 0) {
         tc_fence_after();
-        uint32_t acc = 0u;
-        const uint32_t d2 = tmem_base + a.d2_col;
-        for (int tap = 0; tap < 3; ++tap) {
-          const uint32_t av = a2_addr + tap * 64;
-          issue_term_uniform<P>(leader, d2, av, av + a2_lo, w2_addr, tap, a.kb2, a.cmid_p, a.n2, a.cat2 != 0, idesc2, idesc2c, acc);
-        }
-        if (a.wsc) {
-          // x[s (p0 + i)]: stride 1 -> X row i + 1 + pad; stride 2 -> E row i + 1
-          const uint32_t av = a1_addr + ((a.stride == 2) ? 1 : 1 + pad) * 64;
-          issue_term_uniform<P>(leader, d2, av, av + a1_lo, wsc_addr, 0, a.kb1, a.cin_p, a.n2, a.cat2 != 0, idesc2, idesc2c, acc);
-        }
-        umma_commit_p(leader ? 1u : 0u, &s.bar);
+        replay<P>(list2, a.n_mma2, tmem_base);
+        umma_commit(&s.bar);
       }
-      cta_wait(&s.bar, phase);
+      mbar_wait(&s.bar, phase);
       phase ^= 1;
       tc_fence_after();
     }

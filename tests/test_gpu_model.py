@@ -55,10 +55,11 @@ def oracle_layers(state, x):
                          [pytest.param(f, p, id=f"{f}-precision{k}") for k, (f, p) in enumerate([
                                             (0, (PREC_F16_F8, 1)), (2, (PREC_F16_F8, 1)), (2, (PREC_F16_F8, 3)),
                                             (2, (PREC_F16_X3, "flat")), (0, (PREC_F16, "flat")),
-                                            (2, (PREC_F16_F8, "nopair")), (2, (PREC_F16_F8, "pair2")), (2, (PREC_F16_F8, "pair5")),
-                                            (2, (PREC_F16_F8, "pair192")), (2, (PREC_F16_F8, 6)),
+                                            (2, (PREC_F16_F8, "nopair"))], 11)] +
+                         [pytest.param(f, p, id=f"{f}-precision{k}") for k, (f, p) in enumerate([
+                                            (2, (PREC_F16_F8, 6)),
                                             (2, (PREC_F16_F8, "nofuse23")), (2, (PREC_F16_X3, "nofuse23")),
-                                            (2, (PREC_F16_X3, "nokc")), (2, (PREC_F16_F8, "nokc"))], 11)])
+                                            (2, (PREC_F16_X3, "nokc")), (2, (PREC_F16_F8, "nokc"))], 20)])
 def test_every_layer_against_oracle(fuse, precision, monkeypatch):
     monkeypatch.setenv("RISER_FUSE_L0", str(fuse))
     if isinstance(precision, tuple) and precision[1] == "flat":     # without the even / odd plane layout
@@ -67,23 +68,12 @@ def test_every_layer_against_oracle(fuse, precision, monkeypatch):
     elif isinstance(precision, tuple) and precision[1] == "nopair":   # e4m3 layers on single CTAs (conv_tc_kernel<F8>)
         precision = precision[0]                                       # instead of CTA pairs (cta_group::2, the default)
         monkeypatch.setenv("RISER_PAIR", "0")
-    elif isinstance(precision, tuple) and precision[1] == "pair2":    # CTA pairs, two 256-row sub-tiles per item,
-        precision = precision[0]                                       # one issuing warp each (default: one sub-tile)
-        monkeypatch.setenv("RISER_PAIR_MS", "2")
-    elif isinstance(precision, tuple) and precision[1] == "pair5":    # CTA pairs from layer 5 on, one issuing warp
-        precision = precision[0]
-        monkeypatch.setenv("RISER_PAIR_FROM", "5")
-        monkeypatch.setenv("RISER_PAIR_MS", "2")
-        monkeypatch.setenv("RISER_DUAL_ISSUE", "0")
     elif isinstance(precision, tuple) and precision[1] == "nokc":      # layer 1's hi / lo terms as three plane passes
         precision = precision[0]                                        # (fused01_kernel<2>) instead of one K = 64 pass
         monkeypatch.setenv("RISER_KC", "0")
     elif isinstance(precision, tuple) and precision[1] == "nofuse23":  # layers 2 and 3 as two conv_eo_kernel launches
         precision = precision[0]
         monkeypatch.setenv("RISER_FUSE23", "0")
-    elif isinstance(precision, tuple) and precision[1] == "pair192":  # CTA pairs, 192-wide N tiles (+ narrower last)
-        precision = precision[0]
-        monkeypatch.setenv("RISER_PAIR_NTILE", "192")
     elif isinstance(precision, tuple):                                # first layer that runs the e4m3 correction pass
         precision, f8_from = precision
         monkeypatch.setenv("RISER_F8_FROM", str(f8_from))

@@ -42,9 +42,7 @@ VARIANTS = {
     "f0-f8-from1": (0, PREC_F16_F8, {"RISER_F8_FROM": "1"}), "f2-f8-from1": (2, PREC_F16_F8, {"RISER_F8_FROM": "1"}),
     "f2-f8-from3": (2, PREC_F16_F8, {"RISER_F8_FROM": "3"}), "f2-f8-from6": (2, PREC_F16_F8, {"RISER_F8_FROM": "6"}),
     "f2-x3-flat": (2, PREC_F16_X3, {"RISER_EO": "0"}), "f0-f16-flat": (0, PREC_F16, {"RISER_EO": "0"}),
-    "f2-f8-nopair": (2, PREC_F16_F8, {"RISER_PAIR": "0"}), "f2-f8-pair2": (2, PREC_F16_F8, {"RISER_PAIR_MS": "2"}),
-    "f2-f8-pair5": (2, PREC_F16_F8, {"RISER_PAIR_FROM": "5", "RISER_PAIR_MS": "2", "RISER_DUAL_ISSUE": "0"}),
-    "f2-f8-pair192": (2, PREC_F16_F8, {"RISER_PAIR_NTILE": "192"}),
+    "f2-f8-nopair": (2, PREC_F16_F8, {"RISER_PAIR": "0"}),
     "f2-f8-nofuse23": (2, PREC_F16_F8, {"RISER_FUSE23": "0"}), "f2-x3-nofuse23": (2, PREC_F16_X3, {"RISER_FUSE23": "0"}),
     "f2-x3-nokc": (2, PREC_F16_X3, {"RISER_KC": "0"}), "f2-f8-nokc": (2, PREC_F16_F8, {"RISER_KC": "0"}),
 }

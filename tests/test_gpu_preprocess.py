@@ -287,31 +287,6 @@ def test_many_short_reads_with_gaps(proc):
     check_batch(proc, sigs, start=start, length=length)
 
 
-@pytest.mark.parametrize("env", [{"RISER_NORM_NBUF": "2"}, {"RISER_NORM_F64": "4"}, {"RISER_NORM_F64": "2"}, {"RISER_NORM_F64": "0"}])
-def test_normalise_kernel_variants(env):
-    """The opt-in variants (second staging buffer; all / half of the quotients on the float64 pipe instead of the value table)
-    give the same bits.  The switches are read once per process, hence the subprocess."""
-    import subprocess
-    import sys
-    code = (
-        "import numpy as np\n"
-        "from riser_b200 import Kit, SignalProcessor, synth\n"
-        "from oracle import preprocess_oracle as pp\n"
-        "proc = SignalProcessor(Kit.create_from_version('RNA002'))\n"
-        "rng = np.random.default_rng(5)\n"
-        "sigs = [synth.body(rng, int(n)) for n in rng.integers(4096, 16000, size=700)]\n"
-        "out, _ = proc.mad_normalise_batch(sigs)\n"
-        "out = out.cpu().numpy()\n"
-        "for b in range(0, 700, 9):\n"
-        "    want = np.asarray(pp.mad_normalise(sigs[b]), dtype=np.float64).astype(np.float32)\n"
-        "    assert np.array_equal(out[b, :len(want)], want), b\n"
-        "print('ok')\n")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-c", code], cwd=root, env={**os.environ, **env}, capture_output=True,
-                       text=True, timeout=600)
-    assert r.returncode == 0 and "ok" in r.stdout, r.stderr[-2000:]
-
-
 def test_normalise_cuts_windows_at_max_len():
     """A len[b] above the max_len the caller states must not run past the staging buffer: the window is processed
     as its first max_len samples (include/riser_b200.h)."""

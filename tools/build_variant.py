@@ -1,7 +1,9 @@
-"""Build a timing / A-B variant of libriser_b200.so with extra nvcc flags into build_ab/ (git-ignored, but it travels
-to the GPU box).  Select it at run time with RISER_B200_LIB=build_ab/<name>.so.
+"""Build a timing / A-B variant of libriser_b200.so with extra nvcc flags into build_ab/ (git-ignored).  Select it at
+run time with RISER_B200_LIB=build_ab/<name>.so.  Run in a checkout of another commit, it builds that commit's
+library, which can then be copied into this tree's build_ab/ and timed against it, alternating RISER_B200_LIB.
 
-  python tools/build_variant.py st128 -DRISER_ST128
+  python tools/build_variant.py parent                 (the sources of this checkout, default flags)
+  python tools/build_variant.py maxreg -maxrregcount=128
 """
 import os
 import subprocess

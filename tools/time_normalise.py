@@ -1,6 +1,6 @@
 """Device timing of riser_normalise alone on the bench shape (B x L already-trimmed int16 chunks):
 algorithmic bytes = 6 * L per read (int16 in, fp32 out) against the measured HBM copy peak.
-usage: python tools/time_normalise.py [B] [L]      (RISER_NORM_NBUF=1|2 selects the staging depth)"""
+usage: python tools/time_normalise.py [B] [L]"""
 import json
 import os
 import sys
@@ -44,4 +44,4 @@ if os.path.exists("MEASURED_PEAKS.json"):
     peak = json.load(open("MEASURED_PEAKS.json")).get("hbm_gbs", peak)
 gbs = 6 * n * B / ms / 1e6
 print(json.dumps({"kernel": "normalise_kernel", "B": B, "L": n, "ms": ms, "algorithmic_GBps": gbs,
-                  "hbm_peak_GBps": peak, "frac": gbs / peak, "nbuf": os.environ.get("RISER_NORM_NBUF", "auto")}))
+                  "hbm_peak_GBps": peak, "frac": gbs / peak}))
