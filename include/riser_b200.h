@@ -130,7 +130,7 @@ int riser_normalise_f32_live(const float* sig, const int64_t* off, const int32_t
  *     flight at once need two workspaces.
  * Each call launches a fixed sequence of kernels for a given (B, max_len), so it can be captured in a CUDA
  * graph.  On short windows the shared-memory entry points are faster; callers pick by length
- * (SignalProcessor.mad_normalise_batch sends only windows above riser_normalise_max_len() here).          */
+ * (riser_b200.preprocess.normalise_windows sends only windows above the *_max_len() limits here).        */
 size_t riser_normalise_long_workspace_bytes(int B, int max_len);
 int riser_normalise_long(const int16_t* sig, const int64_t* off, const int32_t* start, const int32_t* len, int B,
                          int max_len, float* out, int64_t ld_out, int32_t* med2_mad4,

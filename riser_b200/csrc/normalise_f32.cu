@@ -6,7 +6,7 @@
 // Exact order statistics come from a 3-pass (11 + 11 + 10 bit) block-wide radix select over
 // the order-preserving integer image of the floats.  Data-prep path: written for exactness,
 // not for the HBM roofline.
-#include "common.cuh"
+#include "normalise.cuh"
 
 #include <algorithm>
 
@@ -25,22 +25,6 @@ struct Scratch {
   uint32_t res[3];       // bin, keys before the bin, keys in the bin
   uint32_t red[kWarps];
 };
-
-__device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t v, uint32_t* warp_sums) {
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  uint32_t inc = v;
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) {
-    const uint32_t n = __shfl_up_sync(0xffffffffu, inc, d);
-    if (lane >= d) inc += n;
-  }
-  if (lane == 31) warp_sums[warp] = inc;
-  __syncthreads();
-  uint32_t base = 0;
-  for (uint32_t w = 0; w < warp; ++w) base += warp_sums[w];
-  __syncthreads();
-  return base + inc - v;
-}
 
 // key of rank k (0-based) among key(0..n-1); *count_le = number of keys <= that key
 template <class KeyFn>
@@ -113,14 +97,6 @@ __device__ void select_middle(KeyFn key, int n, uint32_t k1, uint32_t k2, Scratc
   }
 }
 
-__device__ __forceinline__ uint32_t f2key(float f) {
-  const uint32_t u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float key2f(uint32_t k) {
-  return __uint_as_float((k & 0x80000000u) ? (k ^ 0x80000000u) : ~k);
-}
-
 __global__ void __launch_bounds__(kThreads)
 normalise_f32_kernel(const float* __restrict__ sig, const int64_t* __restrict__ off, const int32_t* __restrict__ len,
                      int B, float lim, float* __restrict__ out, int64_t ld_out, int zero_if_mad0,
@@ -139,11 +115,9 @@ normalise_f32_kernel(const float* __restrict__ sig, const int64_t* __restrict__ 
     const uint32_t k1 = static_cast<uint32_t>((n - 1) >> 1), k2 = static_cast<uint32_t>(n >> 1);
     uint32_t a1, a2;
     select_middle([&](int i) { return f2key(x[i]); }, n, k1, k2, s, a1, a2);
-    // numpy: mean of the two middle float32 values, in float32 (preprocess.py:11)
-    const float med = (k1 == k2) ? key2f(a1) : __fmul_rn(__fadd_rn(key2f(a1), key2f(a2)), 0.5f);
+    const float med = np_median_f32(key2f(a1), key2f(a2), k1 == k2);
     select_middle([&](int i) { return __float_as_uint(fabsf(__fsub_rn(x[i], med))); }, n, k1, k2, s, a1, a2);
-    const float mad = (k1 == k2) ? __uint_as_float(a1)
-                                 : __fmul_rn(__fadd_rn(__uint_as_float(a1), __uint_as_float(a2)), 0.5f);
+    const float mad = np_median_f32(__uint_as_float(a1), __uint_as_float(a2), k1 == k2);
     if (med_mad && tid == 0) {
       med_mad[2 * b] = med;
       med_mad[2 * b + 1] = mad;
@@ -153,26 +127,8 @@ normalise_f32_kernel(const float* __restrict__ sig, const int64_t* __restrict__ 
       __syncthreads();
       continue;
     }
-    const float denom = __fmul_rn(1.4826f, mad);                       // preprocess.py:44
-    auto norm = [&](int i) { return __fdiv_rn(__fsub_rn(x[i], med), denom); };
-    auto clip = [&](float v) { return v > lim ? lim : (v < -lim ? -lim : v); };
-    for (int i = tid; i < n; i += kThreads) {
-      const float v = norm(i);
-      if (!(fabsf(v) > lim)) {
-        o[i] = v;
-        continue;
-      }
-      if (i > 0 && fabsf(norm(i - 1)) > lim) continue;       // the run's first element walks it
-      float prev = (i > 0) ? norm(i - 1) : 0.f;               // preprocess.py:18-33, sequential
-      for (int j = i; j < n && fabsf(norm(j)) > lim; ++j) {
-        float nv;
-        if (j == 0) nv = (n > 1) ? norm(1) : norm(0);
-        else if (j == n - 1) nv = prev;
-        else nv = clip(__fmul_rn(__fadd_rn(prev, norm(j + 1)), 0.5f));
-        o[j] = nv;
-        prev = nv;
-      }
-    }
+    const float denom = __fmul_rn(static_cast<float>(kScalingFactor), mad);       // retrain/preprocess.py:44
+    normalise_span([&](int64_t i) { return __fdiv_rn(__fsub_rn(x[i], med), denom); }, lim, tid, n, n, kThreads, o);
     __syncthreads();
   }
 }

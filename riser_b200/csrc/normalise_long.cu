@@ -1,7 +1,8 @@
 // Normalisation of windows of any length (up to INT32_MAX samples) for sm_100a:
-//   riser_normalise_long      -- int16 windows, the arithmetic of riser_normalise (riser/preprocess.py:108-147)
-//   riser_normalise_f32_long  -- float32 windows, the arithmetic of riser_normalise_f32 / riser_normalise_f32_live
+//   riser_normalise_long      -- int16 windows, the results of riser_normalise (riser/preprocess.py:108-147)
+//   riser_normalise_f32_long  -- float32 windows, the results of riser_normalise_f32 / riser_normalise_f32_live
 //                                (riser/retrain/preprocess.py:8-44; riser/preprocess.py:108-147 on float32 input)
+// The arithmetic that decides those results bit for bit is shared with them (normalise.cuh).
 // The kernels of preprocess.cu and normalise_f32.cu stage a whole window in one CTA's shared memory, which bounds the
 // window (98,304 int16 / 49,152 float32 samples).  Here the window stays in global memory and is worked on by many
 // CTAs at once, a work item being one kChunk-sample chunk of one read:
@@ -13,11 +14,11 @@
 //                int16: median keys x + 32768 (16 bits: 11 + 5), MAD keys |2x - 2 median| (17 bits: 11 + 6) ->
 //                {2 median, 4 MAD} exactly as riser_normalise reports them.  float32: the order-preserving image of
 //                the float (11 + 11 + 10 bits) for the median, the bits of |x - median| for the MAD.
-//   normalise    every sample's quotient, in the operation order of the shared-memory kernels; an outlier run
-//                (the set |v| > limit is fixed up front) is walked sequentially by the thread that owns its first
-//                element -- runs cross chunk boundaries freely since everything is in global memory.
+//   normalise    normalise_span over each chunk: every sample's quotient; an outlier run (the set |v| > limit is
+//                fixed up front) is walked sequentially by the thread that owns its first element -- runs cross
+//                chunk boundaries freely since everything is in global memory.
 // No host synchronisation, no allocation, and for a given (B, max_len) a fixed launch sequence (CUDA-graph capturable).
-#include "common.cuh"
+#include "normalise.cuh"
 
 #include <algorithm>
 
@@ -30,9 +31,6 @@ constexpr int kLBins = 2048;
 constexpr int kLBinsPerThread = kLBins / kLThreads;
 constexpr int kChunk = 16384;               // samples per work item
 constexpr int kBlocksPerSm = 8;             // persistent grid: 8 x 256 threads fill an SM
-
-constexpr double kOutlierLimit = 3.5;       // riser/preprocess.py:6
-constexpr double kScalingFactor = 1.4826;   // riser/preprocess.py:7
 
 // Per-read selection state in the workspace, after the B histograms.
 struct LongState {
@@ -48,30 +46,6 @@ static_assert(sizeof(LongState) == 64, "64-byte state per read");
 struct PassSpec {
   int shift, bits;
 };
-
-__device__ __forceinline__ uint32_t f2key(float f) {
-  const uint32_t u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float key2f(uint32_t k) {
-  return __uint_as_float((k & 0x80000000u) ? (k ^ 0x80000000u) : ~k);
-}
-
-__device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t v, uint32_t* warp_sums) {
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  uint32_t inc = v;
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) {
-    const uint32_t n = __shfl_up_sync(0xffffffffu, inc, d);
-    if (lane >= d) inc += n;
-  }
-  if (lane == 31) warp_sums[warp] = inc;
-  __syncthreads();
-  uint32_t base = 0;
-  for (uint32_t w = 0; w < warp; ++w) base += warp_sums[w];
-  __syncthreads();
-  return base + inc - v;
-}
 
 __device__ __forceinline__ int window_len(const int32_t* len, int b, int max_len) { return min(len[b], max_len); }
 
@@ -150,7 +124,7 @@ long_hist_kernel(const T* __restrict__ sig, const int64_t* __restrict__ off, con
 
 // One CTA per read: locate the bin of rank s.k in the read's histogram (clearing it for the next pass) and narrow the
 // prefix.  After the last pass of a select: the two middle order statistics -> the median (stage 0, and the state is
-// reset for the MAD select) or the MAD (stage 1), combined as the shared-memory kernels combine them.
+// reset for the MAD select) or the MAD (stage 1): 2 median / 4 MAD for int16, numpy's float32 median for float32.
 template <bool F32>
 __global__ void __launch_bounds__(kLThreads)
 long_narrow_kernel(const int32_t* __restrict__ len, int B, int max_len, uint32_t* __restrict__ hist,
@@ -216,38 +190,18 @@ long_narrow_kernel(const int32_t* __restrict__ len, int B, int max_len, uint32_t
     if (tid == 0) {
       LongState& o = st[b];
       if (stage == 0) {
-        if (F32) o.med = (k1 == k2) ? key2f(v1) : __fmul_rn(__fadd_rn(key2f(v1), key2f(v2)), 0.5f);   // numpy: float32 mean of the pair
+        if (F32) o.med = np_median_f32(key2f(v1), key2f(v2), k1 == k2);
         else o.med2 = static_cast<int>(v1) + static_cast<int>(v2) - 65536;
         o.prefix = o.mask = o.below = 0;
         o.k = k1;
         o.min_above = 0xffffffffu;
       } else {
-        if (F32) o.mad = (k1 == k2) ? __uint_as_float(v1)
-                                    : __fmul_rn(__fadd_rn(__uint_as_float(v1), __uint_as_float(v2)), 0.5f);
+        if (F32) o.mad = np_median_f32(__uint_as_float(v1), __uint_as_float(v2), k1 == k2);
         else o.mad4 = static_cast<int32_t>(v1 + v2);
       }
     }
     __syncthreads();
   }
-}
-
-// (x - median) / (1.4826 MAD) in float64 as k / D with k = 2x - 2 median (an exact small integer) and D = 2 * denom
-// (exact): y = RN(1/D), q0 = RN(k y), e = k - q0 D (exact in one FMA), RN(q0 + e y) is the correctly rounded quotient
-// (Markstein's final division step) -- the reference's float64 divide, as normalise_kernel computes it.
-struct Quot16 {
-  double D, y;
-  int med2;
-  __device__ __forceinline__ double operator()(int x) const {
-    const double k = static_cast<double>(2 * x - med2);
-    const double q0 = __dmul_rn(k, y);
-    return __fma_rn(__fma_rn(-q0, D, k), y, q0);
-  }
-};
-
-__device__ __forceinline__ double clip_outlier(double v) {   // riser/preprocess.py:141-147
-  if (v > kOutlierLimit) return kOutlierLimit;
-  if (v < -kOutlierLimit) return -kOutlierLimit;
-  return v;
 }
 
 __global__ void __launch_bounds__(kLThreads)
@@ -274,33 +228,8 @@ long_norm_i16_kernel(const int16_t* __restrict__ sig, const int64_t* __restrict_
       for (int64_t i = i0 + tid; i < i1; i += kLThreads) o[i] = 0.f;
       continue;
     }
-    const double denom = __dmul_rn(kScalingFactor, static_cast<double>(mad4) * 0.25);
-    const double D = __dmul_rn(2.0, denom);
-    const Quot16 q{D, __ddiv_rn(1.0, D), med2};
-    for (int64_t i = i0 + tid; i < i1; i += kLThreads) {
-      const double v = q(g[i]);
-      if (!(fabs(v) > kOutlierLimit)) {
-        o[i] = static_cast<float>(v);
-        continue;
-      }
-      if (i > 0 && fabs(q(g[i - 1])) > kOutlierLimit) continue;     // the run's first element walks it
-      // riser/preprocess.py:130-138: arr[j-1] is already updated, arr[j+1] still raw; the end points of the array
-      // copy their single neighbour and are not clipped
-      double prev = (i > 0) ? q(g[i - 1]) : 0.0;
-      int64_t j = i;
-      double right = (j + 1 < n) ? q(g[j + 1]) : v;
-      for (;;) {
-        double nv;
-        if (j == 0) nv = right;
-        else if (j == n - 1) nv = prev;
-        else nv = clip_outlier(__dmul_rn(__dadd_rn(prev, right), 0.5));
-        o[j] = static_cast<float>(nv);
-        prev = nv;
-        if (j + 1 >= n || !(fabs(right) > kOutlierLimit)) break;
-        ++j;
-        right = (j + 1 < n) ? q(g[j + 1]) : 0.0;
-      }
-    }
+    const Quot16 q(__dmul_rn(kScalingFactor, static_cast<double>(mad4) * 0.25));
+    normalise_span([&](int64_t i) { return q(2 * g[i] - med2); }, kOutlierLimit, i0 + tid, i1, n, kLThreads, o);
   }
 }
 
@@ -310,7 +239,6 @@ long_norm_f32_kernel(const float* __restrict__ sig, const int64_t* __restrict__ 
                      float* __restrict__ out, int64_t ld_out, float* __restrict__ med_mad) {
   const int tid = threadIdx.x;
   const int64_t items = static_cast<int64_t>(B) * n_chunks;
-  auto clip = [&](float v) { return v > lim ? lim : (v < -lim ? -lim : v); };
   for (int64_t it = blockIdx.x; it < items; it += gridDim.x) {
     const int b = static_cast<int>(it / n_chunks);
     const int64_t i0 = (it - static_cast<int64_t>(b) * n_chunks) * kChunk;
@@ -328,30 +256,9 @@ long_norm_f32_kernel(const float* __restrict__ sig, const int64_t* __restrict__ 
       for (int64_t i = i0 + tid; i < i1; i += kLThreads) o[i] = 0.f;
       continue;
     }
-    const float denom = __fmul_rn(1.4826f, mad);        // retrain/preprocess.py:44
-    auto norm = [&](int64_t i) { return __fdiv_rn(__fsub_rn(g[i], med), denom); };
-    for (int64_t i = i0 + tid; i < i1; i += kLThreads) {
-      const float v = norm(i);
-      if (!(fabsf(v) > lim)) {
-        o[i] = v;
-        continue;
-      }
-      if (i > 0 && fabsf(norm(i - 1)) > lim) continue;  // the run's first element walks it
-      float prev = (i > 0) ? norm(i - 1) : 0.f;         // retrain/preprocess.py:18-33, sequential
-      int64_t j = i;
-      float right = (j + 1 < n) ? norm(j + 1) : v;
-      for (;;) {
-        float nv;
-        if (j == 0) nv = right;
-        else if (j == n - 1) nv = prev;
-        else nv = clip(__fmul_rn(__fadd_rn(prev, right), 0.5f));
-        o[j] = nv;
-        prev = nv;
-        if (j + 1 >= n || !(fabsf(right) > lim)) break;
-        ++j;
-        right = (j + 1 < n) ? norm(j + 1) : 0.f;
-      }
-    }
+    const float denom = __fmul_rn(static_cast<float>(kScalingFactor), mad);     // retrain/preprocess.py:44
+    normalise_span([&](int64_t i) { return __fdiv_rn(__fsub_rn(g[i], med), denom); }, lim, i0 + tid, i1, n, kLThreads,
+                   o);
   }
 }
 

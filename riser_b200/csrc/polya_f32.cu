@@ -9,7 +9,7 @@
 // add / multiply / divide is an explicit round-to-nearest intrinsic so that nvcc cannot contract to FMA.
 // One CTA per read, one warp per 500-sample window, the warp's next window fetched while the current one is worked
 // on; the two-state scan over the windows is that of polya_kernel (preprocess.cu).
-#include "common.cuh"
+#include "normalise.cuh"
 
 #include <algorithm>
 #include <utility>
@@ -100,13 +100,6 @@ __device__ __forceinline__ float np_sum_f32(const float* __restrict__ x, int lan
   return np_sum_f32_impl<N>(x, lane, std::make_integer_sequence<int, pw_leaves(N)>{});
 }
 
-__device__ __forceinline__ uint32_t f2key(float f) {
-  const uint32_t u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float key2f(uint32_t k) {
-  return __uint_as_float((k & 0x80000000u) ? (k ^ 0x80000000u) : ~k);
-}
 __device__ __forceinline__ int bits_of(uint32_t v) { return 32 - __clz(v); }
 
 // numpy's median of the warp's 500 keys (padding lanes hold 0xffffffff): the two middle keys (ranks 249, 250) found
@@ -144,9 +137,6 @@ __device__ __forceinline__ void warp_mid_keys(const uint32_t (&key)[kPerLane], u
   k1 = v1;
   k2 = (le > kRes / 2) ? v1 : next;
 }
-
-// numpy's mean of two float32 values (np.median's last step): float32((0 + a + b) / 2)
-__device__ __forceinline__ float mid_mean(float a, float b) { return __fmul_rn(__fadd_rn(__fadd_rn(a, b), 0.f), 0.5f); }
 
 __global__ void __launch_bounds__(kThreads)
 polya_f32_kernel(const float* __restrict__ sig, const int64_t* __restrict__ off, const int32_t* __restrict__ nsamp,
@@ -197,12 +187,12 @@ polya_f32_kernel(const float* __restrict__ sig, const int64_t* __restrict__ off,
 #pragma unroll
       for (int j = 0; j < kPerLane; ++j) key[j] = ok[j] ? f2key(v[j]) : 0xffffffffu;
       warp_mid_keys(key, k1, k2);
-      const float med = mid_mean(key2f(k1), key2f(k2));
+      const float med = np_median_f32(key2f(k1), key2f(k2), kRes % 2);
       // |x - median| >= 0: the float's bit pattern is already order-preserving
 #pragma unroll
       for (int j = 0; j < kPerLane; ++j) key[j] = ok[j] ? __float_as_uint(fabsf(__fsub_rn(v[j], med))) : 0xffffffffu;
       warp_mid_keys(key, k1, k2);
-      const float mad = mid_mean(__uint_as_float(k1), __uint_as_float(k2));
+      const float mad = np_median_f32(__uint_as_float(k1), __uint_as_float(k2), kRes % 2);
       const float mean = __fdiv_rn(np_sum_f32<kRes>(wp, lane), static_cast<float>(kRes));
       float rolling = mean;
       if (w > 2) rolling = __fdiv_rn(np_sum_f32<2 * kRes>(wp - 2 * kRes, lane), static_cast<float>(2 * kRes));

@@ -8,7 +8,7 @@
 // select for whole windows, warp-shuffle bit-descent select for 500-sample windows),
 // float64 arithmetic in the reference's operation order, fp32 results written with
 // 16-byte stores.
-#include "common.cuh"
+#include "normalise.cuh"
 
 #include <algorithm>
 #include <stdlib.h>
@@ -27,9 +27,6 @@ constexpr int kMaxRuns = 512;           // outlier-run start indices collected p
 
 constexpr int kDefaultF64 = 1;          // samples per group of four on the float64 pipe (0 / 1 / 4: 0.1106 / 0.1085 / 0.1085 ms)
 
-constexpr double kOutlierLimit = 3.5;   // riser/preprocess.py:6
-constexpr double kScalingFactor = 1.4826;  // riser/preprocess.py:7
-
 struct SelectScratch {
   uint64_t bar;         // bulk-copy completion of the staging buffer
   alignas(16) uint32_t hist[kBins];
@@ -41,22 +38,6 @@ struct SelectScratch {
   int32_t red[2 * kWarps];
   int32_t runs[kMaxRuns];
 };
-
-__device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t v, uint32_t* warp_sums) {
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  uint32_t inc = v;
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) {
-    uint32_t n = __shfl_up_sync(0xffffffffu, inc, d);
-    if (lane >= d) inc += n;
-  }
-  if (lane == 31) warp_sums[warp] = inc;
-  __syncthreads();
-  uint32_t base = 0;
-  for (uint32_t w = 0; w < warp; ++w) base += warp_sums[w];
-  __syncthreads();
-  return base + inc - v;
-}
 
 // A window of n samples staged in shared memory at the 16-byte phase it has in global memory:
 // sample i is stage[a + i], 0 <= a < 8.  for_each() hands every sample of the window to f, one
@@ -202,13 +183,6 @@ __device__ int select_two(KeyFn key, const StagedWindow& win, uint32_t maxkey, u
   }
   __syncthreads();
   return shift;
-}
-
-__device__ __forceinline__ double clip_outlier(double v) {
-  // riser/preprocess.py:141-147
-  if (v > kOutlierLimit) return kOutlierLimit;
-  if (v < -kOutlierLimit) return -kOutlierLimit;
-  return v;
 }
 
 // Kernel structure (one CTA per read, persistent over reads b = blockIdx.x, + gridDim.x, ...):
@@ -405,19 +379,7 @@ normalise_kernel(const int16_t* __restrict__ sig, const int64_t* __restrict__ of
       }
     } else {
       const double denom = __dmul_rn(kScalingFactor, static_cast<double>(mad4) * 0.25);
-      // (x - median) / denom == k / D with k = 2x - 2*median (an exact small integer) and D = 2 * denom
-      // (exact).  With y = RN(1/D), q0 = RN(k*y), e = k - q0*D (exact in one FMA), RN(q0 + e*y) is the
-      // correctly rounded quotient (Markstein's final division step), i.e. bit-identical to the reference's
-      // float64 divide at 3 FP64 ops instead of a full DDIV.
-      const double Dd = __dmul_rn(2.0, denom);
-      const double yrcp = __ddiv_rn(1.0, Dd);
-      auto quot = [&](int ki) {
-        // (double) ki without an I2F: 2^52 + 2^31 + ki has ki ^ 0x80000000 in its low word; one exact DADD removes the offset
-        const double k = __dadd_rn(__hiloint2double(0x43300000, ki ^ static_cast<int>(0x80000000u)), -4503601774854144.0);
-        const double q0 = __dmul_rn(k, yrcp);
-        const double e = __fma_rn(-q0, Dd, k);
-        return __fma_rn(e, yrcp, q0);
-      };
+      const Quot16 quot(denom);          // (x - median) / denom of sample x is quot(2x - med2)
       // A window holds at most range + 1 distinct values (~1,000 for a squiggle against 4,096-16,000 samples),
       // and the float64 pipe is what bounds this kernel: when the value range fits the histogram, the fp32 result
       // of every VALUE is tabulated once (in the histogram's storage, free after the MAD search) and the per-sample
@@ -471,7 +433,7 @@ normalise_kernel(const int16_t* __restrict__ sig, const int64_t* __restrict__ of
           } else if (j == n - 1) {
             nv = prev;                           // arr[n-1] = arr[n-2] (already updated)
           } else {
-            nv = clip_outlier(__fma_rn(prev, 0.5, rh));
+            nv = clip_outlier(__fma_rn(prev, 0.5, rh), kOutlierLimit);
           }
           o[j] = static_cast<float>(nv);
           prev = nv;

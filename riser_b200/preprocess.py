@@ -170,6 +170,54 @@ def signal_dtype(signals):
     return _F32
 
 
+_long_ws = {}       # device -> workspace of the long-window kernels, grown as needed; its users share one stream
+
+
+def normalise_windows(sig, off, start, len_host, len_dev, out, stats=None, outlier_lim=3.5, live=True):
+    """Median / MAD-normalise window b = ``sig[off[b] + start[b]:][:len_host[b]]`` into row b of ``out`` (fp32 [B, ld]),
+    for int16 or float32 ``sig``.  ``start``: int32 device tensor (int16 only) or None; ``len_dev``: ``len_host`` on the
+    device; ``stats`` (optional): {2 median, 4 MAD} int32 for int16, {median, MAD} float32 for live float32.  float32
+    takes ``outlier_lim``, and ``live`` zeros windows whose MAD is 0 (else numpy's inf / nan, as retraining wants).
+    Windows above the shared-memory kernels' limit go to ``riser_normalise_long`` / ``riser_normalise_f32_long`` (the
+    same results), the rest to ``riser_normalise`` / ``riser_normalise_f32(_live)``; each launch sees the other's
+    windows as length 0."""
+    L, P = _lib.lib(), _lib.ptr
+    f32 = sig.dtype == torch.float32
+    assert not f32 or (start is None and (live or stats is None)), "no float32 kernel takes these arguments"
+    B = len(len_host)
+    max_len = int(len_host.max()) if B else 0
+    if max_len <= 0:
+        return
+    limit = L.riser_normalise_f32_max_len() if f32 else L.riser_normalise_max_len()
+    short_len = len_dev
+    if max_len > limit:
+        is_long = len_host > limit
+        short_len = torch.from_numpy(np.where(is_long, 0, len_host).astype(np.int32)).to(sig.device)
+        long_len = torch.from_numpy(np.where(is_long, len_host, 0).astype(np.int32)).to(sig.device)
+        nbytes = max(L.riser_normalise_long_workspace_bytes(B, max_len), 16)
+        ws = _long_ws.get(sig.device)
+        if ws is None or ws.numel() < nbytes:
+            ws = _long_ws[sig.device] = torch.empty(nbytes, dtype=torch.uint8, device=sig.device)
+        if f32:
+            _lib.check(L.riser_normalise_f32_long(P(sig), P(off), P(long_len), B, max_len, float(outlier_lim),
+                                                  int(live), P(out), out.stride(0), P(stats), P(ws), ws.numel(),
+                                                  _lib.stream_ptr()), "riser_normalise_f32_long")
+        else:
+            _lib.check(L.riser_normalise_long(P(sig), P(off), P(start), P(long_len), B, max_len, P(out),
+                                              out.stride(0), P(stats), P(ws), ws.numel(), _lib.stream_ptr()),
+                       "riser_normalise_long")
+        max_len = limit
+    if not f32:
+        _lib.check(L.riser_normalise(P(sig), P(off), P(start), P(short_len), B, max_len, P(out), out.stride(0),
+                                     P(stats), _lib.stream_ptr()), "riser_normalise")
+    elif live:
+        _lib.check(L.riser_normalise_f32_live(P(sig), P(off), P(short_len), B, max_len, P(out), out.stride(0),
+                                              P(stats), _lib.stream_ptr()), "riser_normalise_f32_live")
+    else:
+        _lib.check(L.riser_normalise_f32(P(sig), P(off), P(short_len), B, max_len, float(outlier_lim), P(out),
+                                         out.stride(0), _lib.stream_ptr()), "riser_normalise_f32")
+
+
 class SignalProcessor():
     def __init__(self, kit):
         self.kit = kit
@@ -287,17 +335,6 @@ class SignalProcessor():
             return np.zeros(n, dtype=np.int64)
         return out[0, :n].double().cpu().numpy()
 
-    def _long_workspace(self, B, max_len):
-        """Workspace of riser_normalise_long / riser_normalise_f32_long for (B, max_len), kept for the next call of
-        the same shape."""
-        key = (B, max_len)
-        ws = getattr(self, "_long_ws", None)
-        if ws is None or ws[0] != key:
-            nbytes = _lib.lib().riser_normalise_long_workspace_bytes(B, max_len)
-            ws = (key, torch.empty(max(nbytes, 16), dtype=torch.uint8, device=_lib.require_device()))
-            self._long_ws = ws
-        return ws[1]
-
     def _mad_normalise_f32(self, signal):
         device = _lib.require_device()
         n = signal.shape[0]
@@ -306,16 +343,7 @@ class SignalProcessor():
         ln = torch.tensor([n], dtype=torch.int32, device=device)
         out = torch.empty(1, n, dtype=torch.float32, device=device)
         med_mad = torch.empty(1, 2, dtype=torch.float32, device=device)
-        if n > _lib.lib().riser_normalise_f32_max_len():
-            ws = self._long_workspace(1, n)
-            _lib.check(_lib.lib().riser_normalise_f32_long(_lib.ptr(sig), _lib.ptr(off), _lib.ptr(ln), 1, n, 3.5, 1,
-                                                           _lib.ptr(out), out.stride(0), _lib.ptr(med_mad),
-                                                           _lib.ptr(ws), ws.numel(), _lib.stream_ptr()),
-                       "riser_normalise_f32_long")
-        else:
-            _lib.check(_lib.lib().riser_normalise_f32_live(_lib.ptr(sig), _lib.ptr(off), _lib.ptr(ln), 1, n,
-                                                           _lib.ptr(out), out.stride(0), _lib.ptr(med_mad),
-                                                           _lib.stream_ptr()), "riser_normalise_f32_live")
+        normalise_windows(sig, off, None, np.array([n], dtype=np.int32), ln, out, med_mad)
         if float(med_mad[0, 1]) == 0.0:
             return np.zeros(n, dtype=np.int64)
         return out[0].cpu().numpy()
@@ -328,9 +356,7 @@ class SignalProcessor():
         (``sig[start:start+length]``); default the whole read.
         Returns (out fp32 [B, ld] on the device, lengths int32 device tensor).
 
-        Windows longer than ``riser_normalise_max_len()`` go to ``riser_normalise_long`` (same results, global-memory
-        passes instead of one CTA's shared memory); the rest to ``riser_normalise``, each launch seeing the other's
-        windows as length 0."""
+        Windows of any length: ``normalise_windows`` routes them by length."""
         device = _lib.require_device()
         batch = signals if isinstance(signals, RaggedBatch) else RaggedBatch(
             [np.ascontiguousarray(s, dtype=np.int16) for s in signals], device)
@@ -339,29 +365,13 @@ class SignalProcessor():
         else:
             len_host = np.asarray(length, dtype=np.int32)
         max_len = int(len_host.max()) if batch.B else 0
-        limit = _lib.lib().riser_normalise_max_len()
         ld = (max_len + 3) & ~3
         if out is None:
             out = torch.zeros(batch.B, max(ld, 4), dtype=torch.float32, device=device)
         start_t = None if start is None else torch.as_tensor(np.asarray(start, dtype=np.int32)).to(device)
         len_t = batch.n if (length is None and start is None) else torch.from_numpy(len_host).to(device)
         stats = torch.zeros(batch.B, 2, dtype=torch.int32, device=device) if return_stats else None
-        short_t = len_t
-        if max_len > limit:
-            is_long = len_host > limit
-            short_t = torch.from_numpy(np.where(is_long, 0, len_host).astype(np.int32)).to(device)
-            long_t = torch.from_numpy(np.where(is_long, len_host, 0).astype(np.int32)).to(device)
-            ws = self._long_workspace(batch.B, max_len)
-            _lib.check(_lib.lib().riser_normalise_long(_lib.ptr(batch.sig), _lib.ptr(batch.off), _lib.ptr(start_t),
-                                                       _lib.ptr(long_t), batch.B, max_len, _lib.ptr(out),
-                                                       out.stride(0), _lib.ptr(stats), _lib.ptr(ws), ws.numel(),
-                                                       _lib.stream_ptr()), "riser_normalise_long")
-            max_len = limit
-        if batch.B and max_len > 0:
-            _lib.check(_lib.lib().riser_normalise(_lib.ptr(batch.sig), _lib.ptr(batch.off), _lib.ptr(start_t),
-                                                  _lib.ptr(short_t), batch.B, max_len, _lib.ptr(out),
-                                                  out.stride(0), _lib.ptr(stats), _lib.stream_ptr()),
-                       "riser_normalise")
+        normalise_windows(batch.sig, batch.off, start_t, len_host, len_t, out, stats)
         if return_stats:
             return out, len_t, stats
         return out, len_t

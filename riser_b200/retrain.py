@@ -7,13 +7,13 @@ import numpy as np
 import torch
 
 from . import _lib
+from .preprocess import normalise_windows
 
 
 def mad_normalise_f32_batch(signals, outlier_lim=3.5):
     """Batched retrain/preprocess.py:8-15 over a list of float32 arrays.  Returns an fp32
-    [B, ld] device tensor and the int32 lengths (device).  Reads longer than
-    ``riser_normalise_f32_max_len()`` go to ``riser_normalise_f32_long`` (same results), the rest to
-    ``riser_normalise_f32``, each launch seeing the other's reads as length 0."""
+    [B, ld] device tensor and the int32 lengths (device).  Reads of any length: ``normalise_windows`` routes
+    them by length."""
     device = _lib.require_device()
     B = len(signals)
     n = np.fromiter((len(s) for s in signals), dtype=np.int64, count=B)
@@ -25,27 +25,12 @@ def mad_normalise_f32_batch(signals, outlier_lim=3.5):
     hv = host.numpy()
     for s, o, k in zip(signals, off[:-1], n):
         hv[o:o + k] = np.asarray(s, dtype=np.float32)
-    max_len = int(n.max())
-    limit = _lib.lib().riser_normalise_f32_max_len()
     sig = host.to(device, non_blocking=True)
     off_d = torch.from_numpy(off).to(device)
-    len_d = torch.from_numpy(n.astype(np.int32)).to(device)
-    out = torch.zeros(B, max_len, dtype=torch.float32, device=device)
-    short_d = len_d
-    if max_len > limit:
-        is_long = n > limit
-        short_d = torch.from_numpy(np.where(is_long, 0, n).astype(np.int32)).to(device)
-        long_d = torch.from_numpy(np.where(is_long, n, 0).astype(np.int32)).to(device)
-        nbytes = _lib.lib().riser_normalise_long_workspace_bytes(B, max_len)
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
-        _lib.check(_lib.lib().riser_normalise_f32_long(_lib.ptr(sig), _lib.ptr(off_d), _lib.ptr(long_d), B, max_len,
-                                                       float(outlier_lim), 0, _lib.ptr(out), out.stride(0), None,
-                                                       _lib.ptr(ws), nbytes, _lib.stream_ptr()),
-                   "riser_normalise_f32_long")
-        max_len = limit
-    _lib.check(_lib.lib().riser_normalise_f32(_lib.ptr(sig), _lib.ptr(off_d), _lib.ptr(short_d), B, max_len,
-                                              float(outlier_lim), _lib.ptr(out), out.stride(0),
-                                              _lib.stream_ptr()), "riser_normalise_f32")
+    n32 = n.astype(np.int32)
+    len_d = torch.from_numpy(n32).to(device)
+    out = torch.zeros(B, int(n.max()), dtype=torch.float32, device=device)
+    normalise_windows(sig, off_d, None, n32, len_d, out, outlier_lim=outlier_lim, live=False)
     return out, len_d
 
 

@@ -301,3 +301,41 @@ def test_long_path_replays_from_a_cuda_graph():
         torch.cuda.synchronize()
         assert np.array_equal(out.cpu().numpy(), want) and np.array_equal(stats.cpu().numpy(), want_stats)
         assert np.array_equal(out32.cpu().numpy(), want32)
+
+
+def zero_median_window(n, seed):
+    """float32 window of n samples whose middle value(s) are -0.0 and whose MAD is 5: 500-sample blocks of 249 x -5,
+    2 x -0.0 and 249 x 5 (shuffled), then one more -0.0 when n is odd; every 500-sample window has the same median."""
+    rng = np.random.default_rng(seed)
+    block = np.float32([-5] * 249 + [-0.0] * 2 + [5] * 249)
+    x = np.concatenate([rng.permutation(block) for _ in range(n // 500)] + [np.float32([-0.0] * (n % 500))])
+    return x.astype(np.float32)
+
+
+def test_median_of_negative_zeros_is_positive_zero(proc):
+    """numpy's median of two -0.0 (or of one, for an odd count) is +0.0, so every -0.0 sample normalises to
+    -0.0 - +0.0 = -0.0; compared as bit patterns, since +0 == -0 as floats."""
+    limit = _lib.lib().riser_normalise_f32_max_len()
+    lengths = [40000, 40001, 60000, 60001]
+    assert lengths[1] < limit < lengths[2]
+    sigs = [zero_median_window(n, n) for n in lengths]
+    bits = lambda a: np.asarray(a, dtype=np.float32).view(np.uint32)
+    for x in sigs:
+        assert np.median(x).view(np.uint32) == 0 and np.median(np.abs(x - np.median(x))) == 5
+        want = cref.mad_normalise_f32(x)
+        assert np.array_equal(bits(want), bits(pp.mad_normalise(x)))
+        assert np.array_equal(bits(proc.mad_normalise(x)), bits(want)), len(x)
+    out, _ = retrain.mad_normalise_f32_batch(sigs)
+    out = out.cpu().numpy()
+    out32, med_mad = long32(sigs, 3.5, 0)
+    for b, x in enumerate(sigs):
+        want = bits(rt.mad_normalise(x))
+        assert np.array_equal(bits(out[b, :len(x)]), want), len(x)
+        assert np.array_equal(bits(out32[b, :len(x)]), want), len(x)
+        assert bits(med_mad[b, 0]) == 0 and med_mad[b, 1] == 5
+    batch = RaggedBatch(sigs, torch.device("cuda"), dtype=np.float32)
+    _, stats = proc.polya_end_device(batch, return_stats=True)
+    stats = stats.cpu().numpy()
+    for b, x in enumerate(sigs):
+        w = len(x) // 500
+        assert np.all(bits(stats[b, :w, 0]) == 0) and np.all(stats[b, :w, 1] == 5), len(x)
