@@ -2680,7 +2680,8 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
     const int rows_in = B * p->Lp[i];
     const bool last = (i == m->n_layers - 1);
     const int a_box_rows = 136;   // 130 needed; a multiple of 8 is what TMA likes
-    const bool fuse01 = (i == 1 && fuse_l0 && L.cin_p == 32 && L.n_tile == 32 && L.n_tiles == 1 &&
+    // fused01_kernel stores fp16 rows only: a last layer (the head reads fp32) runs as layer0_kernel + conv_tc_kernel
+    const bool fuse01 = (i == 1 && fuse_l0 && !last && L.cin_p == 32 && L.n_tile == 32 && L.n_tiles == 1 &&
                          m->layer[0].cout <= 24);
     // 32-channel K blocks (64-byte rows, SWIZZLE_64B) for narrow layers: no zero-filled half rows,
     // twice the pipeline depth / sub-tiles per item in the same shared memory

@@ -21,6 +21,8 @@ PREC_F16_X3 = 2    # three passes, weights and activations split hi + lo: fp32-c
 PREC_F16_F8 = 3    # fp16 pass + one e4m3 pass carrying both hi/lo correction terms (2 pass-equivalents)
 DEFAULT_PRECISION = PREC_F16_F8
 MIN_LENGTH = 4096  # riser/preprocess.py:8 -- 12 stride-2 pools
+MAX_LAYERS = 16            # csrc/convnet.cu kMaxLayers: deeper networks run on GenericConvNet
+MAX_LAYER0_CHANNELS = 64   # layer0_kernel's limit (riser_model_create): wider layers 0 run on GenericConvNet
 # F16_F8 rows carry a8 = e4m3(a * 2^-F8_A_SHIFT) and lo8 = e4m3((a - hi) * 2^(9 - F8_LO_SHIFT)); the weight operands
 # of the e4m3 pass carry the opposite powers of two (csrc/convnet.cu kF8AScale / kF8LoScale, which these must match)
 F8_A_SHIFT = 3
@@ -141,9 +143,10 @@ class Model():
         (riser/nets/cnn.py:8-41, riser/model.py:18-19)."""
         self._generic = None
         if (c.classifier != 'gap_fc' or int(c.depth) != 1 or int(c.n_classes) != 2
-                or any(int(k) != 3 for k in c.kernels[:c.n_layers]) or int(c.n_layers) < 2):
-            # not the shipped shape (riser/model/*.yaml:6-12) the kernels of csrc/convnet.cu are written for: depth > 1,
-            # other odd kernel sizes, 'gap' head, n_classes != 2 run on the generic channel-last ops
+                or any(int(k) != 3 for k in c.kernels[:c.n_layers]) or not 2 <= int(c.n_layers) <= MAX_LAYERS
+                or int(c.channels[0]) > MAX_LAYER0_CHANNELS):
+            # not a shape the kernels of csrc/convnet.cu are written for: depth > 1, other odd kernel sizes, 'gap' head,
+            # n_classes != 2, more than 16 layers or a layer 0 wider than 64 channels run on the generic channel-last ops
             # (riser/nets/cnn.py:8-65 in full; convnet_generic.py says what is still refused and why)
             from .convnet_generic import GenericConvNet
             self._generic = GenericConvNet(sd, c, self.device, self.logger)
@@ -211,9 +214,10 @@ class Model():
             if signal.ndim != 1 or signal.shape[0] < self._generic.min_length:
                 raise RuntimeError(f"signal of length {signal.shape} is shorter than {self._generic.min_length} samples")
             return self._generic.classify(signal)
-        if signal.ndim != 1 or signal.shape[0] < MIN_LENGTH:
-            # the reference dies in the 12th MaxPool1d for shorter input
-            raise RuntimeError(f"signal of length {signal.shape} is shorter than {MIN_LENGTH} samples")
+        min_length = max(MIN_LENGTH, 1 << self.n_layers)
+        if signal.ndim != 1 or signal.shape[0] < min_length:
+            # the reference's preprocessing needs 4096 samples, and its last MaxPool1d dies for fewer than 2 ** n_layers
+            raise RuntimeError(f"signal of length {signal.shape} is shorter than {min_length} samples")
         n = signal.shape[0]
         ld = (n + 1023) & ~1023
         x = torch.zeros(1, ld, dtype=torch.float32, device=self.device)
@@ -223,7 +227,8 @@ class Model():
 
     def classify_batch(self, x, lens, max_len=None, probs=None, feat=None, chunk=None, events=None):
         """x: fp32 [B, ld] normalised signals on the device (8-byte aligned rows, even
-        ld), lens: int32 [B] valid lengths (>= 4096; shorter -> NaN row).
+        ld), lens: int32 [B] valid lengths (>= max(MIN_LENGTH, 2 ** n_layers); a read shorter than
+        2 ** n_layers, length 0 included, gives a NaN row).
         Returns probs fp32 [B, 2] on the device.  No synchronisation.
 
         chunk: optionally run the network over sub-batches of this many reads, one plan

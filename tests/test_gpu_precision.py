@@ -79,13 +79,13 @@ def _state(scale=None):
     return sd
 
 
-def _inputs():
+def _inputs(lengths=LENGTHS, max_len=MAX_LEN):
     rng = np.random.default_rng(0)
-    normed = [pp.mad_normalise(synth.body(rng, n)) for n in LENGTHS]
-    x = torch.full((len(LENGTHS), MAX_LEN), POISON)            # poison beyond each read's length
+    normed = [pp.mad_normalise(synth.body(rng, n)) for n in lengths]
+    x = torch.full((len(lengths), max_len), POISON)            # poison beyond each read's length
     for b, v in enumerate(normed):
         x[b, :len(v)] = torch.from_numpy(np.asarray(v, dtype=np.float64)).float()
-    return x.cuda(), torch.tensor(LENGTHS, dtype=torch.int32).cuda()
+    return x.cuda(), torch.tensor(lengths, dtype=torch.int32).cuda()
 
 
 def _launches(plan, n):
@@ -118,20 +118,18 @@ def _check_format(planes, fmt, val, ctx):
     assert not bool(bad.any()), f"{ctx}: |lo| exceeds half an fp16 ulp of hi (split not round-to-nearest)"
 
 
-def run_variant(fuse, precision, env, monkeypatch, scale=None):
-    """Runs one forward and checks every launch; returns {launch key: (max ratio, rms ratio)}."""
-    monkeypatch.setenv("RISER_FUSE_L0", str(fuse))
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
-    state = _state(scale)
-    model = Model(state, CFG, LOG, "mRNA", precision=precision)
-    x, lens = _inputs()
+def check_every_launch(state, cfg, precision, lengths, max_len, beta, record=None):
+    """One forward of Model(state, cfg) over the reads `lengths` (poison beyond each length, max_len columns), then
+    every tensor-core launch of its plan against the float64 emulation, and the head against the GPU's own last
+    activation.  beta(i, terms, with_layer0) is the bar of the launch that starts at conv layer i.  Every length must
+    leave at least one row for the last pool.  Returns (model, {launch key: (max ratio, rms ratio)})."""
+    model = Model(state, cfg, LOG, "mRNA", precision=precision)
+    x, lens = _inputs(lengths, max_len)
     n = model.n_layers
-    feat = torch.zeros(len(LENGTHS), synth.CHANNELS[-1], device="cuda")
-    probs = model.classify_batch(x, lens, max_len=MAX_LEN, feat=feat)
+    feat = torch.zeros(len(lengths), model.channels[-1], device="cuda")
+    probs = model.classify_batch(x, lens, max_len=max_len, feat=feat)
     torch.cuda.synchronize()
-    plan = model.plan(len(LENGTHS), MAX_LEN)
-    assert plan.fused_layer0 == bool(fuse)
+    plan = model.plan(len(lengths), max_len)
     W = [state[f"layers.{i}.0.weight"].cuda() for i in range(n)]
     Bs = [state[f"layers.{i}.0.bias"].cuda() for i in range(n)]
     packs = {}
@@ -140,16 +138,17 @@ def run_variant(fuse, precision, env, monkeypatch, scale=None):
         fmt_in = plan.layer_format(i)
         fmt_out = plan.layer_format(j + 1) if j + 1 < n else 0
         terms = pe.terms_of(abs(fmt_in), precision)
-        key = f"L{i}{'+' + str(j) if j > i else ''}{'+0' if i == 1 and plan.fused_layer0 else ''}:" \
+        with_l0 = i == 1 and plan.fused_layer0
+        key = f"L{i}{'+' + str(j) if j > i else ''}{'+0' if with_l0 else ''}:" \
               f"{TERMS_NAME[terms]}:{plan.layer_kernel(i)}"
-        src = None if (i == 1 and plan.fused_layer0) else plan.planes(i, n)
+        src = None if with_l0 else plan.planes(i, n)
         out = plan.planes(j + 1, n, fmt_out or None)
         worst, sq, cnt = 0.0, 0.0, 0
-        for b, L0 in enumerate(LENGTHS):
+        for b, L0 in enumerate(lengths):
             rows_in, rows_out = L0 >> i, L0 >> (j + 1)
             if src is None:                                   # layer 0 inside layer 1's launch
                 xs = x[b, :L0]
-                a0 = pe.layer0_tc(xs, state["layers.0.0.weight"].cuda(), state["layers.0.0.bias"].cuda())
+                a0 = pe.layer0_tc(xs, W[0], Bs[0])
                 s_in = pe.layer0_bound(xs, W[0], Bs[0])
                 planes = pe.split_act(a0, fmt_in)
             else:
@@ -181,22 +180,37 @@ def run_variant(fuse, precision, env, monkeypatch, scale=None):
             cnt += d.numel()
         rms = math.sqrt(sq / max(cnt, 1))
         stats[key] = (worst, rms)
-        beta = BETA[terms][i - 1]
-        if worst > beta or rms > RMS_BAR[terms]:
-            failures.append((key, f"max {worst:.3g} (beta {beta:.3g})", f"rms {rms:.3g} (bar {RMS_BAR[terms]:.3g})"))
-    record = os.environ.get("RISER_PRECISION_RECORD")
-    if record:
-        with open(record, "a") as f:
-            f.write(json.dumps({"variant": [fuse, precision, env, scale], "stats": stats}) + "\n")
-    # head: feat = float64 mean of the GPU's own act_n rows; probs = softmax of the head on that feat
+        bar = beta(i, terms, with_l0)
+        if worst > bar or rms > RMS_BAR[terms]:
+            failures.append((key, f"max {worst:.3g} (beta {bar:.3g})", f"rms {rms:.3g} (bar {RMS_BAR[terms]:.3g})"))
+    path = os.environ.get("RISER_PRECISION_RECORD")
+    if path and record is not None:
+        with open(path, "a") as f:
+            f.write(json.dumps({"variant": record, "stats": stats}) + "\n")
+    # head: feat = float64 mean of the GPU's own act_n rows; probs = softmax of the head on that feat.  The head sums
+    # the (non-negative) rows one after another in fp32: each addition may round by 2^-24 of the partial sum
     act = plan.planes(n, n)[0].double()
-    want_feat = torch.stack([act[b, :L0 >> n].mean(0) for b, L0 in enumerate(LENGTHS)])
+    want_feat = torch.stack([act[b, :L0 >> n].mean(0) for b, L0 in enumerate(lengths)])
     fd = (feat.double() - want_feat).abs().max().item()
-    assert fd <= 2.0 ** -22 * want_feat.abs().max().item() + 1e-30, ("feat", fd)
+    rows = max(4, max(lengths) >> n)
+    assert fd <= rows * 2.0 ** -24 * want_feat.abs().max().item() + 1e-30, ("feat", fd)
     logits = feat.double() @ state["classifier.2.weight"].double().cuda().T + state["classifier.2.bias"].double().cuda()
     pd = (probs.double() - torch.softmax(logits, 1)).abs().max().item()
     assert pd <= 1e-6, ("probs", pd)
     assert not failures, failures
+    return model, stats
+
+
+def run_variant(fuse, precision, env, monkeypatch, scale=None):
+    """Runs one forward of the shipped network and checks every launch; returns {launch key: (max ratio, rms ratio)}."""
+    monkeypatch.setenv("RISER_FUSE_L0", str(fuse))
+    for k, v in env.items():
+        monkeypatch.setenv(k, v)
+    model, stats = check_every_launch(_state(scale), CFG, precision, LENGTHS, MAX_LEN,
+                                      lambda i, terms, with_l0: BETA[terms][i - 1],
+                                      record=[fuse, precision, env, scale])
+    assert model.plan(len(LENGTHS), MAX_LEN).fused_layer0 == bool(fuse)
+    return stats
 
 
 @pytest.mark.parametrize("name", list(VARIANTS))

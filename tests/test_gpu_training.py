@@ -334,8 +334,9 @@ def test_loss_falls_on_two_class_data(dev):
     assert np.mean(losses[-5:]) < 0.8 * np.mean(losses[:5])
 
 
-def test_checkpoint_round_trip(dev):
-    cfg = AttrDict({"model": "cnn", "cnn": dict(CNN_SHIPPED), "learning_rate": 1e-4})
+def _round_trip(cnn, dev):
+    """One trainer step, then the checkpoint through Model onto the dedicated kernels and through the reference module."""
+    cfg = AttrDict({"model": "cnn", "cnn": dict(cnn), "learning_rate": 1e-4})
     tr = ConvNetTrainer(cfg, seed=2)
     lens = [4096, 12048, 7000]
     x = _batch(lens, 12048, 9)
@@ -352,6 +353,16 @@ def test_checkpoint_round_trip(dev):
     err = (probs - want).abs().max().item()
     print(f"round trip: max |dp| {err:.2e}")
     assert err < 1e-3
+
+
+def test_checkpoint_round_trip(dev):
+    _round_trip(CNN_SHIPPED, dev)
+
+
+def test_checkpoint_round_trip_other_k3_shape(dev):
+    """A k = 3 network of the user's own shape (7 layers, other widths) also loads onto the dedicated kernels."""
+    _round_trip({"n_layers": 7, "depth": 1, "channels": [24, 32, 33, 47, 80, 129, 257], "kernels": [3] * 7,
+                 "n_classes": 2, "classifier": "gap_fc"}, dev)
 
 
 def test_fit_end_to_end(dev, tmp_path):
