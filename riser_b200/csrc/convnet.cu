@@ -170,6 +170,7 @@ struct LayerPlan {
   int eo = 0;                             // input in the even / odd plane layout -> conv_eo_kernel
   int fused_prev = 0;                     // computed inside the previous layer's launch: its input buffer is never written
   int kind = kTcKernel;                   // kEo2Kernel: this layer and the next one run as ONE conv_eo2_kernel launch
+  int kc = 0;                             // kFused01Kernel: the K-concatenated operand (fused01_kernel<4>)
   union {                                 // the kernel of `kind` (unset when fused_prev)
     ConvKernelFn tc;
     EoKernelFn eo;
@@ -2495,6 +2496,274 @@ int env_int(const char* name, int dflt) {
   return v ? atoi(v) : dflt;
 }
 
+constexpr int kABoxRows = 136;                               // haloed A tile rows: 130 needed; TMA likes multiples of 8
+constexpr size_t kSmemFixed = 1024 + sizeof(ConvSmem) + 64;  // beside a conv kernel's rings: alignment slack, ConvSmem
+
+// Layer i's K blocks and the shared-memory budgets both steps test.  Narrow layers take 32-channel K blocks (64-byte
+// rows, SWIZZLE_64B): no zero-filled half rows, twice the pipeline depth / sub-tiles per item in the same memory.
+struct LayerBudget {
+  bool k32, tc_resident, eo_fits, pair_resident;   // all weights (pair: each CTA's half) stay in shared memory
+  int row_bytes, kplanes, kb16, k_blocks, eo_acc, pair_n;   // kplanes: A tiles per K block; eo_acc: [even | odd] TMEM
+  size_t avail, b_bytes, w_all, a_group1, eo_group1;   // beside kSmemFixed; weight tile(s); a K block's A / E + O tiles
+  size_t pair_a, pair_hb, pair_hw;                 // conv_pair_kernel: A tile; a CTA's half of a weight tile, of all
+};
+LayerBudget layer_budget(const riser_model* m, int i, int max_smem) {
+  const LayerPack& L = m->layer[i];
+  LayerBudget g;
+  g.k32 = L.cin_p <= 80;
+  g.row_bytes = g.k32 ? 64 : 128;
+  g.kplanes = L.f8 ? 1 : m->act_planes;
+  g.kb16 = (L.cin_p + g.row_bytes / 2 - 1) / (g.row_bytes / 2);
+  g.k_blocks = g.kb16 + (L.f8 ? (2 * L.cin_p + g.row_bytes - 1) / g.row_bytes : 0);
+  g.eo_acc = round_up(2 * L.n_tile, 32);
+  g.pair_n = std::min(kMaxNTile, L.cout_p);
+  g.avail = static_cast<size_t>(max_smem) - kSmemFixed;
+  g.b_bytes = static_cast<size_t>(L.n_tile) * g.row_bytes;
+  g.w_all = static_cast<size_t>(L.passes) * 3 * g.k_blocks * g.b_bytes;
+  g.a_group1 = static_cast<size_t>(g.kplanes) * kABoxRows * g.row_bytes;
+  g.eo_group1 = static_cast<size_t>(m->act_planes) * 2 * kEoTile;
+  g.pair_a = static_cast<size_t>(kABoxRows) * 128;
+  g.pair_hb = static_cast<size_t>(g.pair_n / 2) * 128;
+  g.pair_hw = static_cast<size_t>(3) * g.k_blocks * g.pair_hb;
+  g.tc_resident = L.n_tiles == 1 && g.w_all + 2 * g.a_group1 <= g.avail;
+  g.eo_fits = g.w_all + 2 * g.eo_group1 <= g.avail;
+  g.pair_resident = L.n_tiles == 1 && g.pair_hw + 3 * g.pair_a <= g.avail;
+  return g;
+}
+void choose_kernels(riser_plan* p, int max_smem) {
+  const riser_model* m = p->model;
+  // These switches exist so that the test suite can reach, on the shipped network, the kernels that other shapes
+  // select on their own.
+  const bool fuse_l0 = env_int("RISER_FUSE_L0", 1) != 0, eo_on = env_int("RISER_EO", 1) != 0;
+  const bool pair_on = env_int("RISER_PAIR", 1) != 0, kc_on = env_int("RISER_KC", 1) != 0;
+  const bool fuse23 = env_int("RISER_FUSE23", 1) != 0;
+  constexpr int kPairFrom = 6;
+  for (int i = 1; i < m->n_layers; ++i) {
+    const LayerPack& L = m->layer[i];
+    const LayerBudget g = layer_budget(m, i, max_smem);
+    const bool last = (i == m->n_layers - 1);
+    LayerPlan& lp = p->layer[i];
+    // fused01_kernel stores fp16 rows only: a last layer (the head reads fp32) runs as layer0_kernel + conv_tc_kernel
+    if (i == 1 && fuse_l0 && !last && L.cin_p == 32 && L.n_tile == 32 && L.n_tiles == 1 && m->layer[0].cout <= 24) {
+      lp.kind = kFused01Kernel;
+      lp.kc = (L.wkc && m->layer[0].cout <= 20 && kc_on) ? 1 : 0;
+      p->fuse_l0 = 1;
+    } else if (eo_on && i >= 2 && i <= 4 && !last && !L.f8 && L.cin_p <= 80 && L.n_tiles == 1 &&
+               2 * L.n_tile <= kMaxNTile && g.eo_fits) {   // the narrow resident-weight layers 2..4
+      lp.kind = kEoKernel;
+      lp.eo = 1;
+    } else if (pair_on && L.f8 && !g.tc_resident && !g.k32 && (L.n_tile % 16) == 0 &&
+               (i >= kPairFrom || g.pair_resident)) {
+      // CTA pairs take the streamed-weight F16_F8 layers from layer kPairFrom on, and earlier ones (layer 5 of the
+      // shipped network) only when each CTA's half of the weights stays resident
+      lp.kind = kPairKernel;
+    }
+  }
+  // Two consecutive even / odd layers as ONE launch (conv_eo2_kernel): the first such pair (layers 2 + 3 of the shipped
+  // network), when both are hi + lo plane layers, the accumulators fit the TMEM and everything fits shared memory.
+  for (int i = 2; fuse23 && m->act_planes == 2 && i + 1 < m->n_layers - 1; ++i) {
+    const LayerPack &L1 = m->layer[i], &L2 = m->layer[i + 1];
+    const LayerBudget g1 = layer_budget(m, i, max_smem), g2 = layer_budget(m, i + 1, max_smem);
+    if (p->layer[i].eo && p->layer[i + 1].eo && L1.passes == 2 && L2.passes == 2 && !L1.f8 && !L2.f8 &&
+        3 * g1.eo_acc + g2.eo_acc <= kTmemCols && L1.n_tile <= 128 && L2.n_tile <= 128 &&
+        conv_eo2_smem(L1.n_tile, L2.n_tile, g1.k_blocks, g2.k_blocks) <= static_cast<size_t>(max_smem)) {
+      p->layer[i].kind = p->layer[i + 1].kind = kEo2Kernel;
+      p->layer[i + 1].fused_prev = 1;
+      break;
+    }
+  }
+}
+// The ConvArgs fields all conv kernels share: lengths, K and N tiling, output format and layout, pointers
+ConvArgs conv_args(const riser_plan* p, int i, const LayerBudget& g, int m_rows, int n_tile) {
+  const LayerPack& L = p->model->layer[i];
+  const bool last = (i == p->model->n_layers - 1);
+  ConvArgs a = {};
+  a.bias = L.bias;
+  a.out = p->ws + p->act_off[i + 1];
+  a.rows_in = p->B * p->Lp[i];
+  a.Lp_in = p->Lp[i];
+  a.Lp_out = p->Lp[i + 1];
+  a.half_lp = p->Lp[i] / 2;
+  a.half_lp_out = p->Lp[i + 1] / 2;
+  a.n_pairs_out = p->B * p->Lp[i + 1] / 2;
+  a.pair_magic = ((1ull << 40) / static_cast<unsigned long long>(a.half_lp)) + 1ull;
+  a.shift = i + 1;
+  a.cin_p = L.cin_p;
+  a.cout_p = L.cout_p;
+  a.kb16 = g.kb16;
+  a.k_blocks = g.k_blocks;
+  a.k32 = g.k32 ? 1 : 0;
+  a.f8 = L.f8;
+  a.planes = g.kplanes;
+  a.wplanes = L.passes;
+  a.a_tx_bytes = kABoxRows * g.row_bytes;
+  a.n_tile = n_tile;
+  a.n_tiles = (L.cout_p + n_tile - 1) / n_tile;
+  a.idesc = umma_idesc_f16(m_rows, n_tile);
+  a.w_inv_scale = L.w_inv_scale;
+  a.out_fp32 = last ? 1 : 0;
+  a.out_planes = last ? 1 : p->model->act_planes;
+  a.out_f8 = (!last && p->model->layer[i + 1].f8) ? 1 : 0;   // the epilogue writes the format the next layer reads
+  a.out_eo = (!last && p->layer[i + 1].eo) ? 1 : 0;           // ... and the row layout it reads
+  a.epi_sets = kMaxEpiSets;
+  return a;
+}
+// Weight maps (box_rows rows): fp16 [plane][tap][cout_p][cin_p]; e4m3 [tap][cout_p][2 cin_p], or a copy when not F16_F8
+int weight_maps(CUtensorMap* b, CUtensorMap* b8, const LayerPack& L, uint32_t box_rows, bool k32) {
+  const int st = make_tmap(b, L.w, L.cin_p, static_cast<uint64_t>(L.passes) * 3 * L.cout_p, box_rows, k32);
+  if (!st && L.f8) return make_tmap8(b8, L.w8, 2ull * L.cin_p, 2ull * L.cin_p, 3ull * L.cout_p, box_rows, k32);
+  *b8 = *b;
+  return st;
+}
+int flat_maps(LayerPlan& lp, const riser_plan* p, int i, uint32_t b_rows, bool k32) {
+  const LayerPack& L = p->model->layer[i];
+  char* act = p->ws + p->act_off[i];
+  const int rows = p->B * p->Lp[i];
+  int st = make_tmap(&lp.tm_a, act, static_cast<uint64_t>(L.cin_p) * p->model->act_planes, rows, kABoxRows, k32);
+  if (!st && L.f8) st = make_tmap8(&lp.tm_a8, act, 4ull * L.cin_p, 4ull * L.cin_p, rows, kABoxRows, k32);
+  else lp.tm_a8 = lp.tm_a;
+  return st ? st : weight_maps(&lp.tm_b, &lp.tm_b8, L, b_rows, k32);
+}
+int configure_tc(riser_plan* p, int i, const LayerBudget& g, const void** fn) {
+  const LayerPack& L = p->model->layer[i];
+  LayerPlan& lp = p->layer[i];
+  ConvArgs& a = lp.args = conv_args(p, i, g, kBlockM, L.n_tile);
+  a.acc_cols = round_up(L.n_tile, 32);
+  a.resident = g.tc_resident ? 1 : 0;
+  if (a.resident) {
+    // the most 128-row sub-tiles per item that leave >= 2 accumulator stages and A groups (amortises per-item work)
+    for (a.ms = 4; a.ms > 1; a.ms >>= 1)
+      if (2 * a.ms * a.acc_cols <= kTmemCols && g.w_all + 2 * a.ms * g.a_group1 <= g.avail &&
+          static_cast<int64_t>(a.rows_in) / (a.ms * kBlockM) >= 2 * p->model->sm_count)
+        break;
+    a.b_stages = 1;
+    a.a_stages = std::min<int>(kMaxAStages, static_cast<int>((g.avail - g.w_all) / (a.ms * g.a_group1)));
+    lp.smem = kSmemFixed + g.w_all + static_cast<size_t>(a.a_stages) * a.ms * g.a_group1;
+  } else {
+    a.ms = (2 * a.acc_cols <= kTmemCols) ? 2 : 1;
+    if (4 * a.acc_cols <= kTmemCols && 2 * 4 * g.a_group1 + 3 * g.b_bytes <= g.avail)
+      a.ms = 4;       // more rows per streamed weight tile (narrow layers / 32-channel K blocks)
+    // smem split: at least 2 A groups and 2 B stages; a third A group when that still leaves 4+ B stages
+    while (a.ms > 1 && 2 * a.ms * g.a_group1 + 2 * g.b_bytes > g.avail) a.ms >>= 1;
+    const size_t a_group = a.ms * g.a_group1;
+    a.a_stages = (static_cast<int>((g.avail - 2 * a_group) / g.b_bytes) > 4 && 3 * a_group + 4 * g.b_bytes <= g.avail)
+                     ? 3 : 2;
+    a.b_stages = std::max(2, std::min(kMaxBStages, static_cast<int>((g.avail - a.a_stages * a_group) / g.b_bytes)));
+    lp.smem = kSmemFixed + static_cast<size_t>(a.a_stages) * a_group + static_cast<size_t>(a.b_stages) * g.b_bytes;
+  }
+  a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / (a.ms * a.acc_cols)));
+  a.dual = (a.ms == 2 && !a.resident) ? 1 : 0;
+  lp.rows_per_super = a.ms * kBlockM;
+  lp.block = 64 + 128 * a.epi_sets + (a.dual ? 32 : 0);
+  lp.fn.tc = pick_conv_kernel(a.ms, a.planes, a.wplanes, a.resident, a.k32, a.f8);
+  *fn = reinterpret_cast<const void*>(lp.fn.tc);
+  return flat_maps(lp, p, i, L.n_tile, g.k32);
+}
+// layers 0 + 1 on the tensor pipe: work item = 255 pooled outputs = 510 input rows
+int configure_fused01(riser_plan* p, const LayerBudget& g, const void** fn) {
+  const riser_model* m = p->model;
+  const LayerPack& L = m->layer[1];
+  LayerPlan& lp = p->layer[1];
+  ConvArgs& a = lp.args = conv_args(p, 1, g, kBlockM, L.n_tile);
+  a.w0 = m->layer[0].w0;
+  a.b0 = m->layer[0].bias;
+  a.cout0 = m->layer[0].cout;
+  lp.rows_per_super = 2 * kF2Pairs;
+  lp.smem = fused01_smem(m->act_planes, L.f8 ? 2 : L.passes);
+  lp.fn.fused01 = pick_fused01(lp.kc ? 4 : L.f8 ? 3 : (m->act_planes == 2 ? 2 : (L.passes == 2 ? 1 : 0)));
+  lp.block = kF2Threads;
+  *fn = reinterpret_cast<const void*>(lp.fn.fused01);
+  // kc: the three hi / lo terms concatenated along K, [tap][cout_p][64]; same shared-memory footprint
+  if (lp.kc) return make_tmap(&lp.tm_b, L.wkc, 64, 3ull * L.cout_p, 32, false);
+  return weight_maps(&lp.tm_b, &lp.tm_b8, L, L.n_tile, true);
+}
+// conv_eo_kernel; the launch of a conv_eo2_kernel pair reads both layers' maps and arguments (not their launch fields)
+int configure_eo(riser_plan* p, int i, const LayerBudget& g, const void** fn) {
+  const LayerPack& L = p->model->layer[i];
+  LayerPlan& lp = p->layer[i];
+  ConvArgs& a = lp.args = conv_args(p, i, g, kBlockM, L.n_tile);
+  a.acc_cols = g.eo_acc;
+  a.ms = (2 * 2 * a.acc_cols <= kTmemCols && g.w_all + 2 * 2 * g.eo_group1 <= g.avail) ? 2 : 1;
+  a.a_stages = std::min<int>(kMaxAStages, static_cast<int>((g.avail - g.w_all) / (a.ms * g.eo_group1)));
+  a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / (a.ms * a.acc_cols)));
+  lp.rows_per_super = a.ms * 2 * kBlockM;
+  if (lp.kind == kEoKernel) {
+    lp.smem = kSmemFixed + g.w_all + static_cast<size_t>(a.a_stages) * a.ms * g.eo_group1;
+    lp.block = 64 + 128 * a.epi_sets;
+    *fn = reinterpret_cast<const void*>(lp.fn.eo = pick_conv_eo(a.ms, a.planes, a.wplanes));
+  }
+  // E plane = rows [0, n_pairs), O plane = rows [n_pairs, 2 n_pairs) of the same buffer
+  const uint64_t n_pairs = a.rows_in / 2, pitch = static_cast<uint64_t>(L.cin_p) * p->model->act_planes;   // fp16 / row
+  int st = make_tmap(&lp.tm_a, p->ws + p->act_off[i], pitch, n_pairs, kABoxRows, true);
+  if (!st) st = make_tmap(&lp.tm_a8, p->ws + p->act_off[i] + n_pairs * pitch * 2, pitch, n_pairs, kABoxRows, true);
+  return st ? st : weight_maps(&lp.tm_b, &lp.tm_b8, L, L.n_tile, true);
+}
+// layers i and i + 1, each with its configure_eo arguments, as one conv_eo2_kernel launch
+void configure_eo2(riser_plan* p, int i, const void** fn) {
+  LayerPlan& l1 = p->layer[i];
+  const ConvArgs &a1 = l1.args, &a2 = p->layer[i + 1].args;
+  Eo2Args& e = l1.eo2;
+  e.kb1 = a1.k_blocks;
+  e.kb2 = a2.k_blocks;
+  e.n1 = a1.n_tile;
+  e.n2 = a2.n_tile;
+  e.acc1 = a1.acc_cols;
+  e.acc2 = a2.acc_cols;
+  e.bias1 = a1.bias;
+  e.bias2 = a2.bias;
+  e.out = a2.out;
+  e.B = p->B;
+  e.Lp_out = a2.Lp_out;
+  e.n_seg = (e.Lp_out + kE2Rows - 1) / kE2Rows;
+  e.half_lp_in = a1.half_lp;
+  e.half_lp_out = a2.half_lp_out;
+  e.n_pairs_out = a2.n_pairs_out;
+  e.out_eo = a2.out_eo;
+  e.out_f8 = a2.out_f8;
+  e.out_planes = a2.out_planes;
+  e.cout_p2 = a2.cout_p;
+  e.shift1 = a1.shift;
+  e.shift2 = a2.shift;
+  e.cin_p1 = a1.cin_p;
+  e.idesc1_n = a1.idesc;
+  e.idesc1_2n = umma_idesc_f16(kBlockM, 2 * e.n1);
+  e.idesc2_n = a2.idesc;
+  e.idesc2_2n = umma_idesc_f16(kBlockM, 2 * e.n2);
+  e.inv_scale1 = a1.w_inv_scale;
+  e.inv_scale2 = a2.w_inv_scale;
+  l1.grid = std::min(e.B * e.n_seg, p->model->sm_count);
+  l1.smem = conv_eo2_smem(e.n1, e.n2, e.kb1, e.kb2);
+  l1.block = kE2Threads;
+  *fn = reinterpret_cast<const void*>(l1.fn.eo2 = conv_eo2_kernel);
+}
+// conv_pair_kernel: M = 256 over two CTAs, each holds 128 rows of A and half of every weight tile
+int configure_pair(riser_plan* p, int i, const LayerBudget& g, const void** fn) {
+  const LayerPack& L = p->model->layer[i];
+  LayerPlan& lp = p->layer[i];
+  // N tiles 256 wide (the widest M = 256 MMA: fewest shared-memory operand bytes per MAC) with ONE narrower last tile
+  // instead of equal tiles -- cout_p itself (the next layer's K) is unchanged
+  ConvArgs& a = lp.args = conv_args(p, i, g, 256, g.pair_n);
+  a.n_last = L.cout_p - (a.n_tiles - 1) * a.n_tile;
+  a.idesc_last = umma_idesc_f16(256, a.n_last);
+  // item / n_tiles by multiply-high; with one N tile the magic would overflow, and the kernel divides instead
+  a.nt_magic = a.n_tiles > 1 ? static_cast<uint32_t>((1ull << 32) / static_cast<unsigned>(a.n_tiles)) + 1u : 0u;
+  a.acc_cols = round_up(a.n_tile, 32);
+  // One 256-row sub-tile per item and two accumulator stages: layers 6-11 in situ 0.38 / 0.47 / 0.37 / 0.38 / 0.46 /
+  // 0.49 ms, against 0.41 / 0.47 / 0.40 / 0.43 / 0.48 / 0.55 with two sub-tiles (they leave the TMEM one item deep)
+  a.ms = 1;
+  int a_st = 5;         // A stages beside streamed weights (the kernel sets up b_stages even when they are resident)
+  while (a_st > 2 && a_st * g.pair_a + 4 * g.pair_hb > g.avail) --a_st;
+  a.b_stages = std::max(2, std::min<int>(kMaxBStages, static_cast<int>((g.avail - a_st * g.pair_a) / g.pair_hb)));
+  a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / a.acc_cols));
+  a.resident = g.pair_resident ? 1 : 0;
+  a.a_stages = a.resident ? std::min<int>(kMaxAStages, static_cast<int>((g.avail - g.pair_hw) / g.pair_a)) : a_st;
+  lp.rows_per_super = 256;
+  lp.smem = kSmemFixed + a.a_stages * g.pair_a + (a.resident ? g.pair_hw : a.b_stages * g.pair_hb);
+  lp.block = 64 + 128 * a.epi_sets;
+  *fn = reinterpret_cast<const void*>(lp.fn.pair = conv_pair_kernel);
+  const int st = flat_maps(lp, p, i, a.n_tile / 2, false);
+  return st ? st : weight_maps(&lp.tm_bl, &lp.tm_b8l, L, a.n_last / 2, false);
+}
 }  // namespace
 }  // namespace riser
 
@@ -2634,18 +2903,13 @@ extern "C" size_t riser_workspace_bytes(const riser_model* m, int B, int max_len
   return plan_offsets(m, B, Lp, off);
 }
 
+// Two steps: choose_kernels picks the kernel of every conv layer, then that kernel's configure_* function fills in its
+// arguments, tensor maps, shared memory, block and kernel pointer.  Both steps test the budgets of layer_budget.
 extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, int max_len, void* workspace,
                                  size_t workspace_bytes, riser_stream_t stream) {
   RISER_REQUIRE(out && m && workspace, "riser_plan_create: null pointer");
   RISER_REQUIRE(B > 0 && max_len >= kMinLen, "riser_plan_create: need B > 0 and max_len >= %d", kMinLen);
   RISER_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "riser_plan_create: workspace not 256-byte aligned");
-  // These switches exist so that the test suite can reach, on the shipped network, the kernels that other shapes
-  // select on their own.
-  const bool fuse_l0 = env_int("RISER_FUSE_L0", 1) != 0;
-  const bool eo_on = env_int("RISER_EO", 1) != 0;
-  const bool pair_on = env_int("RISER_PAIR", 1) != 0;
-  const bool kc_on = env_int("RISER_KC", 1) != 0;
-  const bool fuse23 = env_int("RISER_FUSE23", 1) != 0;
   std::unique_ptr<riser_plan, int (*)(riser_plan*)> owner(new riser_plan(), riser_plan_destroy);   // freed on every error return
   riser_plan* p = owner.get();
   p->model = m;
@@ -2655,297 +2919,34 @@ extern "C" int riser_plan_create(riser_plan** out, const riser_model* m, int B, 
   int Lmax[kMaxLayers + 1];
   plan_lengths(m, max_len, Lmax, p->Lp);
   const size_t need = plan_offsets(m, B, p->Lp, p->act_off);
-  if (workspace_bytes < need) {
+  if (workspace_bytes < need)
     return fail(RISER_ENOMEM, "riser_plan_create: workspace %zu < %zu bytes", workspace_bytes, need);
-  }
   RISER_REQUIRE(static_cast<int64_t>(B) * p->Lp[1] * 8 < (int64_t(1) << 31), "riser_plan_create: B * L too large");
   RISER_CUDA_TRY(cudaMemsetAsync(workspace, 0, need, as_stream(stream)));
   int max_smem = 0;
   RISER_CUDA_TRY(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, m->device));
 
-  // Even / odd plane layout (conv_eo_kernel) for the narrow resident-weight layers 2..4
-  if (eo_on)
-    for (int i = 2; i < m->n_layers - 1 && i <= 4; ++i) {
-      const LayerPack& L = m->layer[i];
-      const size_t w_all = static_cast<size_t>(L.passes) * ((L.cin_p + 31) / 32) * 3 * L.n_tile * 64;
-      const size_t group1 = static_cast<size_t>(m->act_planes) * 2 * kEoTile;
-      if (!L.f8 && L.cin_p <= 80 && L.n_tiles == 1 && 2 * L.n_tile <= kMaxNTile &&
-          w_all + 2 * group1 + 1024 + sizeof(ConvSmem) + 64 <= static_cast<size_t>(max_smem))
-        p->layer[i].eo = 1;
-    }
-
+  choose_kernels(p, max_smem);
   for (int i = 1; i < m->n_layers; ++i) {
-    const LayerPack& L = m->layer[i];
     LayerPlan& lp = p->layer[i];
-    const int rows_in = B * p->Lp[i];
-    const bool last = (i == m->n_layers - 1);
-    const int a_box_rows = 136;   // 130 needed; a multiple of 8 is what TMA likes
-    // fused01_kernel stores fp16 rows only: a last layer (the head reads fp32) runs as layer0_kernel + conv_tc_kernel
-    const bool fuse01 = (i == 1 && fuse_l0 && !last && L.cin_p == 32 && L.n_tile == 32 && L.n_tiles == 1 &&
-                         m->layer[0].cout <= 24);
-    // 32-channel K blocks (64-byte rows, SWIZZLE_64B) for narrow layers: no zero-filled half rows,
-    // twice the pipeline depth / sub-tiles per item in the same shared memory
-    const bool k32 = fuse01 || L.cin_p <= 80;
-    const int row_bytes = k32 ? 64 : 128;
-    const int k_elems = row_bytes / 2;
-    int st = make_tmap(&lp.tm_a, p->ws + p->act_off[i], static_cast<uint64_t>(L.cin_p) * m->act_planes, rows_in,
-                       a_box_rows, k32);
-    if (!st) st = make_tmap(&lp.tm_b, L.w, L.cin_p, static_cast<uint64_t>(L.passes) * 3 * L.cout_p, L.n_tile, k32);
-    if (!st && L.f8) {
-      st = make_tmap8(&lp.tm_a8, p->ws + p->act_off[i], 4ull * L.cin_p, 4ull * L.cin_p, rows_in, a_box_rows, k32);
-      if (!st) st = make_tmap8(&lp.tm_b8, L.w8, 2ull * L.cin_p, 2ull * L.cin_p, 3ull * L.cout_p, L.n_tile, k32);
-    } else {
-      lp.tm_a8 = lp.tm_a;
-      lp.tm_b8 = lp.tm_b;
-    }
+    const LayerBudget g = layer_budget(m, i, max_smem);
+    const void* fn = nullptr;      // the kernel this layer launches, if any
+    const int st = lp.kind == kFused01Kernel ? configure_fused01(p, g, &fn)
+                   : lp.kind == kPairKernel  ? configure_pair(p, i, g, &fn)
+                   : lp.kind == kTcKernel    ? configure_tc(p, i, g, &fn)
+                                             : configure_eo(p, i, g, &fn);   // also both conv_eo2_kernel layers
     if (st) return st;
-    ConvArgs& a = lp.args;
-    std::memset(&a, 0, sizeof(a));
-    a.bias = L.bias;
-    a.out = p->ws + p->act_off[i + 1];
-    a.rows_in = rows_in;
-    a.Lp_in = p->Lp[i];
-    a.Lp_out = p->Lp[i + 1];
-    a.shift = i + 1;
-    a.cin_p = L.cin_p;
-    a.cout_p = L.cout_p;
-    a.n_tile = L.n_tile;
-    a.n_tiles = L.n_tiles;
-    a.kb16 = (L.cin_p + k_elems - 1) / k_elems;
-    a.k_blocks = a.kb16 + (L.f8 ? (2 * L.cin_p + row_bytes - 1) / row_bytes : 0);
-    a.k32 = k32 ? 1 : 0;
-    a.f8 = L.f8;
-    a.out_f8 = (!last && m->layer[i + 1].f8) ? 1 : 0;   // the epilogue writes the format the next layer reads
-    a.out_eo = (!last && p->layer[i + 1].eo) ? 1 : 0;    // ... and the row layout it reads
-    a.n_pairs_out = B * p->Lp[i + 1] / 2;
-    a.half_lp_out = p->Lp[i + 1] / 2;
-    const int kplanes = L.f8 ? 1 : m->act_planes;      // activation tiles per K block
-    a.planes = kplanes;
-    a.wplanes = L.passes;
-    a.out_fp32 = last ? 1 : 0;
-    a.out_planes = last ? 1 : m->act_planes;
-    a.idesc = umma_idesc_f16(kBlockM, L.n_tile);
-    a.w_inv_scale = L.w_inv_scale;
-    a.acc_cols = round_up(L.n_tile, 32);
-    a.half_lp = p->Lp[i] / 2;
-    a.a_tx_bytes = a_box_rows * row_bytes;
-    a.pair_magic = ((1ull << 40) / static_cast<unsigned long long>(a.half_lp)) + 1ull;
-    const size_t b_bytes = static_cast<size_t>(L.n_tile) * row_bytes;
-    const size_t fixed = 1024 + sizeof(ConvSmem) + 64;
-    const size_t avail = static_cast<size_t>(max_smem) - fixed;
-    const size_t w_all = static_cast<size_t>(L.passes) * 3 * a.k_blocks * b_bytes;
-    const size_t a_group1 = static_cast<size_t>(kplanes) * 136 * row_bytes;
-    if (L.n_tiles == 1 && w_all + 2 * a_group1 <= avail) {
-      // resident weights; as many 128-row sub-tiles per work item as leave >= 2 accumulator
-      // stages and >= 2 A groups in flight (amortises the per-item bookkeeping of small-N layers)
-      a.resident = 1;
-      a.ms = 1;
-      for (int ms = 4; ms > 1; ms >>= 1)
-        if (2 * ms * a.acc_cols <= kTmemCols && w_all + 2 * ms * a_group1 <= avail &&
-            static_cast<int64_t>(rows_in) / (ms * kBlockM) >= 2 * m->sm_count) {
-          a.ms = ms;
-          break;
-        }
-      a.b_stages = 1;
-      a.a_stages = std::min<int>(kMaxAStages, static_cast<int>((avail - w_all) / (a.ms * a_group1)));
-      lp.smem = fixed + w_all + static_cast<size_t>(a.a_stages) * a.ms * a_group1;
-    } else {
-      a.resident = 0;
-      a.ms = (2 * a.acc_cols <= kTmemCols) ? 2 : 1;
-      if (4 * a.acc_cols <= kTmemCols && 2 * 4 * a_group1 + 3 * b_bytes <= avail)
-        a.ms = 4;       // more rows per streamed weight tile (narrow layers / 32-channel K blocks)
-      // smem split: at least 2 A groups and 2 B stages; prefer 3+ B stages
-      while (a.ms > 1 && 2 * a.ms * a_group1 + 2 * b_bytes > avail) a.ms >>= 1;
-      const size_t a_group = a.ms * a_group1;
-      int a_st = 2;
-      int b_st = static_cast<int>((avail - a_st * a_group) / b_bytes);
-      if (b_st > 4 && (a_st + 1) * a_group + 4 * b_bytes <= avail) {
-        a_st = 3;
-        b_st = static_cast<int>((avail - a_st * a_group) / b_bytes);
-      }
-      a.a_stages = a_st;
-      a.b_stages = std::max(2, std::min(kMaxBStages, b_st));
-      lp.smem = fixed + static_cast<size_t>(a.a_stages) * a_group + static_cast<size_t>(a.b_stages) * b_bytes;
-    }
-    a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / (a.ms * a.acc_cols)));
-    a.dual = (a.ms == 2 && !a.resident) ? 1 : 0;
-    a.epi_sets = kMaxEpiSets;
-    lp.rows_per_super = a.ms * kBlockM;
-    bool kc = false;
-    if (fuse01) {
-      // layers 0 + 1 on the tensor pipe (fused01_kernel): work item = 255 pooled outputs = 510 input rows
-      p->fuse_l0 = 1;
-      lp.kind = kFused01Kernel;
-      a.w0 = m->layer[0].w0;
-      a.b0 = m->layer[0].bias;
-      a.cout0 = m->layer[0].cout;
-      lp.rows_per_super = 2 * kF2Pairs;
-      lp.smem = fused01_smem(m->act_planes, L.f8 ? 2 : L.passes);
-      a.planes = m->act_planes;     // fused01_kernel's own modes (see pick_fused01)
-      if (L.wkc && m->layer[0].cout <= 20 && kc_on) {
-        kc = true;      // the three hi / lo terms concatenated along K (fused01_kernel<4>); same shared-memory footprint
-        const int st3 = make_tmap(&lp.tm_b, L.wkc, 64, 3ull * L.cout_p, 32, false);
-        if (st3) return st3;
-      }
-    }
-    if (lp.eo) {
-      // conv_eo_kernel: E plane = rows [0, n_pairs), O plane = rows [n_pairs, 2 n_pairs) of the same buffer
-      lp.kind = kEoKernel;
-      const uint64_t n_pairs = static_cast<uint64_t>(rows_in) / 2;
-      const uint64_t pitch = static_cast<uint64_t>(L.cin_p) * m->act_planes;     // fp16 elements per row
-      int st2 = make_tmap(&lp.tm_a, p->ws + p->act_off[i], pitch, n_pairs, 136, true);
-      if (!st2) st2 = make_tmap(&lp.tm_a8, p->ws + p->act_off[i] + n_pairs * pitch * 2, pitch, n_pairs, 136, true);
-      if (st2) return st2;
-      a.acc_cols = round_up(2 * L.n_tile, 32);
-      const size_t w_eo = static_cast<size_t>(L.passes) * a.k_blocks * 3 * b_bytes;
-      const size_t group1 = static_cast<size_t>(m->act_planes) * 2 * kEoTile;
-      a.ms = (2 * 2 * a.acc_cols <= kTmemCols && w_eo + 2 * 2 * group1 <= avail) ? 2 : 1;
-      a.resident = 1;
-      a.a_stages = std::min<int>(kMaxAStages, static_cast<int>((avail - w_eo) / (a.ms * group1)));
-      a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / (a.ms * a.acc_cols)));
-      a.epi_sets = 4;
-      lp.smem = fixed + w_eo + static_cast<size_t>(a.a_stages) * a.ms * group1;
-      lp.rows_per_super = a.ms * 2 * kBlockM;
-    }
-    // CTA pairs take the streamed-weight F16_F8 layers from layer kPairFrom on, and earlier ones (layer 5 of the shipped
-    // network) only when each CTA's half of the weights stays resident
-    constexpr int kPairFrom = 6;
-    if (L.f8 && !a.resident && !k32 && !lp.eo && (L.n_tile % 16) == 0 && pair_on &&
-        (i >= kPairFrom ||
-         (L.n_tiles == 1 && static_cast<size_t>(3) * a.k_blocks * (L.cout_p / 2) * 128 + 3 * 136 * 128 <= avail))) {
-      // conv_pair_kernel: M = 256 over two CTAs, each holds 128 rows of A and half of every weight tile
-      // N tiles of the pair kernel: 256 wide (the widest M = 256 MMA: fewest shared-memory operand bytes per MAC)
-      // with ONE narrower last tile instead of equal tiles -- cout_p itself (the next layer's K) is unchanged
-      lp.kind = kPairKernel;
-      a.n_tile = std::min(kMaxNTile, L.cout_p);
-      a.n_tiles = (L.cout_p + a.n_tile - 1) / a.n_tile;
-      a.n_last = L.cout_p - (a.n_tiles - 1) * a.n_tile;
-      a.acc_cols = round_up(a.n_tile, 32);
-      int st2 = make_tmap(&lp.tm_b, L.w, L.cin_p, 3ull * L.cout_p, a.n_tile / 2, false);
-      if (!st2) st2 = make_tmap8(&lp.tm_b8, L.w8, 2ull * L.cin_p, 2ull * L.cin_p, 3ull * L.cout_p, a.n_tile / 2, false);
-      if (!st2) st2 = make_tmap(&lp.tm_bl, L.w, L.cin_p, 3ull * L.cout_p, a.n_last / 2, false);
-      if (!st2) st2 = make_tmap8(&lp.tm_b8l, L.w8, 2ull * L.cin_p, 2ull * L.cin_p, 3ull * L.cout_p, a.n_last / 2, false);
-      if (st2) return st2;
-      a.idesc = umma_idesc_f16(256, a.n_tile);
-      a.idesc_last = umma_idesc_f16(256, a.n_last);
-      // One 256-row sub-tile per item and two accumulator stages is the measured optimum (layers 6-11 in situ: 0.38 /
-      // 0.47 / 0.37 / 0.38 / 0.46 / 0.49 ms against 0.41 / 0.47 / 0.40 / 0.43 / 0.48 / 0.55 with two sub-tiles, which
-      // halve the weight bytes streamed per MAC but leave the TMEM one item deep, even with one issuing warp per
-      // sub-tile).
-      a.ms = 1;
-      const size_t a_group = static_cast<size_t>(136) * 128, half_b = static_cast<size_t>(a.n_tile / 2) * 128;
-      a.a_stages = 5;
-      while (a.a_stages > 2 && a.a_stages * a_group + 4 * half_b > avail) --a.a_stages;
-      a.b_stages = std::max(2, std::min<int>(kMaxBStages, static_cast<int>((avail - a.a_stages * a_group) / half_b)));
-      a.acc_stages = std::max(1, std::min(kMaxAccStages, kTmemCols / a.acc_cols));
-      a.dual = 0;
-      a.resident = 0;
-      size_t b_total = a.b_stages * half_b;
-      const size_t w_half = static_cast<size_t>(3) * a.k_blocks * half_b;      // this CTA's half of every tap and K block
-      if (a.n_tiles == 1 && w_half + 3 * a_group <= avail) {
-        a.resident = 1;
-        a.a_stages = std::min<int>(kMaxAStages, static_cast<int>((avail - w_half) / a_group));
-        b_total = w_half;
-      }
-      a.epi_sets = 4;
-      // item / n_tiles by multiply-high; with one N tile the magic would overflow, and the kernel divides instead
-      a.nt_magic = a.n_tiles > 1 ? static_cast<uint32_t>((1ull << 32) / static_cast<unsigned>(a.n_tiles)) + 1u : 0u;
-      lp.smem = fixed + a.a_stages * a_group + b_total;
-      lp.rows_per_super = 256;
-    }
+    if (lp.fused_prev) configure_eo2(p, i - 1, &fn);   // once the second layer has its arguments
     // every launch covers the whole batch
-    a.n_supers = (rows_in + lp.rows_per_super - 1) / lp.rows_per_super;
-    const int n_items = a.n_supers * a.n_tiles;
-    lp.grid = std::min(n_items, m->sm_count);
-    const void* fn = nullptr;
-    switch (lp.kind) {
-      case kFused01Kernel:
-        lp.fn.fused01 = pick_fused01(kc ? 4 : a.f8 ? 3 : (a.planes == 2 ? 2 : (a.wplanes == 2 ? 1 : 0)));
-        lp.block = kF2Threads;
-        fn = reinterpret_cast<const void*>(lp.fn.fused01);
-        break;
-      case kEoKernel:
-        lp.fn.eo = pick_conv_eo(a.ms, a.planes, a.wplanes);
-        lp.block = 64 + 128 * a.epi_sets;
-        fn = reinterpret_cast<const void*>(lp.fn.eo);
-        break;
-      case kPairKernel:
-        lp.fn.pair = conv_pair_kernel;
-        lp.grid = std::min(2 * n_items, m->sm_count & ~1);
-        lp.block = 64 + 128 * a.epi_sets;
-        fn = reinterpret_cast<const void*>(lp.fn.pair);
-        break;
-      default:
-        lp.fn.tc = pick_conv_kernel(a.ms, a.planes, a.wplanes, a.resident, a.k32, a.f8);
-        lp.block = 64 + 128 * a.epi_sets + (a.dual ? 32 : 0);
-        fn = reinterpret_cast<const void*>(lp.fn.tc);
-    }
-    RISER_CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-  }
-  // Two consecutive even / odd layers as ONE launch (conv_eo2_kernel): the first such pair (layers 2 + 3 of the shipped
-  // network), when both are hi + lo plane layers, the accumulators fit the TMEM and everything fits shared memory.
-  if (fuse23 && m->act_planes == 2)
-    for (int i = 2; i + 1 < m->n_layers - 1; ++i) {
-      LayerPlan& l1 = p->layer[i];
-      LayerPlan& l2 = p->layer[i + 1];
-      const LayerPack& L1 = m->layer[i];
-      const LayerPack& L2 = m->layer[i + 1];
-      if (!(l1.eo && l2.eo && L1.passes == 2 && L2.passes == 2 && !L1.f8 && !L2.f8)) continue;
-      Eo2Args& e = l1.eo2;
-      std::memset(&e, 0, sizeof(e));
-      e.kb1 = (L1.cin_p + 31) / 32;
-      e.kb2 = (L2.cin_p + 31) / 32;
-      e.n1 = L1.n_tile;
-      e.n2 = L2.n_tile;
-      e.acc1 = round_up(2 * e.n1, 32);
-      e.acc2 = round_up(2 * e.n2, 32);
-      const size_t smem = conv_eo2_smem(e.n1, e.n2, e.kb1, e.kb2);
-      if (3 * e.acc1 + e.acc2 > kTmemCols || smem > static_cast<size_t>(max_smem) || e.n1 > 128 || e.n2 > 128) continue;
-      e.bias1 = L1.bias;
-      e.bias2 = L2.bias;
-      e.out = l2.args.out;
-      e.B = B;
-      e.Lp_out = l2.args.Lp_out;
-      e.n_seg = (e.Lp_out + kE2Rows - 1) / kE2Rows;
-      e.half_lp_in = l1.args.half_lp;
-      e.half_lp_out = l2.args.half_lp_out;
-      e.n_pairs_out = l2.args.n_pairs_out;
-      e.out_eo = l2.args.out_eo;
-      e.out_f8 = l2.args.out_f8;
-      e.out_planes = l2.args.out_planes;
-      e.cout_p2 = L2.cout_p;
-      e.shift1 = l1.args.shift;
-      e.shift2 = l2.args.shift;
-      e.cin_p1 = L1.cin_p;
-      e.idesc1_n = umma_idesc_f16(kBlockM, e.n1);
-      e.idesc1_2n = umma_idesc_f16(kBlockM, 2 * e.n1);
-      e.idesc2_n = umma_idesc_f16(kBlockM, e.n2);
-      e.idesc2_2n = umma_idesc_f16(kBlockM, 2 * e.n2);
-      e.inv_scale1 = L1.w_inv_scale;
-      e.inv_scale2 = L2.w_inv_scale;
-      l1.kind = l2.kind = kEo2Kernel;
-      l1.fn.eo2 = conv_eo2_kernel;
-      l1.grid = std::min(e.B * e.n_seg, m->sm_count);
-      l1.block = kE2Threads;
-      l1.smem = smem;
-      l2.fused_prev = 1;
-      RISER_CUDA_TRY(cudaFuncSetAttribute(reinterpret_cast<const void*>(conv_eo2_kernel),
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-      break;
-    }
-  // tile activity flags (ragged batches / skipped reads): one byte per M super-tile and layer
-  p->activity.n_layers = 0;
-  p->activity.total = 0;
-  for (int i = 1; i < m->n_layers; ++i) {
-    const ConvArgs& a = p->layer[i].args;
-    ActivityLayer& al = p->activity.layer[p->activity.n_layers++];
-    al.Lp_in = a.Lp_in;
-    al.rows_in = a.rows_in;
-    al.rows_per_super = p->layer[i].rows_per_super;
-    al.shift = a.shift;
-    al.n_supers = a.n_supers;
-    al.flag_off = p->activity.total;
-    p->activity.total += al.n_supers;
+    ConvArgs& a = lp.args;
+    a.n_supers = (a.rows_in + lp.rows_per_super - 1) / lp.rows_per_super;
+    if (lp.kind == kPairKernel) lp.grid = std::min(2 * a.n_supers * a.n_tiles, m->sm_count & ~1);
+    else if (lp.kind != kEo2Kernel) lp.grid = std::min(a.n_supers * a.n_tiles, m->sm_count);
+    if (fn) RISER_CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
+    // tile activity flags (ragged batches / skipped reads): one byte per M super-tile and layer
+    p->activity.layer[p->activity.n_layers++] = {a.Lp_in, a.rows_in, lp.rows_per_super, a.shift, a.n_supers,
+                                                 p->activity.total};
+    p->activity.total += a.n_supers;
   }
   RISER_CUDA_TRY(cudaMalloc(&p->flags, p->activity.total));
   for (int i = 1; i < m->n_layers; ++i) {
