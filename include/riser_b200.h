@@ -369,11 +369,64 @@ size_t riser_conv1d_wgrad_workspace_bytes(int B, int L_pad, int Cin, int Cout, i
 int riser_conv1d_wgrad_cl(const float* dz, const float* x, const int32_t* len, int B, int L_pad, int Cin, int Cout,
                           int K, float* dw, float* db, void* workspace, size_t workspace_bytes, riser_stream_t stream);
 
+/* riser_conv1d_wgrad_cl for any stride and padding (the ResNet's strided and padded convolutions, resnet.py:26-47,79-81):
+ *   dw[co][ci][j] = sum_b sum_{t < len_out[b]} dz[b][t][co] * x[b][t * stride + j - pad][ci]
+ *                   (x = 0 outside [0, len_in[b]))
+ *   db[co]        = sum_b sum_{t < len_out[b]} dz[b][t][co]         (db may be NULL: no bias)
+ * dz [B][Lout_pad][Cout], x [B][Lin_pad][Cin]; rows at or beyond len_out / len_in are never read.  Same kernel,
+ * precision and fixed summation order as riser_conv1d_wgrad_cl, which is this call at stride 1, pad (K - 1) / 2, bit
+ * for bit.  K <= 32, odd or even.  workspace: at least riser_conv1d_wgrad_ex_workspace_bytes(B, Lout_pad, Cin, Cout, K)
+ * bytes (0 = unsupported shape); RISER_ENOMEM when smaller.                                                   */
+size_t riser_conv1d_wgrad_ex_workspace_bytes(int B, int Lout_pad, int Cin, int Cout, int K);
+int riser_conv1d_wgrad_ex(const float* dz, const float* x, const int32_t* len_out, const int32_t* len_in, int B,
+                          int Lout_pad, int Lin_pad, int Cin, int Cout, int K, int stride, int pad, float* dw, float* db,
+                          void* workspace, size_t workspace_bytes, riser_stream_t stream);
+
+/* Input gradient of Conv1d(Cin -> Cout, K, stride, pad) (the strided convolutions of the ResNet; stride-1 ones use
+ * riser_conv1d_cl with the tap-flipped weight):
+ *   dx[b][u][ci] = sum_{t, j : t * stride + j - pad = u, t < len_out[b]} sum_co w[j][co][ci] dz[b][t][co]
+ *                  (+ residual[b][u][ci]) for u < len_in[b], 0 on rows u >= len_in[b].
+ * w [K][Cout][Cin] (taps not flipped); dz [B][Lout_pad][Cout]; residual (optional) and dx [B][Lin_pad][Cin], not
+ * aliased.  fp32, a fixed order per element.  residual carries the gradient of the block's other branch.          */
+int riser_conv1d_dgrad_cl(const float* dz, const int32_t* len_out, const float* w, const float* residual, float* dx,
+                          const int32_t* len_in, int B, int Lout_pad, int Lin_pad, int Cin, int Cout, int K, int stride,
+                          int pad, riser_stream_t stream);
+
+/* BatchNorm1d in training mode (resnet.py:23,29,80; torch's momentum 0.1, eps 1e-5), y [B][L_pad][C] valid for
+ * t < len[b].  The statistics are over the n = sum_b len[b] valid rows (torch's batch statistics at equal lengths),
+ * summed in float64 in a fixed order (the same bits on every run).  workspace: riser_bn_workspace_bytes(C) bytes,
+ * any content, RISER_ENOMEM when smaller; one workspace may serve every call in turn on one stream.
+ * riser_bn_stats_cl: mean [C] and the biased variance var [C].  With running_mean, running_var and
+ *   num_batches_tracked (all three or none): running = (1 - momentum) running + momentum stat, with the unbiased
+ *   variance var n / (n - 1), and num_batches_tracked (int64) + 1.
+ * riser_bn_apply_cl: out = act(gamma (y - mean) / sqrt(var + eps) + beta + r) on valid rows (others not written),
+ *   act = ReLU when relu; r = residual [B][L_pad][C] (optional) or, with res_mean, the same BatchNorm of residual
+ *   with res_mean, res_var, res_gamma, res_beta (a block's BN2(conv2) + BN_sc(conv_sc) + ReLU in one pass).  Eval
+ *   mode: pass the running statistics as mean and var.
+ * riser_bn_bwd_cl: dy = dout * (mask > 0) (mask: the saved activation output; NULL = no ReLU), xhat = (y - mean) /
+ *   sqrt(var + eps); dgamma = sum dy xhat, dbeta = sum dy (float64, fixed order) and
+ *   dx = gamma / sqrt(var + eps) (dy - sum dy / n - xhat sum dy xhat / n) on valid rows, 0 on the others; dy_out
+ *   (optional) gets dy (0 on invalid rows), the gradient the block's shortcut receives.                           */
+size_t riser_bn_workspace_bytes(int C);
+int riser_bn_stats_cl(const float* y, const int32_t* len, int B, int L_pad, int C, float* mean, float* var,
+                      float* running_mean, float* running_var, int64_t* num_batches_tracked, float momentum,
+                      void* workspace, size_t workspace_bytes, riser_stream_t stream);
+int riser_bn_apply_cl(const float* y, const int32_t* len, int B, int L_pad, int C, const float* mean, const float* var,
+                      const float* gamma, const float* beta, const float* residual, const float* res_mean,
+                      const float* res_var, const float* res_gamma, const float* res_beta, float eps, int relu,
+                      float* out, riser_stream_t stream);
+int riser_bn_bwd_cl(const float* dout, const float* mask, const float* y, const int32_t* len, int B, int L_pad, int C,
+                    const float* mean, const float* var, const float* gamma, float eps, float* dgamma, float* dbeta,
+                    float* dx, float* dy_out, void* workspace, size_t workspace_bytes, riser_stream_t stream);
+
 /* Gradient through ReLU + MaxPool1d(2, 2) (pool = 1) or ReLU alone (pool = 0).  y [B][L_pad][C]: the saved
  * post-ReLU convolution output, valid for t < len[b]; dp: the gradient of the pooled output [B][Lp_pad][C] (valid
  * for t < len[b] / 2) or, pool = 0, of y itself [B][L_pad][C] (Lp_pad == L_pad).  Writes every row of dz
  * [B][L_pad][C]: the pooled gradient goes to the larger of each pair (the first on a tie, torch's rule), times
- * (y > 0); the odd trailing row the floor pool drops and rows t >= len[b] get 0.                              */
+ * (y > 0); the odd trailing row the floor pool drops and rows t >= len[b] get 0.
+ * pool = 2: ReLU + the ResNet stem's MaxPool1d(2, 2, padding 1) (resnet.py:83), dp [B][Lp_pad][C] valid for
+ * t < len[b] / 2 + 1, Lp_pad >= L_pad / 2 + 1: window p is (y[2p - 1], y[2p]); the padding is never chosen, and
+ * between two rows the second wins only when it is larger or NaN (torch's rule).                              */
 int riser_relu_pool_bwd_cl(const float* y, const float* dp, const int32_t* len, float* dz, int B, int L_pad,
                            int Lp_pad, int C, int pool, riser_stream_t stream);
 

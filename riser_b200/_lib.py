@@ -60,7 +60,15 @@ SIGNATURES = {
     "riser_gap_linear_softmax": (c_int, [c_void_p] * 5 + [c_int] * 4 + [c_void_p]),
     "riser_conv1d_wgrad_workspace_bytes": (c_size_t, [c_int] * 5),
     "riser_conv1d_wgrad_cl": (c_int, [c_void_p] * 3 + [c_int] * 5 + [c_void_p] * 3 + [c_size_t, c_void_p]),
+    "riser_conv1d_wgrad_ex_workspace_bytes": (c_size_t, [c_int] * 5),
+    "riser_conv1d_wgrad_ex": (c_int, [c_void_p] * 4 + [c_int] * 8 + [c_void_p] * 3 + [c_size_t, c_void_p]),
     "riser_relu_pool_bwd_cl": (c_int, [c_void_p] * 4 + [c_int] * 5 + [c_void_p]),
+    "riser_conv1d_dgrad_cl": (c_int, [c_void_p] * 6 + [c_int] * 8 + [c_void_p]),
+    "riser_bn_workspace_bytes": (c_size_t, [c_int]),
+    "riser_bn_stats_cl": (c_int, [c_void_p] * 2 + [c_int] * 3 + [c_void_p] * 5 + [c_float, c_void_p, c_size_t, c_void_p]),
+    "riser_bn_apply_cl": (c_int, [c_void_p] * 2 + [c_int] * 3 + [c_void_p] * 9 + [c_float, c_int, c_void_p, c_void_p]),
+    "riser_bn_bwd_cl": (c_int, [c_void_p] * 4 + [c_int] * 3 + [c_void_p] * 3 + [c_float] + [c_void_p] * 5 +
+                        [c_size_t, c_void_p]),
     "riser_gap_linear_ce_bwd": (c_int, [c_void_p] * 5 + [c_int] * 4 + [c_void_p] * 9),
     "riser_decide": (c_int, [c_void_p, c_void_p, c_int, c_int, c_float, c_int, c_int, c_void_p, c_void_p]),
 }

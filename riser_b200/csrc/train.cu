@@ -13,7 +13,11 @@
 //     valid row: the centre tap's accumulator column for it is sum_r dZ[r][co].  Each split writes its partial
 //     sums to the workspace and a second launch adds them in split order: no float atomics, the same bits on every
 //     run.
-//   * riser_relu_pool_bwd_cl: the gradient through ReLU and MaxPool1d(2, 2) (or ReLU alone);
+//   riser_conv1d_wgrad_ex is the same kernel for any stride and padding (the ResNet's strided, padded convolutions,
+//   csrc/train_resnet.cu): the B operand of tap j for output row t is x[t * stride + j - pad] and the ones channel is
+//   1 on every valid output row, so the bias gradient does not depend on the taps that read the padding.
+//   * riser_relu_pool_bwd_cl: the gradient through ReLU and MaxPool1d(2, 2), the ResNet stem's MaxPool1d(2, 2,
+//     padding 1), or ReLU alone;
 //   * riser_gap_linear_ce_bwd: AdaptiveAvgPool1d(1) + Linear + CrossEntropyLoss (mean), forward and backward.
 #include "common.cuh"
 
@@ -33,13 +37,15 @@ constexpr uint32_t kWgAPlane = kWgM * 64;   // bytes of one A plane (128 rows x 
 
 struct WgArgs {
   const float* dz;       // [B][L_pad][Cout]
-  const float* x;        // [B][L_pad][Cin]
-  const int32_t* len;    // [B]
+  const float* x;        // [B][Lin_pad][Cin]
+  const int32_t* len;    // [B] output lengths
+  const int32_t* len_in; // [B] input lengths
   float* part;           // [S][K][Cin + 1][Cout]
   int B, L_pad, Cin, Cout, K, pad;
+  int Lin_pad, stride;
   int n;                 // MMA N (input channels per CTA, multiple of 16)
   int S;
-  int64_t rows;          // B * L_pad
+  int64_t rows;          // B * L_pad (output rows)
   int64_t chunks;        // ceil(rows / kWgRows)
   uint32_t stage_bytes, tmem_cols;
 };
@@ -144,15 +150,20 @@ wgrad_tc_kernel(const WgArgs a) {
         *reinterpret_cast<uint4*>(st + sw64(c, 16 * g)) = hi;
         *reinterpret_cast<uint4*>(st + kWgAPlane + sw64(c, 16 * g)) = lo;
       } else {
-        // B_j = X shifted by j - pad: row c = input channel ci0 + c (ci == Cin: 1 on valid rows), K = the chunk's rows
+        // B_j = X at t * stride + j - pad: row c = input channel ci0 + c (ci == Cin: 1 on valid output rows), K = the
+        // chunk's output rows
         const int ci = ci0 + c, sh = j - a.pad;
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
           float val = 0.f;
           if (r < a.rows && ci <= a.Cin) {
-            const int ts = t + sh;
-            if (ts >= 0 && ts < __ldg(a.len + b))
-              val = (ci == a.Cin) ? 1.f : __ldg(a.x + (static_cast<int64_t>(b) * a.L_pad + ts) * a.Cin + ci);
+            if (ci == a.Cin) {
+              if (t < __ldg(a.len + b)) val = 1.f;
+            } else {
+              const int ts = t * a.stride + sh;
+              if (ts >= 0 && ts < __ldg(a.len_in + b))
+                val = __ldg(a.x + (static_cast<int64_t>(b) * a.Lin_pad + ts) * a.Cin + ci);
+            }
           }
           v[e] = val;
           ++r;
@@ -215,14 +226,14 @@ wgrad_tc_kernel(const WgArgs a) {
   }
 }
 
-// dW[co][ci][j] = sum over splits s (in order) of part[s][j][ci][co]; db[co] the same over the ones channel of the
-// centre tap
+// dW[co][ci][j] = sum over splits s (in order) of part[s][j][ci][co]; db[co] the same over the ones channel of tap
+// (K - 1) / 2 (the ones channel is the same in every tap); no db when db is NULL
 __global__ void __launch_bounds__(256)
 wgrad_reduce_kernel(const float* __restrict__ part, float* __restrict__ dw, float* __restrict__ db, int S, int K,
                     int pad, int Cin, int Cout) {
   const int64_t n_w = static_cast<int64_t>(Cout) * Cin * K;
   const int64_t plane = static_cast<int64_t>(Cin + 1) * Cout;
-  for (int64_t idx = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; idx < n_w + Cout;
+  for (int64_t idx = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; idx < n_w + (db ? Cout : 0);
        idx += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     int co, ci, j;
     if (idx < n_w) {
@@ -249,9 +260,10 @@ struct WgPlan {
 };
 
 // Tile and split of a shape: N = the input channels (+ the ones channel) spread evenly over as few tiles as the
-// 512 TMEM columns allow for K accumulators; S row splits so that the tiles fill about one wave.
+// 512 TMEM columns allow for K accumulators (K <= 32); S splits of the output rows so that the tiles fill about one
+// wave.
 bool wg_plan(int B, int L_pad, int Cin, int Cout, int K, WgPlan& p) {
-  if (B <= 0 || L_pad <= 0 || Cin <= 0 || Cout <= 0 || K <= 0 || (K & 1) == 0) return false;
+  if (B <= 0 || L_pad <= 0 || Cin <= 0 || Cout <= 0 || K <= 0) return false;
   const int n_max = std::min(256, (512 / K) / 16 * 16);
   if (n_max < 16) return false;
   const int cin1 = Cin + 1;
@@ -271,7 +283,8 @@ int grid_for(int64_t total) { return static_cast<int>(std::max<int64_t>(1, std::
 
 // ------------------------------------------------------------------ ReLU + MaxPool1d(2, 2) backward
 // dz[b][t][c] = (t < len and t < 2 (len / 2) and t is the first maximum of its pair ? dp[b][t / 2][c] : 0) * (y > 0)
-// (pool = 1); dz = (t < len ? dp[b][t][c] : 0) * (y > 0) (pool = 0)
+// (pool = 1); the same for the windows (t - 1, t) of MaxPool1d(2, 2, padding 1) (pool = 2); dz = (t < len ?
+// dp[b][t][c] : 0) * (y > 0) (pool = 0)
 __global__ void __launch_bounds__(256)
 relu_pool_bwd_kernel(const float* __restrict__ y, const float* __restrict__ dp, const int32_t* __restrict__ len,
                      float* __restrict__ dz, int B, int L_pad, int Lp_pad, int C, int pool) {
@@ -285,7 +298,25 @@ relu_pool_bwd_kernel(const float* __restrict__ y, const float* __restrict__ dp, 
     const int n = len[b];
     float g = 0.f;
     const float yv = (t < n) ? y[idx] : 0.f;
-    if (pool) {
+    if (pool == 2) {
+      // MaxPool1d(2, 2, padding 1): window p is (in[2p - 1], in[2p]); t is the second of window t / 2 (t even) or the
+      // first of window (t + 1) / 2 (t odd).  The padding is never chosen: a window with one row inside the read
+      // takes that row.
+      if (t < n) {
+        const int p = (t + 1) >> 1, i0 = 2 * p - 1, i1 = 2 * p;
+        bool second;
+        if (i0 < 0) {
+          second = true;
+        } else if (i1 >= n) {
+          second = false;
+        } else {
+          const float* yb = y + (static_cast<int64_t>(b) * L_pad) * C + c;
+          const float y0 = yb[static_cast<int64_t>(i0) * C], y1 = yb[static_cast<int64_t>(i1) * C];
+          second = y1 > y0 || y1 != y1;
+        }
+        if ((t == i1) == second) g = dp[(static_cast<int64_t>(b) * Lp_pad + p) * C + c];
+      }
+    } else if (pool) {
       if (t < (n / 2) * 2) {
         const int t0 = t & ~1;
         const float* yb = y + (static_cast<int64_t>(b) * L_pad) * C + c;
@@ -392,28 +423,22 @@ head_reduce_kernel(const float* __restrict__ loss, const float* __restrict__ dlo
 
 using namespace riser;
 
-extern "C" size_t riser_conv1d_wgrad_workspace_bytes(int B, int L_pad, int Cin, int Cout, int K) {
-  WgPlan p;
-  if (!wg_plan(B, L_pad, Cin, Cout, K, p)) return 0;
-  return static_cast<size_t>(p.S) * K * (Cin + 1) * static_cast<size_t>(Cout) * sizeof(float);
-}
+namespace {
 
-extern "C" int riser_conv1d_wgrad_cl(const float* dz, const float* x, const int32_t* len, int B, int L_pad, int Cin,
-                                     int Cout, int K, float* dw, float* db, void* workspace, size_t workspace_bytes,
-                                     riser_stream_t stream) {
-  RISER_REQUIRE(dz && x && len && dw && db && workspace, "riser_conv1d_wgrad_cl: null pointer");
+int wgrad_launch(const char* who, const float* dz, const float* x, const int32_t* len_out, const int32_t* len_in, int B,
+                 int Lout_pad, int Lin_pad, int Cin, int Cout, int K, int stride, int pad, float* dw, float* db,
+                 void* workspace, size_t workspace_bytes, riser_stream_t stream) {
   WgPlan p;
-  RISER_REQUIRE(wg_plan(B, L_pad, Cin, Cout, K, p),
-                "riser_conv1d_wgrad_cl: unsupported shape (B %d, L_pad %d, Cin %d, Cout %d, K %d: odd K <= 31)", B,
-                L_pad, Cin, Cout, K);
-  RISER_REQUIRE(p.chunks < (static_cast<int64_t>(1) << 31), "riser_conv1d_wgrad_cl: too many rows");
-  const size_t need = riser_conv1d_wgrad_workspace_bytes(B, L_pad, Cin, Cout, K);
-  if (workspace_bytes < need)
-    return fail(RISER_ENOMEM, "riser_conv1d_wgrad_cl: workspace %zu bytes < %zu", workspace_bytes, need);
+  RISER_REQUIRE(wg_plan(B, Lout_pad, Cin, Cout, K, p),
+                "%s: unsupported shape (B %d, L_pad %d, Cin %d, Cout %d, K %d)", who, B, Lout_pad, Cin, Cout, K);
+  RISER_REQUIRE(p.chunks < (static_cast<int64_t>(1) << 31), "%s: too many rows", who);
+  const size_t need = static_cast<size_t>(p.S) * K * (Cin + 1) * static_cast<size_t>(Cout) * sizeof(float);
+  if (workspace_bytes < need) return fail(RISER_ENOMEM, "%s: workspace %zu bytes < %zu", who, workspace_bytes, need);
   WgArgs a;
-  a.dz = dz; a.x = x; a.len = len; a.part = static_cast<float*>(workspace);
-  a.B = B; a.L_pad = L_pad; a.Cin = Cin; a.Cout = Cout; a.K = K; a.pad = (K - 1) / 2;
-  a.n = p.n; a.S = p.S; a.rows = static_cast<int64_t>(B) * L_pad; a.chunks = p.chunks;
+  a.dz = dz; a.x = x; a.len = len_out; a.len_in = len_in; a.part = static_cast<float*>(workspace);
+  a.B = B; a.L_pad = Lout_pad; a.Cin = Cin; a.Cout = Cout; a.K = K; a.pad = pad;
+  a.Lin_pad = Lin_pad; a.stride = stride;
+  a.n = p.n; a.S = p.S; a.rows = static_cast<int64_t>(B) * Lout_pad; a.chunks = p.chunks;
   a.stage_bytes = p.stage_bytes; a.tmem_cols = p.tmem_cols;
   // CTAs that share an SM must fit their TMEM allocations in its 512 columns (an allocation that cannot be served
   // waits for a resident CTA to exit): ask for enough shared memory that no more are co-scheduled
@@ -422,21 +447,54 @@ extern "C" int riser_conv1d_wgrad_cl(const float* dz, const float* x, const int3
   int dev = 0, max_smem = 0;
   RISER_CUDA_TRY(cudaGetDevice(&dev));
   RISER_CUDA_TRY(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-  RISER_REQUIRE(smem <= static_cast<size_t>(max_smem), "riser_conv1d_wgrad_cl: %zu bytes of shared memory", smem);
+  RISER_REQUIRE(smem <= static_cast<size_t>(max_smem), "%s: %zu bytes of shared memory", who, smem);
   RISER_CUDA_TRY(cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   wgrad_tc_kernel<<<dim3(p.m_tiles, p.n_tiles, p.S), kWgThreads, smem, as_stream(stream)>>>(a);
   RISER_CUDA_TRY(cudaGetLastError());
-  const int64_t total = static_cast<int64_t>(Cout) * Cin * K + Cout;
-  wgrad_reduce_kernel<<<grid_for(total), 256, 0, as_stream(stream)>>>(a.part, dw, db, p.S, K, a.pad, Cin, Cout);
+  const int64_t total = static_cast<int64_t>(Cout) * Cin * K + (db ? Cout : 0);
+  wgrad_reduce_kernel<<<grid_for(total), 256, 0, as_stream(stream)>>>(a.part, dw, db, p.S, K, (K - 1) / 2, Cin, Cout);
   RISER_CUDA_TRY(cudaGetLastError());
   return RISER_OK;
+}
+
+}  // namespace
+
+extern "C" size_t riser_conv1d_wgrad_ex_workspace_bytes(int B, int Lout_pad, int Cin, int Cout, int K) {
+  WgPlan p;
+  if (!wg_plan(B, Lout_pad, Cin, Cout, K, p)) return 0;
+  return static_cast<size_t>(p.S) * K * (Cin + 1) * static_cast<size_t>(Cout) * sizeof(float);
+}
+
+extern "C" size_t riser_conv1d_wgrad_workspace_bytes(int B, int L_pad, int Cin, int Cout, int K) {
+  return (K & 1) ? riser_conv1d_wgrad_ex_workspace_bytes(B, L_pad, Cin, Cout, K) : 0;
+}
+
+extern "C" int riser_conv1d_wgrad_cl(const float* dz, const float* x, const int32_t* len, int B, int L_pad, int Cin,
+                                     int Cout, int K, float* dw, float* db, void* workspace, size_t workspace_bytes,
+                                     riser_stream_t stream) {
+  RISER_REQUIRE(dz && x && len && dw && db && workspace, "riser_conv1d_wgrad_cl: null pointer");
+  RISER_REQUIRE((K & 1) == 1, "riser_conv1d_wgrad_cl: unsupported shape (K %d: odd K <= 31)", K);
+  return wgrad_launch("riser_conv1d_wgrad_cl", dz, x, len, len, B, L_pad, L_pad, Cin, Cout, K, 1, (K - 1) / 2, dw, db,
+                      workspace, workspace_bytes, stream);
+}
+
+extern "C" int riser_conv1d_wgrad_ex(const float* dz, const float* x, const int32_t* len_out, const int32_t* len_in,
+                                     int B, int Lout_pad, int Lin_pad, int Cin, int Cout, int K, int stride, int pad,
+                                     float* dw, float* db, void* workspace, size_t workspace_bytes,
+                                     riser_stream_t stream) {
+  RISER_REQUIRE(dz && x && len_out && len_in && dw && workspace, "riser_conv1d_wgrad_ex: null pointer");
+  RISER_REQUIRE(Lin_pad > 0 && stride > 0 && pad >= 0 && K <= 32, "riser_conv1d_wgrad_ex: bad shape (Lin_pad %d, "
+                "stride %d, pad %d, K %d <= 32)", Lin_pad, stride, pad, K);
+  return wgrad_launch("riser_conv1d_wgrad_ex", dz, x, len_out, len_in, B, Lout_pad, Lin_pad, Cin, Cout, K, stride, pad,
+                      dw, db, workspace, workspace_bytes, stream);
 }
 
 extern "C" int riser_relu_pool_bwd_cl(const float* y, const float* dp, const int32_t* len, float* dz, int B, int L_pad,
                                       int Lp_pad, int C, int pool, riser_stream_t stream) {
   RISER_REQUIRE(y && dp && len && dz, "riser_relu_pool_bwd_cl: null pointer");
-  RISER_REQUIRE(pool == 0 || pool == 1, "riser_relu_pool_bwd_cl: pool %d (0 or 1)", pool);
-  RISER_REQUIRE(B >= 0 && L_pad > 0 && C > 0 && (pool ? Lp_pad >= L_pad / 2 : Lp_pad == L_pad),
+  RISER_REQUIRE(pool >= 0 && pool <= 2, "riser_relu_pool_bwd_cl: pool %d (0, 1 or 2)", pool);
+  RISER_REQUIRE(B >= 0 && L_pad > 0 && C > 0 &&
+                    (pool == 2 ? Lp_pad >= L_pad / 2 + 1 : pool ? Lp_pad >= L_pad / 2 : Lp_pad == L_pad),
                 "riser_relu_pool_bwd_cl: bad shape");
   const int64_t total = static_cast<int64_t>(B) * L_pad * C;
   if (total == 0) return RISER_OK;

@@ -1,12 +1,14 @@
-"""Time one training step of the shipped ConvNet shape (riser_b200.training.ConvNetTrainer) against the reference
-ConvNet trained with torch autograd + torch.optim.Adam on the same GPU.
+"""Time one training step of the shipped ConvNet shape (riser_b200.training.ConvNetTrainer), or of a synthetic ResNet
+configuration (``--net resnet --config basic|bottleneck``, ResNetTrainer), against the same network trained with torch
+autograd + torch.optim.Adam on the same GPU (cuDNN; the ResNet's BatchNorm in training mode).
 
-    python tools/time_train.py [--steps 10] [--warmup 3] [--batches 32,256] [--length 12048] [--out file.json]
+    python tools/time_train.py [--net cnn|resnet] [--config basic] [--steps 10] [--warmup 3] [--batches 32,256]
+                               [--length 12048] [--out file.json]
 
 Prints the GPU name and power limit, ms per step and reads/s for both at every batch size (every read at the full
-length), and splits the riser_b200 step into forward (convolutions, pools, lengths), head, wgrad, dgrad, the ReLU /
-pool backward and Adam (with the weight repacking) from CUDA events around every launch of an instrumented step.
-Needs a B200."""
+length), and splits the riser_b200 step into forward (convolutions, pools, lengths), BatchNorm forward and backward,
+head, wgrad, dgrad, the ReLU / pool backward and Adam (with the weight repacking) from CUDA events around every launch
+of an instrumented step.  Needs a B200."""
 import argparse
 import json
 import os
@@ -20,8 +22,9 @@ import torch.nn.functional as F
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 from oracle.convnet_module import ConvNet                         # noqa: E402
+from oracle.resnet_module import ResNet                           # noqa: E402
 from riser_b200 import _lib                                      # noqa: E402
-from riser_b200 import training                                   # noqa: E402
+from riser_b200 import synth, training                            # noqa: E402
 from riser_b200.config import CNN_SHIPPED, AttrDict              # noqa: E402
 
 
@@ -52,7 +55,7 @@ class _Recorder:
     """Stands in for the loaded library: every launch function is bracketed by CUDA events under a category."""
 
     def __init__(self, lib):
-        self.lib, self.spans = lib, []
+        self.lib, self.spans, self.backward = lib, [], False
 
     def __getattr__(self, name):
         fn = getattr(self.lib, name)
@@ -61,13 +64,21 @@ class _Recorder:
 
         def call(*args):
             if name == "riser_conv1d_cl":
-                cat = "forward" if args[15] else "dgrad"
+                cat = "dgrad" if self.backward else "forward"          # the launches after the head are dgrad
             elif name in ("riser_maxpool1d_pad_cl", "riser_len_chain"):
                 cat = "forward"
+            elif name in ("riser_bn_stats_cl", "riser_bn_apply_cl"):
+                cat = "bn_forward"
+            elif name == "riser_bn_bwd_cl":
+                cat = "bn_backward"
+            elif name == "riser_conv1d_dgrad_cl":
+                cat = "dgrad"
             elif name == "riser_gap_linear_ce_bwd":
                 cat = "head"
-            elif name == "riser_conv1d_wgrad_cl":
-                cat = "wgrad_layer0" if args[5] == 1 else "wgrad"        # Cin = 1: 2 of the 16 MMA columns are used
+                self.backward = True
+            elif name in ("riser_conv1d_wgrad_cl", "riser_conv1d_wgrad_ex"):
+                cin = args[5] if name == "riser_conv1d_wgrad_cl" else args[7]
+                cat = "wgrad_layer0" if cin == 1 else "wgrad"          # Cin = 1: 2 of the 16 MMA columns are used
             else:
                 cat = "relu_pool_bwd"
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -87,7 +98,10 @@ def breakdown(tr, x, lens, labels):
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s0 = torch.cuda.Event(enable_timing=True)
         s0.record()
-        tr._run(x, lens, labels)
+        if isinstance(tr, training.ResNetTrainer):
+            tr._run(x, lens, labels, "step")
+        else:
+            tr._run(x, lens, labels)
         a.record()
         tr.optimizer.step()
         b.record()
@@ -105,6 +119,9 @@ def breakdown(tr, x, lens, labels):
 
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument("--net", choices=["cnn", "resnet"], default="cnn")
+    ap.add_argument("--config", choices=sorted(synth.RESNET_CONFIGS), default="basic",
+                    help="the synthetic ResNet configuration (--net resnet)")
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--batches", default="32,256")
@@ -115,22 +132,28 @@ def main():
     name, power = gpu_info()
     print(f"GPU: {name}; power.limit, clocks.max.sm: {power}")
     print(f"torch {torch.__version__}; reference convolutions: cudnn.allow_tf32 = {torch.backends.cudnn.allow_tf32}")
-    cfg = AttrDict({"model": "cnn", "cnn": dict(CNN_SHIPPED), "learning_rate": 1e-4})
+    if args.net == "resnet":
+        cfg = AttrDict({"model": "resnet", "resnet": dict(synth.RESNET_CONFIGS[args.config]), "learning_rate": 1e-4})
+        print(f"ResNet '{args.config}': {cfg.resnet}")
+    else:
+        cfg = AttrDict({"model": "cnn", "cnn": dict(CNN_SHIPPED), "learning_rate": 1e-4})
     L = args.length
-    results = {"gpu": name, "power_limit_max_sm_clock": power, "length": L, "rows": []}
+    results = {"gpu": name, "power_limit_max_sm_clock": power, "net": args.net, "length": L, "rows": []}
+    if args.net == "resnet":
+        results["config"] = args.config
     for B in [int(b) for b in args.batches.split(",")]:
         g = torch.Generator(device="cpu").manual_seed(B)
         x = torch.randn(B, L, generator=g).to(dev)
         lens = torch.full((B,), L, dtype=torch.int32, device=dev)
         labels = (torch.arange(B) % 2).to(dev)
-        tr = training.ConvNetTrainer(cfg, seed=0)
+        tr = training.make_trainer(cfg, seed=0)
         ms = timed(lambda: tr.step(x, lens, labels), args.steps, args.warmup)
         parts = breakdown(tr, x, lens, labels)
         del tr
         torch.cuda.empty_cache()
         with torch.random.fork_rng(devices=[]):
             torch.manual_seed(0)
-            net = ConvNet(cfg.cnn).to(dev)
+            net = (ResNet(cfg.resnet) if args.net == "resnet" else ConvNet(cfg.cnn)).to(dev).train()
         opt = torch.optim.Adam(net.parameters(), lr=1e-4)
 
         def ref_step():
