@@ -48,6 +48,9 @@ enum {
   RISER_SKIPPED = 4,
 };
 
+/* Most replicas a data-parallel reduction takes (riser_peer_reduce_f32, riser_bn_*_finalize_cl). */
+enum { RISER_MAX_REPLICAS = 8 };
+
 /* mode argument of riser_decide (riser/riser.py:91-95, control.py:76,78) */
 enum { RISER_MODE_ENRICH = 0, RISER_MODE_DEPLETE = 1 };
 
@@ -419,6 +422,33 @@ int riser_bn_bwd_cl(const float* dout, const float* mask, const float* y, const 
                     const float* mean, const float* var, const float* gamma, float eps, float* dgamma, float* dbeta,
                     float* dx, float* dy_out, void* workspace, size_t workspace_bytes, riser_stream_t stream);
 
+/* The two halves of riser_bn_stats_cl / riser_bn_bwd_cl, for G data-parallel replicas that each hold a slice of the
+ * batch (SyncBatchNorm: the statistics and sums are those of the global batch; riser_b200/parallel.py).
+ *   *_partial_cl: this replica's float64 partial, riser_bn_partial_bytes(C) bytes: [C][2] sums, then the number of
+ *     valid rows.  stats: (sum y, sum y^2); bwd: (sum dy, sum dy xhat), dy and xhat as in riser_bn_bwd_cl with the
+ *     global mean / var.  B = 0 (an empty slice) writes zeros and reads nothing else.
+ *   *_finalize_cl: partials_host is a host array of the G replicas' partials (device pointers, peer pointers for the
+ *     other devices), in device order, G <= RISER_MAX_REPLICAS; they are added in that order, n = the global row count.
+ *     stats: mean, var and the running update as riser_bn_stats_cl with the global n.  bwd: dgamma and dbeta get the
+ *     global sums when owner != 0 and zeros otherwise (one replica owns them, so adding the replicas' gradients
+ *     counts them once); dx and dy_out as riser_bn_bwd_cl for this replica's B reads (none when B = 0).
+ * workspace as for riser_bn_stats_cl (the finalize uses it for the bwd sums).  With G = 1 the results are
+ * riser_bn_stats_cl's and riser_bn_bwd_cl's bit for bit.  A caller must not overwrite a partial while another replica
+ * may still read it.                                                                                              */
+size_t riser_bn_partial_bytes(int C);
+int riser_bn_stats_partial_cl(const float* y, const int32_t* len, int B, int L_pad, int C, double* partial,
+                              void* workspace, size_t workspace_bytes, riser_stream_t stream);
+int riser_bn_stats_finalize_cl(const double* const* partials_host, int G, int C, float* mean, float* var,
+                               float* running_mean, float* running_var, int64_t* num_batches_tracked, float momentum,
+                               riser_stream_t stream);
+int riser_bn_bwd_partial_cl(const float* dout, const float* mask, const float* y, const int32_t* len, int B, int L_pad,
+                            int C, const float* mean, const float* var, float eps, double* partial, void* workspace,
+                            size_t workspace_bytes, riser_stream_t stream);
+int riser_bn_bwd_finalize_cl(const double* const* partials_host, int G, int owner, const float* dout, const float* mask,
+                             const float* y, const int32_t* len, int B, int L_pad, int C, const float* mean,
+                             const float* var, const float* gamma, float eps, float* dgamma, float* dbeta, float* dx,
+                             float* dy_out, void* workspace, size_t workspace_bytes, riser_stream_t stream);
+
 /* Gradient through ReLU + MaxPool1d(2, 2) (pool = 1) or ReLU alone (pool = 0).  y [B][L_pad][C]: the saved
  * post-ReLU convolution output, valid for t < len[b]; dp: the gradient of the pooled output [B][Lp_pad][C] (valid
  * for t < len[b] / 2) or, pool = 0, of y itself [B][L_pad][C] (Lp_pad == L_pad).  Writes every row of dz
@@ -442,6 +472,33 @@ int riser_gap_linear_ce_bwd(const float* h, const int32_t* len, const float* fc_
                             const int64_t* labels, int B, int L_pad, int C, int n_classes, float* loss,
                             float* loss_mean, float* logits, float* dlogits, float* feat, float* dfc_w, float* dfc_b,
                             float* dh, riser_stream_t stream);
+
+/* riser_gap_linear_ce_bwd for one data-parallel replica's B reads of a global batch of B_total >= B:
+ * dlogits = (softmax(z) - onehot) / B_total and loss_mean = sum of this replica's losses / B_total, so every read's
+ * dlogits and dh have the bits of the one-device step and the replicas' dfc_w, dfc_b and loss_mean add up to the
+ * global ones.  riser_gap_linear_ce_bwd is this call with B_total = B.                                           */
+int riser_gap_linear_ce_bwd_ex(const float* h, const int32_t* len, const float* fc_w, const float* fc_b,
+                               const int64_t* labels, int B, int B_total, int L_pad, int C, int n_classes, float* loss,
+                               float* loss_mean, float* logits, float* dlogits, float* feat, float* dfc_w,
+                               float* dfc_b, float* dh, riser_stream_t stream);
+
+/* ------------------------------------------------------------------ data-parallel training (riser_b200/parallel.py)
+ * One process drives G <= RISER_MAX_REPLICAS GPUs of one box; the replicas exchange gradients by peer-to-peer loads
+ * over NVLink in a fixed device order (no NCCL), so every replica holds the same bits and a run is repeatable.      */
+
+/* Enables peer access between every pair of the G listed devices in this process ("already enabled" is success;
+ * repeated entries are skipped).  RISER_ECUDA with a message naming the first pair that cannot access each other.
+ * Changes no device setting.  Restores the calling thread's current device.                                        */
+int riser_peer_enable(const int* devices_host, int G);
+
+/* dst[i] = ((src[0][i] + src[1][i]) + src[2][i]) + ... in fp32, sources in that order, for i in [lo, hi).
+ * src_host: a host array of G <= RISER_MAX_REPLICAS device pointers (peer pointers for other devices: peer access
+ * enabled), passed to the kernel by value; dst may be one of the sources.  G = 1 copies src[0].  An empty range
+ * launches nothing.  16-byte aligned pointers take vector loads.  The all-reduce of parallel.py: replica d reduces
+ * the d-th slice of the flat gradient from every replica into its own buffer, then copies the other slices from
+ * their owners (G = 1), so one owner computes each element.                                                        */
+int riser_peer_reduce_f32(const float* const* src_host, int G, float* dst, int64_t lo, int64_t hi,
+                          riser_stream_t stream);
 
 #ifdef __cplusplus
 }

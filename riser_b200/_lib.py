@@ -70,6 +70,16 @@ SIGNATURES = {
     "riser_bn_bwd_cl": (c_int, [c_void_p] * 4 + [c_int] * 3 + [c_void_p] * 3 + [c_float] + [c_void_p] * 5 +
                         [c_size_t, c_void_p]),
     "riser_gap_linear_ce_bwd": (c_int, [c_void_p] * 5 + [c_int] * 4 + [c_void_p] * 9),
+    "riser_gap_linear_ce_bwd_ex": (c_int, [c_void_p] * 5 + [c_int] * 5 + [c_void_p] * 9),
+    "riser_bn_partial_bytes": (c_size_t, [c_int]),
+    "riser_bn_stats_partial_cl": (c_int, [c_void_p] * 2 + [c_int] * 3 + [c_void_p] * 2 + [c_size_t, c_void_p]),
+    "riser_bn_stats_finalize_cl": (c_int, [c_void_p, c_int, c_int] + [c_void_p] * 5 + [c_float, c_void_p]),
+    "riser_bn_bwd_partial_cl": (c_int, [c_void_p] * 4 + [c_int] * 3 + [c_void_p] * 2 + [c_float] + [c_void_p] * 2 +
+                                [c_size_t, c_void_p]),
+    "riser_bn_bwd_finalize_cl": (c_int, [c_void_p, c_int, c_int] + [c_void_p] * 4 + [c_int] * 3 + [c_void_p] * 3 +
+                                 [c_float] + [c_void_p] * 5 + [c_size_t, c_void_p]),
+    "riser_peer_enable": (c_int, [c_void_p, c_int]),
+    "riser_peer_reduce_f32": (c_int, [c_void_p, c_int, c_void_p, c_i64, c_i64, c_void_p]),
     "riser_decide": (c_int, [c_void_p, c_void_p, c_int, c_int, c_float, c_int, c_int, c_void_p, c_void_p]),
 }
 

@@ -334,12 +334,13 @@ relu_pool_bwd_kernel(const float* __restrict__ y, const float* __restrict__ dp, 
 
 // ------------------------------------------------------------------ head: GAP + Linear + cross entropy
 // One CTA per read, in float64: feat = mean of the valid rows, z = W feat + bias, loss = logsumexp(z) - z[y],
-// dlogits = (softmax(z) - onehot(y)) / B, dh = (W^T dlogits) / len on the valid rows, 0 on the others.  A read with
-// len 0 or a label outside [0, n_classes) gets a NaN loss and no gradient.
+// dlogits = (softmax(z) - onehot(y)) / B_total (B_total = B, or a data-parallel replica's global batch), dh = (W^T dlogits)
+// / len on the valid rows, 0 on the others.  A read with len 0 or a label outside [0, n_classes) gets a NaN loss and no
+// gradient.
 constexpr int kHeadMaxClasses = 32;
 __global__ void __launch_bounds__(256)
 head_ce_kernel(const float* __restrict__ h, const int32_t* __restrict__ len, const float* __restrict__ fc_w,
-               const float* __restrict__ fc_b, const int64_t* __restrict__ labels, int B, int L_pad, int C,
+               const float* __restrict__ fc_b, const int64_t* __restrict__ labels, int B_total, int L_pad, int C,
                int n_classes, float* __restrict__ loss, float* __restrict__ logits, float* __restrict__ dlogits,
                float* __restrict__ feat, float* __restrict__ dh) {
   extern __shared__ double fs[];                    // [C] features, then [C] activation gradient
@@ -372,7 +373,7 @@ head_ce_kernel(const float* __restrict__ h, const int32_t* __restrict__ len, con
     const double lse = m + log(se);
     loss[b] = ok ? static_cast<float>(lse - z[y]) : nanf("");
     for (int k = 0; k < n_classes; ++k) {
-      dz[k] = ok ? (exp(z[k] - lse) - (k == y ? 1.0 : 0.0)) / B : 0.0;
+      dz[k] = ok ? (exp(z[k] - lse) - (k == y ? 1.0 : 0.0)) / B_total : 0.0;
       logits[static_cast<int64_t>(b) * n_classes + k] = static_cast<float>(z[k]);
       dlogits[static_cast<int64_t>(b) * n_classes + k] = static_cast<float>(dz[k]);
     }
@@ -392,10 +393,11 @@ head_ce_kernel(const float* __restrict__ h, const int32_t* __restrict__ len, con
   }
 }
 
-// dfc_w[k][c] = sum_b dlogits[b][k] feat[b][c], dfc_b[k] = sum_b dlogits[b][k] (b in order, float64), and the mean loss
+// dfc_w[k][c] = sum_b dlogits[b][k] feat[b][c], dfc_b[k] = sum_b dlogits[b][k] (b in order, float64), and the loss
+// summed over the reads / B_total
 __global__ void __launch_bounds__(256)
 head_reduce_kernel(const float* __restrict__ loss, const float* __restrict__ dlogits, const float* __restrict__ feat,
-                   int B, int C, int n_classes, float* __restrict__ loss_mean, float* __restrict__ dfc_w,
+                   int B, int B_total, int C, int n_classes, float* __restrict__ loss_mean, float* __restrict__ dfc_w,
                    float* __restrict__ dfc_b) {
   const int64_t n_w = static_cast<int64_t>(n_classes) * C;
   for (int64_t idx = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; idx <= n_w + n_classes;
@@ -413,7 +415,7 @@ head_reduce_kernel(const float* __restrict__ loss, const float* __restrict__ dlo
       dfc_b[k] = static_cast<float>(acc);
     } else {
       for (int b = 0; b < B; ++b) acc += static_cast<double>(loss[b]);
-      *loss_mean = static_cast<float>(acc / B);
+      *loss_mean = static_cast<float>(acc / B_total);
     }
   }
 }
@@ -503,24 +505,33 @@ extern "C" int riser_relu_pool_bwd_cl(const float* y, const float* dp, const int
   return RISER_OK;
 }
 
-extern "C" int riser_gap_linear_ce_bwd(const float* h, const int32_t* len, const float* fc_w, const float* fc_b,
-                                       const int64_t* labels, int B, int L_pad, int C, int n_classes, float* loss,
-                                       float* loss_mean, float* logits, float* dlogits, float* feat, float* dfc_w,
-                                       float* dfc_b, float* dh, riser_stream_t stream) {
+extern "C" int riser_gap_linear_ce_bwd_ex(const float* h, const int32_t* len, const float* fc_w, const float* fc_b,
+                                          const int64_t* labels, int B, int B_total, int L_pad, int C, int n_classes,
+                                          float* loss, float* loss_mean, float* logits, float* dlogits, float* feat,
+                                          float* dfc_w, float* dfc_b, float* dh, riser_stream_t stream) {
   RISER_REQUIRE(h && len && fc_w && fc_b && labels && loss && loss_mean && logits && dlogits && feat && dfc_w && dfc_b &&
                     dh, "riser_gap_linear_ce_bwd: null pointer");
-  RISER_REQUIRE(B > 0 && L_pad > 0 && C > 0 && n_classes >= 1 && n_classes <= kHeadMaxClasses,
-                "riser_gap_linear_ce_bwd: bad shape (n_classes %d <= %d)", n_classes, kHeadMaxClasses);
+  RISER_REQUIRE(B > 0 && B_total >= B && L_pad > 0 && C > 0 && n_classes >= 1 && n_classes <= kHeadMaxClasses,
+                "riser_gap_linear_ce_bwd: bad shape (B %d <= B_total %d, n_classes %d <= %d)", B, B_total, n_classes,
+                kHeadMaxClasses);
   const size_t smem = 2 * sizeof(double) * static_cast<size_t>(C);
   RISER_REQUIRE(smem <= 200 * 1024, "riser_gap_linear_ce_bwd: %d channels", C);
   if (smem > 48 * 1024)
     RISER_CUDA_TRY(cudaFuncSetAttribute(head_ce_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  head_ce_kernel<<<B, 256, smem, as_stream(stream)>>>(h, len, fc_w, fc_b, labels, B, L_pad, C, n_classes, loss, logits,
-                                                      dlogits, feat, dh);
+  head_ce_kernel<<<B, 256, smem, as_stream(stream)>>>(h, len, fc_w, fc_b, labels, B_total, L_pad, C, n_classes, loss,
+                                                      logits, dlogits, feat, dh);
   RISER_CUDA_TRY(cudaGetLastError());
   const int64_t total = static_cast<int64_t>(n_classes) * C + n_classes + 1;
-  head_reduce_kernel<<<grid_for(total), 256, 0, as_stream(stream)>>>(loss, dlogits, feat, B, C, n_classes, loss_mean,
-                                                                     dfc_w, dfc_b);
+  head_reduce_kernel<<<grid_for(total), 256, 0, as_stream(stream)>>>(loss, dlogits, feat, B, B_total, C, n_classes,
+                                                                     loss_mean, dfc_w, dfc_b);
   RISER_CUDA_TRY(cudaGetLastError());
   return RISER_OK;
+}
+
+extern "C" int riser_gap_linear_ce_bwd(const float* h, const int32_t* len, const float* fc_w, const float* fc_b,
+                                       const int64_t* labels, int B, int L_pad, int C, int n_classes, float* loss,
+                                       float* loss_mean, float* logits, float* dlogits, float* feat, float* dfc_w,
+                                       float* dfc_b, float* dh, riser_stream_t stream) {
+  return riser_gap_linear_ce_bwd_ex(h, len, fc_w, fc_b, labels, B, B, L_pad, C, n_classes, loss, loss_mean, logits,
+                                    dlogits, feat, dfc_w, dfc_b, dh, stream);
 }

@@ -8,6 +8,10 @@
 //     every CTA owns a fixed slice of the rows (kBnParts slices, a constant, so the order does not depend on the
 //     device), and a second launch adds the slices in order.  No float atomics: a launch gives the same bits on every
 //     run.
+//   * riser_bn_{stats,bwd}_{partial,finalize}_cl: the two halves of those reductions for data-parallel replicas
+//     (SyncBatchNorm): each replica adds its slices into one float64 partial (valid rows, two sums per channel), and
+//     every replica then adds the G partials in device order.  riser_bn_stats_cl / riser_bn_bwd_cl are G = 1 of it
+//     without the intermediate partial (0.0 + x is exact), so their bits do not change.
 #include "common.cuh"
 
 #include <algorithm>
@@ -121,20 +125,56 @@ __device__ double valid_rows(const int32_t* __restrict__ len, int B) {
   return static_cast<double>(n);
 }
 
+// The partial sums a finishing kernel adds: G buffers (in device order) of S slices [S][C][2] each.  A replica's
+// partial (S = 1) also holds its valid-row count at [2C].
+struct BnParts {
+  const double* p[RISER_MAX_REPLICAS];
+};
+
+__device__ void bn_sums(const BnParts& parts, int G, int S, int C, int c, double& s0, double& s1) {
+  s0 = 0.0;
+  s1 = 0.0;
+  for (int g = 0; g < G; ++g)
+    for (int p = 0; p < S; ++p) {
+      s0 += parts.p[g][(static_cast<int64_t>(p) * C + c) * 2];
+      s1 += parts.p[g][(static_cast<int64_t>(p) * C + c) * 2 + 1];
+    }
+}
+
+// len != NULL: the rows of this launch's batch; else the replicas' counts (S = 1) in order
+__device__ double bn_count(const BnParts& parts, int G, int C, const int32_t* __restrict__ len, int B) {
+  if (len) return valid_rows(len, B);
+  double n = 0.0;
+  for (int g = 0; g < G; ++g) n += parts.p[g][2 * C];
+  return n;
+}
+
+// A replica's partial: its kBnParts slices in order per channel, and its valid-row count
+__global__ void __launch_bounds__(256)
+bn_slices_kernel(const double* __restrict__ part, const int32_t* __restrict__ len, int B, int C,
+                 double* __restrict__ partial) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  BnParts parts{};
+  parts.p[0] = part;
+  double s0, s1;
+  bn_sums(parts, 1, kBnParts, C, c, s0, s1);
+  partial[2 * c] = s0;
+  partial[2 * c + 1] = s1;
+  if (c == 0) partial[2 * C] = valid_rows(len, B);
+}
+
 // Per channel: the slices in order -> mean and biased variance; with update, running = (1 - m) running + m stat
 // (unbiased variance n / (n - 1)) and num_batches_tracked + 1.
 __global__ void __launch_bounds__(256)
-bn_stats_finish_kernel(const double* __restrict__ part, const int32_t* __restrict__ len, int B, int C,
+bn_stats_finish_kernel(BnParts parts, int G, int S, const int32_t* __restrict__ len, int B, int C,
                        float* __restrict__ mean, float* __restrict__ var, float* __restrict__ running_mean,
                        float* __restrict__ running_var, int64_t* __restrict__ num_batches, float momentum) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= C) return;
-  double s = 0.0, ss = 0.0;
-  for (int p = 0; p < kBnParts; ++p) {
-    s += part[(static_cast<int64_t>(p) * C + c) * 2];
-    ss += part[(static_cast<int64_t>(p) * C + c) * 2 + 1];
-  }
-  const double n = valid_rows(len, B);
+  double s, ss;
+  bn_sums(parts, G, S, C, c, s, ss);
+  const double n = bn_count(parts, G, C, len, B);
   const double mu = s / n;
   const double v = fmax(ss / n - mu * mu, 0.0);
   mean[c] = static_cast<float>(mu);
@@ -173,20 +213,18 @@ bn_apply_kernel(const float* __restrict__ y, const int32_t* __restrict__ len, in
   }
 }
 
-// Per channel: the slices in order -> dgamma = sum dy xhat, dbeta = sum dy; sums[c] = (sum dy / n, sum dy xhat / n)
+// Per channel: the slices in order -> dgamma = sum dy xhat, dbeta = sum dy (zeros when !owner: a replica whose
+// gradients are added to the owner's); sums[c] = (sum dy / n, sum dy xhat / n)
 __global__ void __launch_bounds__(256)
-bn_bwd_finish_kernel(const double* __restrict__ part, const int32_t* __restrict__ len, int B, int C,
+bn_bwd_finish_kernel(BnParts parts, int G, int S, const int32_t* __restrict__ len, int B, int C, int owner,
                      float* __restrict__ dgamma, float* __restrict__ dbeta, double* __restrict__ sums) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= C) return;
-  double s0 = 0.0, s1 = 0.0;
-  for (int p = 0; p < kBnParts; ++p) {
-    s0 += part[(static_cast<int64_t>(p) * C + c) * 2];
-    s1 += part[(static_cast<int64_t>(p) * C + c) * 2 + 1];
-  }
-  const double n = valid_rows(len, B);
-  dgamma[c] = static_cast<float>(s1);
-  dbeta[c] = static_cast<float>(s0);
+  double s0, s1;
+  bn_sums(parts, G, S, C, c, s0, s1);
+  const double n = bn_count(parts, G, C, len, B);
+  dgamma[c] = owner ? static_cast<float>(s1) : 0.f;
+  dbeta[c] = owner ? static_cast<float>(s0) : 0.f;
   sums[2 * c] = s0 / n;
   sums[2 * c + 1] = s1 / n;
 }
@@ -243,6 +281,32 @@ extern "C" size_t riser_bn_workspace_bytes(int C) {
   return (static_cast<size_t>(kBnParts) + 1) * 2 * static_cast<size_t>(C) * sizeof(double);
 }
 
+namespace {
+
+BnParts one_part(const double* part) {
+  BnParts p{};
+  p.p[0] = part;
+  return p;
+}
+
+int gather_parts(const char* who, const double* const* partials_host, int G, BnParts& parts) {
+  RISER_REQUIRE(partials_host && G >= 1 && G <= RISER_MAX_REPLICAS, "%s: %d partials (1 to %d)", who, G,
+                RISER_MAX_REPLICAS);
+  parts = BnParts{};
+  for (int g = 0; g < G; ++g) {
+    RISER_REQUIRE(partials_host[g], "%s: partial %d is null", who, g);
+    parts.p[g] = partials_host[g];
+  }
+  return RISER_OK;
+}
+
+}  // namespace
+
+extern "C" size_t riser_bn_partial_bytes(int C) {
+  if (C <= 0) return 0;
+  return (2 * static_cast<size_t>(C) + 1) * sizeof(double);
+}
+
 extern "C" int riser_bn_stats_cl(const float* y, const int32_t* len, int B, int L_pad, int C, float* mean, float* var,
                                  float* running_mean, float* running_var, int64_t* num_batches_tracked, float momentum,
                                  void* workspace, size_t workspace_bytes, riser_stream_t stream) {
@@ -257,8 +321,47 @@ extern "C" int riser_bn_stats_cl(const float* y, const int32_t* len, int B, int 
   bn_partial_kernel<false><<<dim3(kBnParts, (C + 31) / 32), dim3(32, kBnRowLanes), 0, as_stream(stream)>>>(
       y, nullptr, nullptr, nullptr, nullptr, 0.f, len, B, L_pad, C, part);
   RISER_CUDA_TRY(cudaGetLastError());
-  bn_stats_finish_kernel<<<(C + 255) / 256, 256, 0, as_stream(stream)>>>(part, len, B, C, mean, var, running_mean,
-                                                                         running_var, num_batches_tracked, momentum);
+  bn_stats_finish_kernel<<<(C + 255) / 256, 256, 0, as_stream(stream)>>>(one_part(part), 1, kBnParts, len, B, C, mean,
+                                                                         var, running_mean, running_var,
+                                                                         num_batches_tracked, momentum);
+  RISER_CUDA_TRY(cudaGetLastError());
+  return RISER_OK;
+}
+
+extern "C" int riser_bn_stats_partial_cl(const float* y, const int32_t* len, int B, int L_pad, int C, double* partial,
+                                         void* workspace, size_t workspace_bytes, riser_stream_t stream) {
+  RISER_REQUIRE(partial && workspace && (B == 0 || (y && len)), "riser_bn_stats_partial_cl: null pointer");
+  RISER_REQUIRE(B >= 0 && L_pad > 0 && C > 0, "riser_bn_stats_partial_cl: bad shape");
+  const size_t need = riser_bn_workspace_bytes(C);
+  if (workspace_bytes < need)
+    return fail(RISER_ENOMEM, "riser_bn_stats_partial_cl: workspace %zu bytes < %zu", workspace_bytes, need);
+  if (B == 0) {
+    RISER_CUDA_TRY(cudaMemsetAsync(partial, 0, riser_bn_partial_bytes(C), as_stream(stream)));
+    return RISER_OK;
+  }
+  double* part = static_cast<double*>(workspace);
+  bn_partial_kernel<false><<<dim3(kBnParts, (C + 31) / 32), dim3(32, kBnRowLanes), 0, as_stream(stream)>>>(
+      y, nullptr, nullptr, nullptr, nullptr, 0.f, len, B, L_pad, C, part);
+  RISER_CUDA_TRY(cudaGetLastError());
+  bn_slices_kernel<<<(C + 255) / 256, 256, 0, as_stream(stream)>>>(part, len, B, C, partial);
+  RISER_CUDA_TRY(cudaGetLastError());
+  return RISER_OK;
+}
+
+extern "C" int riser_bn_stats_finalize_cl(const double* const* partials_host, int G, int C, float* mean, float* var,
+                                          float* running_mean, float* running_var, int64_t* num_batches_tracked,
+                                          float momentum, riser_stream_t stream) {
+  RISER_REQUIRE(mean && var, "riser_bn_stats_finalize_cl: null pointer");
+  RISER_REQUIRE((running_mean == nullptr) == (running_var == nullptr) &&
+                    (running_mean == nullptr) == (num_batches_tracked == nullptr),
+                "riser_bn_stats_finalize_cl: running_mean, running_var and num_batches_tracked go together");
+  RISER_REQUIRE(C > 0, "riser_bn_stats_finalize_cl: bad shape");
+  BnParts parts;
+  const int rc = gather_parts("riser_bn_stats_finalize_cl", partials_host, G, parts);
+  if (rc != RISER_OK) return rc;
+  bn_stats_finish_kernel<<<(C + 255) / 256, 256, 0, as_stream(stream)>>>(parts, G, 1, nullptr, 0, C, mean, var,
+                                                                         running_mean, running_var,
+                                                                         num_batches_tracked, momentum);
   RISER_CUDA_TRY(cudaGetLastError());
   return RISER_OK;
 }
@@ -293,9 +396,58 @@ extern "C" int riser_bn_bwd_cl(const float* dout, const float* mask, const float
   bn_partial_kernel<true><<<dim3(kBnParts, (C + 31) / 32), dim3(32, kBnRowLanes), 0, as_stream(stream)>>>(
       y, dout, mask, mean, var, eps, len, B, L_pad, C, part);
   RISER_CUDA_TRY(cudaGetLastError());
-  bn_bwd_finish_kernel<<<(C + 255) / 256, 256, 0, as_stream(stream)>>>(part, len, B, C, dgamma, dbeta, sums);
+  bn_bwd_finish_kernel<<<(C + 255) / 256, 256, 0, as_stream(stream)>>>(one_part(part), 1, kBnParts, len, B, C, 1,
+                                                                       dgamma, dbeta, sums);
   RISER_CUDA_TRY(cudaGetLastError());
   const int64_t total = static_cast<int64_t>(B) * L_pad * C;
+  bn_bwd_dx_kernel<<<grid_for(total), 256, 0, as_stream(stream)>>>(y, dout, mask, len, B, L_pad, C, mean, var, gamma,
+                                                                   eps, sums, dx, dy_out);
+  RISER_CUDA_TRY(cudaGetLastError());
+  return RISER_OK;
+}
+
+extern "C" int riser_bn_bwd_partial_cl(const float* dout, const float* mask, const float* y, const int32_t* len, int B,
+                                       int L_pad, int C, const float* mean, const float* var, float eps, double* partial,
+                                       void* workspace, size_t workspace_bytes, riser_stream_t stream) {
+  RISER_REQUIRE(partial && workspace && (B == 0 || (dout && y && len && mean && var)),
+                "riser_bn_bwd_partial_cl: null pointer");
+  RISER_REQUIRE(B >= 0 && L_pad > 0 && C > 0, "riser_bn_bwd_partial_cl: bad shape");
+  const size_t need = riser_bn_workspace_bytes(C);
+  if (workspace_bytes < need)
+    return fail(RISER_ENOMEM, "riser_bn_bwd_partial_cl: workspace %zu bytes < %zu", workspace_bytes, need);
+  if (B == 0) {
+    RISER_CUDA_TRY(cudaMemsetAsync(partial, 0, riser_bn_partial_bytes(C), as_stream(stream)));
+    return RISER_OK;
+  }
+  double* part = static_cast<double*>(workspace);
+  bn_partial_kernel<true><<<dim3(kBnParts, (C + 31) / 32), dim3(32, kBnRowLanes), 0, as_stream(stream)>>>(
+      y, dout, mask, mean, var, eps, len, B, L_pad, C, part);
+  RISER_CUDA_TRY(cudaGetLastError());
+  bn_slices_kernel<<<(C + 255) / 256, 256, 0, as_stream(stream)>>>(part, len, B, C, partial);
+  RISER_CUDA_TRY(cudaGetLastError());
+  return RISER_OK;
+}
+
+extern "C" int riser_bn_bwd_finalize_cl(const double* const* partials_host, int G, int owner, const float* dout,
+                                        const float* mask, const float* y, const int32_t* len, int B, int L_pad, int C,
+                                        const float* mean, const float* var, const float* gamma, float eps,
+                                        float* dgamma, float* dbeta, float* dx, float* dy_out, void* workspace,
+                                        size_t workspace_bytes, riser_stream_t stream) {
+  RISER_REQUIRE(dgamma && dbeta && workspace && (B == 0 || (dout && y && len && mean && var && gamma && dx)),
+                "riser_bn_bwd_finalize_cl: null pointer");
+  RISER_REQUIRE(B >= 0 && L_pad > 0 && C > 0, "riser_bn_bwd_finalize_cl: bad shape");
+  const size_t need = riser_bn_workspace_bytes(C);
+  if (workspace_bytes < need)
+    return fail(RISER_ENOMEM, "riser_bn_bwd_finalize_cl: workspace %zu bytes < %zu", workspace_bytes, need);
+  BnParts parts;
+  const int rc = gather_parts("riser_bn_bwd_finalize_cl", partials_host, G, parts);
+  if (rc != RISER_OK) return rc;
+  double* sums = static_cast<double*>(workspace) + static_cast<size_t>(kBnParts) * 2 * C;
+  bn_bwd_finish_kernel<<<(C + 255) / 256, 256, 0, as_stream(stream)>>>(parts, G, 1, nullptr, 0, C, owner, dgamma,
+                                                                       dbeta, sums);
+  RISER_CUDA_TRY(cudaGetLastError());
+  const int64_t total = static_cast<int64_t>(B) * L_pad * C;
+  if (total == 0) return RISER_OK;
   bn_bwd_dx_kernel<<<grid_for(total), 256, 0, as_stream(stream)>>>(y, dout, mask, len, B, L_pad, C, mean, var, gamma,
                                                                    eps, sums, dx, dy_out);
   RISER_CUDA_TRY(cudaGetLastError());

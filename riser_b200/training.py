@@ -18,6 +18,8 @@ package's own kernels, not a restatement of Lightning:
     ``CombinedLoader`` --, validates, and writes ``<prefix>_latest.pth`` and, on a new lowest validation loss,
     ``<prefix>_best.pth``.
 No CPU path: every op is a kernel of libriser_b200.so."""
+import functools
+
 import numpy as np
 import torch
 from torch import nn
@@ -25,6 +27,16 @@ from torch import nn
 from . import _lib
 from .config import AttrDict
 from .convnet_generic import check_supported
+
+
+def _on_own_device(method):
+    """Runs a trainer method with the trainer's device current, whatever device the calling thread has current: every
+    launch goes to _lib.stream_ptr(), the current device's stream, and must go to the device that holds the buffers."""
+    @functools.wraps(method)
+    def guarded(self, *args, **kwargs):
+        with torch.cuda.device(self.device):
+            return method(self, *args, **kwargs)
+    return guarded
 
 
 def _cnn_config(config):
@@ -112,6 +124,7 @@ class ConvNetTrainer:
         self.n_chain = len(chain)
         self.chain = torch.tensor(chain, dtype=torch.int32).to(self.device)
         self._bufs = {}
+        self.reducer = None           # a data-parallel replica's side of the reductions (riser_b200.parallel)
 
     # ------------------------------------------------------------------ buffers of one (B, L) shape
     def _shape_bufs(self, B, L):
@@ -146,6 +159,7 @@ class ConvNetTrainer:
         return s
 
     # ------------------------------------------------------------------ inputs
+    @_on_own_device
     def _inputs(self, x, lens, labels):
         if x.dim() != 2:
             raise ValueError(f"x must be [B, L], got {tuple(x.shape)}")
@@ -203,10 +217,7 @@ class ConvNetTrainer:
         fc_w, fc_b = self.params[self.head_w], self.params[self.head_b]
         # without the backward pass (evaluate) the head's gradients go to scratch: the parameters' .grad stay as they were
         dw, db = (fc_w.grad, fc_b.grad) if backward else (s["dfc_w"], s["dfc_b"])
-        _lib.check(lib.riser_gap_linear_ce_bwd(ptr(h), ptr(n_in), ptr(fc_w), ptr(fc_b), ptr(labels), B, Li, C,
-                                               self.n_classes, ptr(s["loss"]), ptr(s["loss_mean"]), ptr(s["logits"]),
-                                               ptr(s["dlogits"]), ptr(s["feat"]), ptr(dw), ptr(db), ptr(gh), stream),
-                   "riser_gap_linear_ce_bwd")
+        _head(self.reducer if backward else None, h, n_in, fc_w, fc_b, labels, Li, C, self.n_classes, s, dw, db, gh)
         if backward:
             self._backward(s, x, lens, conv_len, B, L)
         return s
@@ -252,6 +263,7 @@ class ConvNetTrainer:
                                                           Li, cout, 0, stream), "riser_relu_pool_bwd_cl")
 
     # ------------------------------------------------------------------ public surface
+    @_on_own_device
     def step(self, x, lens, labels):
         """One Adam step on the batch: x fp32 [B, ld] normalised windows, read b valid for lens[b] samples
         (2**n_layers <= lens[b] <= ld), labels int64 class indices.  Returns the mean loss as a 0-dim device tensor
@@ -264,12 +276,14 @@ class ConvNetTrainer:
         self.optimizer.step()
         return s["loss_mean"][0]
 
+    @_on_own_device
     def gradients(self, x, lens, labels):
         """The loss gradients of the batch at the current weights, keyed like the state-dict (device tensors)."""
         x, lens, labels = self._inputs(x, lens, labels)
         self._run(x, lens, labels)
         return {k: p.grad.clone() for k, p in self.params.items()}
 
+    @_on_own_device
     def evaluate(self, x, lens, labels):
         """(mean loss, number of reads whose argmax class is the label) at the current weights."""
         x, lens, labels = self._inputs(x, lens, labels)
@@ -438,6 +452,7 @@ class ResNetTrainer:
         self.bn_ws = torch.empty(lib.riser_bn_workspace_bytes(max(cv[3] for cv in self.convs)) // 4 + 4,
                                  device=self.device)
         self._bufs = {}
+        self.reducer = None           # a data-parallel replica's side of the reductions (riser_b200.parallel)
 
     # ------------------------------------------------------------------ buffers of one (B, L) shape
     def _shape_bufs(self, B, L):
@@ -506,6 +521,7 @@ class ResNetTrainer:
                 raise ValueError(f"op {j} leaves {int(n.sum())} value per channel for BatchNorm's batch statistics "
                                  "(more than 1 needed)")
 
+    @_on_own_device
     def _inputs(self, x, lens, labels):
         if x.dim() != 2:
             raise ValueError(f"x must be [B, L], got {tuple(x.shape)}")
@@ -539,6 +555,9 @@ class ResNetTrainer:
         run = [None] * 3
         if mode == "step":
             run = [self.buffers[cv[1] + k] for k in (".running_mean", ".running_var", ".num_batches_tracked")]
+        if self.reducer is not None:
+            self.reducer.bn_stats(cv, y, n, mean, var, run)
+            return mean, var
         _lib.check(_lib.lib().riser_bn_stats_cl(_lib.ptr(y), _lib.ptr(n), y.shape[0], y.shape[1], cv[3], _lib.ptr(mean),
                                                 _lib.ptr(var), *[_lib.ptr(t) for t in run], BN_MOMENTUM,
                                                 _lib.ptr(self.bn_ws), self.bn_ws.numel() * 4, _lib.stream_ptr()),
@@ -601,15 +620,16 @@ class ResNetTrainer:
         gh = s["gH"][self.blocks[-1][0]]
         fc_w, fc_b = self.params["decoder.2.weight"], self.params["decoder.2.bias"]
         dw, db = (fc_w.grad, fc_b.grad) if mode != "eval" else (s["dfc_w"], s["dfc_b"])
-        _lib.check(lib.riser_gap_linear_ce_bwd(ptr(h), ptr(n), ptr(fc_w), ptr(fc_b), ptr(labels), B, Lh, C,
-                                               self.n_classes, ptr(s["loss"]), ptr(s["loss_mean"]), ptr(s["logits"]),
-                                               ptr(s["dlogits"]), ptr(s["feat"]), ptr(dw), ptr(db), ptr(gh),
-                                               _lib.stream_ptr()), "riser_gap_linear_ce_bwd")
+        _head(self.reducer if mode != "eval" else None, h, n, fc_w, fc_b, labels, Lh, C, self.n_classes, s, dw, db,
+              gh)
         if mode != "eval":
             self._backward(s, x, lens, n_all, stats, trace)
         return s
 
     def _bn_bwd(self, cv, dout, mask, y, n, stats, dx, dy_out=None):
+        if self.reducer is not None:
+            self.reducer.bn_bwd(cv, dout, mask, y, n, stats, dx, dy_out)
+            return
         P = _lib.ptr
         g = self.params[cv[1] + ".weight"]
         _lib.check(_lib.lib().riser_bn_bwd_cl(P(dout), P(mask), P(y), P(n), y.shape[0], y.shape[1], cv[3],
@@ -635,6 +655,13 @@ class ResNetTrainer:
             _lib.check(lib.riser_conv1d_dgrad_cl(P(dz), P(n_out), P(self._wd[cv[0]]), P(residual), P(dx), P(n_in),
                                                  dz.shape[0], dz.shape[1], dx.shape[1], cv[2], cv[3], cv[4], cv[5],
                                                  cv[6], _lib.stream_ptr()), "riser_conv1d_dgrad_cl")
+
+    def _bn_backward_order(self):
+        """The convolutions whose BatchNorm _backward differentiates, in its order (self.convs is the forward's)."""
+        order = []
+        for _, convs, sc, applied in reversed(self.blocks):
+            order += [convs[-1]] + ([sc] if applied else []) + convs[-2::-1]
+        return order + [self.stem]
 
     def _backward(self, s, x, lens, n_all, stats, trace):
         for cv in self.convs:
@@ -679,6 +706,7 @@ class ResNetTrainer:
         self._wgrad(s, st, s["gY"][st[0]], n_all[0], x.view(B, L, 1), lens, db=self.params[st[0] + ".bias"].grad)
 
     # ------------------------------------------------------------------ public surface
+    @_on_own_device
     def step(self, x, lens, labels):
         """One Adam step on the batch (x fp32 [B, ld] normalised windows, read b valid for lens[b] samples, labels
         int64), with BatchNorm's batch statistics; the running statistics and num_batches_tracked are updated once.
@@ -690,6 +718,7 @@ class ResNetTrainer:
         self.optimizer.step()
         return s["loss_mean"][0]
 
+    @_on_own_device
     def gradients(self, x, lens, labels):
         """The loss gradients of the batch at the current weights (batch statistics; the running statistics stay as
         they are), keyed like the state-dict (device tensors)."""
@@ -697,6 +726,7 @@ class ResNetTrainer:
         self._run(x, lens, labels, "train")
         return {k: p.grad.clone() for k, p in self.params.items()}
 
+    @_on_own_device
     def evaluate(self, x, lens, labels):
         """(mean loss, number of reads whose argmax class is the label) in eval mode (the running statistics)."""
         x, lens, labels = self._inputs(x, lens, labels)
@@ -717,15 +747,44 @@ class ResNetTrainer:
         return out
 
 
-def make_trainer(config, state=None, seed=0, logger=None):
-    """ConvNetTrainer or ResNetTrainer by ``config.model`` ('cnn' when absent), as the reference's train.py:175-184
-    and riser_b200.Model choose the network."""
+def _head(reducer, h, n, fc_w, fc_b, labels, L_pad, C, n_classes, s, dw, db, dh):
+    """The loss head (riser_gap_linear_ce_bwd).  A data-parallel replica in training (reducer set) divides by the
+    global batch and writes its share of the mean loss where the replicas' gradient exchange adds them up."""
+    lib, ptr, B = _lib.lib(), _lib.ptr, h.shape[0]
+    if reducer is None:
+        _lib.check(lib.riser_gap_linear_ce_bwd(ptr(h), ptr(n), ptr(fc_w), ptr(fc_b), ptr(labels), B, L_pad, C,
+                                               n_classes, ptr(s["loss"]), ptr(s["loss_mean"]), ptr(s["logits"]),
+                                               ptr(s["dlogits"]), ptr(s["feat"]), ptr(dw), ptr(db), ptr(dh),
+                                               _lib.stream_ptr()), "riser_gap_linear_ce_bwd")
+    else:
+        _lib.check(lib.riser_gap_linear_ce_bwd_ex(ptr(h), ptr(n), ptr(fc_w), ptr(fc_b), ptr(labels), B, reducer.batch,
+                                                  L_pad, C, n_classes, ptr(s["loss"]), ptr(reducer.loss),
+                                                  ptr(s["logits"]), ptr(s["dlogits"]), ptr(s["feat"]), ptr(dw), ptr(db),
+                                                  ptr(dh), _lib.stream_ptr()), "riser_gap_linear_ce_bwd_ex")
+
+
+def model_of(config):
+    """``config.model`` ('cnn' when absent)."""
     model = (config.get("model") if isinstance(config, dict) else getattr(config, "model", None)) or "cnn"
-    if model == "resnet":
-        return ResNetTrainer(config, state=state, seed=seed, logger=logger)
-    if model == "cnn":
-        return ConvNetTrainer(config, state=state, seed=seed, logger=logger)
-    raise NotImplementedError(f"model {model!r}: 'cnn' or 'resnet'")
+    if model not in ("cnn", "resnet"):
+        raise NotImplementedError(f"model {model!r}: 'cnn' or 'resnet'")
+    return model
+
+
+def make_trainer(config, state=None, seed=0, logger=None, devices=None):
+    """ConvNetTrainer or ResNetTrainer by ``config.model`` ('cnn' when absent), as the reference's train.py:175-184
+    and riser_b200.Model choose the network.  ``devices`` naming more than one GPU: a
+    riser_b200.parallel.DataParallelTrainer over them; one device: the single-device trainer built on it."""
+    model = model_of(config)
+    if devices is not None:
+        from .parallel import DataParallelTrainer, check_devices
+        devices = check_devices(devices)
+        if len(devices) > 1:
+            return DataParallelTrainer(config, devices, state=state, seed=seed, logger=logger)
+        with torch.cuda.device(devices[0]):
+            return make_trainer(config, state=state, seed=seed, logger=logger)
+    cls = ResNetTrainer if model == "resnet" else ConvNetTrainer
+    return cls(config, state=state, seed=seed, logger=logger)
 
 
 # ---------------------------------------------------------------- data (riser/data.py)
